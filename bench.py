@@ -2,12 +2,21 @@
 """Benchmark of the hot path: UNetSCN forward+backward on synthetic nuScenes-shaped scans.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--mode fp32|tf32] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch (default 8 scans per GPU, BASELINE.json
 configs[1]): structure build (voxel hash, 7-level pyramid, rule tables), UNetSCN forward, backward
 to the point features and all parameters, and -- for N > 1 -- the flat-gradient all-reduce.
 Prints ONE JSON line (rank 0).  ``--impl reference`` times the CPU restatement of the reference's
 SparseConvNet path (oracle/, the dependency itself is not installable here) on the host cores.
+
+``--dump-outputs DIR`` writes what the last timed step computed as ``DIR/<name>.npy``: the point
+features ``out``, ``grad_feats`` and one ``grad.<parameter>`` per parameter.  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
+``--steps K`` sets the number of timed steps of every measured loop: the headline, the end-to-end
+loop, the side modes and, with ``--full-step``, the 3D-branch figures.  The kernel pass times each
+launch on its own (3 repetitions); the CPU baseline of the GPU arm times 5 scans.
+The benchmark writes nothing into the source tree.
 """
 from __future__ import annotations
 
@@ -31,7 +40,7 @@ NET_KW = dict(in_channels=3, m=16, block_reps=1, residual_blocks=False, full_sca
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps of every measured loop (see the module docstring)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     # BASELINE.json configs[1] names both arithmetic modes; the tensor-core one (tcgen05 kind::tf32, FP32
@@ -45,13 +54,52 @@ def parse_args():
     ap.add_argument("--no-pipeline", dest="pipeline", action="store_false",
                     help="build each step's sparse structure inline on the compute stream instead of one step ahead")
     ap.add_argument("--no-kernel-pass", action="store_true")
+    ap.add_argument("--kernel-pass-json", metavar="FILE", help="write the kernel pass's per-launch rows to FILE")
     ap.add_argument("--graph-2d", action="store_true",
                     help="--full-step: replay the dense 2D network (forward and backward, source and target pass) from CUDA graphs")
     ap.add_argument("--ab", default="", help="development: NAME=VALUE, time alternating blocks of steps with that variable set / unset")
     ap.add_argument("--full-step", action="store_true",
                     help="BASELINE configs[2]: whole MM2D3D training step (2D ResNet34-UNet stand-in on stock cuDNN + lift + "
                          "UNetSCN + heads + losses + optimiser), source and target batch, single GPU")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs and gradients of the last timed step as DIR/<name>.npy (at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.full_step):
+        ap.error("--dump-outputs applies to the UNetSCN measurement (--impl ours without --full-step)")
+    return args
+
+
+DUMP_BYTES = 64_000_000  # file sizes included (.npy headers: < 1 kB each)
+
+
+def to_host(tensors):
+    """Host copies of ``{name: tensor}`` in float32 (float64 stays float64), for :func:`dump_outputs`."""
+    import numpy as np
+
+    out = {}
+    for k, t in tensors.items():
+        a = t.detach().cpu().numpy()
+        out[k] = a if a.dtype == np.float64 else a.astype(np.float32)
+    return out
+
+
+def dump_outputs(path, per_point, whole):
+    """Write every array as ``path/<name>.npy``.  ``per_point`` arrays share their row count; if everything
+    together exceeds DUMP_BYTES they keep the same fixed, seeded sample of rows (sorted), so that two runs with the
+    same arguments write the same rows.  ``whole`` arrays are written whole."""
+    import numpy as np
+
+    n = next(iter(per_point.values())).shape[0]
+    row_bytes = sum(a[:1].nbytes for a in per_point.values())
+    budget = DUMP_BYTES - sum(a.nbytes + 1024 for a in whole.values()) - 1024 * len(per_point)
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n, budget // row_bytes, replace=False))
+        per_point = {k: a[rows] for k, a in per_point.items()}
+    os.makedirs(path, exist_ok=True)
+    for k, a in {**per_point, **whole}.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def peaks():
@@ -394,7 +442,7 @@ def run_ours(args):
             in_flight.append(ev)
             if len(in_flight) > 1:
                 in_flight.pop(0).synchronize()
-        return out
+        return out, x
 
     # End to end: every step's inputs come from pinned host memory and its scalar result goes back to the host.
     # The upload of step i+1 is issued on a copy stream while step i computes (what a prefetching data loader does);
@@ -469,12 +517,20 @@ def run_ours(args):
     launches0 = _lib.lib.mm3d_kernel_launches()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for i in range(args.steps):
+    for i in range(args.steps - 1):
         step(i)
+    # only the last step's result is kept (for --dump-outputs): a step's output holds its whole activation arena
+    last = step(args.steps - 1)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = _lib.lib.mm3d_kernel_launches() - launches0
+    dumped = None
+    if args.dump_outputs and rank == 0:  # copied before any further step overwrites the gradients; written later
+        out, x = last
+        dumped = (to_host({"out": out, "grad_feats": x.grad}),
+                  to_host({"grad." + k: p.grad for k, p in net.named_parameters()}))
+    del last
     # a short timed region can fall between two 50 ms samples: run on under the sampler for ~0.4 s (the same number
     # of extra steps on every rank, decided by rank 0, because steps contain a collective)
     extra = torch.tensor([0 if os.environ.get("MM3D_BENCH_NO_RUNON") else
@@ -487,6 +543,8 @@ def run_ours(args):
             torch.cuda.synchronize()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, *dumped)
 
     if args.ab and world == 1:
         # development aid: alternate blocks of steps with an environment switch of the library set / unset (switches
@@ -505,11 +563,11 @@ def run_ours(args):
                 barrier()
                 a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 a0.record()
-                for i in range(20):
+                for i in range(args.steps):
                     step(i)
                 a1.record()
                 barrier()
-                rows[which].append(a0.elapsed_time(a1) / 20)
+                rows[which].append(a0.elapsed_time(a1) / args.steps)
         os.environ.pop(name, None)
         for which in rows:
             v = sorted(rows[which])
@@ -566,9 +624,12 @@ def run_ours(args):
             roofline["share_note"] = ("conv_total_ms sums launches timed one by one with a cold L2; inside a step the weight-"
                                       "gradient kernels run on a second stream beside dgrad/BatchNorm and the caches are warm, "
                                       "so the sum can exceed the step time")
-            os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-            with open(os.path.join(ROOT, "gpurun_out", f"kernel_pass_{args.mode}.json"), "w") as f:
-                json.dump(rows, f, indent=0)
+            if args.kernel_pass_json:
+                try:
+                    with open(args.kernel_pass_json, "w") as f:
+                        json.dump(rows, f, indent=0)
+                except OSError as e:  # a side table: the benchmark line is printed regardless
+                    print(f"bench.py: could not write {args.kernel_pass_json}: {e}", file=sys.stderr)
         if world == 1 and not args.no_cpu_baseline:
             cpu = cpu_reference_scans_per_s(5, 1, args.shape)
             cpu = {k: cpu[k] for k in ("value", "unit", "cores", "kind", "sample")}
@@ -587,7 +648,7 @@ def run_ours(args):
                 scn_mod.set_conv_mode(smode)
                 prepared.clear()  # (row plans are built per mode)
                 try:
-                    n_f = 20
+                    n_f = args.steps
                     for i in range(3):
                         step(i)
                     barrier()
@@ -770,10 +831,10 @@ def run_full_step(args):
     torch.cuda.synchronize()
     clocks = sampler.stop()
     # the 3D branch alone, same batches: mask + UNetSCN forward (events inside the step), and forward+backward
-    for i in range(4):
+    for i in range(args.steps):
         step(i, time3d=True)
     torch.cuda.synchronize()
-    fwd3d = sum(a.elapsed_time(b) for a, b in ev3d) / 4
+    fwd3d = sum(a.elapsed_time(b) for a, b in ev3d) / args.steps
 
     def only3d(i):
         for dom in ("src", "trg"):
@@ -788,11 +849,11 @@ def run_full_step(args):
     torch.cuda.synchronize()
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     f0.record()
-    for i in range(10):
+    for i in range(args.steps):
         only3d(i)
     f1.record()
     torch.cuda.synchronize()
-    ms3d = f0.elapsed_time(f1) / 10
+    ms3d = f0.elapsed_time(f1) / args.steps
     scans = 2 * args.batch
     line = {
         "impl": "ours", "metric": "full MM2D3D training step scans/sec (source + target)", "value": scans / (ms * 1e-3), "unit": UNIT,

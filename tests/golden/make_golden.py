@@ -15,8 +15,12 @@ the lift fixture):  ``python tests/golden/make_golden.py``.
   16-channel pass-through), 3D cross-modal term by the torch lines of ``train.py:174-182``.
 * ``heads_ref.npz`` -- RGB mask by the REFERENCE's ``Net3DSeg.forward`` (``3d_net/model.py:44-58``, backbone replaced by
   a pass-through), cross-modal KL term by the torch lines of ``train.py:157-184``.
+* ``unetscn_tree.json`` -- the SPEC of the reference's ``UNetSCN(in_channels=3)`` module tree (``3d_net/scn_unet.py:8-126``)
+  as state_dict keys in order with their shapes, spelled out from SURVEY.md Appendix B without ``mm2d3d_b200``.  It is
+  not produced by running the reference; where the reference is at hand, its own tree is what to store here.
 """
 import importlib.util
+import json
 import os
 import sys
 
@@ -258,6 +262,37 @@ def heads3d_from_reference():
         d_w2=net.aux.linear_point.weight.grad.numpy(), d_b2=net.aux.linear_point.bias.grad.numpy())
 
 
+def unetscn_tree(in_channels=3, m=16, num_planes=7):
+    """``unetscn_tree.json``: SURVEY.md Appendix B's recursion -- level l at ``prefix`` with p = m(l+1) planes holds
+    BN-ReLU ``.0.0`` and SMC ``.0.1``; every level but the deepest adds BN-ReLU ``.1.1.0``, Conv 2/2 ``.1.1.1``, the
+    next level ``.1.1.2``, BN-ReLU ``.1.1.3``, Deconv 2/2 ``.1.1.4``, then BN-ReLU ``.3.0`` and SMC ``.3.1`` on 2p."""
+    tree = []
+
+    def bn(prefix, c):
+        tree.extend([f"{prefix}.{k}", [c]] for k in ("weight", "bias", "running_mean", "running_var"))
+
+    def level(prefix, lvl):
+        p = m * (lvl + 1)
+        bn(f"{prefix}.0.0", p)
+        tree.append([f"{prefix}.0.1.weight", [27, 1, p, p]])
+        if lvl + 1 < num_planes:
+            q = m * (lvl + 2)
+            bn(f"{prefix}.1.1.0", p)
+            tree.append([f"{prefix}.1.1.1.weight", [8, 1, p, q]])
+            level(f"{prefix}.1.1.2", lvl + 1)
+            bn(f"{prefix}.1.1.3", q)
+            tree.append([f"{prefix}.1.1.4.weight", [8, 1, q, p]])
+            bn(f"{prefix}.3.0", 2 * p)
+            tree.append([f"{prefix}.3.1.weight", [27, 1, 2 * p, p]])
+
+    tree.append(["layer2.weight", [27, 1, in_channels, m]])
+    level("layer3", 0)
+    bn("layer4", m)
+    with open(os.path.join(HERE, "unetscn_tree.json"), "w") as f:
+        json.dump({"in_channels": in_channels, "m": m, "num_planes": num_planes, "state_dict": tree}, f, indent=0)
+        f.write("\n")
+
+
 if __name__ == "__main__":
     only = sys.argv[1] if len(sys.argv) > 1 else None  # e.g. `make_golden.py augment` regenerates one fixture
     if only in (None, "lift"):
@@ -272,6 +307,8 @@ if __name__ == "__main__":
         heads_from_reference()
     if only in (None, "heads3d"):
         heads3d_from_reference()
+    if only in (None, "tree"):
+        unetscn_tree()
     for f in sorted(os.listdir(HERE)):
-        if f.endswith(".npz"):
+        if f.endswith((".npz", ".json")):
             print(f, os.path.getsize(os.path.join(HERE, f)))

@@ -1294,9 +1294,9 @@ class _ForeignUNet(torch.nn.Module):
     """A host network assembled from the raw ``scn.*`` surface the way the reference's 3d_net/scn_unet.py:90-126 does
     (five members layer1..layer5 called in sequence, InputLayer with its default prebuild of ONE level) -- i.e. NOT
     mm2d3d_b200.unet.UNetSCN, so neither the whole-network executor nor the pre-built pyramid is involved and every
-    coarser level is built lazily by the first layer that needs it.  The reference file itself cannot run on the GPU
-    box (/root/reference does not travel, and it may not be copied); tests/test_oracle.py and tests/test_cabi.py load
-    the real file in the build container and pin that its module tree equals the one built here."""
+    coarser level is built lazily by the first layer that needs it.  The reference file itself is not part of this
+    repository; tests/test_oracle.py and tests/test_cabi.py pin UNetSCN's module tree to the one SURVEY.md Appendix B
+    records for it (tests/golden/unetscn_tree.json)."""
 
     def __init__(self, scn, in_channels, m, num_planes, full_scale):
         super().__init__()

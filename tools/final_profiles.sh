@@ -3,7 +3,7 @@
 set -u
 O=gpurun_out
 mkdir -p $O
-timeout 600 python bench.py --steps 50 --warmup 5 > $O/r2_final_bench.json 2> $O/r2_final_bench.err
+timeout 600 python bench.py --steps 50 --warmup 5 --kernel-pass-json $O/kernel_pass_tf32.json > $O/r2_final_bench.json 2> $O/r2_final_bench.err
 timeout 300 python bench.py --mode tf32x3 --steps 30 --warmup 5 --no-cpu-baseline > $O/r2_tf32x3_bench.json 2>/dev/null
 timeout 300 python bench.py --mode bf16 --steps 30 --warmup 5 --no-cpu-baseline > $O/r2_bf16_bench.json 2>/dev/null
 timeout 300 python bench.py --impl reference --steps 3 --warmup 1 > $O/r2_reference_arm.json 2>/dev/null
