@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MM3D_ABI_VERSION 6
+#define MM3D_ABI_VERSION 7
 
 #define MM3D_OK 0
 #define MM3D_ERR_INVALID 1     /* bad argument */
@@ -302,16 +302,30 @@ MM3D_API int mm3d_heads3d_bwd(const float* feat, int64_t n, int f, int C, const 
                      float* d_w1, float* d_b1, float* d_w2, float* d_b2, void* ws, size_t ws_bytes, mm3d_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
- * Whole-network executor: UNetSCN (3d_net/scn_unet.py:90-126, VGG blocks, block_reps == 1) forward and
- * backward as one call each -- the same kernels as above, driven natively instead of from ~110
- * Python autograd nodes.  level_desc: MM3D_LEVEL_DESC_WORDS int64 per level {rows, nbr table ptr, table
- * stride, parent ptr, off ptr, child ptr, plan of the 3^3 table, plan of the child table, plan of the
- * (parent, off) table, plan capacity} (plans may be 0 in MM3D_MODE_FP32).  params / grads: HOST arrays of device pointers in module-tree order:
- *   stem.w | per level: pre_bn{gamma,beta,running_mean,running_var} pre.w [dn_bn{4} dn.w <deeper level>
- *   up_bn{4} up.w post_bn{4} post.w] | head_bn{4}          (mm3d_unet_num_params slots; grads ignore
- * the running-stat slots).  act: activations kept from forward to backward; tmp: backward temporaries.
+ * Whole-network executor: UNetSCN (3d_net/scn_unet.py:36-126) forward and backward as one call each -- the
+ * same kernels as above, driven natively instead of from ~110 Python autograd nodes (about twice that with
+ * block_reps == 2).  Every configuration of the constructor's block topology is covered: block_reps >= 1 blocks per
+ * pre / post group, VGG blocks (residual == 0) or pre-activation residual blocks (residual == 1), whose
+ * NetworkInNetwork shortcut runs as a K = 1 rule-table convolution.  The mm3d_unet_* functions are the
+ * reference configuration (block_reps == 1, VGG) of the mm3d_unet_topo_* ones.  level_desc:
+ * MM3D_LEVEL_DESC_WORDS int64 per level {rows, nbr table ptr, table stride, parent ptr, off ptr, child ptr, plan of
+ * the 3^3 table, plan of the child table, plan of the (parent, off) table, plan capacity} (plans may be 0 in
+ * MM3D_MODE_FP32).  params / grads: HOST arrays of device pointers in module-tree order:
+ *   stem.w | per level: pre blocks [dn_bn{gamma,beta,running_mean,running_var} dn.w <deeper level>
+ *   up_bn{4} up.w post blocks] | head_bn{4}
+ * with a VGG block = bn{4} smc.w and a residual block = [nin.w] bn{4} smc.w bn{4} smc.w (the NetworkInNetwork
+ * weight [a, b] only where the block changes the channel count: the first post block of a level).
+ * (mm3d_unet_topo_num_params slots; grads ignore the running-stat slots.)  act: activations kept from forward to
+ * backward; tmp: backward temporaries.
  * ---------------------------------------------------------------------------------------- */
 #define MM3D_LEVEL_DESC_WORDS 10
+MM3D_API int64_t mm3d_unet_topo_num_params(int num_planes, int block_reps, int residual);
+MM3D_API size_t mm3d_unet_topo_act_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                const int64_t* level_desc, int64_t n_points);
+MM3D_API size_t mm3d_unet_topo_bwd_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                const int64_t* level_desc, int64_t n_points);
+MM3D_API size_t mm3d_unet_topo_scratch_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode);
+/* the reference configuration: block_reps = 1, residual = 0 */
 MM3D_API int64_t mm3d_unet_num_params(int num_planes);
 MM3D_API size_t mm3d_unet_act_bytes(int in_channels, int m, int num_planes, int mode, const int64_t* level_desc,
                            int64_t n_points);
@@ -329,6 +343,16 @@ typedef struct {
   void* ws;           /* backward only: (in_channels + 1) doubles */
   size_t ws_bytes;
 } mm3d_unet_mask;
+MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                           int training, float eps, float momentum, const int64_t* level_desc, int64_t n_points,
+                           const int32_t* p2v, const int32_t* npts, const float* feats, float* out, void* const* params,
+                           void* act, size_t act_bytes, void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask,
+                           mm3d_stream_t stream);
+MM3D_API int mm3d_unet_topo_backward(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                            int training, const int64_t* level_desc, int64_t n_points, const int32_t* p2v,
+                            const int32_t* npts, const float* d_out, float* d_feats, void* const* params,
+                            void* const* grads, void* act, size_t act_bytes, void* tmp, size_t tmp_bytes, void* scratch,
+                            size_t scratch_bytes, const mm3d_unet_mask* mask, mm3d_stream_t stream);
 MM3D_API int mm3d_unet_forward(int in_channels, int m, int num_planes, int mode, int training, float eps, float momentum,
                       const int64_t* level_desc, int64_t n_points, const int32_t* p2v, const int32_t* npts,
                       const float* feats, float* out, void* const* params, void* act, size_t act_bytes,

@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmm3d.so")
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 
 class UnetMask(C.Structure):
@@ -81,6 +81,12 @@ SIGNATURES = {
     "mm3d_kl_logits_bwd": (_i, [_p, _p, _i64, _i, _p, _p, _p]),
     "mm3d_heads3d_fwd": (_i, [_p, _i64, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "mm3d_heads3d_bwd": (_i, [_p, _i64, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "mm3d_unet_topo_num_params": (_i64, [_i, _i, _i]),
+    "mm3d_unet_topo_act_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _p, _i64]),
+    "mm3d_unet_topo_bwd_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _p, _i64]),
+    "mm3d_unet_topo_scratch_bytes": (_sz, [_i, _i, _i, _i, _i, _i]),
+    "mm3d_unet_topo_forward": (_i, [_i, _i, _i, _i, _i, _i, _i, _f, _f, _p, _i64, _p, _p, _p, _p, _p, _p, _sz, _p, _sz, _p, _p]),
+    "mm3d_unet_topo_backward": (_i, [_i, _i, _i, _i, _i, _i, _i, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _sz, _p, _sz, _p, _p]),
     "mm3d_unet_num_params": (_i64, [_i]),
     "mm3d_unet_act_bytes": (_sz, [_i, _i, _i, _i, _p, _i64]),
     "mm3d_unet_bwd_bytes": (_sz, [_i, _i, _i, _i, _p, _i64]),

@@ -322,6 +322,7 @@ k_bn_bwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
   // bit 1: same for the high column block dx_hi
   // bit 2: those outputs carry a hi and a lo plane (TF32x3 mode), the lo plane n * (row length) floats behind
   // bit 3: ... a TF32-rounded FP32 plane and a BF16 plane behind it (BF16 mode)
+  // bit 4: `add` carries a lo plane n * add_ld floats behind its hi plane (a TF32x3 operand): both are added
   const int rnd = (round_flags & ((dx_hi && hi) ? 2 : 1)) ? ((round_flags & 8) ? 3 : (round_flags & 4) ? 2 : 1) : 0;
   float* dx0 = (dx_hi && hi) ? dx_hi : dx;  // base of the tensor this thread writes
   const int64_t dplane = n * dxld;
@@ -413,6 +414,11 @@ k_bn_bwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
         vload<VEC>(add + (row + u * stride) * add_ld + v * VEC, a_);
 #pragma unroll
         for (int j = 0; j < VEC; ++j) g[u][j] += a_[j];
+        if (round_flags & 16) {
+          vload<VEC>(add + n * add_ld + (row + u * stride) * add_ld + v * VEC, a_);
+#pragma unroll
+          for (int j = 0; j < VEC; ++j) g[u][j] += a_[j];
+        }
       }
       store_planes<VEC>(dx0, dxb + (row + u * stride) * dxld, g[u], rnd, dplane);
     }
@@ -433,6 +439,11 @@ k_bn_bwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
       vload<VEC>(add + row * add_ld + v * VEC, a_);
 #pragma unroll
       for (int j = 0; j < VEC; ++j) g[j] += a_[j];
+      if (round_flags & 16) {
+        vload<VEC>(add + n * add_ld + row * add_ld + v * VEC, a_);
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) g[j] += a_[j];
+      }
     }
     store_planes<VEC>(dx0, dxb + row * dxld, g, rnd, dplane);
   }
@@ -539,7 +550,6 @@ int mm3d_bnrelu_bwd_impl(const float* x, const float* x_hi, int c_lo, const floa
                          void* ws, size_t ws_bytes, bool ws_clean, int round_flags, const float* add, int64_t add_ld,
                          cudaStream_t stream) {
   MM3D_REQUIRE(c > 0 && n >= 0, MM3D_ERR_INVALID, "bad sizes");
-  MM3D_REQUIRE(!add || !dx_hi, MM3D_ERR_INVALID, "bnrelu_bwd: an addend is only supported for a single output block");
   const bool vec4 = (c % 4 == 0) && (c_lo % 4 == 0) && (!add || add_ld % 4 == 0) &&
                     ((((uintptr_t)x | (uintptr_t)x_hi | (uintptr_t)dy | (uintptr_t)dx | (uintptr_t)dx_hi | (uintptr_t)add) & 15) == 0);
   const int cv = vec4 ? c / 4 : c;

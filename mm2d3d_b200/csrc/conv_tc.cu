@@ -57,7 +57,7 @@ struct TcParams {
   int S;        // ring stages = producer warps
   int n_pad, num_tiles, tmem_cols;
   int n_local;  // tiles per CTA (upper bound) = ceil(num_tiles / grid)
-  int accumulate; // epilogue adds to `out` instead of overwriting it
+  const float* add;  // epilogue: out[row] = acc + add[row] (NULL: out = acc; add == out accumulates)
   int x3;         // TF32x3 mode: every stage also holds the lo planes of the gathered rows and of the weight block, and
                   // an item is three products into the same accumulator: hi.Whi + lo.Whi + hi.Wlo
  const float* in_lo;
@@ -358,8 +358,8 @@ k_conv_tc(const __grid_constant__ TcParams p) {
             for (int jj = 0; jj < 16; jj += 4)
               if (c0 + jj < p.c_out) {
                 float4 o = make_float4(acc[jj], acc[jj + 1], acc[jj + 2], acc[jj + 3]);
-                if (p.accumulate) {  // (each row is owned by one thread: a plain read-modify-write)
-                  const float4 t = *reinterpret_cast<const float4*>(dst + jj);
+                if (p.add) {  // (each row is owned by one thread: a plain read-modify-write when add == out)
+                  const float4 t = *reinterpret_cast<const float4*>(p.add + (int64_t)row * p.c_out + c0 + jj);
                   o.x += t.x; o.y += t.y; o.z += t.z; o.w += t.w;
                 }
                 *reinterpret_cast<float4*>(dst + jj) = o;
@@ -367,7 +367,7 @@ k_conv_tc(const __grid_constant__ TcParams p) {
           } else {
 #pragma unroll
             for (int jj = 0; jj < 16; ++jj)
-              if (c0 + jj < p.c_out) dst[jj] = p.accumulate ? dst[jj] + acc[jj] : acc[jj];
+              if (c0 + jj < p.c_out) dst[jj] = p.add ? p.add[(int64_t)row * p.c_out + c0 + jj] + acc[jj] : acc[jj];
           }
         }
       }
@@ -593,7 +593,7 @@ int mm3d_conv_tc_build_images(const float* const* weights, float* const* images,
 }
 
 int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
-                         const float* wimg, int K, const void* plan, int64_t plan_cap, int accumulate, cudaStream_t stream,
+                         const float* wimg, int K, const void* plan, int64_t plan_cap, const float* add, cudaStream_t stream,
                          const float* wimg_lo = nullptr, int bf16 = 0);
 
 int mm3d_conv_fwd_tc(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
@@ -614,8 +614,8 @@ int mm3d_conv_fwd_tc(const float* in, int64_t n_in, int c_in, float* out, int64_
       weight, wimg, K, c_in, c_out, nb, n_pad, tr ? 1 : 0, mir ? 1 : 0, 0, bf16);
   mm3d_count_launches(1);
   // BF16 mode: `in` holds an FP32 plane and, n_in * c_in floats behind it, the BF16 plane that is gathered
-  if (bf16) return mm3d_conv_fwd_tc_img(in + n_in * (int64_t)c_in, n_in, c_in, out, n_out, c_out, wimg, K, plan, plan_cap, 0, stream, nullptr, 1);
-  if (!(flags & MM3D_CONV_X3)) return mm3d_conv_fwd_tc_img(in, n_in, c_in, out, n_out, c_out, wimg, K, plan, plan_cap, 0, stream);
+  if (bf16) return mm3d_conv_fwd_tc_img(in + n_in * (int64_t)c_in, n_in, c_in, out, n_out, c_out, wimg, K, plan, plan_cap, nullptr, stream, nullptr, 1);
+  if (!(flags & MM3D_CONV_X3)) return mm3d_conv_fwd_tc_img(in, n_in, c_in, out, n_out, c_out, wimg, K, plan, plan_cap, nullptr, stream);
   // Error-compensated mode: `in` holds two planes, hi = tf32(x) and lo = tf32(x - hi) ([n_in, c_in] each), the
   // workspace two weight images; out = hi.Whi + lo.Whi + hi.Wlo, accumulated in FP32 (the dropped lo.Wlo term and the
   // roundings of the lo parts are ~2^-22 relative)
@@ -623,14 +623,14 @@ int mm3d_conv_fwd_tc(const float* in, int64_t n_in, int c_in, float* out, int64_
   k_weight_image<<<mm3d_grid((int64_t)K * nb * n_pad * kKBlock, 256), 256, 0, stream>>>(weight, wimg_lo, K, c_in, c_out, nb,
                                                                                     n_pad, tr ? 1 : 0, mir ? 1 : 0, 1, 0);
   mm3d_count_launches(1);
-  return mm3d_conv_fwd_tc_img(in, n_in, c_in, out, n_out, c_out, wimg, K, plan, plan_cap, 0, stream, wimg_lo);
+  return mm3d_conv_fwd_tc_img(in, n_in, c_in, out, n_out, c_out, wimg, K, plan, plan_cap, nullptr, stream, wimg_lo);
 }
 
 // the convolution proper, from a prebuilt weight image
 // wimg_lo != NULL: the TF32x3 form -- `in` carries a lo plane n_in * c_in floats behind the hi one, wimg_lo is the image of
 // the weights' TF32 remainder, and every item is three products (one launch, one gather of both planes)
 int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
-                         const float* wimg, int K, const void* plan, int64_t plan_cap, int accumulate, cudaStream_t stream,
+                         const float* wimg, int K, const void* plan, int64_t plan_cap, const float* add, cudaStream_t stream,
                          const float* wimg_lo, int bf16) {
   int nb, n_pad;
   MM3D_REQUIRE(!(bf16 && wimg_lo), MM3D_ERR_INVALID, "tcgen05 conv: BF16 and TF32x3 exclude each other");
@@ -639,7 +639,7 @@ int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, in
   MM3D_REQUIRE(n_out < (1ll << 31) && n_in * (int64_t)c_in < (1ll << 32), MM3D_ERR_UNSUPPORTED,
                "tcgen05 conv: tensor too large for 32-bit element offsets");
   MM3D_REQUIRE(plan && plan_cap >= n_out, MM3D_ERR_INVALID, "tcgen05 conv: needs a row plan covering n_out rows");
-  MM3D_REQUIRE((((uintptr_t)in | (uintptr_t)out | (uintptr_t)wimg) & 15) == 0, MM3D_ERR_INVALID,
+  MM3D_REQUIRE((((uintptr_t)in | (uintptr_t)out | (uintptr_t)wimg | (uintptr_t)add) & 15) == 0, MM3D_ERR_INVALID,
                "tcgen05 conv: pointers must be 16-byte aligned");
   if (n_out == 0) return MM3D_OK;
   const Mm3dPlanView pv = mm3d_plan_view(plan, plan_cap);
@@ -653,7 +653,7 @@ int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, in
   p.n_pad = n_pad;
   p.num_tiles = (int)mm3d_cdiv(n_out, kTileM);
   p.err = mm3d_device_err_flag();
-  p.accumulate = accumulate;
+  p.add = add;
   p.x3 = wimg_lo ? 1 : 0;
   p.in_lo = in + n_in * (int64_t)c_in;
   p.wimg_lo = wimg_lo;

@@ -2,20 +2,25 @@
 //
 // The per-layer entry points are enough for a drop-in, but driving ~110 autograd nodes from
 // Python costs ~8 ms of host time per step -- as much as the GPU work itself.  The executor walks
-// the fixed U-Net topology of 3d_net/scn_unet.py:55-84 (VGG blocks, block_reps == 1) natively:
-// it carves every activation out of one caller-provided workspace with a bump allocator that
-// forward and backward replay identically, and issues the same kernels the modules use.
+// the U-Net topology of 3d_net/scn_unet.py:36-84 natively, for any number of blocks per level
+// (block_reps) and for VGG or pre-activation residual blocks: it carves every activation out of one
+// caller-provided workspace with a bump allocator that forward and backward replay identically, and
+// issues the same kernels the modules use.
 //
 //   level l (p = m(l+1), q = m(l+2)):
-//     X_l --BN--> A_l --SMC--> Y_l                                   ("pre" block)
+//     X_l --[block p->p] x reps--> Y_l                                           ("pre" blocks)
 //     if l < L-1:  Y_l --BN--> B_l --Conv 2/2--> X_{l+1} ... R_{l+1} --BN--> E_l --Deconv 2/2--> F_l
-//                  J_l = [Y_l | F_l] --BN--> G_l --SMC(2p->p)--> R_l   ("post" block)
+//                  J_l = [Y_l | F_l] --block 2p->p--> --[block p->p] x (reps-1)--> R_l   ("post" blocks)
 //     else         R_l = Y_l
+//   VGG block:      x --BN--> A --SMC--> out
+//   residual block: x --BN--> A --SMC--> H --BN--> A2 --SMC(+ shortcut)--> out, shortcut = x (a == b) or
+//                   NetworkInNetwork(x) (a != b: only the first post block, on J), run as a K = 1 rule-table
+//                   convolution over an identity row plan; the add happens in the second SMC's epilogue
 //   stem: V (InputLayer mean) --SMC(in->m)--> X_0 ;  head: R_0 --BN--> Z --OutputLayer--> out
 //
 // Parameter pointers come in the module tree's order (Appendix B of SURVEY.md):
-//   stem.w | per level: pre_bn{gamma,beta,rmean,rvar} pre.w [dn_bn{4} dn.w <deeper level> up_bn{4}
-//   up.w post_bn{4} post.w] | head_bn{4}
+//   stem.w | per level: pre blocks [dn_bn{gamma,beta,rmean,rvar} dn.w <deeper level> up_bn{4} up.w post blocks]
+//   | head_bn{4};  VGG block: bn{4} smc.w;  residual block: [nin.w] bn{4} smc.w bn{4} smc.w
 #include <cuda_bf16.h>
 #include <stdlib.h>
 
@@ -23,6 +28,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "plan.cuh"
 
 // bnrelu.cu
 int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, int64_t n, int c, const float* gamma,
@@ -41,8 +47,13 @@ int mm3d_conv_tc_supported(int c_in, int c_out, int K);
 int mm3d_conv_tc_build_images(const float* const* weights, float* const* images, const int* K, const int* c_in,
                               const int* c_out, const int* flags, int n, cudaStream_t stream);
 int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
-                         const float* wimg, int K, const void* plan, int64_t plan_cap, int accumulate, cudaStream_t stream,
+                         const float* wimg, int K, const void* plan, int64_t plan_cap, const float* add, cudaStream_t stream,
                          const float* wimg_lo = nullptr, int bf16 = 0);
+// conv_simt.cu
+int mm3d_conv_fwd_simt(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
+                       const float* weight, int K, const int32_t* tbl, int64_t tbl_stride,
+                       const uint8_t* onehot_off, int flags, void* ws, size_t ws_bytes, cudaStream_t stream,
+                       const float* add);
 
 namespace {
 
@@ -61,22 +72,35 @@ struct Bump {
   char* base;
   size_t off, cap;
   bool ok;
-  float* f(int64_t n, int64_t c) {
-    size_t bytes = mm3d_align(sizeof(float) * (size_t)n * (size_t)c);
+  void* bytes(size_t n) {
     size_t o = off;
-    off += bytes;
+    off += mm3d_align(n);
     if (off > cap) ok = false;
-    return base ? reinterpret_cast<float*>(base + o) : nullptr;
+    return base ? base + o : nullptr;
   }
+  float* f(int64_t n, int64_t c) { return (float*)bytes(sizeof(float) * (size_t)n * (size_t)c); }
+};
+
+// one VGG or residual block, a -> b channels
+struct BlockBufs {
+  int a, b;
+  int pidx;            // first parameter slot
+  float *A, *s1;       // first BatchNorm's output (operand form) and its save_mean | save_invstd ([2][a])
+  float *H, *A2, *s2;  // residual: first SMC's output, second BatchNorm's output (operand form), its save
+  float* out;          // [n, b]
 };
 
 struct LevelBufs {
-  float *X, *A, *Y, *B, *E, *F, *J, *G, *R;
-  float *s_pre, *s_dn, *s_up, *s_post;  // BN save_mean | save_invstd ([2][C])
+  float *X, *Y, *B, *E, *F, *J, *R;
+  float* Jop;           // NiN shortcut: J in operand form (== J in FP32 mode)
+  float *s_dn, *s_up;   // BN save_mean | save_invstd ([2][C])
+  void* id_plan;        // NiN shortcut: identity row plan of the level's rows (capacity n)
+  std::vector<BlockBufs> pre, post;
 };
 
 struct Net {
   int L, m, cin, cin_k;  // cin_k = stem input channels as seen by the kernels (padded to 16 in TC modes)
+  int reps, res;         // blocks per pre / post group; residual blocks
   int mode;
   std::vector<LevelMeta> lv;
   std::vector<LevelBufs> b;
@@ -91,7 +115,41 @@ struct Net {
   int rmode() const { return mode == MM3D_MODE_TF32X3 ? 2 : mode == MM3D_MODE_BF16 ? 3 : mode == MM3D_MODE_TF32 ? 1 : 0; }
   bool x3() const { return mode == MM3D_MODE_TF32X3; }
   bool bf16() const { return mode == MM3D_MODE_BF16; }
+  bool nin(int a, int b) const { return res && a != b; }
+  int block_slots(int a, int b) const { return res ? (nin(a, b) ? 11 : 10) : 5; }
 };
+
+// parameter slots of level l and everything below it
+int level_slots(const Net& net, int l) {
+  const int p = net.planes(l);
+  int s = net.reps * net.block_slots(p, p);
+  if (l + 1 < net.L) s += 5 + level_slots(net, l + 1) + 5 + net.block_slots(2 * p, p) + (net.reps - 1) * net.block_slots(p, p);
+  return s;
+}
+// first slot of level l (the stem weight is slot 0)
+int level_base(const Net& net, int l) {
+  int base = 1;
+  for (int i = 0; i < l; ++i) base += net.reps * net.block_slots(net.planes(i), net.planes(i)) + 5;
+  return base;
+}
+// first slot of level l's post blocks
+int post_base(const Net& net, int l) {
+  return level_base(net, l) + net.reps * net.block_slots(net.planes(l), net.planes(l)) + 5 + level_slots(net, l + 1) + 5;
+}
+
+BlockBufs carve_block(const Net& net, Bump& bp, int64_t n, int a, int b, int pidx, float* out) {
+  BlockBufs k{};
+  k.a = a; k.b = b; k.pidx = pidx;
+  k.A = bp.f(n, (int64_t)a * net.pl());
+  k.s1 = bp.f(2, a);
+  if (net.res) {
+    k.H = bp.f(n, b);
+    k.A2 = bp.f(n, (int64_t)b * net.pl());
+    k.s2 = bp.f(2, b);
+  }
+  k.out = out ? out : bp.f(n, b);
+  return k;
+}
 
 // the same carving in forward, backward and the size query
 void carve(Net& net, Bump& bp) {
@@ -105,9 +163,10 @@ void carve(Net& net, Bump& bp) {
     const int p = net.planes(l);
     LevelBufs& B = net.b[l];
     B.X = bp.f(n, p);
-    B.A = bp.f(n, (int64_t)p * pl);
-    B.Y = bp.f(n, p);
-    B.s_pre = bp.f(2, p);
+    int pidx = level_base(net, l);
+    for (int r = 0; r < net.reps; ++r, pidx += net.block_slots(p, p))
+      B.pre.push_back(carve_block(net, bp, n, p, p, pidx, nullptr));
+    B.Y = B.pre.back().out;
     if (l + 1 < net.L) {
       const int q = net.planes(l + 1);
       B.B = bp.f(n, (int64_t)p * pl);
@@ -116,15 +175,56 @@ void carve(Net& net, Bump& bp) {
       B.s_up = bp.f(2, q);
       B.F = bp.f(n, p);
       B.J = bp.f(n, 2 * p);
-      B.G = bp.f(n, (int64_t)2 * p * pl);
-      B.s_post = bp.f(2, 2 * p);
-      B.R = bp.f(n, p);
+      B.Jop = B.J;
+      if (net.nin(2 * p, p)) {
+        if (net.mode != MM3D_MODE_FP32) B.Jop = bp.f(n, (int64_t)2 * p * pl);
+        B.id_plan = bp.bytes(mm3d_plan_size(n, 1));
+      }
+      pidx = post_base(net, l);
+      for (int r = 0; r < net.reps; ++r) {
+        const int a = r == 0 ? 2 * p : p;
+        B.post.push_back(carve_block(net, bp, n, a, p, pidx, nullptr));
+        pidx += net.block_slots(a, p);
+      }
+      B.R = B.post.back().out;
     } else {
       B.R = B.Y;
     }
   }
   net.Z = bp.f(n0, net.m);
   net.s_head = bp.f(2, net.m);
+}
+
+// Identity row plans (NetworkInNetwork as a K = 1 rule-table convolution): perm = iota (-1 past the rows), one
+// offset per tile, tiles in natural order, table = perm.  All levels' plans in one launch (blockIdx.y = level).
+constexpr int kMaxIdPlans = 16;
+struct IdPlans {
+  void* plan[kMaxIdPlans];
+  int64_t rows[kMaxIdPlans];
+};
+__global__ void k_identity_plans(const __grid_constant__ IdPlans ps) {
+  mm3d_griddep_launch();
+  mm3d_griddep_wait();
+  char* base = (char*)ps.plan[blockIdx.y];
+  if (!base) return;
+  const int64_t n = ps.rows[blockIdx.y];
+  const int64_t T = mm3d_plan_tiles(n);
+  int32_t* perm = (int32_t*)base;
+  uint32_t* mask = (uint32_t*)(base + mm3d_plan_off_mask(n));
+  int32_t* order = (int32_t*)(base + mm3d_plan_off_order(n));
+  uint32_t* off_tiles = (uint32_t*)(base + mm3d_plan_off_cnt(n));
+  int32_t* tbl = (int32_t*)(base + mm3d_plan_off_tbl(n));
+  const int64_t step = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < T * 128; i += step) {
+    const int32_t v = i < n ? (int32_t)i : -1;
+    perm[i] = v;
+    tbl[i] = v;
+    if (i < T) {
+      mask[i] = 1u;
+      order[i] = (int32_t)i;
+    }
+    if (i < 32) off_tiles[i] = i == 0 ? (uint32_t)T : 0u;
+  }
 }
 
 __global__ void k_copy_cols(const float* __restrict__ src, int64_t n, int c_src, float* __restrict__ dst, int c_dst,
@@ -312,16 +412,18 @@ void bn_fwd(Ctx& c, int pidx, const float* x, float* y, int64_t n, int ch, float
                           tc_mode(c) && to_conv ? c.net->rmode() : 0, c.stream));
 }
 // round: bit 0 = dx (its low column block when split) feeds a convolution as d_out, bit 1 = dx_hi does
-// add (rows add_ld floats apart): another gradient of the same tensor, summed into dx before it is stored
+// add (rows add_ld floats apart): another gradient of the same tensor, summed into dx before it is stored;
+// add_lo: `add` is a TF32x3 operand whose lo plane (n * add_ld floats behind) is summed too
 void bn_bwd(Ctx& c, int pidx, const float* x, const float* dy, float* dx, int64_t n, int ch, const float* save,
             int round, const float* x_hi = nullptr, int c_lo = 0, float* dx_hi = nullptr, const float* add = nullptr,
-            int64_t add_ld = 0) {
+            int64_t add_ld = 0, bool add_lo = false) {
   if (abl_skip("bn")) return;
+  const int flags = tc_mode(c) ? (round | (c.net->x3() ? 4 : c.net->bf16() ? 8 : 0) | (add_lo ? 16 : 0)) : 0;
   EX(mm3d_bnrelu_bwd_impl(x, x_hi, c_lo, dy, dx, dx_hi, n, ch, P(c, pidx), P(c, pidx + 1), save, save + ch, Gp(c, pidx), Gp(c, pidx + 1), 0.f,
-                          c.training, c.bn_ws, c.bn_ws_bytes, true, tc_mode(c) ? (round | (c.net->x3() ? 4 : c.net->bf16() ? 8 : 0)) : 0, add, add_ld,
-                          c.stream));
+                          c.training, c.bn_ws, c.bn_ws_bytes, true, flags, add, add_ld, c.stream));
 }
-enum Kind { SMC, DOWN, UP };
+// NIN: NetworkInNetwork, a K = 1 convolution over the level's identity row plan
+enum Kind { SMC, DOWN, UP, NIN };
 
 const float* find_img(const Ctx& c, const float* w) {
   for (size_t i = 0; i < c.img_key.size(); ++i)
@@ -335,76 +437,87 @@ const float* find_img_lo(const Ctx& c, const float* w) {
 }
 // One rule-table convolution from prebuilt weight images.  TF32x3 mode: hi.Whi + lo.Whi + hi.Wlo inside one launch (`in`
 // carries the lo plane n_in * c_in floats behind the hi one, both planes are gathered into every ring stage).
+// add != NULL: out = conv + add (add == out accumulates)
 int conv_img(const Ctx& c, const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out, const float* im,
-             const float* im_lo, int K, const void* plan, int64_t plan_cap) {
+             const float* im_lo, int K, const void* plan, int64_t plan_cap, const float* add = nullptr) {
   if (c.net->x3() && !im_lo) { mm3d_set_error("tf32x3: missing lo weight image"); return MM3D_ERR_INVALID; }
   if (c.net->bf16())  // the BF16 plane sits n_in * c_in floats behind the FP32 one
-    return mm3d_conv_fwd_tc_img(in + n_in * (int64_t)c_in, n_in, c_in, out, n_out, c_out, im, K, plan, plan_cap, 0, c.stream, nullptr, 1);
-  return mm3d_conv_fwd_tc_img(in, n_in, c_in, out, n_out, c_out, im, K, plan, plan_cap, 0, c.stream, c.net->x3() ? im_lo : nullptr);
+    return mm3d_conv_fwd_tc_img(in + n_in * (int64_t)c_in, n_in, c_in, out, n_out, c_out, im, K, plan, plan_cap, add, c.stream, nullptr, 1);
+  return mm3d_conv_fwd_tc_img(in, n_in, c_in, out, n_out, c_out, im, K, plan, plan_cap, add, c.stream, c.net->x3() ? im_lo : nullptr);
 }
-// forward of layer type `kind` whose FINE level is l
-void conv_fwd(Ctx& c, Kind kind, int l, const float* in, int c_in, float* out, int c_out, const float* w) {
-  if (abl_skip("conv")) return;
+
+// the rule table of a layer type at FINE level l, as the convolutions take it
+struct Table {
+  int K;
+  const int32_t* tbl;
+  int64_t stride;
+  const uint8_t* onehot;
+  const void* plan;
+  int64_t cap;
+  int64_t n_in, n_out;
+};
+Table table(const Ctx& c, Kind kind, int l) {
   const LevelMeta& f = c.net->lv[l];
+  const int64_t nc = l + 1 < c.net->L ? c.net->lv[l + 1].n : 0;
+  switch (kind) {
+    case SMC: return {27, f.nbr, f.tstride, nullptr, f.plan_smc, f.plan_cap, f.n, f.n};
+    case DOWN: return {8, f.child, f.tstride, nullptr, f.plan_down, f.plan_cap, f.n, nc};
+    case UP: return {8, f.parent, 0, f.off, f.plan_up, f.plan_cap, nc, f.n};
+    default: {
+      const void* plan = c.net->b[l].id_plan;
+      return {1, mm3d_plan_view(plan, f.n).tbl, mm3d_plan_tiles(f.n) * 128, nullptr, plan, f.n, f.n, f.n};
+    }
+  }
+}
+// the table of the transposed layer (dgrad): SMC and NIN are their own transpose, DOWN <-> UP
+Table table_t(const Ctx& c, Kind kind, int l) {
+  Table t = table(c, kind == DOWN ? UP : kind == UP ? DOWN : kind, l);
+  return t;
+}
+
+// forward of layer type `kind` whose FINE level is l; add != NULL: out = conv + add (add may be out)
+void conv_fwd(Ctx& c, Kind kind, int l, const float* in, int c_in, float* out, int c_out, const float* w,
+              const float* add = nullptr) {
+  if (abl_skip("conv")) return;
+  const Table t = table(c, kind, l);
   if (const float* im = find_img(c, w)) {  // prebuilt weight image: the tcgen05 kernel directly
-    const int64_t nc = l + 1 < c.net->L ? c.net->lv[l + 1].n : 0;
-    const float* il = find_img_lo(c, w);
-    if (kind == SMC) EX(conv_img(c, in, f.n, c_in, out, f.n, c_out, im, il, 27, f.plan_smc, f.plan_cap));
-    else if (kind == DOWN) EX(conv_img(c, in, f.n, c_in, out, nc, c_out, im, il, 8, f.plan_down, f.plan_cap));
-    else EX(conv_img(c, in, nc, c_in, out, f.n, c_out, im, il, 8, f.plan_up, f.plan_cap));
+    EX(conv_img(c, in, t.n_in, c_in, out, t.n_out, c_out, im, find_img_lo(c, w), t.K, t.plan, t.cap, add));
     return;
   }
-  if (kind == SMC)
-    EX(mm3d_conv_fwd(in, f.n, c_in, out, f.n, c_out, w, 27, f.nbr, f.tstride, nullptr, f.plan_smc, f.plan_cap, 0,
-                     c.net->mode, c.scratch, c.scratch_bytes, c.stream));
-  else if (kind == DOWN)
-    EX(mm3d_conv_fwd(in, f.n, c_in, out, c.net->lv[l + 1].n, c_out, w, 8, f.child, f.tstride, nullptr, f.plan_down,
-                     f.plan_cap, 0, c.net->mode, c.scratch, c.scratch_bytes, c.stream));
-  else
-    EX(mm3d_conv_fwd(in, c.net->lv[l + 1].n, c_in, out, f.n, c_out, w, 8, f.parent, 0, f.off, f.plan_up, f.plan_cap, 0,
+  if (add) {  // (no weight image: FP32 mode, or a TF32 shape the tensor cores do not take) the SIMT kernel with the addend
+    if (c.net->x3() || c.net->bf16()) {
+      mm3d_set_error("unet: conv c_in %d c_out %d has no tensor-core weight image in this mode", c_in, c_out);
+      if (c.rc == 0) c.rc = MM3D_ERR_UNSUPPORTED;
+      return;
+    }
+    EX(mm3d_conv_fwd_simt(in, t.n_in, c_in, out, t.n_out, c_out, w, t.K, t.tbl, t.stride, t.onehot, 0, c.scratch,
+                          c.scratch_bytes, c.stream, add));
+  } else
+    EX(mm3d_conv_fwd(in, t.n_in, c_in, out, t.n_out, c_out, w, t.K, t.tbl, t.stride, t.onehot, t.plan, t.cap, 0,
                      c.net->mode, c.scratch, c.scratch_bytes, c.stream));
 }
 // dgrad (d_in from d_out) and wgrad of the same layer; c_in / c_out are the FORWARD layer's
 void conv_bwd(Ctx& c, Kind kind, int l, const float* in, int c_in, const float* d_out, int c_out, const float* w,
               float* d_in, float* d_w) {
-  const LevelMeta& f = c.net->lv[l];
-  const int64_t nc = l + 1 < c.net->L ? c.net->lv[l + 1].n : 0;
   const int md = c.net->mode;
+  const Table t = table(c, kind, l), tt = table_t(c, kind, l);
   cudaStream_t ws = wgrad_stream(c);  // d_out is complete on the main stream at this point
   const float* im = find_img(c, w);   // prebuilt dgrad image (tensor-core modes)
   const float* il = find_img_lo(c, w);
   // parameter gradients inside the caller's (pre-zeroed) flat buffer accumulate; temporaries are overwritten
   const int acc = c.wgrad_acc && c.grad_lo <= (const char*)d_w && (const char*)d_w < c.grad_hi;
-  const bool do_wg = !abl_skip("wgrad") && d_w != nullptr, do_dg = !abl_skip("conv");  // (frozen weight: no d_w)
+  const bool do_wg = !abl_skip("wgrad") && d_w != nullptr, do_dg = !abl_skip("conv") && d_in != nullptr;  // (frozen weight: no d_w)
   // The weight gradient (side stream) is enqueued before the data gradient.  (Measured with the in-process A/B of
   // bench.py on the final kernels: the order makes no difference, 2.959 vs 2.958 ms per step -- the step is bound by
   // the total work of both streams, not by which kernel gets the SMs first.)
-  if (kind == SMC) {
-    if (do_wg)
-      EX(mm3d_conv_wgrad(in, f.n, c_in, d_out, f.n, c_out, d_w, 27, f.nbr, f.tstride, nullptr, f.plan_smc, f.plan_cap, acc,
-                         md, nullptr, 0, ws));
-    if (d_in && im && do_dg)
-      EX(conv_img(c, d_out, f.n, c_out, d_in, f.n, c_in, im, il, 27, f.plan_smc, f.plan_cap));
-    else if (d_in && do_dg)
-      EX(mm3d_conv_fwd(d_out, f.n, c_out, d_in, f.n, c_in, w, 27, f.nbr, f.tstride, nullptr, f.plan_smc, f.plan_cap,
-                       MM3D_CONV_TRANSPOSE_W | MM3D_CONV_MIRROR_K, md, c.scratch, c.scratch_bytes, c.stream));
-  } else if (kind == DOWN) {  // in: fine rows, d_out: coarse rows
-    if (do_wg)
-      EX(mm3d_conv_wgrad(in, f.n, c_in, d_out, nc, c_out, d_w, 8, f.child, f.tstride, nullptr, f.plan_down, f.plan_cap, acc,
-                         md, nullptr, 0, ws));
-    if (im && do_dg) EX(conv_img(c, d_out, nc, c_out, d_in, f.n, c_in, im, il, 8, f.plan_up, f.plan_cap));
-    else if (do_dg)
-      EX(mm3d_conv_fwd(d_out, nc, c_out, d_in, f.n, c_in, w, 8, f.parent, 0, f.off, f.plan_up, f.plan_cap,
-                       MM3D_CONV_TRANSPOSE_W, md, c.scratch, c.scratch_bytes, c.stream));
-  } else {  // UP: in: coarse rows, d_out: fine rows
-    if (do_wg)
-      EX(mm3d_conv_wgrad(in, nc, c_in, d_out, f.n, c_out, d_w, 8, f.parent, 0, f.off, f.plan_up, f.plan_cap, acc, md,
-                         nullptr, 0, ws));
-    if (im && do_dg) EX(conv_img(c, d_out, f.n, c_out, d_in, nc, c_in, im, il, 8, f.plan_down, f.plan_cap));
-    else if (do_dg)
-      EX(mm3d_conv_fwd(d_out, f.n, c_out, d_in, nc, c_in, w, 8, f.child, f.tstride, nullptr, f.plan_down, f.plan_cap,
-                       MM3D_CONV_TRANSPOSE_W, md, c.scratch, c.scratch_bytes, c.stream));
-  }
+  if (do_wg)
+    EX(mm3d_conv_wgrad(in, t.n_in, c_in, d_out, t.n_out, c_out, d_w, t.K, t.tbl, t.stride, t.onehot, t.plan, t.cap, acc,
+                       md, nullptr, 0, ws));
+  if (im && do_dg)
+    EX(conv_img(c, d_out, t.n_out, c_out, d_in, t.n_in, c_in, im, il, t.K, tt.plan, tt.cap));
+  else if (do_dg)
+    EX(mm3d_conv_fwd(d_out, t.n_out, c_out, d_in, t.n_in, c_in, w, t.K, tt.tbl, tt.stride, tt.onehot, tt.plan, tt.cap,
+                     MM3D_CONV_TRANSPOSE_W | (kind == SMC ? MM3D_CONV_MIRROR_K : 0), md, c.scratch, c.scratch_bytes, c.stream));
 }
 
 // main stream waits for everything enqueued on the side stream so far
@@ -427,34 +540,58 @@ void launch_pad_cols(Ctx& c, const float* src, int64_t n, int c_src, float* dst,
   if (mm3d_launch_pdl(k_pad_cols, dim3(mm3d_grid(n * c_dst, 256)), dim3(256), 0, c.stream, src, n, c_src, dst, c_dst, round_tf32) != cudaSuccess) c.rc = MM3D_ERR_CUDA;
   mm3d_count_launches(1);
 }
-
-// parameter index bookkeeping: number of pointer slots a level (and everything below it) uses
-int level_slots(int l, int L) { return l + 1 < L ? 5 + 5 + level_slots(l + 1, L) + 5 + 5 : 5; }
+// JoinTable: j = [y | f] ([n, p] each)
+void launch_join(Ctx& c, const float* y, const float* f, int64_t n, int p, float* j) {
+  if ((p & 3) == 0) {
+    if (n && !c.rc) {
+      if (mm3d_launch_pdl(k_concat2, dim3(mm3d_grid(n * p / 2 + 1, 256)), dim3(256), 0, c.stream, y, f, n, p, j) != cudaSuccess)
+        c.rc = MM3D_ERR_CUDA;
+      mm3d_count_launches(1);
+    }
+  } else {
+    launch_copy_cols(c, y, n, p, j, 2 * p, 0, p);
+    launch_copy_cols(c, f, n, p, j, 2 * p, p, p);
+  }
+}
 
 struct ConvInfo {
   int pidx, K, c_in, c_out, smc;
 };
-// every convolution of the network below level l (slot layout as in level_fwd)
-void list_convs(const Net& net, int l, int pbase, std::vector<ConvInfo>& v) {
-  const int p = net.planes(l);
-  v.push_back({pbase + 4, 27, p, p, 1});
-  if (l + 1 < net.L) {
-    const int q = net.planes(l + 1);
-    const int dn = pbase + 5, deeper = pbase + 10, up = deeper + level_slots(l + 1, net.L), post = up + 5;
-    v.push_back({dn + 4, 8, p, q, 0});
-    list_convs(net, l + 1, deeper, v);
-    v.push_back({up + 4, 8, q, p, 0});
-    v.push_back({post + 4, 27, 2 * p, p, 1});
+void list_block_convs(const Net& net, const BlockBufs& k, std::vector<ConvInfo>& v) {
+  if (!net.res) {
+    v.push_back({k.pidx + 4, 27, k.a, k.b, 1});
+    return;
   }
+  const int o = net.nin(k.a, k.b) ? 1 : 0;
+  if (o) v.push_back({k.pidx, 1, k.a, k.b, 0});
+  v.push_back({k.pidx + o + 4, 27, k.a, k.b, 1});
+  v.push_back({k.pidx + o + 9, 27, k.b, k.b, 1});
+}
+// every convolution of the network below level l, in slot order (the blocks' slots come from `carve`, which
+// needs no buffers: a shape-only Net carved with a NULL base works)
+void list_convs(const Net& net, int l, std::vector<ConvInfo>& v) {
+  const LevelBufs& B = net.b[l];
+  for (const BlockBufs& k : B.pre) list_block_convs(net, k, v);
+  if (l + 1 < net.L) {
+    const int p = net.planes(l), q = net.planes(l + 1);
+    const int dn = B.pre.back().pidx + net.block_slots(p, p), up = post_base(net, l) - 5;
+    v.push_back({dn + 4, 8, p, q, 0});
+    list_convs(net, l + 1, v);
+    v.push_back({up + 4, 8, q, p, 0});
+    for (const BlockBufs& k : B.post) list_block_convs(net, k, v);
+  }
+}
+std::vector<ConvInfo> all_convs(const Net& net, int cin) {
+  std::vector<ConvInfo> v;
+  v.push_back({0, 27, cin, net.m, 1});
+  list_convs(net, 0, v);
+  return v;
 }
 
 size_t img_region_bytes(const Net& net) {
   if (net.mode == MM3D_MODE_FP32) return 0;
-  std::vector<ConvInfo> v;
-  v.push_back({0, 27, net.cin_k, net.m, 1});
-  list_convs(net, 0, 1, v);
   size_t fwd = 0, bwd = 0;
-  for (const ConvInfo& ci : v) {
+  for (const ConvInfo& ci : all_convs(net, net.cin_k)) {
     fwd += mm3d_align(mm3d_conv_tc_workspace_bytes(ci.c_in, ci.c_out, ci.K));
     bwd += mm3d_align(mm3d_conv_tc_workspace_bytes(ci.c_out, ci.c_in, ci.K));
   }
@@ -465,14 +602,11 @@ size_t img_region_bytes(const Net& net) {
 int build_images(Ctx& c, bool backward, const float* w_stem) {
   const Net& net = *c.net;
   if (net.mode == MM3D_MODE_FP32 || !c.img_ws) return MM3D_OK;
-  std::vector<ConvInfo> v;
-  v.push_back({0, 27, net.cin_k, net.m, 1});
-  list_convs(net, 0, 1, v);
   std::vector<const float*> w;
   std::vector<float*> img;
   std::vector<int> K, ci, co, fl;
   char* at = (char*)c.img_ws;
-  for (const ConvInfo& x : v) {
+  for (const ConvInfo& x : all_convs(net, net.cin_k)) {
     const int a = backward ? x.c_out : x.c_in, b = backward ? x.c_in : x.c_out;
     if (!mm3d_conv_tc_supported(a, b, x.K)) continue;
     const size_t bytes = mm3d_align(mm3d_conv_tc_workspace_bytes(a, b, x.K));
@@ -504,83 +638,170 @@ int build_images(Ctx& c, bool backward, const float* w_stem) {
   return MM3D_OK;
 }
 
-void level_fwd(Ctx& c, int l, int pbase) {
+// the identity row plans of every level with a NetworkInNetwork shortcut, one launch
+void build_identity_plans(Ctx& c) {
+  const Net& net = *c.net;
+  IdPlans ps{};
+  int64_t most = 0;
+  bool any = false;
+  for (int l = 0; l < net.L && l < kMaxIdPlans; ++l) {
+    ps.plan[l] = net.b[l].id_plan;
+    ps.rows[l] = net.lv[l].n;
+    if (ps.plan[l]) {
+      any = true;
+      if (net.lv[l].n > most) most = net.lv[l].n;
+    }
+  }
+  if (!any || c.rc) return;
+  if (net.L > kMaxIdPlans) { mm3d_set_error("unet: more than %d levels", kMaxIdPlans); c.rc = MM3D_ERR_UNSUPPORTED; return; }
+  const int blocks = mm3d_grid(mm3d_plan_tiles(most) * 128 + 1, 256);
+  if (mm3d_launch_pdl(k_identity_plans, dim3(blocks, net.L), dim3(256), 0, c.stream, ps) != cudaSuccess) c.rc = MM3D_ERR_CUDA;
+  mm3d_count_launches(1);
+}
+
+// A block's forward.  x: its input [n, a]; the first post block of a level (join) reads [Y | F] instead.
+void block_fwd(Ctx& c, int l, const BlockBufs& k, const float* x, bool join) {
+  Net& net = *c.net;
+  LevelBufs& B = net.b[l];
+  const int64_t n = net.lv[l].n;
+  const int o = net.nin(k.a, k.b) ? 1 : 0;
+  const int bn1 = k.pidx + o;
+  if (join) {
+    const int p = k.b;
+    const bool split = (p & 3) == 0 && c.training;  // JoinTable never materialised: BatchNorm reads [Y | F] directly
+    // the shortcut gathers J: it is written (the BatchNorm of an unsplit join reads the unrounded J)
+    if (!split || o) launch_join(c, B.Y, B.F, n, p, split ? B.Jop : B.J);
+    if (split) bn_fwd(c, bn1, B.Y, k.A, n, 2 * p, k.s1, B.F, p);
+    else bn_fwd(c, bn1, B.J, k.A, n, 2 * p, k.s1);
+    if (o && tc_mode(c))  // J in operand form (rounded; + second plane)
+      launch_pad_cols(c, split ? B.Jop : B.J, n, 2 * p, B.Jop, 2 * p, net.rmode());
+    MARK("bn_fwd post", l);
+  } else {
+    bn_fwd(c, bn1, x, k.A, n, k.a, k.s1);
+    MARK("bn_fwd block", l);
+  }
+  if (!net.res) {
+    conv_fwd(c, SMC, l, k.A, k.a, k.out, k.b, P(c, k.pidx + 4));
+    MARK("smc_fwd block", l);
+    return;
+  }
+  conv_fwd(c, SMC, l, k.A, k.a, k.H, k.b, P(c, bn1 + 4));
+  bn_fwd(c, bn1 + 5, k.H, k.A2, n, k.b, k.s2);
+  if (o) {  // NetworkInNetwork shortcut writes `out`, the second convolution adds onto it
+    conv_fwd(c, NIN, l, B.Jop, k.a, k.out, k.b, P(c, k.pidx));
+    conv_fwd(c, SMC, l, k.A2, k.b, k.out, k.b, P(c, bn1 + 9), k.out);
+  } else {  // identity shortcut: the block input is the second convolution's addend
+    conv_fwd(c, SMC, l, k.A2, k.b, k.out, k.b, P(c, bn1 + 9), x);
+  }
+  MARK("residual block fwd", l);
+}
+
+void level_fwd(Ctx& c, int l) {
   Net& net = *c.net;
   LevelBufs& B = net.b[l];
   const int64_t n = net.lv[l].n;
   const int p = net.planes(l);
-  bn_fwd(c, pbase, B.X, B.A, n, p, B.s_pre);
-  MARK("bn_fwd pre", l);
-  conv_fwd(c, SMC, l, B.A, p, B.Y, p, P(c, pbase + 4));
-  MARK("smc_fwd pre", l);
+  const float* x = B.X;
+  for (const BlockBufs& k : B.pre) {
+    block_fwd(c, l, k, x, false);
+    x = k.out;
+  }
   if (l + 1 < net.L) {
     const int q = net.planes(l + 1);
-    const int dn = pbase + 5, deeper = pbase + 10, up = deeper + level_slots(l + 1, net.L), post = up + 5;
+    const int dn = B.pre.back().pidx + net.block_slots(p, p), up = post_base(net, l) - 5;
     bn_fwd(c, dn, B.Y, B.B, n, p, B.s_dn);
     MARK("bn_fwd dn", l);
     conv_fwd(c, DOWN, l, B.B, p, net.b[l + 1].X, q, P(c, dn + 4));
     MARK("down_fwd", l);
-    level_fwd(c, l + 1, deeper);
+    level_fwd(c, l + 1);
     bn_fwd(c, up, net.b[l + 1].R, B.E, net.lv[l + 1].n, q, B.s_up);
     MARK("bn_fwd up", l);
     conv_fwd(c, UP, l, B.E, q, B.F, p, P(c, up + 4));
     MARK("up_fwd", l);
-    if ((p & 3) == 0 && c.training) {
-      // JoinTable is never materialised: BatchNorm reads the two column blocks [Y | F] directly
-      bn_fwd(c, post, B.Y, B.G, n, 2 * p, B.s_post, B.F, p);
-      MARK("bn_fwd post", l);
-    } else {
-      if ((p & 3) == 0) {
-        if (n && !c.rc) {
-          if (mm3d_launch_pdl(k_concat2, dim3(mm3d_grid(n * p / 2 + 1, 256)), dim3(256), 0, c.stream, (const float*)B.Y,
-                              (const float*)B.F, n, p, B.J) != cudaSuccess)
-            c.rc = MM3D_ERR_CUDA;
-          mm3d_count_launches(1);
-        }
-      } else {
-        launch_copy_cols(c, B.Y, n, p, B.J, 2 * p, 0, p);
-        launch_copy_cols(c, B.F, n, p, B.J, 2 * p, p, p);
-      }
-      bn_fwd(c, post, B.J, B.G, n, 2 * p, B.s_post);
-    }
-    conv_fwd(c, SMC, l, B.G, 2 * p, B.R, p, P(c, post + 4));
-    MARK("smc_fwd post", l);
+    for (size_t r = 0; r < B.post.size(); ++r) block_fwd(c, l, B.post[r], r ? B.post[r - 1].out : nullptr, r == 0);
   }
 }
 
-// d_R: gradient w.r.t. the level's output R_l; returns (in d_X) the gradient w.r.t. X_l.
+// A block's backward.  d_o: gradient w.r.t. its output (operand form); writes d_x, the gradient w.r.t. its input,
+// in operand form.  The first post block (join) instead writes the skip half d_J[:, :p] (unrounded; all of d_J
+// when the join is not split) and d_F, the deconvolution's d_out (operand form).
+void block_bwd(Ctx& c, Bump& g, int l, const BlockBufs& k, const float* x, const float* d_o, float* d_x, bool join,
+               float* d_J = nullptr, float* d_F = nullptr) {
+  Net& net = *c.net;
+  LevelBufs& B = net.b[l];
+  const int64_t n = net.lv[l].n;
+  const int pl = net.pl();
+  const int o = net.nin(k.a, k.b) ? 1 : 0;
+  const int bn1 = k.pidx + o;
+  const float* add = nullptr;  // the shortcut's gradient, summed into the first BatchNorm's backward
+  int64_t add_ld = 0;
+  bool add_lo = false;
+  float* d_A = g.f(n, k.a);
+  if (!net.res) {
+    conv_bwd(c, SMC, l, k.A, k.a, d_o, k.b, P(c, k.pidx + 4), d_A, Gp(c, k.pidx + 4));
+  } else {
+    float* d_A2 = g.f(n, k.b);
+    conv_bwd(c, SMC, l, k.A2, k.b, d_o, k.b, P(c, bn1 + 9), d_A2, Gp(c, bn1 + 9));
+    float* d_H = g.f(n, (int64_t)k.b * pl);
+    bn_bwd(c, bn1 + 5, k.H, d_A2, d_H, n, k.b, k.s2, 1);
+    conv_bwd(c, SMC, l, k.A, k.a, d_H, k.b, P(c, bn1 + 4), d_A, Gp(c, bn1 + 4));
+    if (o) {
+      float* d_S = g.f(n, k.a);
+      conv_bwd(c, NIN, l, B.Jop, k.a, d_o, k.b, P(c, k.pidx), d_S, Gp(c, k.pidx));
+      add = d_S;
+      add_ld = k.a;
+    } else {  // identity: d_o itself, FP32-exact in TF32x3 mode through its lo plane
+      add = d_o;
+      add_ld = k.b;
+      add_lo = net.x3();
+    }
+  }
+  MARK("block conv bwd", l);
+  if (!join) {
+    bn_bwd(c, bn1, x, d_A, d_x, n, k.a, k.s1, 1, nullptr, 0, nullptr, add, add_ld, add_lo);
+    MARK("bn_bwd block", l);
+    return;
+  }
+  const int p = k.b;
+  if ((p & 3) == 0 && c.training) {  // as in the forward: [Y | F] was never concatenated
+    bn_bwd(c, bn1, B.Y, d_A, d_J, n, 2 * p, k.s1, 2, B.F, p, d_F, add, add_ld);  // d_F is the deconvolution's d_out
+  } else {
+    bn_bwd(c, bn1, B.J, d_A, d_J, n, 2 * p, k.s1, 0, nullptr, 0, nullptr, add, add_ld);  // (eval-mode backward: d_F stays unrounded)
+    // d_F = d_J[:, p:]; the skip half is combined with the branch gradient further down
+    if (n && !c.rc) {
+      if (mm3d_launch_pdl(k_copy_cols, dim3(mm3d_grid(n * p / 4 + 1, 256)), dim3(256), 0, c.stream, (const float*)d_J, n, 2 * p, d_F, p, 0, p, p) != cudaSuccess) c.rc = MM3D_ERR_CUDA;
+      mm3d_count_launches(1);
+      if (tc_mode(c)) launch_pad_cols(c, d_F, n, p, d_F, p, net.rmode());  // round in place (+ second plane): d_F is the deconvolution's d_out
+    }
+  }
+  MARK("bn_bwd post", l);
+}
+
+// d_R: gradient w.r.t. the level's output R_l (operand form); returns (in d_X) the gradient w.r.t. X_l.
 // Gradient temporaries come from the backward bump allocator `g`.
-void level_bwd(Ctx& c, Bump& g, int l, int pbase, const float* d_R, float* d_X) {
+void level_bwd(Ctx& c, Bump& g, int l, const float* d_R, float* d_X) {
   Net& net = *c.net;
   LevelBufs& B = net.b[l];
   const int64_t n = net.lv[l].n;
   const int p = net.planes(l);
+  const int pl = net.pl();  // conv d_out tensors carry a second plane in the TF32x3 and BF16 modes
   const float* d_Y = d_R;
   const size_t mark = g.off;
   if (l + 1 < net.L) {
     const int q = net.planes(l + 1);
     const int64_t nc = net.lv[l + 1].n;
-    const int dn = pbase + 5, deeper = pbase + 10, up = deeper + level_slots(l + 1, net.L), post = up + 5;
-    float* d_G = g.f(n, 2 * p);
-    conv_bwd(c, SMC, l, B.G, 2 * p, d_R, p, P(c, post + 4), d_G, Gp(c, post + 4));
-    MARK("smc_dgrad post", l);
-    const bool split = (p & 3) == 0 && c.training;  // as in the forward: [Y | F] was never concatenated
-    float* d_J = g.f(n, split ? p : 2 * p);         // split: only the skip half d_J[:, :p]
-    const int pl = net.pl();  // conv d_out tensors carry a second plane in the TF32x3 and BF16 modes
+    const int dn = B.pre.back().pidx + net.block_slots(p, p), up = post_base(net, l) - 5;
+    const float* d_o = d_R;
+    for (size_t r = B.post.size() - 1; r >= 1; --r) {
+      float* d_x = g.f(n, (int64_t)p * pl);
+      block_bwd(c, g, l, B.post[r], B.post[r - 1].out, d_o, d_x, false);
+      d_o = d_x;
+    }
+    const bool split = (p & 3) == 0 && c.training;
+    float* d_J = g.f(n, split ? p : 2 * p);  // split: only the skip half d_J[:, :p]
     float* d_F = g.f(n, (int64_t)p * pl);
     float* d_Yskip = g.f(n, (int64_t)p * pl);
-    if (split) {
-      bn_bwd(c, post, B.Y, d_G, d_J, n, 2 * p, B.s_post, 2, B.F, p, d_F);  // d_F is the deconvolution's d_out
-      MARK("bn_bwd post", l);
-    } else {
-      bn_bwd(c, post, B.J, d_G, d_J, n, 2 * p, B.s_post, 0);  // (eval-mode backward: d_F stays unrounded)
-      // d_F = d_J[:, p:]; the skip half is combined with the branch gradient further down
-      if (n && !c.rc) {
-        if (mm3d_launch_pdl(k_copy_cols, dim3(mm3d_grid(n * p / 4 + 1, 256)), dim3(256), 0, c.stream, (const float*)d_J, n, 2 * p, d_F, p, 0, p, p) != cudaSuccess) c.rc = MM3D_ERR_CUDA;
-        mm3d_count_launches(1);
-        if (tc_mode(c)) launch_pad_cols(c, d_F, n, p, d_F, p, net.rmode());  // round in place (+ second plane): d_F is the deconvolution's d_out
-      }
-    }
+    block_bwd(c, g, l, B.post[0], nullptr, d_o, nullptr, true, d_J, d_F);
     float* d_E = g.f(nc, q);
     conv_bwd(c, UP, l, B.E, q, d_F, p, P(c, up + 4), d_E, Gp(c, up + 4));
     MARK("up_dgrad", l);
@@ -588,7 +809,7 @@ void level_bwd(Ctx& c, Bump& g, int l, int pbase, const float* d_R, float* d_X) 
     bn_bwd(c, up, net.b[l + 1].R, d_E, d_Rn, nc, q, B.s_up, 1);
     MARK("bn_bwd up", l);
     float* d_Xn = g.f(nc, (int64_t)q * pl);
-    level_bwd(c, g, l + 1, deeper, d_Rn, d_Xn);
+    level_bwd(c, g, l + 1, d_Rn, d_Xn);
     float* d_B = g.f(n, p);
     conv_bwd(c, DOWN, l, B.B, p, d_Xn, q, P(c, dn + 4), d_B, Gp(c, dn + 4));
     MARK("down_dgrad", l);
@@ -598,25 +819,29 @@ void level_bwd(Ctx& c, Bump& g, int l, int pbase, const float* d_R, float* d_X) 
     MARK("bn_bwd dn", l);
     d_Y = d_Yskip;
   }
-  float* d_A = g.f(n, p);
-  conv_bwd(c, SMC, l, B.A, p, d_Y, p, P(c, pbase + 4), d_A, Gp(c, pbase + 4));
-  MARK("smc_dgrad pre", l);
-  bn_bwd(c, pbase, B.X, d_A, d_X, n, p, B.s_pre, 1);
-  MARK("bn_bwd pre", l);
+  for (size_t r = B.pre.size(); r-- > 0;) {
+    float* d_x = r ? g.f(n, (int64_t)p * pl) : d_X;
+    block_bwd(c, g, l, B.pre[r], r ? B.pre[r - 1].out : B.X, d_Y, d_x, false);
+    d_Y = d_x;
+  }
   if (!c.side) g.off = mark;  // temporaries of this level are dead once d_X is written -- unless the side stream
                               // may still be reading a d_out (the workspace bound assumes no reuse anyway)
 }
 
-int fill_net(Net& net, int in_channels, int m, int num_planes, int mode, const int64_t* level_desc, int64_t n_points) {
+int fill_net(Net& net, int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+             const int64_t* level_desc, int64_t n_points) {
   MM3D_REQUIRE(num_planes >= 1 && num_planes <= 16 && m > 0 && in_channels > 0, MM3D_ERR_INVALID, "bad network shape");
+  MM3D_REQUIRE(block_reps >= 1 && block_reps <= 16 && (residual == 0 || residual == 1), MM3D_ERR_INVALID,
+               "bad block topology: block_reps %d residual %d", block_reps, residual);
   MM3D_REQUIRE(mode == MM3D_MODE_FP32 || mode == MM3D_MODE_TF32 || mode == MM3D_MODE_TF32X3 || mode == MM3D_MODE_BF16, MM3D_ERR_UNSUPPORTED,
                "conv mode %d not implemented in this build", mode);
   net.L = num_planes; net.m = m; net.cin = in_channels; net.mode = mode; net.n_points = n_points;
+  net.reps = block_reps; net.res = residual;
   // tensor-core kernels gather rows in 64-byte pieces: pad the stem input to a multiple of 16 channels
   net.cin_k = in_channels;
   if (mode != MM3D_MODE_FP32) net.cin_k = (in_channels + 15) / 16 * 16;
-  net.lv.resize(num_planes);
-  for (int l = 0; l < num_planes; ++l) {
+  net.lv.assign(num_planes, LevelMeta{});
+  for (int l = 0; l < num_planes && level_desc; ++l) {
     const int64_t* d = level_desc + MM3D_LEVEL_DESC_WORDS * l;
     net.lv[l] = LevelMeta{d[0], (const int32_t*)d[1], d[2], (const int32_t*)d[3], (const uint8_t*)d[4], (const int32_t*)d[5],
                           (const void*)d[6], (const void*)d[7], (const void*)d[8], d[9]};
@@ -629,13 +854,18 @@ size_t bwd_temp_bytes(const Net& net) {
   size_t total = 0;
   for (int l = 0; l < net.L; ++l) {
     const size_t n = (size_t)net.lv[l].n, p = (size_t)net.planes(l);
+    const bool deeper = l + 1 < net.L;
     size_t rows = 0;
-    if (l + 1 < net.L) {
+    if (deeper) {
       const size_t nc = (size_t)net.lv[l + 1].n, q = (size_t)net.planes(l + 1);
       rows = n * (2 * p + 2 * p + p + p + p + p) + nc * (3 * q);
     }
     rows += n * p;
-    total += mm3d_align(sizeof(float) * rows) + 16 * 256;
+    // further blocks (d_A + d_x each); residual blocks (d_A2 + d_H each, + the NetworkInNetwork's d_in)
+    const size_t blocks = (size_t)net.reps * (deeper ? 2 : 1);
+    rows += n * (blocks - (deeper ? 2 : 1)) * 2 * p;
+    if (net.res) rows += n * (blocks * 2 * p + (deeper ? 2 * p : 0));
+    total += mm3d_align(sizeof(float) * rows) + 16 * 256 + (blocks - (deeper ? 2 : 1) + (net.res ? 2 * blocks : 0)) * 2 * 256;
   }
   const size_t n0 = (size_t)net.lv[0].n;
   total += mm3d_align(4 * n0 * (size_t)net.m) * 3 + mm3d_align(4 * n0 * (size_t)(net.cin + net.cin_k)) * 2 + 8 * 256;
@@ -643,50 +873,38 @@ size_t bwd_temp_bytes(const Net& net) {
   return total * (size_t)net.pl();
 }
 
-}  // namespace
-
-extern "C" {
-
-// level_desc: MM3D_LEVEL_DESC_WORDS int64 per level = {n rows, nbr table ptr, table stride, parent ptr, off ptr,
-// child ptr, plan of the 3^3 table, plan of the child table, plan of the (parent, off) table, plan capacity}
-MM3D_API int64_t mm3d_unet_num_params(int num_planes) { return 1 + level_slots(0, num_planes) + 4; }
-
-MM3D_API size_t mm3d_unet_act_bytes(int in_channels, int m, int num_planes, int mode, const int64_t* level_desc,
-                                    int64_t n_points) {
-  Net net;
-  if (fill_net(net, in_channels, m, num_planes, mode, level_desc, n_points)) return 0;
-  Bump bp{nullptr, 0, ~(size_t)0, true};
-  carve(net, bp);
-  return bp.off + 256;
+// number of BatchNorm channels of the whole network (each has a gamma and a beta gradient)
+size_t bn_channels(const Net& net) {
+  size_t ch = (size_t)net.m;  // head
+  for (int l = 0; l < net.L; ++l) {
+    const size_t p = (size_t)net.planes(l);
+    const size_t per_block = net.res ? 2 : 1;  // (the first post block's first BatchNorm has 2p channels)
+    ch += net.reps * per_block * p;
+    if (l + 1 < net.L) ch += p + (size_t)net.planes(l + 1) + net.reps * per_block * p + p;
+  }
+  return ch;
 }
 
-MM3D_API size_t mm3d_unet_bwd_bytes(int in_channels, int m, int num_planes, int mode, const int64_t* level_desc,
-                                    int64_t n_points) {
-  Net net;
-  if (fill_net(net, in_channels, m, num_planes, mode, level_desc, n_points)) return 0;
-  return bwd_temp_bytes(net);
-}
-
-MM3D_API size_t mm3d_unet_scratch_bytes(int in_channels, int m, int num_planes, int mode) {
+size_t scratch_bytes(const Net& shape) {
+  const int m = shape.m, num_planes = shape.L;
   size_t best = mm3d_bnrelu_workspace_bytes(2 * m * num_planes);
-  const int cin_k = (in_channels + 15) / 16 * 16;
-  size_t s = mm3d_conv_workspace_bytes(0, 0, cin_k, m, 27, mode);
+  size_t s = mm3d_conv_workspace_bytes(0, 0, shape.cin_k, m, 27, shape.mode);
   if (s > best) best = s;
   for (int l = 0; l < num_planes; ++l) {
     const int p = m * (l + 1);
-    s = mm3d_conv_workspace_bytes(0, 0, 2 * p, p, 27, mode);
+    s = mm3d_conv_workspace_bytes(0, 0, 2 * p, p, 27, shape.mode);
     if (s > best) best = s;
-    s = mm3d_conv_workspace_bytes(0, 0, p + m, p, 8, mode);
+    s = mm3d_conv_workspace_bytes(0, 0, p + m, p, 8, shape.mode);
     if (s > best) best = s;
   }
-  Net shape;
-  shape.L = num_planes; shape.m = m; shape.cin = in_channels; shape.cin_k = cin_k; shape.mode = mode;
   return best + img_region_bytes(shape) + mm3d_bnrelu_workspace_bytes(2 * m * num_planes) +
-         mm3d_align(4 * (size_t)27 * cin_k * m) + 256;
+         mm3d_align(4 * (size_t)27 * shape.cin_k * m) + 256;
 }
 
+}  // namespace
+
 // carve the executor's private tail of the scratch buffer: [... | BatchNorm workspace | padded stem weight]
-int carve_tail(Ctx& c, const Net& net) {
+static int carve_tail(Ctx& c, const Net& net) {
   const size_t wp_bytes = mm3d_align(4 * (size_t)27 * net.cin_k * net.m);
   c.bn_ws_bytes = mm3d_bnrelu_workspace_bytes(2 * net.m * net.L);
   c.img_ws_bytes = img_region_bytes(net) / 256 * 256;
@@ -700,12 +918,61 @@ int carve_tail(Ctx& c, const Net& net) {
   return MM3D_OK;
 }
 
-MM3D_API int mm3d_unet_forward(int in_channels, int m, int num_planes, int mode, int training, float eps, float momentum,
-                               const int64_t* level_desc, int64_t n_points, const int32_t* p2v, const int32_t* npts,
-                               const float* feats, float* out, void* const* params, void* act, size_t act_bytes,
-                               void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask, mm3d_stream_t stream_) {
+extern "C" {
+
+// level_desc: MM3D_LEVEL_DESC_WORDS int64 per level = {n rows, nbr table ptr, table stride, parent ptr, off ptr,
+// child ptr, plan of the 3^3 table, plan of the child table, plan of the (parent, off) table, plan capacity}
+MM3D_API int64_t mm3d_unet_topo_num_params(int num_planes, int block_reps, int residual) {
   Net net;
-  int rc = fill_net(net, in_channels, m, num_planes, mode, level_desc, n_points);
+  if (fill_net(net, 1, 1, num_planes, block_reps, residual, MM3D_MODE_FP32, nullptr, 0)) return -1;
+  return 1 + level_slots(net, 0) + 4;
+}
+MM3D_API int64_t mm3d_unet_num_params(int num_planes) { return mm3d_unet_topo_num_params(num_planes, 1, 0); }
+
+MM3D_API size_t mm3d_unet_topo_act_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                         const int64_t* level_desc, int64_t n_points) {
+  Net net;
+  if (!level_desc || fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points)) return 0;
+  Bump bp{nullptr, 0, ~(size_t)0, true};
+  carve(net, bp);
+  return bp.off + 256;
+}
+MM3D_API size_t mm3d_unet_act_bytes(int in_channels, int m, int num_planes, int mode, const int64_t* level_desc,
+                                    int64_t n_points) {
+  return mm3d_unet_topo_act_bytes(in_channels, m, num_planes, 1, 0, mode, level_desc, n_points);
+}
+
+MM3D_API size_t mm3d_unet_topo_bwd_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                         const int64_t* level_desc, int64_t n_points) {
+  Net net;
+  if (!level_desc || fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points)) return 0;
+  return bwd_temp_bytes(net);
+}
+MM3D_API size_t mm3d_unet_bwd_bytes(int in_channels, int m, int num_planes, int mode, const int64_t* level_desc,
+                                    int64_t n_points) {
+  return mm3d_unet_topo_bwd_bytes(in_channels, m, num_planes, 1, 0, mode, level_desc, n_points);
+}
+
+MM3D_API size_t mm3d_unet_topo_scratch_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode) {
+  Net shape;
+  if (fill_net(shape, in_channels, m, num_planes, block_reps, residual, mode, nullptr, 0)) return 0;
+  shape.cin_k = (in_channels + 15) / 16 * 16;
+  Bump bp{nullptr, 0, ~(size_t)0, true};
+  carve(shape, bp);  // (block slots for the weight-image list; no buffers)
+  return scratch_bytes(shape);
+}
+MM3D_API size_t mm3d_unet_scratch_bytes(int in_channels, int m, int num_planes, int mode) {
+  return mm3d_unet_topo_scratch_bytes(in_channels, m, num_planes, 1, 0, mode);
+}
+
+MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                    int training, float eps, float momentum, const int64_t* level_desc, int64_t n_points,
+                                    const int32_t* p2v, const int32_t* npts, const float* feats, float* out,
+                                    void* const* params, void* act, size_t act_bytes, void* scratch, size_t scratch_bytes,
+                                    const mm3d_unet_mask* mask, mm3d_stream_t stream_) {
+  MM3D_REQUIRE(level_desc, MM3D_ERR_INVALID, "unet forward: no level descriptors");
+  Net net;
+  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points);
   if (rc) return rc;
   Bump bp{(char*)act, 0, act_bytes, true};
   carve(net, bp);
@@ -737,11 +1004,12 @@ MM3D_API int mm3d_unet_forward(int in_channels, int m, int num_planes, int mode,
     w_stem = wp;
   }
   EX(build_images(c, false, w_stem));
+  build_identity_plans(c);  // (kept in `act`: the backward reuses them)
   MARK("pad + weight images", -1);
   conv_fwd(c, SMC, 0, net.Vp, net.cin_k, net.b[0].X, m, w_stem);
   MARK("stem fwd", -1);
-  level_fwd(c, 0, 1);
-  const int head = 1 + level_slots(0, net.L);
+  level_fwd(c, 0);
+  const int head = 1 + level_slots(net, 0);
   bn_fwd(c, head, net.b[0].R, net.Z, n0, m, net.s_head, nullptr, 0, /*to_conv=*/false);
   MARK("bn_fwd head", -1);
   EX(mm3d_output_fwd(net.Z, p2v, n_points, m, out, c.stream));
@@ -749,14 +1017,24 @@ MM3D_API int mm3d_unet_forward(int in_channels, int m, int num_planes, int mode,
   return c.rc;
 }
 
+MM3D_API int mm3d_unet_forward(int in_channels, int m, int num_planes, int mode, int training, float eps, float momentum,
+                               const int64_t* level_desc, int64_t n_points, const int32_t* p2v, const int32_t* npts,
+                               const float* feats, float* out, void* const* params, void* act, size_t act_bytes,
+                               void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask, mm3d_stream_t stream_) {
+  return mm3d_unet_topo_forward(in_channels, m, num_planes, 1, 0, mode, training, eps, momentum, level_desc, n_points, p2v,
+                                npts, feats, out, params, act, act_bytes, scratch, scratch_bytes, mask, stream_);
+}
+
 // grads: same slot order as params (running-stat slots ignored); d_feats may be NULL.
-MM3D_API int mm3d_unet_backward(int in_channels, int m, int num_planes, int mode, int training,
-                                const int64_t* level_desc, int64_t n_points, const int32_t* p2v, const int32_t* npts,
-                                const float* d_out, float* d_feats, void* const* params, void* const* grads,
-                                void* act, size_t act_bytes, void* tmp, size_t tmp_bytes, void* scratch,
-                                size_t scratch_bytes, const mm3d_unet_mask* mask, mm3d_stream_t stream_) {
+MM3D_API int mm3d_unet_topo_backward(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                     int training, const int64_t* level_desc, int64_t n_points, const int32_t* p2v,
+                                     const int32_t* npts, const float* d_out, float* d_feats, void* const* params,
+                                     void* const* grads, void* act, size_t act_bytes, void* tmp, size_t tmp_bytes,
+                                     void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask,
+                                     mm3d_stream_t stream_) {
+  MM3D_REQUIRE(level_desc, MM3D_ERR_INVALID, "unet backward: no level descriptors");
   Net net;
-  int rc = fill_net(net, in_channels, m, num_planes, mode, level_desc, n_points);
+  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points);
   if (rc) return rc;
   Bump bp{(char*)act, 0, act_bytes, true};
   carve(net, bp);
@@ -769,16 +1047,13 @@ MM3D_API int mm3d_unet_backward(int in_channels, int m, int num_planes, int mode
   if (rc) return rc;
   Bump g{(char*)tmp, 0, tmp_bytes, true};
   const int64_t n0 = net.lv[0].n;
-  const int head = 1 + level_slots(0, net.L);
+  const int head = 1 + level_slots(net, 0);
   {  // One memset instead of one per layer when the gradient buffers are one contiguous block (the shipped host
      // code hands out views of one flat tensor): slot sizes follow from the network shape.
-    std::vector<ConvInfo> v;
-    v.push_back({0, 27, net.cin, net.m, 1});
-    list_convs(net, 0, 1, v);
     const char *lo = nullptr, *hi = nullptr;
     size_t bytes = 0;
     bool all = true;
-    for (const ConvInfo& x : v) {
+    for (const ConvInfo& x : all_convs(net, net.cin)) {
       const char* g0 = (const char*)grads[x.pidx];
       if (!g0) { all = false; break; }
       const size_t nb_ = sizeof(float) * (size_t)x.K * x.c_in * x.c_out;
@@ -787,12 +1062,7 @@ MM3D_API int mm3d_unet_backward(int in_channels, int m, int num_planes, int mode
       bytes += nb_;
     }
     // BatchNorm gradients (2 * channels each) may sit in between: allow the span to be at most their size larger
-    size_t bn_bytes = 0;
-    for (int l = 0; l < net.L; ++l) {
-      const size_t pl = (size_t)net.planes(l);
-      bn_bytes += sizeof(float) * 2 * (l + 1 < net.L ? 4 * pl + (size_t)net.planes(l + 1) : pl);  // pre, dn, up, post
-    }
-    bn_bytes += sizeof(float) * 2 * (size_t)net.m;  // head
+    const size_t bn_bytes = sizeof(float) * 2 * bn_channels(net);
     if (all && lo && (size_t)(hi - lo) <= bytes + bn_bytes) {
       MM3D_CUDA(cudaMemsetAsync((void*)lo, 0, (size_t)(hi - lo), c.stream));
       c.grad_lo = lo; c.grad_hi = hi; c.wgrad_acc = 1;
@@ -814,7 +1084,7 @@ MM3D_API int mm3d_unet_backward(int in_channels, int m, int num_planes, int mode
   bn_bwd(c, head, net.b[0].R, d_Z, d_R0, n0, m, net.s_head, 1);
   MARK("bn_bwd head", -1);
   float* d_X0 = g.f(n0, (int64_t)m * net.pl());
-  level_bwd(c, g, 0, 1, d_R0, d_X0);
+  level_bwd(c, g, 0, d_R0, d_X0);
   // stem
   const float* w_stem = P(c, 0);
   float* d_w = Gp(c, 0);
@@ -850,6 +1120,16 @@ MM3D_API int mm3d_unet_backward(int in_channels, int m, int num_planes, int mode
   MARK("join wgrad stream", -1);
   MM3D_REQUIRE(g.ok, MM3D_ERR_WORKSPACE, "backward workspace overflow");
   return c.rc;
+}
+
+MM3D_API int mm3d_unet_backward(int in_channels, int m, int num_planes, int mode, int training,
+                                const int64_t* level_desc, int64_t n_points, const int32_t* p2v, const int32_t* npts,
+                                const float* d_out, float* d_feats, void* const* params, void* const* grads,
+                                void* act, size_t act_bytes, void* tmp, size_t tmp_bytes, void* scratch,
+                                size_t scratch_bytes, const mm3d_unet_mask* mask, mm3d_stream_t stream_) {
+  return mm3d_unet_topo_backward(in_channels, m, num_planes, 1, 0, mode, training, level_desc, n_points, p2v, npts, d_out,
+                                 d_feats, params, grads, act, act_bytes, tmp, tmp_bytes, scratch, scratch_bytes, mask,
+                                 stream_);
 }
 
 // out[i] = in[i] rounded to TF32 (round-to-nearest, ties away); in == out allowed.  The module-by-module path uses

@@ -1,9 +1,13 @@
 """Fused execution of ``UNetSCN``: the whole forward (and the whole backward) is ONE call into
-``libmm3d`` (``csrc/unet_exec.cu``) instead of ~110 Python autograd nodes.
+``libmm3d`` (``csrc/unet_exec.cu``) instead of ~110 Python autograd nodes (about twice that with
+``block_reps=2``).
 
-``UNetSCN.forward`` uses this path when the network has the reference's shape (VGG blocks,
-``block_reps == 1``, InputLayer mode 4 -- ``config/config.yaml:22-28``); any other configuration
-runs module by module.  Results are the same kernels in the same order, so parity is unchanged.
+``UNetSCN.forward`` uses this path for every block topology of the constructor (any ``block_reps``,
+VGG or residual blocks) with InputLayer mode 4 (``config/config.yaml:22-28``); what the executor does
+not implement (per-layer conv modes, conv or NetworkInNetwork bias, leaky ReLU) runs module by module.
+Results are the same kernels in the same order, so parity is unchanged; the one exception is the
+residual blocks' NetworkInNetwork, which the module path runs as an FP32 torch matmul and the executor
+as this library's K = 1 rule-table convolution in the network's convolution mode.
 """
 from __future__ import annotations
 
@@ -18,29 +22,27 @@ from .metadata import Metadata
 
 
 def collect_slots(net):
-    """Parameters and BN buffers of ``net`` in the executor's slot order (module-tree order):
-    stem.w | per level: pre_bn{w,b,rm,rv} pre.w [dn_bn dn.w <deeper> up_bn up.w post_bn post.w] | head_bn."""
-
-    def bn(mod):
-        return [mod.weight, mod.bias, mod.running_mean, mod.running_var]
-
-    def level(seq):
-        mods = list(seq._modules.values())
-        out = bn(mods[0][0]) + [mods[0][1].weight]
-        if len(mods) > 1:
-            branch = list(mods[1][1]._modules.values())  # ConcatTable[Identity, Sequential[BN, Conv, U, BN, Deconv]]
-            out += bn(branch[0]) + [branch[1].weight]
-            out += level(branch[2])
-            out += bn(branch[3]) + [branch[4].weight]
-            out += bn(mods[3][0]) + [mods[3][1].weight]
-        return out
-
+    """Parameters and BN buffers of ``net`` in the executor's slot order, which is module-tree order: per
+    BatchNorm ``weight, bias, running_mean, running_var``, per convolution or NetworkInNetwork ``weight``.
+    For the reference configuration: stem.w | per level: pre_bn pre.w [dn_bn dn.w <deeper> up_bn up.w post_bn
+    post.w] | head_bn."""
+    from . import scn
     cached = getattr(net, "_exec_slots", None)
     if cached is not None and cached[0] is net.layer2.weight and cached[-1] is net.layer4.running_var:
         return cached  # (the module walk costs ~0.1 ms per call; parameters are updated in place by optimisers / .to())
-    slots = [net.layer2.weight] + level(net.layer3) + bn(net.layer4)
+    slots = []
+    for mod in net.modules():
+        if isinstance(mod, scn.BatchNormLeakyReLU):
+            slots += [mod.weight, mod.bias, mod.running_mean, mod.running_var]
+        elif isinstance(mod, (scn._ConvBase, scn.NetworkInNetwork)):
+            slots.append(mod.weight)
     net._exec_slots = slots
     return slots
+
+
+def topology(net):
+    """``(block_reps, residual)`` of a ``UNetSCN``: the block topology argument of the ``mm3d_unet_topo_*`` calls."""
+    return int(getattr(net, "_block_reps", 1)), int(bool(getattr(net, "_residual", False)))
 
 
 def fusable(net) -> bool:
@@ -49,9 +51,11 @@ def fusable(net) -> bool:
     from . import scn
     mods = getattr(net, "_exec_mods", None)
     if mods is None:
-        mods = net._exec_mods = [m for m in net.modules() if isinstance(m, (scn._ConvBase, scn.BatchNormLeakyReLU))]
+        mods = net._exec_mods = [m for m in net.modules()
+                                 if isinstance(m, (scn._ConvBase, scn.NetworkInNetwork, scn.BatchNormLeakyReLU))]
     key = (net.layer1.mode if isinstance(net.layer1, scn.InputLayer) else None,
-           tuple((m.mode, hasattr(m, "bias")) if isinstance(m, scn._ConvBase) else m.leakiness for m in mods))
+           tuple((m.mode, hasattr(m, "bias")) if isinstance(m, scn._ConvBase)
+                 else hasattr(m, "bias") if isinstance(m, scn.NetworkInNetwork) else m.leakiness for m in mods))
     cached = getattr(net, "_exec_fusable", None)
     if cached is not None and cached[0] == key:
         return cached[1]
@@ -64,10 +68,12 @@ def _fusable(net) -> bool:
     from . import scn
     if not isinstance(net.layer1, scn.InputLayer) or net.layer1.mode != 4:
         return False
-    if getattr(net, "_block_reps", 1) != 1 or getattr(net, "_residual", False):
+    if int(getattr(net, "_block_reps", 1)) < 1:
         return False
     for mod in net.modules():
         if isinstance(mod, scn._ConvBase) and (mod.mode is not None or hasattr(mod, "bias")):
+            return False
+        if isinstance(mod, scn.NetworkInNetwork) and hasattr(mod, "bias"):
             return False
         if isinstance(mod, scn.BatchNormLeakyReLU) and mod.leakiness != 0:
             return False
@@ -108,7 +114,7 @@ def _level_desc(meta: Metadata, num_planes: int, spatial0: int, plans: bool):
 class UNetSCNFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, feats, meta, cfg, mask_w, mask_b, *slots):
-        in_ch, m, L, mode, training, eps, momentum, spatial0 = cfg
+        in_ch, m, L, mode, training, eps, momentum, spatial0, reps, res = cfg
         feats = feats.float().contiguous()
         dev = feats.device
         # optional RGB mask of Net3DSeg.forward (3d_net/model.py:46-48), folded into the InputLayer scatter
@@ -121,9 +127,9 @@ class UNetSCNFn(torch.autograd.Function):
             # sticky device-error words (mapped host memory): whatever a kernel of an earlier call raised surfaces
             # here -- no synchronisation, a few nanoseconds
             _lib.raise_device_errors("UNetSCN.forward")
-            act_bytes = lib.mm3d_unet_act_bytes(in_ch, m, L, mode, desc, n_points)
+            act_bytes = lib.mm3d_unet_topo_act_bytes(in_ch, m, L, reps, res, mode, desc, n_points)
             act = torch.empty(act_bytes, dtype=torch.uint8, device=dev)
-            scr = F.scratch(lib.mm3d_unet_scratch_bytes(in_ch, m, L, mode), dev)
+            scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes(in_ch, m, L, reps, res, mode), dev)
             out = torch.empty(n_points, m, dtype=torch.float32, device=dev)
             params = (C.c_void_p * len(slots))(*[t.data_ptr() for t in slots])
             mask, wb, gate = None, None, None
@@ -131,9 +137,9 @@ class UNetSCNFn(torch.autograd.Function):
                 wb = torch.cat([mask_w.detach().reshape(-1), mask_b.detach().reshape(-1)]).float().contiguous()
                 gate = torch.empty(max(n_points, 1), dtype=torch.float32, device=dev)
                 mask = C.byref(_lib.UnetMask(wb.data_ptr(), gate.data_ptr(), None, None, None, 0))
-            check(lib.mm3d_unet_forward(in_ch, m, L, mode, int(training), eps, momentum, desc, n_points, meta.p2v_ptr,
+            check(lib.mm3d_unet_topo_forward(in_ch, m, L, reps, res, mode, int(training), eps, momentum, desc, n_points, meta.p2v_ptr,
                                         meta.npts_ptr, feats.data_ptr(), out.data_ptr(), params, act.data_ptr(), act_bytes,
-                                        scr.data_ptr(), scr.numel(), mask, _lib.stream_ptr()), "mm3d_unet_forward")
+                                        scr.data_ptr(), scr.numel(), mask, _lib.stream_ptr()), "mm3d_unet_topo_forward")
         ctx.meta, ctx.cfg, ctx.desc, ctx.act, ctx.slots = meta, cfg, desc, act, slots
         ctx.feats_shape = feats.shape
         ctx.mask = (feats, wb, gate, mask_w.shape, mask_b.shape) if masked else None
@@ -141,7 +147,7 @@ class UNetSCNFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, d_out):
-        in_ch, m, L, mode, training, eps, momentum, spatial0 = ctx.cfg
+        in_ch, m, L, mode, training, eps, momentum, spatial0, reps, res = ctx.cfg
         meta, slots, desc, act = ctx.meta, ctx.slots, ctx.desc, ctx.act
         d_out = d_out.float().contiguous()
         dev = d_out.device
@@ -166,9 +172,9 @@ class UNetSCNFn(torch.autograd.Function):
             d_feats = torch.empty(ctx.feats_shape, dtype=torch.float32, device=dev) if need_feats else None
             if need_feats and ctx.feats_shape[0] > n_points:
                 d_feats.zero_()
-            tmp_bytes = lib.mm3d_unet_bwd_bytes(in_ch, m, L, mode, desc, n_points)
+            tmp_bytes = lib.mm3d_unet_topo_bwd_bytes(in_ch, m, L, reps, res, mode, desc, n_points)
             tmp = torch.empty(tmp_bytes, dtype=torch.uint8, device=dev)
-            scr = F.scratch(lib.mm3d_unet_scratch_bytes(in_ch, m, L, mode), dev)
+            scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes(in_ch, m, L, reps, res, mode), dev)
             params = (C.c_void_p * len(slots))(*[t.data_ptr() for t in slots])
             gp = (C.c_void_p * len(slots))(*gptrs)
             mask, d_mw, d_mb = None, None, None
@@ -179,10 +185,10 @@ class UNetSCNFn(torch.autograd.Function):
                 mask = C.byref(_lib.UnetMask(wb.data_ptr(), gate.data_ptr(), feats.data_ptr(), d_wb.data_ptr(), mws.data_ptr(),
                                              mws.numel() * 8))
                 d_mw, d_mb = d_wb[:in_ch].reshape(w_shape), d_wb[in_ch:].reshape(b_shape)
-            check(lib.mm3d_unet_backward(in_ch, m, L, mode, int(training), desc, n_points, meta.p2v_ptr, meta.npts_ptr,
+            check(lib.mm3d_unet_topo_backward(in_ch, m, L, reps, res, mode, int(training), desc, n_points, meta.p2v_ptr, meta.npts_ptr,
                                          d_out.data_ptr(), d_feats.data_ptr() if need_feats else None, params, gp,
                                          act.data_ptr(), act.numel(), tmp.data_ptr(), tmp_bytes, scr.data_ptr(),
-                                         scr.numel(), mask, _lib.stream_ptr()), "mm3d_unet_backward")
+                                         scr.numel(), mask, _lib.stream_ptr()), "mm3d_unet_topo_backward")
         return (d_feats, None, None, d_mw, d_mb, *grads)
 
 
@@ -281,7 +287,7 @@ def run(net, coords, feats, rgb_mask=None):
         raise ValueError(f"UNetSCN: {feats.shape[0]} feature rows for {meta.n_points} points")
     bn0 = net.layer4
     cfg = (net.in_channels, net.out_channels, L, _lib.MODES[F.DEFAULT_MODE], bool(net.training), float(bn0.eps),
-           float(bn0.momentum), spatial0)
+           float(bn0.momentum), spatial0, *topology(net))
     mask_w, mask_b = rgb_mask if rgb_mask is not None else (None, None)
     with torch.autocast("cuda", enabled=False):
         return UNetSCNFn.apply(feats, meta, cfg, mask_w, mask_b, *collect_slots(net))
