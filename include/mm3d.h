@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MM3D_ABI_VERSION 7
+#define MM3D_ABI_VERSION 8
 
 #define MM3D_OK 0
 #define MM3D_ERR_INVALID 1     /* bad argument */
@@ -49,6 +49,15 @@ extern "C" {
                             * FP32-grade results (1e-4 bar) on the tensor cores.  The gathered operands (`in` of
                             * mm3d_conv_fwd; `in` and `d_out` of mm3d_conv_wgrad) carry TWO planes of [rows, c] floats,
                             * hi = tf32(x) then lo = tf32(x - hi) (mm3d_split_tf32) */
+
+/* Deterministic mode: the `flags` bit of the *_ex entry points below.  With it, an op whose default form adds into
+ * its output with floating-point atomics (so that the result depends on the order in which they land) sums in a
+ * fixed order instead and returns the same bits on every run.  The scatter-adds of the point -> voxel and point ->
+ * pixel sums become segmented sums over group-by-key lists (mm3d_point_csr, mm3d_lift_csr and the *_csr ops); the
+ * small FP64 totals (RGB-mask weight gradient, KL loss, heads3d loss and weight gradients) keep one partial vector per
+ * CTA, at most MM3D_DET_CTAS CTAs, summed in CTA order by the launch that converts them to float. */
+#define MM3D_DETERMINISTIC 0x100
+#define MM3D_DET_CTAS 592
 
 /* flags of mm3d_conv_fwd */
 #define MM3D_CONV_TRANSPOSE_W 1 /* use W[k]^T: weight is [K, c_out, c_in] as stored by the forward layer (dgrad) */
@@ -194,6 +203,20 @@ MM3D_API int mm3d_output_fwd(const float* vox, const int32_t* p2v, int64_t n_poi
                     mm3d_stream_t stream);
 MM3D_API int mm3d_output_bwd(const float* d_out, const int32_t* p2v, int64_t n_points, int64_t n_vox, int c,
                     float* d_vox, mm3d_stream_t stream);
+/* Deterministic forms (MM3D_DETERMINISTIC).  mm3d_point_csr: the points of every voxel in ascending point index,
+ * vox_pts[vox_start[v] .. vox_start[v + 1]) (vox_start [n_vox + 1], vox_pts [n_points]), from p2v and npts of
+ * mm3d_voxelize; ws: mm3d_point_csr_workspace_bytes(n_vox).  The lists depend only on p2v, so a structure builds
+ * them once for all its forward and backward passes.  Cost: linear in points and voxels, except that one thread sorts
+ * each voxel's list (O(k log k) for k points), so a voxel holding a large share of all points serialises that part. */
+MM3D_API size_t mm3d_point_csr_workspace_bytes(int64_t n_vox);
+MM3D_API int mm3d_point_csr(const int32_t* p2v, const int32_t* npts, int64_t n_points, int64_t n_vox, int32_t* vox_start,
+                   int32_t* vox_pts, void* ws, size_t ws_bytes, mm3d_stream_t stream);
+/* mm3d_input_fwd / mm3d_output_bwd over those lists: every voxel row is written once (no memset, no atomics).  Mode 4
+ * sums f / count in point order, so a voxel of one point gets the bits of mm3d_input_fwd. */
+MM3D_API int mm3d_input_fwd_csr(const float* feats, const int32_t* vox_start, const int32_t* vox_pts, int64_t n_vox, int c,
+                       int mode, float* out_vox, mm3d_stream_t stream);
+MM3D_API int mm3d_output_bwd_csr(const float* d_out, const int32_t* vox_start, const int32_t* vox_pts, int64_t n_vox, int c,
+                        float* d_vox, mm3d_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * Rule-table convolution (replaces SubmanifoldConvolution_/Convolution_/Deconvolution_
@@ -263,6 +286,22 @@ MM3D_API int mm3d_lift2d_bilinear_fwd(const void* fmap, int dtype, int B, int C,
 MM3D_API int mm3d_lift2d_bilinear_bwd(const void* d_out, int dtype, int B, int C, int H, int W, int64_t sb, int64_t sc,
                              int64_t sh, int64_t sw, const float* uv, const int64_t* sample_offsets, int64_t n, void* d_fmap,
                              mm3d_stream_t stream);
+/* Deterministic forms of the two backward passes (MM3D_DETERMINISTIC).  mm3d_lift_csr groups the lift's entries by
+ * pixel key (b H + r) W + c: with idx (uv NULL) the entries are the points, indices normalised as mm3d_lift2d_bwd
+ * takes them (an index outside the map gets no entry and raises device-error bit 2); with uv (idx NULL) they are the
+ * (point, tap) pairs 4 p + q of the bilinear lift, q = 2 (row step) + (column step), a tap outside the map or of weight
+ * zero dropped.  pix_start [B H W + 1], pix_ent [n] (idx) or [4 n] (uv), each pixel's entries in ascending order;
+ * ws: mm3d_lift_csr_workspace_bytes(B, H, W, n, uv != NULL); cost as for mm3d_point_csr, per pixel.  The *_bwd_csr ops sum every pixel's entries in that
+ * order in FP32, round once to the map's dtype and store into the caller's zero-filled d_fmap (strides as in
+ * mm3d_lift2d_fwd); uv of the bilinear form is the one the lists were built from. */
+MM3D_API size_t mm3d_lift_csr_workspace_bytes(int B, int H, int W, int64_t n, int bilinear);
+MM3D_API int mm3d_lift_csr(const int64_t* idx, const float* uv, const int64_t* sample_offsets, int B, int H, int W, int64_t n,
+                  int32_t* pix_start, int32_t* pix_ent, void* ws, size_t ws_bytes, mm3d_stream_t stream);
+MM3D_API int mm3d_lift2d_bwd_csr(const void* d_out, int dtype, int B, int C, int H, int W, int64_t sb, int64_t sc, int64_t sh,
+                        int64_t sw, const int32_t* pix_start, const int32_t* pix_ent, void* d_fmap, mm3d_stream_t stream);
+MM3D_API int mm3d_lift2d_bilinear_bwd_csr(const void* d_out, int dtype, int B, int C, int H, int W, int64_t sb, int64_t sc,
+                                 int64_t sh, int64_t sw, const float* uv, const int32_t* pix_start, const int32_t* pix_ent,
+                                 void* d_fmap, mm3d_stream_t stream);
 
 /* Point values -> image (the loaders' sparse depth and 2D label maps, lib/dataset/nuscenes_dataloader.py:275-278):
  * out[b, idx[i,0], idx[i,1]] = vals[i] over a map pre-filled with `fill`; where several points share a pixel the
@@ -280,11 +319,17 @@ MM3D_API int mm3d_rgb_mask_fwd(const float* x, int64_t n, int c, const float* w,
                       mm3d_stream_t stream);
 MM3D_API int mm3d_rgb_mask_bwd(const float* x, const float* s, const float* dy, int64_t n, int c, const float* w, float* dx,
                       float* dw, float* db, void* ws, size_t ws_bytes, mm3d_stream_t stream);
+/* flags 0 = mm3d_rgb_mask_bwd; MM3D_DETERMINISTIC: ws MM3D_DET_CTAS * (c + 1) doubles */
+MM3D_API int mm3d_rgb_mask_bwd_ex(const float* x, const float* s, const float* dy, int64_t n, int c, const float* w, float* dx,
+                         float* dw, float* db, void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags);
 /* Cross-modal loss, train.py:157-184:  loss[0] = mean over the n rows of sum_c q_c (log q_c - log p_c) with
  * p = softmax(pred[n, :]), q = softmax(target[n, :]) (target detached); pred, target float32 [n, C] logits; ws: one
  * double.  Backward: dpred = dloss[0] * (p - q) / n. */
 MM3D_API int mm3d_kl_logits_fwd(const float* pred, const float* target, int64_t n, int C, float* loss, void* ws, size_t ws_bytes,
                        mm3d_stream_t stream);
+/* flags 0 = mm3d_kl_logits_fwd; MM3D_DETERMINISTIC: ws MM3D_DET_CTAS doubles */
+MM3D_API int mm3d_kl_logits_fwd_ex(const float* pred, const float* target, int64_t n, int C, float* loss, void* ws,
+                          size_t ws_bytes, mm3d_stream_t stream, int flags);
 MM3D_API int mm3d_kl_logits_bwd(const float* pred, const float* target, int64_t n, int C, const float* dloss, float* dpred,
                        mm3d_stream_t stream);
 /* The two point-wise heads of the 3D branch and the 3D side of the cross-modal loss in ONE pass over the features
@@ -300,6 +345,15 @@ MM3D_API int mm3d_heads3d_fwd(const float* feat, int64_t n, int f, int C, const 
 MM3D_API int mm3d_heads3d_bwd(const float* feat, int64_t n, int f, int C, const float* w1, const float* w2, const float* b2,
                      const float* target, const float* d_logit1, const float* d_logit2, const float* d_loss, float* d_feat,
                      float* d_w1, float* d_b1, float* d_w2, float* d_b2, void* ws, size_t ws_bytes, mm3d_stream_t stream);
+/* flags 0 = the functions above; MM3D_DETERMINISTIC: ws MM3D_DET_CTAS doubles (forward with a loss) and
+ * MM3D_DET_CTAS * (2 C f + 2 C) doubles (backward) */
+MM3D_API int mm3d_heads3d_fwd_ex(const float* feat, int64_t n, int f, int C, const float* w1, const float* b1, const float* w2,
+                        const float* b2, const float* target, float* logit1, float* logit2, float* loss, void* ws,
+                        size_t ws_bytes, mm3d_stream_t stream, int flags);
+MM3D_API int mm3d_heads3d_bwd_ex(const float* feat, int64_t n, int f, int C, const float* w1, const float* w2, const float* b2,
+                        const float* target, const float* d_logit1, const float* d_logit2, const float* d_loss,
+                        float* d_feat, float* d_w1, float* d_b1, float* d_w2, float* d_b2, void* ws, size_t ws_bytes,
+                        mm3d_stream_t stream, int flags);
 
 /* ------------------------------------------------------------------------------------------
  * Whole-network executor: UNetSCN (3d_net/scn_unet.py:36-126) forward and backward as one call each -- the

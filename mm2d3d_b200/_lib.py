@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmm3d.so")
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 
 class UnetMask(C.Structure):
@@ -24,6 +24,8 @@ LEVEL_DESC_WORDS = 10
 MODE_FP32, MODE_TF32, MODE_BF16, MODE_TF32X3 = 0, 1, 2, 3
 MODES = {"fp32": MODE_FP32, "tf32": MODE_TF32, "bf16": MODE_BF16, "tf32x3": MODE_TF32X3}
 CONV_TRANSPOSE_W, CONV_MIRROR_K = 1, 2
+DETERMINISTIC = 0x100  # MM3D_DETERMINISTIC: the flags bit of the *_ex entry points
+DET_CTAS = 592         # MM3D_DET_CTAS: partial slots of a deterministic reduction
 STATUS_BAD_COORD = 1
 STATUS_DROPPED = 2
 
@@ -95,6 +97,18 @@ SIGNATURES = {
     "mm3d_unet_backward": (_i, [_i, _i, _i, _i, _i, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _sz, _p, _sz, _p, _p]),
     "mm3d_input_masked_fwd": (_i, [_p, _p, _p, _i64, _i64, _i, _i, _p, _p, _p, _p]),
     "mm3d_input_masked_bwd": (_i, [_p, _p, _p, _p, _p, _i64, _i, _i, _p, _p, _p, _p, _sz, _p]),
+    "mm3d_point_csr_workspace_bytes": (_sz, [_i64]),
+    "mm3d_point_csr": (_i, [_p, _p, _i64, _i64, _p, _p, _p, _sz, _p]),
+    "mm3d_input_fwd_csr": (_i, [_p, _p, _p, _i64, _i, _i, _p, _p]),
+    "mm3d_output_bwd_csr": (_i, [_p, _p, _p, _i64, _i, _p, _p]),
+    "mm3d_lift_csr_workspace_bytes": (_sz, [_i, _i, _i, _i64, _i]),
+    "mm3d_lift_csr": (_i, [_p, _p, _p, _i, _i, _i, _i64, _p, _p, _p, _sz, _p]),
+    "mm3d_lift2d_bwd_csr": (_i, [_p, _i, _i, _i, _i, _i, _i64, _i64, _i64, _i64, _p, _p, _p, _p]),
+    "mm3d_lift2d_bilinear_bwd_csr": (_i, [_p, _i, _i, _i, _i, _i, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p]),
+    "mm3d_rgb_mask_bwd_ex": (_i, [_p, _p, _p, _i64, _i, _p, _p, _p, _p, _p, _sz, _p, _i]),
+    "mm3d_kl_logits_fwd_ex": (_i, [_p, _p, _i64, _i, _p, _p, _sz, _p, _i]),
+    "mm3d_heads3d_fwd_ex": (_i, [_p, _i64, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _i]),
+    "mm3d_heads3d_bwd_ex": (_i, [_p, _i64, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _i]),
 }
 
 class PlanDesc(C.Structure):

@@ -21,6 +21,12 @@ int mm3d_sm_count();
 void mm3d_set_error(const char* fmt, ...);
 void mm3d_count_launches(int n);  // bookkeeping for mm3d_kernel_launches()
 
+// groupby.cu: CSR lists start[n_keys + 1] / list[] of the entries of every key in ascending entry index (key < 0 = no
+// key); `counts` = the per-key counts when the caller has them (NULL: counted here)
+size_t mm3d_group_by_workspace_bytes(int64_t n_keys);
+int mm3d_group_by(const int32_t* key, const int32_t* counts, int64_t n, int64_t n_keys, int32_t* start, int32_t* list,
+                  void* ws, size_t ws_bytes, cudaStream_t stream);
+
 #define MM3D_REQUIRE(cond, code, ...)     \
   do {                                    \
     if (!(cond)) {                        \

@@ -12,6 +12,40 @@ namespace {
 
 constexpr int kMaxC = 64;
 
+// Deterministic mode (MM3D_DETERMINISTIC): instead of adding its block total to a global FP64 word atomically, every
+// CTA stores it to its own slot part[blockIdx.x][...] (the in-block sum in a fixed warp order), and the finalize launch
+// that converts the totals to float -- one the default path has too -- sums the slots in CTA order.  At most
+// MM3D_DET_CTAS CTAs, independent of the device.
+template <int NW>
+__device__ __forceinline__ double block_sum_ordered(double v) {  // valid in thread 0
+  __shared__ double wsum[NW];
+  for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double t = 0.0;
+  if (threadIdx.x == 0)
+    for (int w = 0; w < NW; ++w) t += wsum[w];
+  return t;
+}
+
+struct PartOuts {  // where word j of the summed slots goes: the first n[0] words to p[0], the next n[1] to p[1], ...
+  float* p[4];
+  int n[4];
+};
+
+__global__ void k_sum_parts(const double* __restrict__ part, int nparts, int words, double scale, PartOuts o) {
+  mm3d_griddep_wait();
+  for (int j = threadIdx.x; j < words; j += blockDim.x) {
+    double t = 0.0;
+    for (int b = 0; b < nparts; ++b) t += part[(int64_t)b * words + j];
+    int k = 0, jj = j;
+    while (jj >= o.n[k]) jj -= o.n[k++];
+    o.p[k][jj] = (float)(t * scale);
+  }
+}
+
+static inline int det_grid(int64_t g) { return (int)(g < MM3D_DET_CTAS ? g : MM3D_DET_CTAS); }
+
 __global__ void k_rgb_mask_fwd(const float* x, int64_t n, int c, const float* __restrict__ w,
                                const float* __restrict__ b, float* y, float* __restrict__ s_out) {
   mm3d_griddep_wait();
@@ -32,6 +66,7 @@ __global__ void k_rgb_mask_fwd(const float* x, int64_t n, int c, const float* __
 }
 
 // dx = dy s + t w,  t = (dy . x) s (1 - s);   dw = sum_n t x,  db = sum_n t   (FP64 totals, one atomic per CTA)
+template <bool DET>
 __global__ void k_rgb_mask_bwd(const float* __restrict__ x, const float* __restrict__ s_in, const float* __restrict__ dy,
                                int64_t n, int c, const float* __restrict__ w, float* __restrict__ dx,
                                double* __restrict__ dwb) {
@@ -54,14 +89,31 @@ __global__ void k_rgb_mask_bwd(const float* __restrict__ x, const float* __restr
       if (j < c) loc[j] += (double)(t * __ldg(x + i * c + j));
     loc[8] += (double)t;
   }
+  if constexpr (DET) {  // dwb = this CTA's slot of c + 1 doubles; 256 threads = 8 warps
+    __shared__ double wred[8][9];
 #pragma unroll
-  for (int j = 0; j < 9; ++j) {
-    double v = loc[j];
-    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if ((threadIdx.x & 31) == 0 && (j < c || j == 8)) atomicAdd(&red[j == 8 ? c : j], v);
+    for (int j = 0; j < 9; ++j) {
+      double v = loc[j];
+      for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+      if ((threadIdx.x & 31) == 0) wred[threadIdx.x >> 5][j] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x <= c) {
+      const int j = threadIdx.x == c ? 8 : threadIdx.x;
+      double t = 0.0;
+      for (int w = 0; w < 8; ++w) t += wred[w][j];
+      dwb[(int64_t)blockIdx.x * (c + 1) + threadIdx.x] = t;
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < 9; ++j) {
+      double v = loc[j];
+      for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+      if ((threadIdx.x & 31) == 0 && (j < c || j == 8)) atomicAdd(&red[j == 8 ? c : j], v);
+    }
+    __syncthreads();
+    for (int j = threadIdx.x; j <= c; j += blockDim.x) atomicAdd(dwb + j, red[j]);
   }
-  __syncthreads();
-  for (int j = threadIdx.x; j <= c; j += blockDim.x) atomicAdd(dwb + j, red[j]);
 }
 
 __global__ void k_f64_to_f32(const double* __restrict__ src, float* __restrict__ dst, int n, double scale) {
@@ -87,19 +139,25 @@ __device__ __forceinline__ double kl_row(const float* __restrict__ pr, const flo
   return kl;
 }
 
+template <bool DET>
 __global__ void k_kl_fwd(const float* __restrict__ pred, const float* __restrict__ target, int64_t n, int C,
                          double* __restrict__ total) {
   mm3d_griddep_wait();
   double loc = 0.0;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
     loc += kl_row(pred + i * C, target + i * C, C, nullptr, 0.f);
-  for (int o = 16; o; o >>= 1) loc += __shfl_xor_sync(0xffffffffu, loc, o);
-  __shared__ double red;
-  if (threadIdx.x == 0) red = 0.0;
-  __syncthreads();
-  if ((threadIdx.x & 31) == 0) atomicAdd(&red, loc);
-  __syncthreads();
-  if (threadIdx.x == 0) atomicAdd(total, red);
+  if constexpr (DET) {  // total = this CTA's slot
+    const double t = block_sum_ordered<8>(loc);
+    if (threadIdx.x == 0) total[blockIdx.x] = t;
+  } else {
+    for (int o = 16; o; o >>= 1) loc += __shfl_xor_sync(0xffffffffu, loc, o);
+    __shared__ double red;
+    if (threadIdx.x == 0) red = 0.0;
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0) atomicAdd(&red, loc);
+    __syncthreads();
+    if (threadIdx.x == 0) atomicAdd(total, red);
+  }
 }
 
 __global__ void k_kl_bwd(const float* __restrict__ pred, const float* __restrict__ target, int64_t n, int C,
@@ -151,6 +209,7 @@ __device__ __forceinline__ float heads_dot(const float (&fr)[kHeadMaxF], const f
   return acc;
 }
 
+template <bool DET>
 __global__ void __launch_bounds__(kHeadTile)
 k_heads3d_fwd(const float* __restrict__ feat, int64_t n, int f, int C, const float* __restrict__ w1, const float* __restrict__ b1,
               const float* __restrict__ w2, const float* __restrict__ b2, const float* __restrict__ target,
@@ -193,7 +252,10 @@ k_heads3d_fwd(const float* __restrict__ feat, int64_t n, int f, int C, const flo
       }
     }
   }
-  if (total) {
+  if (total && DET) {  // total = the slots, one per CTA
+    const double t = block_sum_ordered<kHeadTile / 32>(loc);
+    if (threadIdx.x == 0) total[blockIdx.x] = t;
+  } else if (total) {
     for (int o = 16; o; o >>= 1) loc += __shfl_xor_sync(0xffffffffu, loc, o);
     if ((threadIdx.x & 31) == 0) atomicAdd(&red, loc);
     __syncthreads();
@@ -201,7 +263,8 @@ k_heads3d_fwd(const float* __restrict__ feat, int64_t n, int f, int C, const flo
   }
 }
 
-// tot: [C f | C | C f | C] doubles = d_w1, d_b1, d_w2, d_b2 (zero on entry)
+// tot: [C f | C | C f | C] doubles = d_w1, d_b1, d_w2, d_b2 (zero on entry; DET: one such slot per CTA, written)
+template <bool DET>
 __global__ void __launch_bounds__(kHeadTile)
 k_heads3d_bwd(const float* __restrict__ feat, int64_t n, int f, int C, const float* __restrict__ w1, const float* __restrict__ w2,
               const float* __restrict__ b2, const float* __restrict__ target, const float* __restrict__ d_logit1,
@@ -292,7 +355,8 @@ k_heads3d_bwd(const float* __restrict__ feat, int64_t n, int f, int C, const flo
     else if (o < 2 * C * f) dst = C * f + C + (o - C * f);
     else if (o < 2 * C * f + C) dst = C * f + (o - 2 * C * f);
     else dst = 2 * C * f + C + (o - 2 * C * f - C);
-    atomicAdd(tot + dst, (double)acc[a]);
+    if (DET) tot[(int64_t)blockIdx.x * n_out + dst] = (double)acc[a];
+    else atomicAdd(tot + dst, (double)acc[a]);
   }
 }
 
@@ -315,16 +379,32 @@ int mm3d_rgb_mask_fwd(const float* x, int64_t n, int c, const float* w, const fl
 }
 
 // x: the UNMASKED features; dx may be NULL (the features are data); dw [c], db [1]; ws: (c + 1) doubles
-int mm3d_rgb_mask_bwd(const float* x, const float* s, const float* dy, int64_t n, int c, const float* w, float* dx,
-                      float* dw, float* db, void* ws, size_t ws_bytes, mm3d_stream_t stream_) {
+// flags: MM3D_DETERMINISTIC -> ws: MM3D_DET_CTAS * (c + 1) doubles
+int mm3d_rgb_mask_bwd_ex(const float* x, const float* s, const float* dy, int64_t n, int c, const float* w, float* dx,
+                         float* dw, float* db, void* ws, size_t ws_bytes, mm3d_stream_t stream_, int flags) {
   cudaStream_t stream = (cudaStream_t)stream_;
   MM3D_REQUIRE(n >= 0 && c > 0 && c <= 8, MM3D_ERR_INVALID, "rgb_mask: 1..8 feature channels supported, got %d", c);
-  MM3D_REQUIRE(dw && db && ws && ws_bytes >= sizeof(double) * (size_t)(c + 1), MM3D_ERR_WORKSPACE, "rgb_mask: workspace too small");
+  MM3D_REQUIRE((flags & ~MM3D_DETERMINISTIC) == 0, MM3D_ERR_INVALID, "rgb_mask: unknown flags %#x", flags);
+  const bool det = flags & MM3D_DETERMINISTIC;
+  MM3D_REQUIRE(dw && db && ws && ws_bytes >= sizeof(double) * (size_t)(c + 1) * (det ? MM3D_DET_CTAS : 1), MM3D_ERR_WORKSPACE,
+               "rgb_mask: workspace too small");
   double* tot = (double*)ws;
+  if (det) {
+    const int grid = n > 0 ? det_grid(mm3d_grid(n, 256, 2)) : 0;
+    if (n > 0) {
+      MM3D_REQUIRE(x && s && dy && w, MM3D_ERR_INVALID, "rgb_mask: null pointer");
+      MM3D_CUDA(mm3d_launch_pdl(k_rgb_mask_bwd<true>, dim3(grid), dim3(256), 0, stream, x, s, dy, n, c, w, dx, tot));
+    }
+    const PartOuts o = {{dw, db, nullptr, nullptr}, {c, 1, 0, 0}};
+    MM3D_CUDA(mm3d_launch_pdl(k_sum_parts, dim3(1), dim3(32), 0, stream, (const double*)tot, grid, c + 1, 1.0, o));
+    mm3d_count_launches(n > 0 ? 2 : 1);
+    MM3D_CHECK_LAUNCH("mm3d_rgb_mask_bwd");
+    return MM3D_OK;
+  }
   MM3D_CUDA(cudaMemsetAsync(tot, 0, sizeof(double) * (size_t)(c + 1), stream));
   if (n > 0) {
     MM3D_REQUIRE(x && s && dy && w, MM3D_ERR_INVALID, "rgb_mask: null pointer");
-    MM3D_CUDA(mm3d_launch_pdl(k_rgb_mask_bwd, dim3(mm3d_grid(n, 256, 2)), dim3(256), 0, stream, x, s, dy, n, c, w, dx, tot));
+    MM3D_CUDA(mm3d_launch_pdl(k_rgb_mask_bwd<false>, dim3(mm3d_grid(n, 256, 2)), dim3(256), 0, stream, x, s, dy, n, c, w, dx, tot));
   }
   MM3D_CUDA(mm3d_launch_pdl(k_f64_to_f32, dim3(1), dim3(32), 0, stream, (const double*)tot, dw, c, 1.0));
   MM3D_CUDA(mm3d_launch_pdl(k_f64_to_f32, dim3(1), dim3(32), 0, stream, (const double*)(tot + c), db, 1, 1.0));
@@ -333,18 +413,41 @@ int mm3d_rgb_mask_bwd(const float* x, const float* s, const float* dy, int64_t n
   return MM3D_OK;
 }
 
+int mm3d_rgb_mask_bwd(const float* x, const float* s, const float* dy, int64_t n, int c, const float* w, float* dx,
+                      float* dw, float* db, void* ws, size_t ws_bytes, mm3d_stream_t stream) {
+  return mm3d_rgb_mask_bwd_ex(x, s, dy, n, c, w, dx, dw, db, ws, ws_bytes, stream, 0);
+}
+
 // loss[0] = mean_n sum_c q (log q - log p),  p = softmax(pred[n, :]), q = softmax(target[n, :]);  ws: one double
-int mm3d_kl_logits_fwd(const float* pred, const float* target, int64_t n, int C, float* loss, void* ws, size_t ws_bytes,
-                       mm3d_stream_t stream_) {
+// (flags MM3D_DETERMINISTIC: MM3D_DET_CTAS doubles)
+int mm3d_kl_logits_fwd_ex(const float* pred, const float* target, int64_t n, int C, float* loss, void* ws, size_t ws_bytes,
+                          mm3d_stream_t stream_, int flags) {
   cudaStream_t stream = (cudaStream_t)stream_;
   MM3D_REQUIRE(n > 0 && C > 0 && C <= 4096, MM3D_ERR_INVALID, "kl_logits: bad sizes");
-  MM3D_REQUIRE(pred && target && loss && ws && ws_bytes >= sizeof(double), MM3D_ERR_WORKSPACE, "kl_logits: workspace too small");
+  MM3D_REQUIRE((flags & ~MM3D_DETERMINISTIC) == 0, MM3D_ERR_INVALID, "kl_logits: unknown flags %#x", flags);
+  const bool det = flags & MM3D_DETERMINISTIC;
+  MM3D_REQUIRE(pred && target && loss && ws && ws_bytes >= sizeof(double) * (det ? MM3D_DET_CTAS : 1), MM3D_ERR_WORKSPACE,
+               "kl_logits: workspace too small");
+  if (det) {
+    const int grid = det_grid(mm3d_grid(n, 256, 2));
+    MM3D_CUDA(mm3d_launch_pdl(k_kl_fwd<true>, dim3(grid), dim3(256), 0, stream, pred, target, n, C, (double*)ws));
+    const PartOuts o = {{loss, nullptr, nullptr, nullptr}, {1, 0, 0, 0}};
+    MM3D_CUDA(mm3d_launch_pdl(k_sum_parts, dim3(1), dim3(32), 0, stream, (const double*)ws, grid, 1, 1.0 / (double)n, o));
+    mm3d_count_launches(2);
+    MM3D_CHECK_LAUNCH("mm3d_kl_logits_fwd");
+    return MM3D_OK;
+  }
   MM3D_CUDA(cudaMemsetAsync(ws, 0, sizeof(double), stream));
-  MM3D_CUDA(mm3d_launch_pdl(k_kl_fwd, dim3(mm3d_grid(n, 256, 2)), dim3(256), 0, stream, pred, target, n, C, (double*)ws));
+  MM3D_CUDA(mm3d_launch_pdl(k_kl_fwd<false>, dim3(mm3d_grid(n, 256, 2)), dim3(256), 0, stream, pred, target, n, C, (double*)ws));
   MM3D_CUDA(mm3d_launch_pdl(k_f64_to_f32, dim3(1), dim3(32), 0, stream, (const double*)ws, loss, 1, 1.0 / (double)n));
   mm3d_count_launches(2);
   MM3D_CHECK_LAUNCH("mm3d_kl_logits_fwd");
   return MM3D_OK;
+}
+
+int mm3d_kl_logits_fwd(const float* pred, const float* target, int64_t n, int C, float* loss, void* ws, size_t ws_bytes,
+                       mm3d_stream_t stream) {
+  return mm3d_kl_logits_fwd_ex(pred, target, n, C, loss, ws, ws_bytes, stream, 0);
 }
 
 // dpred = dloss[0] * (softmax(pred) - softmax(target)) / n   (the target side is detached in the reference)
@@ -362,25 +465,33 @@ int mm3d_kl_logits_bwd(const float* pred, const float* target, int64_t n, int C,
 
 // The two Linear(f -> C) heads of the 3D branch (weights [C, f] as nn.Linear stores them) and, when `target` is given,
 // loss[0] = mean_n KL(softmax(target_n) || softmax(logit2_n)) in one pass over feat [n, f].  logit2 and loss may be NULL.
-// f: multiple of 4, <= 32; C <= 20.  ws: one double.
-int mm3d_heads3d_fwd(const float* feat, int64_t n, int f, int C, const float* w1, const float* b1, const float* w2,
-                     const float* b2, const float* target, float* logit1, float* logit2, float* loss, void* ws,
-                     size_t ws_bytes, mm3d_stream_t stream_) {
+// f: multiple of 4, <= 32; C <= 20.  ws: one double (flags MM3D_DETERMINISTIC: MM3D_DET_CTAS doubles).
+int mm3d_heads3d_fwd_ex(const float* feat, int64_t n, int f, int C, const float* w1, const float* b1, const float* w2,
+                        const float* b2, const float* target, float* logit1, float* logit2, float* loss, void* ws,
+                        size_t ws_bytes, mm3d_stream_t stream_, int flags) {
   cudaStream_t stream = (cudaStream_t)stream_;
   MM3D_REQUIRE(n >= 0 && f > 0 && f <= kHeadMaxF && (f & 3) == 0 && C > 0 && C <= kHeadMaxC, MM3D_ERR_INVALID,
                "heads3d: f must be a multiple of 4 up to %d and C at most %d (got %d, %d)", kHeadMaxF, kHeadMaxC, f, C);
-  MM3D_REQUIRE(!loss || (target && ws && ws_bytes >= sizeof(double)), MM3D_ERR_WORKSPACE, "heads3d: the loss needs a target and a workspace");
-  if (loss) MM3D_CUDA(cudaMemsetAsync(ws, 0, sizeof(double), stream));
+  MM3D_REQUIRE((flags & ~MM3D_DETERMINISTIC) == 0, MM3D_ERR_INVALID, "heads3d: unknown flags %#x", flags);
+  const bool det = flags & MM3D_DETERMINISTIC;
+  MM3D_REQUIRE(!loss || (target && ws && ws_bytes >= sizeof(double) * (det ? MM3D_DET_CTAS : 1)), MM3D_ERR_WORKSPACE,
+               "heads3d: the loss needs a target and a workspace");
+  if (loss && !det) MM3D_CUDA(cudaMemsetAsync(ws, 0, sizeof(double), stream));
   if (n == 0) {
     if (loss) MM3D_CUDA(cudaMemsetAsync(loss, 0, sizeof(float), stream));
     return MM3D_OK;
   }
   MM3D_REQUIRE(feat && w1 && b1 && w2 && b2 && logit1, MM3D_ERR_INVALID, "heads3d: null pointer");
   MM3D_REQUIRE((((uintptr_t)feat) & 15) == 0, MM3D_ERR_INVALID, "heads3d: feat must be 16-byte aligned");
-  MM3D_CUDA(mm3d_launch_pdl(k_heads3d_fwd, dim3(mm3d_grid(n, kHeadTile, 2)), dim3(kHeadTile), 0, stream, feat, n, f, C, w1, b1, w2, b2,
-                            loss ? target : (const float*)nullptr, logit1, logit2, loss ? (double*)ws : (double*)nullptr));
+  const int grid = det ? det_grid(mm3d_grid(n, kHeadTile, 2)) : mm3d_grid(n, kHeadTile, 2);
+  MM3D_CUDA(mm3d_launch_pdl(det ? k_heads3d_fwd<true> : k_heads3d_fwd<false>, dim3(grid), dim3(kHeadTile), 0, stream, feat, n, f, C,
+                            w1, b1, w2, b2, loss ? target : (const float*)nullptr, logit1, logit2, loss ? (double*)ws : (double*)nullptr));
   mm3d_count_launches(1);
-  if (loss) {
+  if (loss && det) {
+    const PartOuts o = {{loss, nullptr, nullptr, nullptr}, {1, 0, 0, 0}};
+    MM3D_CUDA(mm3d_launch_pdl(k_sum_parts, dim3(1), dim3(32), 0, stream, (const double*)ws, grid, 1, 1.0 / (double)n, o));
+    mm3d_count_launches(1);
+  } else if (loss) {
     MM3D_CUDA(mm3d_launch_pdl(k_f64_to_f32, dim3(1), dim3(32), 0, stream, (const double*)ws, loss, 1, 1.0 / (double)n));
     mm3d_count_launches(1);
   }
@@ -388,26 +499,52 @@ int mm3d_heads3d_fwd(const float* feat, int64_t n, int f, int C, const float* w1
   return MM3D_OK;
 }
 
+int mm3d_heads3d_fwd(const float* feat, int64_t n, int f, int C, const float* w1, const float* b1, const float* w2,
+                     const float* b2, const float* target, float* logit1, float* logit2, float* loss, void* ws,
+                     size_t ws_bytes, mm3d_stream_t stream) {
+  return mm3d_heads3d_fwd_ex(feat, n, f, C, w1, b1, w2, b2, target, logit1, logit2, loss, ws, ws_bytes, stream, 0);
+}
+
 // Gradients of the above.  d_logit1 / d_logit2: upstream gradients of the two logit tensors ([n, C], either may be NULL);
 // d_loss: upstream gradient of the loss ([1], NULL = the loss was not used; needs `target`).  d_feat [n, f] may be NULL.
-// d_w1, d_w2 [C, f], d_b1, d_b2 [C] are overwritten.  ws: (2 C f + 2 C) doubles.
-int mm3d_heads3d_bwd(const float* feat, int64_t n, int f, int C, const float* w1, const float* w2, const float* b2,
-                     const float* target, const float* d_logit1, const float* d_logit2, const float* d_loss, float* d_feat,
-                     float* d_w1, float* d_b1, float* d_w2, float* d_b2, void* ws, size_t ws_bytes, mm3d_stream_t stream_) {
+// d_w1, d_w2 [C, f], d_b1, d_b2 [C] are overwritten.  ws: (2 C f + 2 C) doubles (flags MM3D_DETERMINISTIC:
+// MM3D_DET_CTAS times that).
+int mm3d_heads3d_bwd_ex(const float* feat, int64_t n, int f, int C, const float* w1, const float* w2, const float* b2,
+                        const float* target, const float* d_logit1, const float* d_logit2, const float* d_loss, float* d_feat,
+                        float* d_w1, float* d_b1, float* d_w2, float* d_b2, void* ws, size_t ws_bytes, mm3d_stream_t stream_,
+                        int flags) {
   cudaStream_t stream = (cudaStream_t)stream_;
   MM3D_REQUIRE(n >= 0 && f > 0 && f <= kHeadMaxF && (f & 3) == 0 && C > 0 && C <= kHeadMaxC, MM3D_ERR_INVALID,
                "heads3d: f must be a multiple of 4 up to %d and C at most %d (got %d, %d)", kHeadMaxF, kHeadMaxC, f, C);
+  MM3D_REQUIRE((flags & ~MM3D_DETERMINISTIC) == 0, MM3D_ERR_INVALID, "heads3d: unknown flags %#x", flags);
+  const bool det = flags & MM3D_DETERMINISTIC;
   const size_t words = 2 * (size_t)C * f + 2 * (size_t)C;
-  MM3D_REQUIRE(d_w1 && d_b1 && d_w2 && d_b2 && ws && ws_bytes >= sizeof(double) * words, MM3D_ERR_WORKSPACE, "heads3d: workspace too small");
+  MM3D_REQUIRE(d_w1 && d_b1 && d_w2 && d_b2 && ws && ws_bytes >= sizeof(double) * words * (det ? MM3D_DET_CTAS : 1), MM3D_ERR_WORKSPACE,
+               "heads3d: workspace too small");
   MM3D_REQUIRE(!d_loss || target, MM3D_ERR_INVALID, "heads3d: a loss gradient needs the target");
   double* tot = (double*)ws;
+  if (det) {
+    const int64_t tiles = (n + kHeadTile - 1) / kHeadTile;
+    const int grid = n > 0 ? det_grid(tiles) : 0;
+    if (n > 0) {
+      MM3D_REQUIRE(feat && w1 && w2 && b2, MM3D_ERR_INVALID, "heads3d: null pointer");
+      MM3D_REQUIRE((((uintptr_t)feat) & 15) == 0, MM3D_ERR_INVALID, "heads3d: feat must be 16-byte aligned");
+      MM3D_CUDA(mm3d_launch_pdl(k_heads3d_bwd<true>, dim3(grid), dim3(kHeadTile), 0, stream, feat, n, f, C, w1, w2, b2, target, d_logit1,
+                                d_logit2, d_loss, 1.f / (float)n, d_feat, tot));
+    }
+    const PartOuts o = {{d_w1, d_b1, d_w2, d_b2}, {C * f, C, C * f, C}};
+    MM3D_CUDA(mm3d_launch_pdl(k_sum_parts, dim3(1), dim3(256), 0, stream, (const double*)tot, grid, (int)words, 1.0, o));
+    mm3d_count_launches(n > 0 ? 2 : 1);
+    MM3D_CHECK_LAUNCH("mm3d_heads3d_bwd");
+    return MM3D_OK;
+  }
   MM3D_CUDA(cudaMemsetAsync(tot, 0, sizeof(double) * words, stream));
   if (n > 0) {
     MM3D_REQUIRE(feat && w1 && w2 && b2, MM3D_ERR_INVALID, "heads3d: null pointer");
     MM3D_REQUIRE((((uintptr_t)feat) & 15) == 0, MM3D_ERR_INVALID, "heads3d: feat must be 16-byte aligned");
     int64_t tiles = (n + kHeadTile - 1) / kHeadTile;
     const int64_t cap = (int64_t)mm3d_sm_count() * 4;
-    MM3D_CUDA(mm3d_launch_pdl(k_heads3d_bwd, dim3((unsigned)(tiles < cap ? tiles : cap)), dim3(kHeadTile), 0, stream, feat, n, f, C, w1, w2, b2,
+    MM3D_CUDA(mm3d_launch_pdl(k_heads3d_bwd<false>, dim3((unsigned)(tiles < cap ? tiles : cap)), dim3(kHeadTile), 0, stream, feat, n, f, C, w1, w2, b2,
                               target, d_logit1, d_logit2, d_loss, 1.f / (float)n, d_feat, tot));
     mm3d_count_launches(1);
   }
@@ -418,6 +555,13 @@ int mm3d_heads3d_bwd(const float* feat, int64_t n, int f, int C, const float* w1
   mm3d_count_launches(4);
   MM3D_CHECK_LAUNCH("mm3d_heads3d_bwd");
   return MM3D_OK;
+}
+
+int mm3d_heads3d_bwd(const float* feat, int64_t n, int f, int C, const float* w1, const float* w2, const float* b2,
+                     const float* target, const float* d_logit1, const float* d_logit2, const float* d_loss, float* d_feat,
+                     float* d_w1, float* d_b1, float* d_w2, float* d_b2, void* ws, size_t ws_bytes, mm3d_stream_t stream) {
+  return mm3d_heads3d_bwd_ex(feat, n, f, C, w1, w2, b2, target, d_logit1, d_logit2, d_loss, d_feat, d_w1, d_b1, d_w2, d_b2, ws,
+                             ws_bytes, stream, 0);
 }
 
 }  // extern "C"

@@ -303,6 +303,7 @@ template <class T> __device__ __forceinline__ float lift_to_f32(T v) { return (f
 struct BilinearTaps {
   int64_t off[4];  // element offset of the tap inside the sample's map (without the channel term)
   float w[4];      // 0 for a tap outside the map
+  int rr[4], cc[4];  // the tap's pixel (valid where w != 0)
 };
 
 __device__ __forceinline__ BilinearTaps bilinear_taps(float r, float c, int H, int W, int64_t sh, int64_t sw) {
@@ -318,6 +319,8 @@ __device__ __forceinline__ BilinearTaps bilinear_taps(float r, float c, int H, i
     const float w = ((q >> 1) ? fr : 1.f - fr) * ((q & 1) ? fc : 1.f - fc);
     t.w[q] = in ? w : 0.f;
     t.off[q] = in ? rr * sh + cc * sw : 0;
+    t.rr[q] = rr;
+    t.cc[q] = cc;
   }
   return t;
 }
@@ -375,6 +378,113 @@ k_lift_bilinear_bwd(const T* __restrict__ d_out, int B, int C, int H, int W, int
         for (int j = 0; j < G; ++j) lift_atomic_add(base + t.off[q] + j * sc, T(t.w[q] * g[j]));
       }
     }
+  }
+}
+
+// ------------------------------------------------------------------ deterministic forms: segmented sums
+// Each output row (voxel) or pixel is written ONCE by the thread that owns it, summing its entries in the ascending
+// entry order of the group-by-key lists (groupby.cu): no memset, no atomics, the same bits on every run.
+
+// InputLayer forward.  Mode 4 sums f / cnt in point order -- the terms of k_input_fwd -- so a voxel of one point gets
+// exactly the bits of the default path.
+__global__ void __launch_bounds__(256)
+k_input_fwd_csr(const float* __restrict__ feats, const int32_t* __restrict__ vstart, const int32_t* __restrict__ vpts,
+                int64_t n_vox, int c, int mode, float* __restrict__ out) {
+  mm3d_griddep_wait();
+  const int64_t total = n_vox * c;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t v = i / c;
+    const int j = (int)(i - v * c);
+    const int32_t b = __ldg(vstart + v), e = __ldg(vstart + v + 1), cnt = e - b;
+    float acc;
+    if (cnt == 1) {
+      acc = __ldg(feats + (int64_t)__ldg(vpts + b) * c + j);
+    } else {
+      acc = 0.f;
+      for (int32_t q = b; q < e; ++q) {
+        const float f = __ldg(feats + (int64_t)__ldg(vpts + q) * c + j);
+        acc += mode == 4 ? f / (float)cnt : f;
+      }
+    }
+    out[i] = acc;
+  }
+}
+
+// OutputLayer backward: a voxel's gradient = the sum of its points' gradients, in point order
+__global__ void __launch_bounds__(256)
+k_output_bwd_csr(const float* __restrict__ d_out, const int32_t* __restrict__ vstart, const int32_t* __restrict__ vpts,
+                 int64_t n_vox, int c, float* __restrict__ d_vox) {
+  mm3d_griddep_wait();
+  const int64_t total = n_vox * c;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t v = i / c;
+    const int j = (int)(i - v * c);
+    const int32_t b = __ldg(vstart + v), e = __ldg(vstart + v + 1);
+    float acc = 0.f;
+    for (int32_t q = b; q < e; ++q) acc += __ldg(d_out + (int64_t)__ldg(vpts + q) * c + j);
+    d_vox[i] = acc;
+  }
+}
+
+// Keys of the lift's pixel lists: pixel (b H + r) W + c of every point (integer lift, negative indices wrapped as
+// k_lift_bwd does; an index outside the map gets no key and raises error word 1 like there), or of every (point, tap)
+// entry 4 p + q of the bilinear lift (a tap outside the map, or of weight zero, gets no key: k_lift_bilinear_bwd
+// skips it too)
+__global__ void k_lift_keys(const int64_t* __restrict__ idx, const float* __restrict__ uv, const int64_t* __restrict__ offs,
+                            int B, int H, int W, int64_t n, int32_t* __restrict__ key, int* err) {
+  mm3d_griddep_wait();
+  for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t base = (int64_t)find_sample(offs, B, p) * H;
+    if (idx) {
+      const longlong2 rc = __ldg(reinterpret_cast<const longlong2*>(idx) + p);
+      int64_t r = rc.x, col = rc.y;
+      if (r < 0) r += H;
+      if (col < 0) col += W;
+      if ((uint64_t)r >= (uint64_t)H || (uint64_t)col >= (uint64_t)W) {
+        key[p] = -1;
+        mm3d_raise(err, 1);
+      } else {
+        key[p] = (int32_t)((base + r) * W + col);
+      }
+    } else {
+      const float2 rc = __ldg(reinterpret_cast<const float2*>(uv) + p);
+      const BilinearTaps t = bilinear_taps(rc.x, rc.y, H, W, 0, 0);
+#pragma unroll
+      for (int q = 0; q < 4; ++q) key[4 * p + q] = t.w[q] != 0.f ? (int32_t)((base + t.rr[q]) * W + t.cc[q]) : -1;
+    }
+  }
+}
+
+// Lift backward over the pixel lists: one thread per (pixel, channel), channel fastest; FP32 accumulation in entry
+// order, rounded once to T and stored into the caller's zero-filled map.  BIL: entries are (point, tap) pairs 4 p + q
+// and a term is w_q * g as in k_lift_bilinear_bwd.
+template <class T, bool BIL>
+__global__ void __launch_bounds__(256)
+k_lift_bwd_csr(const T* __restrict__ d_out, int C, int H, int W, int64_t sb, int64_t sc, int64_t sh, int64_t sw,
+               const float* __restrict__ uv, const int32_t* __restrict__ pstart, const int32_t* __restrict__ pent,
+               int64_t n_pix, T* __restrict__ d_fmap) {
+  mm3d_griddep_wait();
+  const int64_t total = n_pix * C;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t pix = i / C;
+    const int ch = (int)(i - pix * C);
+    const int32_t b0 = __ldg(pstart + pix), e0 = __ldg(pstart + pix + 1);
+    if (b0 == e0) continue;
+    float acc = 0.f;
+    for (int32_t q = b0; q < e0; ++q) {
+      const int32_t ent = __ldg(pent + q);
+      if (BIL) {
+        const int64_t p = ent >> 2;
+        const float2 rc = __ldg(reinterpret_cast<const float2*>(uv) + p);
+        const BilinearTaps t = bilinear_taps(rc.x, rc.y, H, W, 0, 0);
+        acc += t.w[ent & 3] * lift_to_f32(d_out[p * C + ch]);
+      } else {
+        acc += lift_to_f32(d_out[(int64_t)ent * C + ch]);
+      }
+    }
+    const int64_t hw = (int64_t)H * W;
+    const int64_t b = pix / hw, rem = pix - b * hw, r = rem / W, col = rem - r * W;
+    d_fmap[b * sb + ch * sc + r * sh + col * sw] = T(acc);
   }
 }
 
@@ -582,6 +692,100 @@ extern "C" int mm3d_lift2d_bilinear_bwd(const void* d_out, int dtype, int B, int
   mm3d_count_launches(1);
   MM3D_CHECK_LAUNCH("mm3d_lift2d_bilinear_bwd");
   return MM3D_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Deterministic forms (MM3D_DETERMINISTIC): segmented sums over the group-by-key lists of groupby.cu
+// ------------------------------------------------------------------------------------------------
+extern "C" int mm3d_input_fwd_csr(const float* feats, const int32_t* vox_start, const int32_t* vox_pts, int64_t n_vox, int c,
+                                  int mode, float* out_vox, mm3d_stream_t stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  MM3D_REQUIRE(mode == 3 || mode == 4, MM3D_ERR_UNSUPPORTED, "InputLayer mode %d not implemented (3=sum, 4=mean)", mode);
+  MM3D_REQUIRE(c > 0 && n_vox >= 0, MM3D_ERR_INVALID, "bad sizes");
+  if (n_vox == 0) return MM3D_OK;
+  MM3D_REQUIRE(feats && vox_start && vox_pts && out_vox, MM3D_ERR_INVALID, "input_fwd_csr: null pointer");
+  MM3D_CUDA(mm3d_launch_pdl(k_input_fwd_csr, dim3(mm3d_grid(n_vox * c, 256, 16)), dim3(256), 0, stream, feats, vox_start,
+                            vox_pts, n_vox, c, mode, out_vox));
+  mm3d_count_launches(1);
+  MM3D_CHECK_LAUNCH("mm3d_input_fwd_csr");
+  return MM3D_OK;
+}
+
+extern "C" int mm3d_output_bwd_csr(const float* d_out, const int32_t* vox_start, const int32_t* vox_pts, int64_t n_vox, int c,
+                                   float* d_vox, mm3d_stream_t stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  MM3D_REQUIRE(c > 0 && n_vox >= 0, MM3D_ERR_INVALID, "bad sizes");
+  if (n_vox == 0) return MM3D_OK;
+  MM3D_REQUIRE(d_out && vox_start && vox_pts && d_vox, MM3D_ERR_INVALID, "output_bwd_csr: null pointer");
+  MM3D_CUDA(mm3d_launch_pdl(k_output_bwd_csr, dim3(mm3d_grid(n_vox * c, 256, 16)), dim3(256), 0, stream, d_out, vox_start,
+                            vox_pts, n_vox, c, d_vox));
+  mm3d_count_launches(1);
+  MM3D_CHECK_LAUNCH("mm3d_output_bwd_csr");
+  return MM3D_OK;
+}
+
+extern "C" size_t mm3d_lift_csr_workspace_bytes(int B, int H, int W, int64_t n, int bilinear) {
+  const int64_t n_ent = (bilinear ? 4 : 1) * (n > 0 ? n : 1);
+  return mm3d_align(sizeof(int32_t) * (size_t)n_ent) + mm3d_group_by_workspace_bytes((int64_t)B * H * W);
+}
+
+extern "C" int mm3d_lift_csr(const int64_t* idx, const float* uv, const int64_t* sample_offsets, int B, int H, int W, int64_t n,
+                             int32_t* pix_start, int32_t* pix_ent, void* ws, size_t ws_bytes, mm3d_stream_t stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  MM3D_REQUIRE(B > 0 && H > 0 && W > 0 && n >= 0, MM3D_ERR_INVALID, "lift_csr: bad sizes");
+  MM3D_REQUIRE((idx == nullptr) != (uv == nullptr), MM3D_ERR_INVALID, "lift_csr: give exactly one of idx and uv");
+  const int64_t n_pix = (int64_t)B * H * W, n_ent = (uv ? 4 : 1) * n;
+  MM3D_REQUIRE(n_pix < (1ll << 31) && n_ent < (1ll << 31), MM3D_ERR_INVALID, "lift_csr: more than 2^31 pixels or entries");
+  MM3D_REQUIRE(ws && ws_bytes >= mm3d_lift_csr_workspace_bytes(B, H, W, n, uv != nullptr), MM3D_ERR_WORKSPACE,
+               "lift_csr: workspace too small");
+  MM3D_REQUIRE(((uintptr_t)idx & 15) == 0 && ((uintptr_t)uv & 7) == 0, MM3D_ERR_INVALID, "lift_csr: misaligned idx / uv");
+  int32_t* key = (int32_t*)ws;
+  const size_t key_bytes = mm3d_align(sizeof(int32_t) * (size_t)(n_ent > 0 ? n_ent : 1));
+  if (n > 0) {
+    MM3D_REQUIRE(sample_offsets, MM3D_ERR_INVALID, "lift_csr: null sample_offsets");
+    MM3D_CUDA(mm3d_launch_pdl(k_lift_keys, dim3(mm3d_grid(n, 256, 16)), dim3(256), 0, stream, idx, uv, sample_offsets, B, H, W, n,
+                              key, mm3d_device_err_flag()));
+    mm3d_count_launches(1);
+  }
+  return mm3d_group_by(key, nullptr, n_ent, n_pix, pix_start, pix_ent, (char*)ws + key_bytes, ws_bytes - key_bytes, stream);
+}
+
+#define LIFT_CSR_LAUNCH(T, BIL)                                                                                          \
+  MM3D_CUDA(mm3d_launch_pdl(k_lift_bwd_csr<T, BIL>, dim3(mm3d_grid(n_pix * C, 256, 16)), dim3(256), 0, stream,           \
+                            (const T*)d_out, C, H, W, sb, sc, sh, sw, uv, pix_start, pix_ent, n_pix, (T*)d_fmap))
+
+static int lift_bwd_csr(const void* d_out, int dtype, int B, int C, int H, int W, int64_t sb, int64_t sc, int64_t sh, int64_t sw,
+                        const float* uv, const int32_t* pix_start, const int32_t* pix_ent, void* d_fmap, cudaStream_t stream,
+                        const char* name) {
+  MM3D_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, MM3D_ERR_INVALID, "bad lift sizes");
+  MM3D_REQUIRE(sb > 0 && sc > 0 && sh > 0 && sw > 0, MM3D_ERR_INVALID, "bad lift strides");
+  MM3D_REQUIRE(d_out && pix_start && pix_ent && d_fmap, MM3D_ERR_INVALID, "%s: null pointer", name);
+  const int64_t n_pix = (int64_t)B * H * W;
+  const bool bil = uv != nullptr;
+  switch (dtype) {
+    case 0: if (bil) LIFT_CSR_LAUNCH(float, true); else LIFT_CSR_LAUNCH(float, false); break;
+    case 1: if (bil) LIFT_CSR_LAUNCH(__half, true); else LIFT_CSR_LAUNCH(__half, false); break;
+    case 2: if (bil) LIFT_CSR_LAUNCH(__nv_bfloat16, true); else LIFT_CSR_LAUNCH(__nv_bfloat16, false); break;
+    default: MM3D_REQUIRE(false, MM3D_ERR_UNSUPPORTED, "lift dtype %d (0=f32,1=f16,2=bf16)", dtype);
+  }
+  mm3d_count_launches(1);
+  MM3D_CHECK_LAUNCH(name);
+  return MM3D_OK;
+}
+
+extern "C" int mm3d_lift2d_bwd_csr(const void* d_out, int dtype, int B, int C, int H, int W, int64_t sb, int64_t sc, int64_t sh,
+                                   int64_t sw, const int32_t* pix_start, const int32_t* pix_ent, void* d_fmap,
+                                   mm3d_stream_t stream) {
+  return lift_bwd_csr(d_out, dtype, B, C, H, W, sb, sc, sh, sw, nullptr, pix_start, pix_ent, d_fmap, (cudaStream_t)stream,
+                      "mm3d_lift2d_bwd_csr");
+}
+
+extern "C" int mm3d_lift2d_bilinear_bwd_csr(const void* d_out, int dtype, int B, int C, int H, int W, int64_t sb, int64_t sc,
+                                            int64_t sh, int64_t sw, const float* uv, const int32_t* pix_start,
+                                            const int32_t* pix_ent, void* d_fmap, mm3d_stream_t stream) {
+  MM3D_REQUIRE(uv && (((uintptr_t)uv) & 7) == 0, MM3D_ERR_INVALID, "lift: the coordinate array must be 8-byte aligned");
+  return lift_bwd_csr(d_out, dtype, B, C, H, W, sb, sc, sh, sw, uv, pix_start, pix_ent, d_fmap, (cudaStream_t)stream,
+                      "mm3d_lift2d_bilinear_bwd_csr");
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -115,6 +115,9 @@ class UNetSCNFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, feats, meta, cfg, mask_w, mask_b, *slots):
         in_ch, m, L, mode, training, eps, momentum, spatial0, reps, res = cfg
+        if F.deterministic():
+            F.alert_not_deterministic("the whole-network UNetSCN executor (weight gradients, BatchNorm statistics, "
+                                      "point->voxel sums)")
         feats = feats.float().contiguous()
         dev = feats.device
         # optional RGB mask of Net3DSeg.forward (3d_net/model.py:46-48), folded into the InputLayer scatter

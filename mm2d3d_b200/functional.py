@@ -8,6 +8,8 @@ argument, defaulting to the module-level :data:`DEFAULT_MODE`.
 """
 from __future__ import annotations
 
+import warnings
+
 import torch
 from torch.amp import custom_bwd, custom_fwd
 
@@ -15,6 +17,22 @@ from . import _lib
 from ._lib import MODES, check, lib, ptr
 
 DEFAULT_MODE = "fp32"
+
+# Deterministic mode (scn.set_deterministic): None follows torch.are_deterministic_algorithms_enabled()
+DETERMINISTIC = None
+
+
+def deterministic() -> bool:
+    """Whether the ops called now take their deterministic (fixed summation order) forms."""
+    return torch.are_deterministic_algorithms_enabled() if DETERMINISTIC is None else bool(DETERMINISTIC)
+
+
+def alert_not_deterministic(what: str) -> None:
+    """Called by an op that has no deterministic form yet while the mode is on: a UserWarning that its result can
+    still differ between runs (Python shows it once per call site)."""
+    warnings.warn(f"mm2d3d_b200: {what} has no deterministic form yet -- its result can differ in the last bits "
+                  "between runs although the deterministic mode is on (see INTEGRATION.md, Deterministic mode)",
+                  UserWarning, stacklevel=3)
 
 _scratch: dict = {}
 
@@ -51,8 +69,13 @@ class InputLayerFn(torch.autograd.Function):
             raise ValueError("InputLayer: fewer feature rows than coordinates")
         out = torch.empty(meta.n_voxels, c, dtype=torch.float32, device=feats.device)
         with torch.cuda.device(feats.device):
-            check(lib.mm3d_input_fwd(ptr(feats), meta.p2v_ptr, meta.npts_ptr, n, meta.n_voxels, c, mode, ptr(out),
-                                     _lib.stream_ptr()), "mm3d_input_fwd")
+            if deterministic():
+                start, pts = meta.point_csr()
+                check(lib.mm3d_input_fwd_csr(ptr(feats), ptr(start), ptr(pts), meta.n_voxels, c, mode, ptr(out),
+                                             _lib.stream_ptr()), "mm3d_input_fwd_csr")
+            else:
+                check(lib.mm3d_input_fwd(ptr(feats), meta.p2v_ptr, meta.npts_ptr, n, meta.n_voxels, c, mode, ptr(out),
+                                         _lib.stream_ptr()), "mm3d_input_fwd")
         ctx.meta, ctx.mode, ctx.rows = meta, mode, feats.shape[0]
         return out
 
@@ -81,7 +104,7 @@ class OutputLayerFn(torch.autograd.Function):
         with torch.cuda.device(vox.device):
             check(lib.mm3d_output_fwd(ptr(vox), meta.p2v_ptr, meta.n_points, c, ptr(out), _lib.stream_ptr()),
                   "mm3d_output_fwd")
-        ctx.meta = meta
+        ctx.meta, ctx.det = meta, deterministic()
         return out
 
     @staticmethod
@@ -92,8 +115,13 @@ class OutputLayerFn(torch.autograd.Function):
         c = d_out.shape[1]
         d_vox = torch.empty(meta.n_voxels, c, dtype=torch.float32, device=d_out.device)
         with torch.cuda.device(d_out.device):
-            check(lib.mm3d_output_bwd(ptr(d_out), meta.p2v_ptr, meta.n_points, meta.n_voxels, c, ptr(d_vox),
-                                      _lib.stream_ptr()), "mm3d_output_bwd")
+            if ctx.det:
+                start, pts = meta.point_csr()
+                check(lib.mm3d_output_bwd_csr(ptr(d_out), ptr(start), ptr(pts), meta.n_voxels, c, ptr(d_vox),
+                                              _lib.stream_ptr()), "mm3d_output_bwd_csr")
+            else:
+                check(lib.mm3d_output_bwd(ptr(d_out), meta.p2v_ptr, meta.n_points, meta.n_voxels, c, ptr(d_vox),
+                                          _lib.stream_ptr()), "mm3d_output_bwd")
         return d_vox, None
 
 
@@ -196,6 +224,7 @@ class TableConvFn(torch.autograd.Function):
                                     _lib.stream_ptr()), "mm3d_conv_fwd")
         ctx.save_for_backward(x, w)
         ctx.meta, ctx.tables, ctx.mode, ctx.wshape = meta, (fwd_t, bwd_t, bwd_flags), m, weight.shape
+        ctx.det = deterministic()
         return out
 
     @staticmethod
@@ -221,6 +250,8 @@ class TableConvFn(torch.autograd.Function):
                                         bwd_t.tbl, bwd_t.stride, bwd_t.onehot, bwd_t.plan, bwd_t.plan_cap, bwd_flags, m,
                                         ptr(ws), ws.numel(), stream), "mm3d_conv_fwd(dgrad)")
             if ctx.needs_input_grad[1]:
+                if ctx.det:
+                    alert_not_deterministic("the sparse-convolution weight gradient")
                 d_w = torch.empty(w.shape, dtype=torch.float32, device=x.device)
                 check(lib.mm3d_conv_wgrad(ptr(x), fwd_t.n_in, c_in, ptr(d_out), fwd_t.n_out, c_out, ptr(d_w), K,
                                           fwd_t.tbl, fwd_t.stride, fwd_t.onehot, fwd_t.plan, fwd_t.plan_cap, 0, m, ptr(ws),
@@ -237,6 +268,8 @@ class BatchNormReLUFn(torch.autograd.Function):
     @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
     def forward(ctx, x, gamma, beta, running_mean, running_var, eps, momentum, leakiness, training):
         _require_cuda(x, "BatchNormReLU")
+        if training and deterministic():
+            alert_not_deterministic("BatchNorm in training mode (batch statistics, gamma / beta gradients)")
         x = _f32c(x)
         n, c = x.shape
         y = torch.empty_like(x)
@@ -272,6 +305,21 @@ class BatchNormReLUFn(torch.autograd.Function):
 _LIFT_DTYPES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
 
 
+def lift_csr(idx, uv, offsets, B, H, W):
+    """(pix_start int32 [B H W + 1], pix_ent int32 [n or 4 n]): the lift's entries grouped by pixel in ascending
+    order (``mm3d_lift_csr``), on the current stream.  ``idx`` int64 [n, 2] or, for the bilinear lift, ``uv``."""
+    t = idx if idx is not None else uv
+    n = int(t.shape[0])
+    bil = uv is not None
+    start = torch.empty(B * H * W + 1, dtype=torch.int32, device=t.device)
+    ent = torch.empty(max((4 if bil else 1) * n, 1), dtype=torch.int32, device=t.device)
+    with torch.cuda.device(t.device):
+        ws = torch.empty(lib.mm3d_lift_csr_workspace_bytes(B, H, W, n, int(bil)), dtype=torch.uint8, device=t.device)
+        check(lib.mm3d_lift_csr(ptr(idx), ptr(uv), ptr(offsets), B, H, W, n, ptr(start), ptr(ent), ptr(ws), ws.numel(),
+                                _lib.stream_ptr()), "mm3d_lift_csr")
+    return start, ent
+
+
 def _dense_map(t):
     """The map as it is when its memory is dense in NCHW or channels-last (NHWC) order, else a contiguous copy."""
     if t.is_contiguous() or t.is_contiguous(memory_format=torch.channels_last):
@@ -281,7 +329,8 @@ def _dense_map(t):
 
 class Lift2DFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, fmap, idx, offsets):
+    def forward(ctx, fmap, idx, offsets, lists=None):
+        """``lists``: an object whose ``pixel_lists(B, H, W)`` caches the pixel lists of ``idx`` (LiftIndices)."""
         _require_cuda(fmap, "lift2d")
         if fmap.dtype not in _LIFT_DTYPES:
             raise TypeError(f"lift2d: unsupported dtype {fmap.dtype}")
@@ -295,6 +344,7 @@ class Lift2DFn(torch.autograd.Function):
         ctx.save_for_backward(idx, offsets)
         ctx.shape = (B, C, H, W)
         ctx.channels_last = not fmap.is_contiguous()
+        ctx.lists, ctx.det = lists, deterministic()
         return out
 
     @staticmethod
@@ -306,9 +356,15 @@ class Lift2DFn(torch.autograd.Function):
         d_fmap = torch.empty(B, C, H, W, dtype=d_out.dtype, device=d_out.device,
                              memory_format=torch.channels_last if ctx.channels_last else torch.contiguous_format).zero_()
         with torch.cuda.device(d_out.device):
-            check(lib.mm3d_lift2d_bwd(ptr(d_out), _LIFT_DTYPES[d_out.dtype], B, C, H, W, *d_fmap.stride(), ptr(idx), ptr(offsets),
-                                      idx.shape[0], ptr(d_fmap), _lib.stream_ptr()), "mm3d_lift2d_bwd")
-        return d_fmap, None, None
+            if ctx.det:
+                start, ent = (ctx.lists.pixel_lists(B, H, W) if ctx.lists is not None
+                              else lift_csr(idx, None, offsets, B, H, W))
+                check(lib.mm3d_lift2d_bwd_csr(ptr(d_out), _LIFT_DTYPES[d_out.dtype], B, C, H, W, *d_fmap.stride(), ptr(start),
+                                              ptr(ent), ptr(d_fmap), _lib.stream_ptr()), "mm3d_lift2d_bwd_csr")
+            else:
+                check(lib.mm3d_lift2d_bwd(ptr(d_out), _LIFT_DTYPES[d_out.dtype], B, C, H, W, *d_fmap.stride(), ptr(idx),
+                                          ptr(offsets), idx.shape[0], ptr(d_fmap), _lib.stream_ptr()), "mm3d_lift2d_bwd")
+        return d_fmap, None, None, None
 
 
 class Lift2DBilinearFn(torch.autograd.Function):
@@ -329,6 +385,7 @@ class Lift2DBilinearFn(torch.autograd.Function):
         ctx.save_for_backward(uv, offsets)
         ctx.shape = (B, C, H, W)
         ctx.channels_last = not fmap.is_contiguous()
+        ctx.det = deterministic()
         return out
 
     @staticmethod
@@ -339,7 +396,13 @@ class Lift2DBilinearFn(torch.autograd.Function):
         d_fmap = torch.empty(B, C, H, W, dtype=d_out.dtype, device=d_out.device,
                              memory_format=torch.channels_last if ctx.channels_last else torch.contiguous_format).zero_()
         with torch.cuda.device(d_out.device):
-            check(lib.mm3d_lift2d_bilinear_bwd(ptr(d_out), _LIFT_DTYPES[d_out.dtype], B, C, H, W, *d_fmap.stride(), ptr(uv),
-                                               ptr(offsets), uv.shape[0], ptr(d_fmap), _lib.stream_ptr()),
-                  "mm3d_lift2d_bilinear_bwd")
+            if ctx.det:  # (point, tap) lists of this call's coordinates
+                start, ent = lift_csr(None, uv, offsets, B, H, W)
+                check(lib.mm3d_lift2d_bilinear_bwd_csr(ptr(d_out), _LIFT_DTYPES[d_out.dtype], B, C, H, W, *d_fmap.stride(),
+                                                       ptr(uv), ptr(start), ptr(ent), ptr(d_fmap), _lib.stream_ptr()),
+                      "mm3d_lift2d_bilinear_bwd_csr")
+            else:
+                check(lib.mm3d_lift2d_bilinear_bwd(ptr(d_out), _LIFT_DTYPES[d_out.dtype], B, C, H, W, *d_fmap.stride(),
+                                                   ptr(uv), ptr(offsets), uv.shape[0], ptr(d_fmap), _lib.stream_ptr()),
+                      "mm3d_lift2d_bilinear_bwd")
         return d_fmap, None, None

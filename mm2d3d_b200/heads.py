@@ -13,6 +13,12 @@ import torch
 
 from . import _lib
 from ._lib import check, lib, ptr
+from .functional import deterministic
+
+
+def _det_flags():
+    """(flags, partial slots of a reduction's workspace) of the deterministic mode as it is now"""
+    return (_lib.DETERMINISTIC, _lib.DET_CTAS) if deterministic() else (0, 1)
 
 
 def _f32c(t):
@@ -34,6 +40,7 @@ class _RgbMaskFn(torch.autograd.Function):
             check(lib.mm3d_rgb_mask_fwd(ptr(x), n, c, ptr(w), ptr(b), ptr(y), ptr(s), _lib.stream_ptr()), "mm3d_rgb_mask_fwd")
         ctx.save_for_backward(x, s, w)
         ctx.shapes = (weight.shape, bias.shape)
+        ctx.det = _det_flags()
         return y
 
     @staticmethod
@@ -43,10 +50,11 @@ class _RgbMaskFn(torch.autograd.Function):
         n, c = x.shape
         dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
         dwb = torch.empty(c + 1, dtype=torch.float32, device=x.device)
-        ws = torch.empty(c + 1, dtype=torch.float64, device=x.device)
+        flags, slots = ctx.det
+        ws = torch.empty((c + 1) * slots, dtype=torch.float64, device=x.device)
         with torch.cuda.device(x.device):
-            check(lib.mm3d_rgb_mask_bwd(ptr(x), ptr(s), ptr(dy), n, c, ptr(w), ptr(dx), ptr(dwb), dwb.data_ptr() + 4 * c,
-                                        ptr(ws), ws.numel() * 8, _lib.stream_ptr()), "mm3d_rgb_mask_bwd")
+            check(lib.mm3d_rgb_mask_bwd_ex(ptr(x), ptr(s), ptr(dy), n, c, ptr(w), ptr(dx), ptr(dwb), dwb.data_ptr() + 4 * c,
+                                           ptr(ws), ws.numel() * 8, _lib.stream_ptr(), flags), "mm3d_rgb_mask_bwd")
         return dx, dwb[:c].reshape(ctx.shapes[0]), dwb[c:].reshape(ctx.shapes[1])
 
 
@@ -65,9 +73,11 @@ class _KlFn(torch.autograd.Function):
             raise ValueError("cross_modal_kl: two non-empty [N, C] logit tensors expected")
         n, C = p.shape
         loss = torch.empty((), dtype=torch.float32, device=p.device)
-        ws = torch.empty(1, dtype=torch.float64, device=p.device)
+        flags, slots = _det_flags()
+        ws = torch.empty(slots, dtype=torch.float64, device=p.device)
         with torch.cuda.device(p.device):
-            check(lib.mm3d_kl_logits_fwd(ptr(p), ptr(t), n, C, ptr(loss), ptr(ws), 8, _lib.stream_ptr()), "mm3d_kl_logits_fwd")
+            check(lib.mm3d_kl_logits_fwd_ex(ptr(p), ptr(t), n, C, ptr(loss), ptr(ws), ws.numel() * 8, _lib.stream_ptr(), flags),
+                  "mm3d_kl_logits_fwd")
         ctx.save_for_backward(p, t)
         return loss
 
@@ -103,11 +113,13 @@ class _Heads3DFn(torch.autograd.Function):
         l1 = torch.empty(n, C, dtype=torch.float32, device=x.device)
         l2 = torch.empty(n, C, dtype=torch.float32, device=x.device)
         loss = torch.zeros((), dtype=torch.float32, device=x.device)
-        ws = torch.empty(1, dtype=torch.float64, device=x.device)
+        flags, slots = ctx.det = _det_flags()
+        ws = torch.empty(slots, dtype=torch.float64, device=x.device)
         with torch.cuda.device(x.device):
-            check(lib.mm3d_heads3d_fwd(ptr(x), n, f, C, ptr(w1c), ptr(b1c), ptr(w2c), ptr(b2c), ptr(t) if t is not None else None,
-                                       ptr(l1), ptr(l2), ptr(loss) if t is not None and n else None, ptr(ws), 8,
-                                       _lib.stream_ptr()), "mm3d_heads3d_fwd")
+            check(lib.mm3d_heads3d_fwd_ex(ptr(x), n, f, C, ptr(w1c), ptr(b1c), ptr(w2c), ptr(b2c),
+                                          ptr(t) if t is not None else None, ptr(l1), ptr(l2),
+                                          ptr(loss) if t is not None and n else None, ptr(ws), ws.numel() * 8,
+                                          _lib.stream_ptr(), flags), "mm3d_heads3d_fwd")
         ctx.save_for_backward(x, w1c, w2c, b2c, *([t] if t is not None else []))
         ctx.has_target = t is not None
         return l1, l2, loss
@@ -125,13 +137,14 @@ class _Heads3DFn(torch.autograd.Function):
         dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
         dw1, db1 = torch.empty_like(w1), torch.empty(C, dtype=torch.float32, device=x.device)
         dw2, db2 = torch.empty_like(w2), torch.empty(C, dtype=torch.float32, device=x.device)
-        ws = torch.empty(2 * C * f + 2 * C, dtype=torch.float64, device=x.device)
+        flags, slots = ctx.det
+        ws = torch.empty((2 * C * f + 2 * C) * slots, dtype=torch.float64, device=x.device)
         with torch.cuda.device(x.device):
-            check(lib.mm3d_heads3d_bwd(ptr(x), n, f, C, ptr(w1), ptr(w2), ptr(b2), ptr(t) if t is not None else None,
-                                       ptr(d1) if d1 is not None else None, ptr(d2) if d2 is not None else None,
-                                       ptr(dl) if dl is not None else None, ptr(dx) if dx is not None else None,
-                                       ptr(dw1), ptr(db1), ptr(dw2), ptr(db2), ptr(ws), ws.numel() * 8, _lib.stream_ptr()),
-                  "mm3d_heads3d_bwd")
+            check(lib.mm3d_heads3d_bwd_ex(ptr(x), n, f, C, ptr(w1), ptr(w2), ptr(b2), ptr(t) if t is not None else None,
+                                          ptr(d1) if d1 is not None else None, ptr(d2) if d2 is not None else None,
+                                          ptr(dl) if dl is not None else None, ptr(dx) if dx is not None else None,
+                                          ptr(dw1), ptr(db1), ptr(dw2), ptr(db2), ptr(ws), ws.numel() * 8, _lib.stream_ptr(),
+                                          flags), "mm3d_heads3d_bwd")
         return dx, dw1, db1, dw2, db2, None
 
 

@@ -18,7 +18,7 @@ import numpy as np
 import torch
 
 from . import _lib  # noqa: F401  (raises when the library is missing)
-from .functional import Lift2DBilinearFn, Lift2DFn
+from .functional import Lift2DBilinearFn, Lift2DFn, lift_csr
 
 
 class LiftIndices:
@@ -39,6 +39,14 @@ class LiftIndices:
         self.hi = (int(cat[:, 0].max()), int(cat[:, 1].max())) if len(cat) else (-1, -1)
         self.idx = torch.from_numpy(np.ascontiguousarray(cat)).to(device, non_blocking=True)
         self.offsets = torch.from_numpy(offs).to(device, non_blocking=True)
+        self._pixel_lists = {}
+
+    def pixel_lists(self, B, H, W):
+        """The points grouped by pixel of a [B, ., H, W] map (deterministic lift backward), built on first use."""
+        key = (int(B), int(H), int(W))
+        if key not in self._pixel_lists:
+            self._pixel_lists[key] = lift_csr(self.idx, None, self.offsets, *key)
+        return self._pixel_lists[key]
 
     @property
     def n(self):
@@ -55,7 +63,7 @@ def lift2d(fmap: torch.Tensor, img_indices) -> torch.Tensor:
     if img_indices.lo[0] < -H or img_indices.hi[0] >= H or img_indices.lo[1] < -W or img_indices.hi[1] >= W:
         raise IndexError(f"lift2d: pixel index out of range for a {H}x{W} map "
                          f"(rows {img_indices.lo[0]}..{img_indices.hi[0]}, columns {img_indices.lo[1]}..{img_indices.hi[1]})")
-    return Lift2DFn.apply(fmap, img_indices.idx, img_indices.offsets)
+    return Lift2DFn.apply(fmap, img_indices.idx, img_indices.offsets, img_indices)
 
 
 def lift2d_bilinear(fmap: torch.Tensor, pixel_coords) -> torch.Tensor:

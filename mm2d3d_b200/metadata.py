@@ -69,6 +69,7 @@ class Metadata:
             self.device = coords.device
             self.n_points = int(coords.shape[0])
         self._pending = None
+        self._point_csr = None
         self.spatial_size0 = int(spatial_size)
         self.levels: dict[int, Level] = {}
         self._order: list[Level] = []
@@ -216,11 +217,27 @@ class Metadata:
         seen = set()
         bufs = [self._buf, self._counts] + [lv.buf for lv in self._order]
         bufs += [pl[0] for lv in self._order for pl in lv.plans.values()]
+        bufs += list(self._point_csr or ())
         for b in bufs:
             key = b.untyped_storage().data_ptr()
             if key not in seen:
                 seen.add(key)
                 b.record_stream(stream)
+
+    def point_csr(self):
+        """(vox_start int32 [n_voxels + 1], vox_pts int32 [n_points]): the points of every voxel in ascending point
+        index, for the deterministic InputLayer forward and OutputLayer backward.  Built on the current stream at
+        first use and kept."""
+        if self._point_csr is None:
+            nv, n = self.n_voxels, self.n_points
+            start = torch.empty(nv + 1, dtype=torch.int32, device=self.device)
+            pts = torch.empty(max(n, 1), dtype=torch.int32, device=self.device)
+            with torch.cuda.device(self.device):
+                ws = torch.empty(lib.mm3d_point_csr_workspace_bytes(nv), dtype=torch.uint8, device=self.device)
+                check(lib.mm3d_point_csr(self.p2v_ptr, self.npts_ptr, n, nv, start.data_ptr(), pts.data_ptr(),
+                                         ws.data_ptr(), ws.numel(), _lib.stream_ptr()), "mm3d_point_csr")
+            self._point_csr = (start, pts)
+        return self._point_csr
 
     # ------------------------------------------------------------------ lookups used by the layers
     def level(self, spatial_size: int) -> Level:

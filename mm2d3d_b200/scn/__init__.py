@@ -22,7 +22,7 @@ from ..metadata import Metadata
 __all__ = [
     "SparseConvNetTensor", "Sequential", "ConcatTable", "JoinTable", "AddTable", "Identity", "InputLayer",
     "OutputLayer", "SubmanifoldConvolution", "Convolution", "Deconvolution", "BatchNormReLU",
-    "BatchNormLeakyReLU", "NetworkInNetwork", "set_conv_mode", "get_conv_mode",
+    "BatchNormLeakyReLU", "NetworkInNetwork", "set_conv_mode", "get_conv_mode", "set_deterministic", "get_deterministic",
 ]
 
 
@@ -38,6 +38,27 @@ def set_conv_mode(mode: str) -> None:
 
 def get_conv_mode() -> str:
     return F.DEFAULT_MODE
+
+
+def set_deterministic(flag) -> None:
+    """Deterministic mode: ``True`` makes the ops below sum in a fixed order, so that they return the same bits on
+    every run and in every process (same device model, build, inputs and settings); ``False`` keeps the default
+    kernels, whose floating-point atomics may land in any order; ``None`` (the default) follows
+    ``torch.use_deterministic_algorithms`` (what Lightning's ``Trainer(deterministic=True)`` sets).  The setting is
+    read when an op runs forward, and its backward keeps that choice.
+
+    Covered: the InputLayer forward and OutputLayer backward of the module path, the lift backward (``lift2d``,
+    ``lift2d_bilinear``), ``rgb_mask``, ``cross_modal_kl`` and ``heads3d``.  Not yet covered: the convolution weight
+    gradients, the BatchNorm statistics and the whole-network executor (``UNetSCN``'s fused path); while the mode is
+    on, these issue a ``UserWarning`` when they run."""
+    if flag is not None and not isinstance(flag, bool):
+        raise TypeError(f"set_deterministic: True, False or None expected, got {flag!r}")
+    F.DETERMINISTIC = flag
+
+
+def get_deterministic() -> bool:
+    """Whether the deterministic mode is on now (the setting of :func:`set_deterministic`, resolved)."""
+    return F.deterministic()
 
 
 class SparseConvNetTensor:
