@@ -370,7 +370,8 @@ MM3D_API int mm3d_heads3d_bwd_ex(const float* feat, int64_t n, int f, int C, con
  * with a VGG block = bn{4} smc.w and a residual block = [nin.w] bn{4} smc.w bn{4} smc.w (the NetworkInNetwork
  * weight [a, b] only where the block changes the channel count: the first post block of a level).
  * (mm3d_unet_topo_num_params slots; grads ignore the running-stat slots.)  act: activations kept from forward to
- * backward; tmp: backward temporaries.
+ * backward; tmp: backward temporaries, mm3d_unet_topo_bwd_bytes, which is the exact need.  Forward and backward check
+ * every buffer against its query before they issue any CUDA call and return MM3D_ERR_WORKSPACE when one is short.
  * ---------------------------------------------------------------------------------------- */
 #define MM3D_LEVEL_DESC_WORDS 10
 MM3D_API int64_t mm3d_unet_topo_num_params(int num_planes, int block_reps, int residual);

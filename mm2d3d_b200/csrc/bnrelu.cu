@@ -490,7 +490,6 @@ int* mm3d_device_err_flag();  // conv_tc.cu
 // workspace: two regions of [kSlots copies of 2*c doubles of totals | kSlots + 1 barrier counters]
 static size_t bn_region_bytes(int c) { return mm3d_align(sizeof(double) * (kSlots * 2 * (size_t)c + 8)); }
 extern "C" size_t mm3d_bnrelu_workspace_bytes(int c) { return 2 * bn_region_bytes(c); }
-static int g_bn_parity = 0;  // (host threads launching BatchNorm concurrently on one device must use separate workspaces)
 
 #define BN_DISPATCH(KERNEL, ...)                                                        \
   do {                                                                                  \
@@ -506,12 +505,14 @@ static int g_bn_parity = 0;  // (host threads launching BatchNorm concurrently o
                 MM3D_CUDA(mm3d_launch_pdl(KERNEL<1>, dim3(grid), dim3(kThreads), smem, stream, __VA_ARGS__)); } \
   } while (0)
 
-// ws_clean: the workspace is known to be all zero (the kernels leave it that way), skip the memset
+// parity == NULL: the workspace is not known to be clean: zero it, use region 0.  Otherwise it is all zero (the kernels
+// leave it that way, no memset), and the launches that use it alternate between its two regions by toggling *parity,
+// which the caller keeps with the workspace.
 int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, int64_t n, int c, const float* gamma,
                          const float* beta,
                          float* running_mean, float* running_var, float* save_mean, float* save_invstd,
                          float eps, float momentum, float leakiness, int training,
-                         void* ws, size_t ws_bytes, bool ws_clean, int round_tf32, cudaStream_t stream) {
+                         void* ws, size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream) {
   MM3D_REQUIRE(c > 0 && n >= 0, MM3D_ERR_INVALID, "bad sizes");
   const bool vec4 = (c % 4 == 0) && (c_lo % 4 == 0) && ((((uintptr_t)x | (uintptr_t)x_hi | (uintptr_t)y) & 15) == 0);
   const int cv = vec4 ? c / 4 : c;
@@ -519,20 +520,20 @@ int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, 
   MM3D_REQUIRE(ws_bytes >= mm3d_bnrelu_workspace_bytes(c) && ws, MM3D_ERR_WORKSPACE, "bnrelu workspace too small");
   MM3D_REQUIRE(!x_hi || (training && c_lo > 0 && c_lo < c), MM3D_ERR_INVALID, "split input needs training mode and 0 < c_lo < c");
   if (n == 0) return MM3D_OK;
-  // region `parity` is this launch's (all zero: memset below, or zeroed by the previous launch), the other one is
+  // region `half` is this launch's (all zero: memset below, or zeroed by the previous launch), the other one is
   // zeroed by this launch for the next.  Region size follows the workspace size (the executor shares one workspace
   // among layers of different widths), so consecutive launches agree on where the regions are.
   const size_t region = ws_bytes / 2 / 256 * 256;
-  const int parity = (ws_clean && training) ? (g_bn_parity ^= 1) : 0;  // (only launches that use the workspace alternate)
-  double* sums = (double*)((char*)ws + (size_t)parity * region);
-  double* other = (double*)((char*)ws + (size_t)(parity ^ 1) * region);
+  const int half = (parity && training) ? (*parity ^= 1) : 0;  // (only launches that use the workspace alternate)
+  double* sums = (double*)((char*)ws + (size_t)half * region);
+  double* other = (double*)((char*)ws + (size_t)(half ^ 1) * region);
   unsigned int* sync = (unsigned int*)(sums + kSlots * 2 * c);
   const int other_words = (int)(region / 8);
   const size_t smem = sizeof(double) * 2 * c > sizeof(float) * 2 * (kThreads / cv) * (size_t)c
                           ? sizeof(double) * 2 * c : sizeof(float) * 2 * (kThreads / cv) * (size_t)c;
   if (training) {
     MM3D_REQUIRE(save_mean && save_invstd && running_mean && running_var, MM3D_ERR_INVALID, "training needs stat buffers");
-    if (!ws_clean) MM3D_CUDA(cudaMemsetAsync(ws, 0, 2 * region, stream));
+    if (!parity) MM3D_CUDA(cudaMemsetAsync(ws, 0, 2 * region, stream));
     BN_DISPATCH_PDL(k_bn_fwd_fused, x, x_hi, c_lo, y, n, c, gamma, beta, running_mean, running_var, save_mean, save_invstd, sums, sync,
                 other, other_words, eps, momentum, leakiness, round_tf32, mm3d_device_err_flag());
   } else {
@@ -547,7 +548,7 @@ int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, 
 int mm3d_bnrelu_bwd_impl(const float* x, const float* x_hi, int c_lo, const float* dy, float* dx, float* dx_hi,
                          int64_t n, int c, const float* gamma, const float* beta, const float* save_mean, const float* save_invstd,
                          float* d_gamma, float* d_beta, float leakiness, int training,
-                         void* ws, size_t ws_bytes, bool ws_clean, int round_flags, const float* add, int64_t add_ld,
+                         void* ws, size_t ws_bytes, int* parity, int round_flags, const float* add, int64_t add_ld,
                          cudaStream_t stream) {
   MM3D_REQUIRE(c > 0 && n >= 0, MM3D_ERR_INVALID, "bad sizes");
   const bool vec4 = (c % 4 == 0) && (c_lo % 4 == 0) && (!add || add_ld % 4 == 0) &&
@@ -561,12 +562,12 @@ int mm3d_bnrelu_bwd_impl(const float* x, const float* x_hi, int c_lo, const floa
     return MM3D_OK;
   }
   const size_t region = ws_bytes / 2 / 256 * 256;
-  const int parity = ws_clean ? (g_bn_parity ^= 1) : 0;
-  double* sums = (double*)((char*)ws + (size_t)parity * region);
-  double* other = (double*)((char*)ws + (size_t)(parity ^ 1) * region);
+  const int half = parity ? (*parity ^= 1) : 0;
+  double* sums = (double*)((char*)ws + (size_t)half * region);
+  double* other = (double*)((char*)ws + (size_t)(half ^ 1) * region);
   unsigned int* sync = (unsigned int*)(sums + kSlots * 2 * c);
   const int other_words = (int)(region / 8);
-  if (!ws_clean) MM3D_CUDA(cudaMemsetAsync(ws, 0, 2 * region, stream));
+  if (!parity) MM3D_CUDA(cudaMemsetAsync(ws, 0, 2 * region, stream));
   const size_t smem = sizeof(double) * 2 * c > sizeof(float) * 2 * (kThreads / cv) * (size_t)c
                           ? sizeof(double) * 2 * c : sizeof(float) * 2 * (kThreads / cv) * (size_t)c;
   BN_DISPATCH_PDL(k_bn_bwd_fused, x, x_hi, c_lo, dy, dx, dx_hi, n, c, gamma, beta, save_mean, save_invstd, leakiness, sums, sync, other, other_words, d_gamma,
@@ -581,7 +582,7 @@ extern "C" int mm3d_bnrelu_fwd(const float* x, float* y, int64_t n, int c, const
                                float eps, float momentum, float leakiness, int training,
                                void* ws, size_t ws_bytes, mm3d_stream_t stream) {
   return mm3d_bnrelu_fwd_impl(x, nullptr, 0, y, n, c, gamma, beta, running_mean, running_var, save_mean, save_invstd, eps, momentum,
-                              leakiness, training, ws, ws_bytes, false, 0, (cudaStream_t)stream);
+                              leakiness, training, ws, ws_bytes, nullptr, 0, (cudaStream_t)stream);
 }
 
 extern "C" int mm3d_bnrelu_bwd(const float* x, const float* dy, float* dx, int64_t n, int c, const float* gamma,
@@ -589,5 +590,5 @@ extern "C" int mm3d_bnrelu_bwd(const float* x, const float* dy, float* dx, int64
                                float* d_gamma, float* d_beta, float leakiness, int training,
                                void* ws, size_t ws_bytes, mm3d_stream_t stream) {
   return mm3d_bnrelu_bwd_impl(x, nullptr, 0, dy, dx, nullptr, n, c, gamma, beta, save_mean, save_invstd, d_gamma, d_beta, leakiness, training,
-                              ws, ws_bytes, false, 0, nullptr, 0, (cudaStream_t)stream);
+                              ws, ws_bytes, nullptr, 0, nullptr, 0, (cudaStream_t)stream);
 }

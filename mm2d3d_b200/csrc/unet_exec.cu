@@ -3,9 +3,9 @@
 // The per-layer entry points are enough for a drop-in, but driving ~110 autograd nodes from
 // Python costs ~8 ms of host time per step -- as much as the GPU work itself.  The executor walks
 // the U-Net topology of 3d_net/scn_unet.py:36-84 natively, for any number of blocks per level
-// (block_reps) and for VGG or pre-activation residual blocks: it carves every activation out of one
-// caller-provided workspace with a bump allocator that forward and backward replay identically, and
-// issues the same kernels the modules use.
+// (block_reps) and for VGG or pre-activation residual blocks, and issues the same kernels the modules use.  One
+// walk over the module tree (`Carve`) assigns the parameter slots and lays out every activation, every backward
+// temporary and the scratch buffer in the caller's workspaces; forward, backward and the size queries all run it.
 //
 //   level l (p = m(l+1), q = m(l+2)):
 //     X_l --[block p->p] x reps--> Y_l                                           ("pre" blocks)
@@ -34,11 +34,11 @@
 int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, int64_t n, int c, const float* gamma,
                          const float* beta, float* running_mean, float* running_var, float* save_mean,
                          float* save_invstd, float eps, float momentum, float leakiness, int training, void* ws,
-                         size_t ws_bytes, bool ws_clean, int round_tf32, cudaStream_t stream);
+                         size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream);
 int mm3d_bnrelu_bwd_impl(const float* x, const float* x_hi, int c_lo, const float* dy, float* dx, float* dx_hi,
                          int64_t n, int c, const float* gamma, const float* beta, const float* save_mean,
                          const float* save_invstd, float* d_gamma, float* d_beta, float leakiness, int training,
-                         void* ws, size_t ws_bytes, bool ws_clean, int round_flags, const float* add, int64_t add_ld,
+                         void* ws, size_t ws_bytes, int* parity, int round_flags, const float* add, int64_t add_ld,
                          cudaStream_t stream);
 
 // conv_tc.cu
@@ -68,17 +68,22 @@ struct LevelMeta {
   int64_t plan_cap;
 };
 
+// hands out consecutive 256-byte aligned pieces of a buffer; a NULL base only counts the bytes
 struct Bump {
   char* base;
-  size_t off, cap;
-  bool ok;
+  size_t off;
   void* bytes(size_t n) {
     size_t o = off;
     off += mm3d_align(n);
-    if (off > cap) ok = false;
     return base ? base + o : nullptr;
   }
   float* f(int64_t n, int64_t c) { return (float*)bytes(sizeof(float) * (size_t)n * (size_t)c); }
+};
+
+// one convolution of the network: its weight's parameter slot, kernel volume and channels (the stem's c_in is cin_k,
+// as the kernels see it)
+struct ConvInfo {
+  int pidx, K, c_in, c_out, smc;
 };
 
 // one VGG or residual block, a -> b channels
@@ -88,6 +93,9 @@ struct BlockBufs {
   float *A, *s1;       // first BatchNorm's output (operand form) and its save_mean | save_invstd ([2][a])
   float *H, *A2, *s2;  // residual: first SMC's output, second BatchNorm's output (operand form), its save
   float* out;          // [n, b]
+  // backward: gradients w.r.t. A, A2, H (operand form), the NetworkInNetwork's input, and the block's input (operand
+  // form; the level's d_X for its first pre block, none for its first post block, which writes d_J and d_F)
+  float *d_A, *d_A2, *d_H, *d_S, *d_x;
 };
 
 struct LevelBufs {
@@ -95,7 +103,11 @@ struct LevelBufs {
   float* Jop;           // NiN shortcut: J in operand form (== J in FP32 mode)
   float *s_dn, *s_up;   // BN save_mean | save_invstd ([2][C])
   void* id_plan;        // NiN shortcut: identity row plan of the level's rows (capacity n)
+  int dn, up;           // first parameter slot of the down and the up branch (BatchNorm, then the convolution at + 4)
   std::vector<BlockBufs> pre, post;
+  // backward: gradients w.r.t. J ([n, 2p]; a split join writes only its skip half, [n, p]), F, Y (skip + branch),
+  // E, R_{l+1} and X_{l+1} (all three of the next level's rows), and B.  All but d_J, d_E and d_B in operand form.
+  float *d_J, *d_F, *d_Yskip, *d_E, *d_Rn, *d_Xn, *d_B;
 };
 
 struct Net {
@@ -105,6 +117,17 @@ struct Net {
   std::vector<LevelMeta> lv;
   std::vector<LevelBufs> b;
   float *V, *Vp, *Z, *s_head;
+  float *d_Z, *d_R0, *d_X0, *d_Vp;        // backward: gradients w.r.t. Z, R_0, X_0 (operand form) and Vp
+  float *d_wp = nullptr, *d_V = nullptr;  // backward, padded stem input only: gradients w.r.t. wp and V
+  int head, n_params;                     // the head BatchNorm's first parameter slot; the number of slots
+  std::vector<ConvInfo> convs;            // every convolution, in slot order
+  size_t bn_channels = 0;                 // of all BatchNorms (each has a gamma and a beta gradient)
+  // The scratch buffer: [convolution workspace | weight images | BatchNorm workspace | padded stem weight].  Weight
+  // images (tensor-core modes): every layer's, for this call's direction, built by one launch up front.  BatchNorm
+  // workspace: totals and barrier counters, zeroed at the start of each call; the kernels keep it clean.
+  void *conv_ws, *img_ws, *bn_ws;
+  size_t conv_ws_bytes, img_ws_bytes, bn_ws_bytes;
+  float* wp;  // the stem weight with zeros for the padded input channels (cin_k != cin only)
   int64_t n_points;
   int planes(int l) const { return m * (l + 1); }
   // TF32x3 mode: every tensor a convolution gathers carries a hi and a lo plane ([rows, c] floats each)
@@ -116,83 +139,145 @@ struct Net {
   bool x3() const { return mode == MM3D_MODE_TF32X3; }
   bool bf16() const { return mode == MM3D_MODE_BF16; }
   bool nin(int a, int b) const { return res && a != b; }
-  int block_slots(int a, int b) const { return res ? (nin(a, b) ? 11 : 10) : 5; }
 };
 
-// parameter slots of level l and everything below it
-int level_slots(const Net& net, int l) {
-  const int p = net.planes(l);
-  int s = net.reps * net.block_slots(p, p);
-  if (l + 1 < net.L) s += 5 + level_slots(net, l + 1) + 5 + net.block_slots(2 * p, p) + (net.reps - 1) * net.block_slots(p, p);
-  return s;
-}
-// first slot of level l (the stem weight is slot 0)
-int level_base(const Net& net, int l) {
-  int base = 1;
-  for (int i = 0; i < l; ++i) base += net.reps * net.block_slots(net.planes(i), net.planes(i)) + 5;
-  return base;
-}
-// first slot of level l's post blocks
-int post_base(const Net& net, int l) {
-  return level_base(net, l) + net.reps * net.block_slots(net.planes(l), net.planes(l)) + 5 + level_slots(net, l + 1) + 5;
-}
+// One walk over the module tree, in its order: it assigns the parameter slots with a running counter, lists the
+// convolutions, counts the BatchNorm channels, and carves the activations out of `act` and the backward temporaries
+// out of `tmp`.  A NULL base only sizes (the queries, and `tmp` in the forward).
+struct Carve {
+  Net& net;
+  Bump &act, &tmp;
+  int pi = 0;  // next parameter slot
 
-BlockBufs carve_block(const Net& net, Bump& bp, int64_t n, int a, int b, int pidx, float* out) {
-  BlockBufs k{};
-  k.a = a; k.b = b; k.pidx = pidx;
-  k.A = bp.f(n, (int64_t)a * net.pl());
-  k.s1 = bp.f(2, a);
-  if (net.res) {
-    k.H = bp.f(n, b);
-    k.A2 = bp.f(n, (int64_t)b * net.pl());
-    k.s2 = bp.f(2, b);
+  int bn(int ch) {
+    net.bn_channels += ch;
+    pi += 4;  // gamma, beta, running mean, running var
+    return pi - 4;
   }
-  k.out = out ? out : bp.f(n, b);
-  return k;
-}
+  void conv(int K, int c_in, int c_out, int smc) { net.convs.push_back({pi++, K, c_in, c_out, smc}); }
 
-// the same carving in forward, backward and the size query
-void carve(Net& net, Bump& bp) {
-  const int64_t n0 = net.lv[0].n;
-  net.V = bp.f(n0, net.cin);
-  const int pl = net.pl();
-  net.Vp = (net.cin_k != net.cin || pl == 2) ? bp.f(n0, (int64_t)net.cin_k * pl) : net.V;
-  net.b.assign(net.L, LevelBufs());
-  for (int l = 0; l < net.L; ++l) {
-    const int64_t n = net.lv[l].n;
-    const int p = net.planes(l);
-    LevelBufs& B = net.b[l];
-    B.X = bp.f(n, p);
-    int pidx = level_base(net, l);
-    for (int r = 0; r < net.reps; ++r, pidx += net.block_slots(p, p))
-      B.pre.push_back(carve_block(net, bp, n, p, p, pidx, nullptr));
-    B.Y = B.pre.back().out;
-    if (l + 1 < net.L) {
-      const int q = net.planes(l + 1);
-      B.B = bp.f(n, (int64_t)p * pl);
-      B.s_dn = bp.f(2, p);
-      B.E = bp.f(net.lv[l + 1].n, (int64_t)q * pl);
-      B.s_up = bp.f(2, q);
-      B.F = bp.f(n, p);
-      B.J = bp.f(n, 2 * p);
-      B.Jop = B.J;
-      if (net.nin(2 * p, p)) {
-        if (net.mode != MM3D_MODE_FP32) B.Jop = bp.f(n, (int64_t)2 * p * pl);
-        B.id_plan = bp.bytes(mm3d_plan_size(n, 1));
-      }
-      pidx = post_base(net, l);
-      for (int r = 0; r < net.reps; ++r) {
-        const int a = r == 0 ? 2 * p : p;
-        B.post.push_back(carve_block(net, bp, n, a, p, pidx, nullptr));
-        pidx += net.block_slots(a, p);
-      }
-      B.R = B.post.back().out;
-    } else {
-      B.R = B.Y;
+  BlockBufs block(int64_t n, int a, int b) {
+    const int pl = net.pl();
+    BlockBufs k{};
+    k.a = a; k.b = b; k.pidx = pi;
+    if (net.nin(a, b)) {
+      conv(1, a, b, 0);
+      k.d_S = tmp.f(n, a);
     }
+    bn(a);
+    conv(27, a, b, 1);
+    k.A = act.f(n, (int64_t)a * pl);
+    k.s1 = act.f(2, a);
+    k.d_A = tmp.f(n, a);
+    if (net.res) {
+      bn(b);
+      conv(27, b, b, 1);
+      k.H = act.f(n, b);
+      k.A2 = act.f(n, (int64_t)b * pl);
+      k.s2 = act.f(2, b);
+      k.d_A2 = tmp.f(n, b);
+      k.d_H = tmp.f(n, (int64_t)b * pl);
+    }
+    k.out = act.f(n, b);
+    return k;
   }
-  net.Z = bp.f(n0, net.m);
-  net.s_head = bp.f(2, net.m);
+
+  // level l; d_X: the gradient w.r.t. its input X_l, carved by the caller
+  void level(int l, float* d_X) {
+    const int64_t n = net.lv[l].n;
+    const int p = net.planes(l), pl = net.pl();
+    LevelBufs& B = net.b[l];
+    B.X = act.f(n, p);
+    for (int r = 0; r < net.reps; ++r) {
+      B.pre.push_back(block(n, p, p));
+      B.pre.back().d_x = r ? tmp.f(n, (int64_t)p * pl) : d_X;
+    }
+    B.Y = B.pre.back().out;
+    if (l + 1 == net.L) {
+      B.R = B.Y;
+      return;
+    }
+    const int q = net.planes(l + 1);
+    const int64_t nc = net.lv[l + 1].n;
+    B.dn = bn(p);
+    conv(8, p, q, 0);
+    B.B = act.f(n, (int64_t)p * pl);
+    B.s_dn = act.f(2, p);
+    B.d_B = tmp.f(n, p);
+    B.d_Xn = tmp.f(nc, (int64_t)q * pl);
+    level(l + 1, B.d_Xn);
+    B.up = bn(q);
+    conv(8, q, p, 0);
+    B.E = act.f(nc, (int64_t)q * pl);
+    B.s_up = act.f(2, q);
+    B.d_Rn = tmp.f(nc, (int64_t)q * pl);
+    B.d_E = tmp.f(nc, q);
+    B.F = act.f(n, p);
+    B.J = act.f(n, 2 * p);
+    B.Jop = B.J;
+    if (net.nin(2 * p, p)) {
+      if (net.mode != MM3D_MODE_FP32) B.Jop = act.f(n, (int64_t)2 * p * pl);
+      B.id_plan = act.bytes(mm3d_plan_size(n, 1));
+    }
+    B.d_J = tmp.f(n, 2 * p);
+    B.d_F = tmp.f(n, (int64_t)p * pl);
+    B.d_Yskip = tmp.f(n, (int64_t)p * pl);
+    for (int r = 0; r < net.reps; ++r) {
+      B.post.push_back(block(n, r ? p : 2 * p, p));
+      if (r) B.post.back().d_x = tmp.f(n, (int64_t)p * pl);
+    }
+    B.R = B.post.back().out;
+  }
+
+  void run() {
+    const int64_t n0 = net.lv[0].n;
+    const int pl = net.pl();
+    net.V = act.f(n0, net.cin);
+    net.Vp = (net.cin_k != net.cin || pl == 2) ? act.f(n0, (int64_t)net.cin_k * pl) : net.V;
+    net.d_Vp = tmp.f(n0, net.cin_k);
+    if (net.cin_k != net.cin) {
+      net.d_V = tmp.f(n0, net.cin);
+      net.d_wp = tmp.f(27, (int64_t)net.cin_k * net.m);
+    }
+    conv(27, net.cin_k, net.m, 1);  // the stem
+    net.d_X0 = tmp.f(n0, (int64_t)net.m * pl);
+    net.b.assign(net.L, LevelBufs());
+    level(0, net.d_X0);
+    net.head = bn(net.m);
+    net.n_params = pi;
+    net.Z = act.f(n0, net.m);
+    net.s_head = act.f(2, net.m);
+    net.d_Z = tmp.f(n0, net.m);
+    net.d_R0 = tmp.f(n0, (int64_t)net.m * pl);
+  }
+};
+
+// the region of the weight images: the larger direction's images, twice in TF32x3 mode (hi and lo)
+size_t img_region_bytes(const Net& net) {
+  if (net.mode == MM3D_MODE_FP32) return 0;
+  size_t fwd = 0, bwd = 0;
+  for (const ConvInfo& ci : net.convs) {  // (0 bytes for a shape the tensor cores do not take)
+    fwd += mm3d_align(mm3d_conv_tc_workspace_bytes(ci.c_in, ci.c_out, ci.K));
+    bwd += mm3d_align(mm3d_conv_tc_workspace_bytes(ci.c_out, ci.c_in, ci.K));
+  }
+  return (fwd > bwd ? fwd : bwd) * (net.x3() ? 2 : 1);
+}
+
+// the layout of the scratch buffer (after the walk: it needs the convolution list), the same in forward, backward and
+// the size query
+void carve_scratch(Net& net, Bump& bp) {
+  size_t conv = 0;
+  for (const ConvInfo& ci : net.convs) {
+    const size_t s = mm3d_conv_workspace_bytes(0, 0, ci.c_in, ci.c_out, ci.K, net.mode);  // (covers dgrad and wgrad)
+    if (s > conv) conv = s;
+  }
+  net.conv_ws_bytes = conv;
+  net.conv_ws = bp.bytes(conv);
+  net.img_ws_bytes = img_region_bytes(net);
+  net.img_ws = bp.bytes(net.img_ws_bytes);
+  net.bn_ws_bytes = mm3d_bnrelu_workspace_bytes(2 * net.m * net.L);
+  net.bn_ws = bp.bytes(net.bn_ws_bytes);
+  net.wp = net.cin_k != net.cin ? bp.f(27, (int64_t)net.cin_k * net.m) : nullptr;
 }
 
 // Identity row plans (NetworkInNetwork as a K = 1 rule-table convolution): perm = iota (-1 past the rows), one
@@ -326,19 +411,12 @@ struct Ctx {
   Net* net;
   void* const* params;
   void* const* grads;  // backward only
-  void* scratch;
-  size_t scratch_bytes;
   cudaStream_t stream;
   float eps, momentum;
   int training;
-  int pi;  // running parameter index
   int rc;
   SideStream* side = nullptr;  // backward only; NULL = everything on `stream`
-  void* bn_ws = nullptr;       // BatchNorm totals + barrier counters: zeroed once per call, the kernels keep it clean
-  size_t bn_ws_bytes = 0;
-  // tensor-core modes: the weight images of all layers of this direction, built by one launch up front
-  void* img_ws = nullptr;
-  size_t img_ws_bytes = 0;
+  int bn_parity = 0;  // which half of bn_ws the BatchNorms of this call alternate to (bnrelu.cu); bn_ws is zeroed first
   const char *grad_lo = nullptr, *grad_hi = nullptr;  // span of the caller's gradient buffers when contiguous
   int wgrad_acc = 0;  // 1: the weight-gradient buffers were zeroed by one memset up front, wgrad kernels accumulate
   std::vector<const float*> img_key;  // weight pointer ...
@@ -408,7 +486,7 @@ void bn_fwd(Ctx& c, int pidx, const float* x, float* y, int64_t n, int ch, float
             int c_lo = 0, bool to_conv = true) {
   if (abl_skip("bn")) return;
   EX(mm3d_bnrelu_fwd_impl(x, x_hi, c_lo, y, n, ch, P(c, pidx), P(c, pidx + 1), (float*)c.params[pidx + 2], (float*)c.params[pidx + 3],
-                          save, save + ch, c.eps, c.momentum, 0.f, c.training, c.bn_ws, c.bn_ws_bytes, true,
+                          save, save + ch, c.eps, c.momentum, 0.f, c.training, c.net->bn_ws, c.net->bn_ws_bytes, &c.bn_parity,
                           tc_mode(c) && to_conv ? c.net->rmode() : 0, c.stream));
 }
 // round: bit 0 = dx (its low column block when split) feeds a convolution as d_out, bit 1 = dx_hi does
@@ -420,7 +498,7 @@ void bn_bwd(Ctx& c, int pidx, const float* x, const float* dy, float* dx, int64_
   if (abl_skip("bn")) return;
   const int flags = tc_mode(c) ? (round | (c.net->x3() ? 4 : c.net->bf16() ? 8 : 0) | (add_lo ? 16 : 0)) : 0;
   EX(mm3d_bnrelu_bwd_impl(x, x_hi, c_lo, dy, dx, dx_hi, n, ch, P(c, pidx), P(c, pidx + 1), save, save + ch, Gp(c, pidx), Gp(c, pidx + 1), 0.f,
-                          c.training, c.bn_ws, c.bn_ws_bytes, true, flags, add, add_ld, c.stream));
+                          c.training, c.net->bn_ws, c.net->bn_ws_bytes, &c.bn_parity, flags, add, add_ld, c.stream));
 }
 // NIN: NetworkInNetwork, a K = 1 convolution over the level's identity row plan
 enum Kind { SMC, DOWN, UP, NIN };
@@ -490,11 +568,11 @@ void conv_fwd(Ctx& c, Kind kind, int l, const float* in, int c_in, float* out, i
       if (c.rc == 0) c.rc = MM3D_ERR_UNSUPPORTED;
       return;
     }
-    EX(mm3d_conv_fwd_simt(in, t.n_in, c_in, out, t.n_out, c_out, w, t.K, t.tbl, t.stride, t.onehot, 0, c.scratch,
-                          c.scratch_bytes, c.stream, add));
+    EX(mm3d_conv_fwd_simt(in, t.n_in, c_in, out, t.n_out, c_out, w, t.K, t.tbl, t.stride, t.onehot, 0, c.net->conv_ws,
+                          c.net->conv_ws_bytes, c.stream, add));
   } else
     EX(mm3d_conv_fwd(in, t.n_in, c_in, out, t.n_out, c_out, w, t.K, t.tbl, t.stride, t.onehot, t.plan, t.cap, 0,
-                     c.net->mode, c.scratch, c.scratch_bytes, c.stream));
+                     c.net->mode, c.net->conv_ws, c.net->conv_ws_bytes, c.stream));
 }
 // dgrad (d_in from d_out) and wgrad of the same layer; c_in / c_out are the FORWARD layer's
 void conv_bwd(Ctx& c, Kind kind, int l, const float* in, int c_in, const float* d_out, int c_out, const float* w,
@@ -517,7 +595,8 @@ void conv_bwd(Ctx& c, Kind kind, int l, const float* in, int c_in, const float* 
     EX(conv_img(c, d_out, t.n_out, c_out, d_in, t.n_in, c_in, im, il, t.K, tt.plan, tt.cap));
   else if (do_dg)
     EX(mm3d_conv_fwd(d_out, t.n_out, c_out, d_in, t.n_in, c_in, w, t.K, tt.tbl, tt.stride, tt.onehot, tt.plan, tt.cap,
-                     MM3D_CONV_TRANSPOSE_W | (kind == SMC ? MM3D_CONV_MIRROR_K : 0), md, c.scratch, c.scratch_bytes, c.stream));
+                     MM3D_CONV_TRANSPOSE_W | (kind == SMC ? MM3D_CONV_MIRROR_K : 0), md, c.net->conv_ws, c.net->conv_ws_bytes,
+                     c.stream));
 }
 
 // main stream waits for everything enqueued on the side stream so far
@@ -554,63 +633,19 @@ void launch_join(Ctx& c, const float* y, const float* f, int64_t n, int p, float
   }
 }
 
-struct ConvInfo {
-  int pidx, K, c_in, c_out, smc;
-};
-void list_block_convs(const Net& net, const BlockBufs& k, std::vector<ConvInfo>& v) {
-  if (!net.res) {
-    v.push_back({k.pidx + 4, 27, k.a, k.b, 1});
-    return;
-  }
-  const int o = net.nin(k.a, k.b) ? 1 : 0;
-  if (o) v.push_back({k.pidx, 1, k.a, k.b, 0});
-  v.push_back({k.pidx + o + 4, 27, k.a, k.b, 1});
-  v.push_back({k.pidx + o + 9, 27, k.b, k.b, 1});
-}
-// every convolution of the network below level l, in slot order (the blocks' slots come from `carve`, which
-// needs no buffers: a shape-only Net carved with a NULL base works)
-void list_convs(const Net& net, int l, std::vector<ConvInfo>& v) {
-  const LevelBufs& B = net.b[l];
-  for (const BlockBufs& k : B.pre) list_block_convs(net, k, v);
-  if (l + 1 < net.L) {
-    const int p = net.planes(l), q = net.planes(l + 1);
-    const int dn = B.pre.back().pidx + net.block_slots(p, p), up = post_base(net, l) - 5;
-    v.push_back({dn + 4, 8, p, q, 0});
-    list_convs(net, l + 1, v);
-    v.push_back({up + 4, 8, q, p, 0});
-    for (const BlockBufs& k : B.post) list_block_convs(net, k, v);
-  }
-}
-std::vector<ConvInfo> all_convs(const Net& net, int cin) {
-  std::vector<ConvInfo> v;
-  v.push_back({0, 27, cin, net.m, 1});
-  list_convs(net, 0, v);
-  return v;
-}
-
-size_t img_region_bytes(const Net& net) {
-  if (net.mode == MM3D_MODE_FP32) return 0;
-  size_t fwd = 0, bwd = 0;
-  for (const ConvInfo& ci : all_convs(net, net.cin_k)) {
-    fwd += mm3d_align(mm3d_conv_tc_workspace_bytes(ci.c_in, ci.c_out, ci.K));
-    bwd += mm3d_align(mm3d_conv_tc_workspace_bytes(ci.c_out, ci.c_in, ci.K));
-  }
-  return (fwd > bwd ? fwd : bwd) * (size_t)net.pl() + 256;
-}
-
 // One launch builds the weight images of every layer for this direction (dgrad: W^T, mirrored for 3^3 layers).
 int build_images(Ctx& c, bool backward, const float* w_stem) {
   const Net& net = *c.net;
-  if (net.mode == MM3D_MODE_FP32 || !c.img_ws) return MM3D_OK;
+  if (net.mode == MM3D_MODE_FP32) return MM3D_OK;
   std::vector<const float*> w;
   std::vector<float*> img;
   std::vector<int> K, ci, co, fl;
-  char* at = (char*)c.img_ws;
-  for (const ConvInfo& x : all_convs(net, net.cin_k)) {
+  char* at = (char*)net.img_ws;
+  for (const ConvInfo& x : net.convs) {
     const int a = backward ? x.c_out : x.c_in, b = backward ? x.c_in : x.c_out;
     if (!mm3d_conv_tc_supported(a, b, x.K)) continue;
     const size_t bytes = mm3d_align(mm3d_conv_tc_workspace_bytes(a, b, x.K));
-    MM3D_REQUIRE((size_t)(at - (char*)c.img_ws) + bytes <= c.img_ws_bytes, MM3D_ERR_WORKSPACE, "weight image region too small");
+    MM3D_REQUIRE((size_t)(at - (char*)net.img_ws) + bytes <= net.img_ws_bytes, MM3D_ERR_WORKSPACE, "weight image region too small");
     w.push_back(x.pidx == 0 ? w_stem : (const float*)c.params[x.pidx]);
     img.push_back((float*)at);
     K.push_back(x.K); ci.push_back(a); co.push_back(b);
@@ -626,7 +661,7 @@ int build_images(Ctx& c, bool backward, const float* w_stem) {
     std::vector<float*> lo;
     for (size_t i = 0; i < w.size(); ++i) {
       const size_t bytes = mm3d_align(mm3d_conv_tc_workspace_bytes(ci[i], co[i], K[i]));
-      MM3D_REQUIRE((size_t)(at - (char*)c.img_ws) + bytes <= c.img_ws_bytes, MM3D_ERR_WORKSPACE, "weight image region too small");
+      MM3D_REQUIRE((size_t)(at - (char*)net.img_ws) + bytes <= net.img_ws_bytes, MM3D_ERR_WORKSPACE, "weight image region too small");
       lo.push_back((float*)at);
       at += bytes;
       fl[i] |= MM3D_CONV_WEIGHT_LO;
@@ -708,47 +743,40 @@ void level_fwd(Ctx& c, int l) {
   }
   if (l + 1 < net.L) {
     const int q = net.planes(l + 1);
-    const int dn = B.pre.back().pidx + net.block_slots(p, p), up = post_base(net, l) - 5;
-    bn_fwd(c, dn, B.Y, B.B, n, p, B.s_dn);
+    bn_fwd(c, B.dn, B.Y, B.B, n, p, B.s_dn);
     MARK("bn_fwd dn", l);
-    conv_fwd(c, DOWN, l, B.B, p, net.b[l + 1].X, q, P(c, dn + 4));
+    conv_fwd(c, DOWN, l, B.B, p, net.b[l + 1].X, q, P(c, B.dn + 4));
     MARK("down_fwd", l);
     level_fwd(c, l + 1);
-    bn_fwd(c, up, net.b[l + 1].R, B.E, net.lv[l + 1].n, q, B.s_up);
+    bn_fwd(c, B.up, net.b[l + 1].R, B.E, net.lv[l + 1].n, q, B.s_up);
     MARK("bn_fwd up", l);
-    conv_fwd(c, UP, l, B.E, q, B.F, p, P(c, up + 4));
+    conv_fwd(c, UP, l, B.E, q, B.F, p, P(c, B.up + 4));
     MARK("up_fwd", l);
     for (size_t r = 0; r < B.post.size(); ++r) block_fwd(c, l, B.post[r], r ? B.post[r - 1].out : nullptr, r == 0);
   }
 }
 
-// A block's backward.  d_o: gradient w.r.t. its output (operand form); writes d_x, the gradient w.r.t. its input,
+// A block's backward.  d_o: gradient w.r.t. its output (operand form); writes k.d_x, the gradient w.r.t. its input,
 // in operand form.  The first post block (join) instead writes the skip half d_J[:, :p] (unrounded; all of d_J
 // when the join is not split) and d_F, the deconvolution's d_out (operand form).
-void block_bwd(Ctx& c, Bump& g, int l, const BlockBufs& k, const float* x, const float* d_o, float* d_x, bool join,
-               float* d_J = nullptr, float* d_F = nullptr) {
+void block_bwd(Ctx& c, int l, const BlockBufs& k, const float* x, const float* d_o, bool join) {
   Net& net = *c.net;
   LevelBufs& B = net.b[l];
   const int64_t n = net.lv[l].n;
-  const int pl = net.pl();
   const int o = net.nin(k.a, k.b) ? 1 : 0;
   const int bn1 = k.pidx + o;
   const float* add = nullptr;  // the shortcut's gradient, summed into the first BatchNorm's backward
   int64_t add_ld = 0;
   bool add_lo = false;
-  float* d_A = g.f(n, k.a);
   if (!net.res) {
-    conv_bwd(c, SMC, l, k.A, k.a, d_o, k.b, P(c, k.pidx + 4), d_A, Gp(c, k.pidx + 4));
+    conv_bwd(c, SMC, l, k.A, k.a, d_o, k.b, P(c, k.pidx + 4), k.d_A, Gp(c, k.pidx + 4));
   } else {
-    float* d_A2 = g.f(n, k.b);
-    conv_bwd(c, SMC, l, k.A2, k.b, d_o, k.b, P(c, bn1 + 9), d_A2, Gp(c, bn1 + 9));
-    float* d_H = g.f(n, (int64_t)k.b * pl);
-    bn_bwd(c, bn1 + 5, k.H, d_A2, d_H, n, k.b, k.s2, 1);
-    conv_bwd(c, SMC, l, k.A, k.a, d_H, k.b, P(c, bn1 + 4), d_A, Gp(c, bn1 + 4));
+    conv_bwd(c, SMC, l, k.A2, k.b, d_o, k.b, P(c, bn1 + 9), k.d_A2, Gp(c, bn1 + 9));
+    bn_bwd(c, bn1 + 5, k.H, k.d_A2, k.d_H, n, k.b, k.s2, 1);
+    conv_bwd(c, SMC, l, k.A, k.a, k.d_H, k.b, P(c, bn1 + 4), k.d_A, Gp(c, bn1 + 4));
     if (o) {
-      float* d_S = g.f(n, k.a);
-      conv_bwd(c, NIN, l, B.Jop, k.a, d_o, k.b, P(c, k.pidx), d_S, Gp(c, k.pidx));
-      add = d_S;
+      conv_bwd(c, NIN, l, B.Jop, k.a, d_o, k.b, P(c, k.pidx), k.d_S, Gp(c, k.pidx));
+      add = k.d_S;
       add_ld = k.a;
     } else {  // identity: d_o itself, FP32-exact in TF32x3 mode through its lo plane
       add = d_o;
@@ -758,74 +786,59 @@ void block_bwd(Ctx& c, Bump& g, int l, const BlockBufs& k, const float* x, const
   }
   MARK("block conv bwd", l);
   if (!join) {
-    bn_bwd(c, bn1, x, d_A, d_x, n, k.a, k.s1, 1, nullptr, 0, nullptr, add, add_ld, add_lo);
+    bn_bwd(c, bn1, x, k.d_A, k.d_x, n, k.a, k.s1, 1, nullptr, 0, nullptr, add, add_ld, add_lo);
     MARK("bn_bwd block", l);
     return;
   }
   const int p = k.b;
   if ((p & 3) == 0 && c.training) {  // as in the forward: [Y | F] was never concatenated
-    bn_bwd(c, bn1, B.Y, d_A, d_J, n, 2 * p, k.s1, 2, B.F, p, d_F, add, add_ld);  // d_F is the deconvolution's d_out
+    bn_bwd(c, bn1, B.Y, k.d_A, B.d_J, n, 2 * p, k.s1, 2, B.F, p, B.d_F, add, add_ld);  // d_F is the deconvolution's d_out
   } else {
-    bn_bwd(c, bn1, B.J, d_A, d_J, n, 2 * p, k.s1, 0, nullptr, 0, nullptr, add, add_ld);  // (eval-mode backward: d_F stays unrounded)
+    bn_bwd(c, bn1, B.J, k.d_A, B.d_J, n, 2 * p, k.s1, 0, nullptr, 0, nullptr, add, add_ld);  // (eval-mode backward: d_F stays unrounded)
     // d_F = d_J[:, p:]; the skip half is combined with the branch gradient further down
     if (n && !c.rc) {
-      if (mm3d_launch_pdl(k_copy_cols, dim3(mm3d_grid(n * p / 4 + 1, 256)), dim3(256), 0, c.stream, (const float*)d_J, n, 2 * p, d_F, p, 0, p, p) != cudaSuccess) c.rc = MM3D_ERR_CUDA;
+      if (mm3d_launch_pdl(k_copy_cols, dim3(mm3d_grid(n * p / 4 + 1, 256)), dim3(256), 0, c.stream, (const float*)B.d_J, n, 2 * p, B.d_F, p, 0, p, p) != cudaSuccess) c.rc = MM3D_ERR_CUDA;
       mm3d_count_launches(1);
-      if (tc_mode(c)) launch_pad_cols(c, d_F, n, p, d_F, p, net.rmode());  // round in place (+ second plane): d_F is the deconvolution's d_out
+      if (tc_mode(c)) launch_pad_cols(c, B.d_F, n, p, B.d_F, p, net.rmode());  // round in place (+ second plane): d_F is the deconvolution's d_out
     }
   }
   MARK("bn_bwd post", l);
 }
 
-// d_R: gradient w.r.t. the level's output R_l (operand form); returns (in d_X) the gradient w.r.t. X_l.
-// Gradient temporaries come from the backward bump allocator `g`.
-void level_bwd(Ctx& c, Bump& g, int l, const float* d_R, float* d_X) {
+// d_R: gradient w.r.t. the level's output R_l (operand form); writes the gradient w.r.t. X_l, B.pre[0].d_x.
+void level_bwd(Ctx& c, int l, const float* d_R) {
   Net& net = *c.net;
   LevelBufs& B = net.b[l];
   const int64_t n = net.lv[l].n;
   const int p = net.planes(l);
-  const int pl = net.pl();  // conv d_out tensors carry a second plane in the TF32x3 and BF16 modes
   const float* d_Y = d_R;
-  const size_t mark = g.off;
   if (l + 1 < net.L) {
     const int q = net.planes(l + 1);
     const int64_t nc = net.lv[l + 1].n;
-    const int dn = B.pre.back().pidx + net.block_slots(p, p), up = post_base(net, l) - 5;
     const float* d_o = d_R;
     for (size_t r = B.post.size() - 1; r >= 1; --r) {
-      float* d_x = g.f(n, (int64_t)p * pl);
-      block_bwd(c, g, l, B.post[r], B.post[r - 1].out, d_o, d_x, false);
-      d_o = d_x;
+      block_bwd(c, l, B.post[r], B.post[r - 1].out, d_o, false);
+      d_o = B.post[r].d_x;
     }
-    const bool split = (p & 3) == 0 && c.training;
-    float* d_J = g.f(n, split ? p : 2 * p);  // split: only the skip half d_J[:, :p]
-    float* d_F = g.f(n, (int64_t)p * pl);
-    float* d_Yskip = g.f(n, (int64_t)p * pl);
-    block_bwd(c, g, l, B.post[0], nullptr, d_o, nullptr, true, d_J, d_F);
-    float* d_E = g.f(nc, q);
-    conv_bwd(c, UP, l, B.E, q, d_F, p, P(c, up + 4), d_E, Gp(c, up + 4));
+    block_bwd(c, l, B.post[0], nullptr, d_o, true);
+    conv_bwd(c, UP, l, B.E, q, B.d_F, p, P(c, B.up + 4), B.d_E, Gp(c, B.up + 4));
     MARK("up_dgrad", l);
-    float* d_Rn = g.f(nc, (int64_t)q * pl);
-    bn_bwd(c, up, net.b[l + 1].R, d_E, d_Rn, nc, q, B.s_up, 1);
+    bn_bwd(c, B.up, net.b[l + 1].R, B.d_E, B.d_Rn, nc, q, B.s_up, 1);
     MARK("bn_bwd up", l);
-    float* d_Xn = g.f(nc, (int64_t)q * pl);
-    level_bwd(c, g, l + 1, d_Rn, d_Xn);
-    float* d_B = g.f(n, p);
-    conv_bwd(c, DOWN, l, B.B, p, d_Xn, q, P(c, dn + 4), d_B, Gp(c, dn + 4));
+    level_bwd(c, l + 1, B.d_Rn);
+    conv_bwd(c, DOWN, l, B.B, p, B.d_Xn, q, P(c, B.dn + 4), B.d_B, Gp(c, B.dn + 4));
     MARK("down_dgrad", l);
     // d_Y = d_J[:, :p] (the skip half of the join's gradient) + the branch gradient: summed inside the BatchNorm
     // backward of the down-branch, stored rounded (it is the pre-block convolution's d_out)
-    bn_bwd(c, dn, B.Y, d_B, d_Yskip, n, p, B.s_dn, 1, nullptr, 0, nullptr, d_J, split ? p : 2 * p);
+    const bool split = (p & 3) == 0 && c.training;
+    bn_bwd(c, B.dn, B.Y, B.d_B, B.d_Yskip, n, p, B.s_dn, 1, nullptr, 0, nullptr, B.d_J, split ? p : 2 * p);
     MARK("bn_bwd dn", l);
-    d_Y = d_Yskip;
+    d_Y = B.d_Yskip;
   }
   for (size_t r = B.pre.size(); r-- > 0;) {
-    float* d_x = r ? g.f(n, (int64_t)p * pl) : d_X;
-    block_bwd(c, g, l, B.pre[r], r ? B.pre[r - 1].out : B.X, d_Y, d_x, false);
-    d_Y = d_x;
+    block_bwd(c, l, B.pre[r], r ? B.pre[r - 1].out : B.X, d_Y, false);
+    d_Y = B.pre[r].d_x;
   }
-  if (!c.side) g.off = mark;  // temporaries of this level are dead once d_X is written -- unless the side stream
-                              // may still be reading a d_out (the workspace bound assumes no reuse anyway)
 }
 
 int fill_net(Net& net, int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
@@ -849,74 +862,18 @@ int fill_net(Net& net, int in_channels, int m, int num_planes, int block_reps, i
   return MM3D_OK;
 }
 
-size_t bwd_temp_bytes(const Net& net) {
-  // upper bound of the live gradient temporaries along the recursion
-  size_t total = 0;
-  for (int l = 0; l < net.L; ++l) {
-    const size_t n = (size_t)net.lv[l].n, p = (size_t)net.planes(l);
-    const bool deeper = l + 1 < net.L;
-    size_t rows = 0;
-    if (deeper) {
-      const size_t nc = (size_t)net.lv[l + 1].n, q = (size_t)net.planes(l + 1);
-      rows = n * (2 * p + 2 * p + p + p + p + p) + nc * (3 * q);
-    }
-    rows += n * p;
-    // further blocks (d_A + d_x each); residual blocks (d_A2 + d_H each, + the NetworkInNetwork's d_in)
-    const size_t blocks = (size_t)net.reps * (deeper ? 2 : 1);
-    rows += n * (blocks - (deeper ? 2 : 1)) * 2 * p;
-    if (net.res) rows += n * (blocks * 2 * p + (deeper ? 2 * p : 0));
-    total += mm3d_align(sizeof(float) * rows) + 16 * 256 + (blocks - (deeper ? 2 : 1) + (net.res ? 2 * blocks : 0)) * 2 * 256;
-  }
-  const size_t n0 = (size_t)net.lv[0].n;
-  total += mm3d_align(4 * n0 * (size_t)net.m) * 3 + mm3d_align(4 * n0 * (size_t)(net.cin + net.cin_k)) * 2 + 8 * 256;
-  total += mm3d_align(4 * (size_t)27 * net.cin_k * net.m) * 2;
-  return total * (size_t)net.pl();
-}
-
-// number of BatchNorm channels of the whole network (each has a gamma and a beta gradient)
-size_t bn_channels(const Net& net) {
-  size_t ch = (size_t)net.m;  // head
-  for (int l = 0; l < net.L; ++l) {
-    const size_t p = (size_t)net.planes(l);
-    const size_t per_block = net.res ? 2 : 1;  // (the first post block's first BatchNorm has 2p channels)
-    ch += net.reps * per_block * p;
-    if (l + 1 < net.L) ch += p + (size_t)net.planes(l + 1) + net.reps * per_block * p + p;
-  }
-  return ch;
-}
-
-size_t scratch_bytes(const Net& shape) {
-  const int m = shape.m, num_planes = shape.L;
-  size_t best = mm3d_bnrelu_workspace_bytes(2 * m * num_planes);
-  size_t s = mm3d_conv_workspace_bytes(0, 0, shape.cin_k, m, 27, shape.mode);
-  if (s > best) best = s;
-  for (int l = 0; l < num_planes; ++l) {
-    const int p = m * (l + 1);
-    s = mm3d_conv_workspace_bytes(0, 0, 2 * p, p, 27, shape.mode);
-    if (s > best) best = s;
-    s = mm3d_conv_workspace_bytes(0, 0, p + m, p, 8, shape.mode);
-    if (s > best) best = s;
-  }
-  return best + img_region_bytes(shape) + mm3d_bnrelu_workspace_bytes(2 * m * num_planes) +
-         mm3d_align(4 * (size_t)27 * shape.cin_k * m) + 256;
+// What the walk and the scratch layout need of each of the caller's three buffers.  A NULL base only sizes.
+struct Sizes {
+  size_t act, tmp, scratch;
+};
+Sizes lay_out(Net& net, void* act, void* tmp, void* scratch) {
+  Bump a{(char*)act, 0}, t{(char*)tmp, 0}, s{(char*)scratch, 0};
+  Carve{net, a, t}.run();
+  carve_scratch(net, s);
+  return {a.off, t.off, s.off};
 }
 
 }  // namespace
-
-// carve the executor's private tail of the scratch buffer: [... | BatchNorm workspace | padded stem weight]
-static int carve_tail(Ctx& c, const Net& net) {
-  const size_t wp_bytes = mm3d_align(4 * (size_t)27 * net.cin_k * net.m);
-  c.bn_ws_bytes = mm3d_bnrelu_workspace_bytes(2 * net.m * net.L);
-  c.img_ws_bytes = img_region_bytes(net) / 256 * 256;
-  MM3D_REQUIRE(c.scratch_bytes >= wp_bytes + c.bn_ws_bytes + c.img_ws_bytes + 256, MM3D_ERR_WORKSPACE,
-               "unet scratch too small");
-  const size_t end = c.scratch_bytes / 256 * 256;
-  c.bn_ws = (char*)c.scratch + end - wp_bytes - c.bn_ws_bytes;
-  c.img_ws = c.img_ws_bytes ? (char*)c.bn_ws - c.img_ws_bytes : nullptr;
-  c.scratch_bytes = end - wp_bytes - c.bn_ws_bytes - c.img_ws_bytes;  // what the convolutions may use
-  MM3D_CUDA(cudaMemsetAsync(c.bn_ws, 0, c.bn_ws_bytes, c.stream));
-  return MM3D_OK;
-}
 
 extern "C" {
 
@@ -925,7 +882,8 @@ extern "C" {
 MM3D_API int64_t mm3d_unet_topo_num_params(int num_planes, int block_reps, int residual) {
   Net net;
   if (fill_net(net, 1, 1, num_planes, block_reps, residual, MM3D_MODE_FP32, nullptr, 0)) return -1;
-  return 1 + level_slots(net, 0) + 4;
+  lay_out(net, nullptr, nullptr, nullptr);
+  return net.n_params;
 }
 MM3D_API int64_t mm3d_unet_num_params(int num_planes) { return mm3d_unet_topo_num_params(num_planes, 1, 0); }
 
@@ -933,9 +891,7 @@ MM3D_API size_t mm3d_unet_topo_act_bytes(int in_channels, int m, int num_planes,
                                          const int64_t* level_desc, int64_t n_points) {
   Net net;
   if (!level_desc || fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points)) return 0;
-  Bump bp{nullptr, 0, ~(size_t)0, true};
-  carve(net, bp);
-  return bp.off + 256;
+  return lay_out(net, nullptr, nullptr, nullptr).act + 256;
 }
 MM3D_API size_t mm3d_unet_act_bytes(int in_channels, int m, int num_planes, int mode, const int64_t* level_desc,
                                     int64_t n_points) {
@@ -946,7 +902,7 @@ MM3D_API size_t mm3d_unet_topo_bwd_bytes(int in_channels, int m, int num_planes,
                                          const int64_t* level_desc, int64_t n_points) {
   Net net;
   if (!level_desc || fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points)) return 0;
-  return bwd_temp_bytes(net);
+  return lay_out(net, nullptr, nullptr, nullptr).tmp;
 }
 MM3D_API size_t mm3d_unet_bwd_bytes(int in_channels, int m, int num_planes, int mode, const int64_t* level_desc,
                                     int64_t n_points) {
@@ -954,12 +910,9 @@ MM3D_API size_t mm3d_unet_bwd_bytes(int in_channels, int m, int num_planes, int 
 }
 
 MM3D_API size_t mm3d_unet_topo_scratch_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode) {
-  Net shape;
-  if (fill_net(shape, in_channels, m, num_planes, block_reps, residual, mode, nullptr, 0)) return 0;
-  shape.cin_k = (in_channels + 15) / 16 * 16;
-  Bump bp{nullptr, 0, ~(size_t)0, true};
-  carve(shape, bp);  // (block slots for the weight-image list; no buffers)
-  return scratch_bytes(shape);
+  Net net;
+  if (fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, nullptr, 0)) return 0;
+  return lay_out(net, nullptr, nullptr, nullptr).scratch;  // (independent of the row counts)
 }
 MM3D_API size_t mm3d_unet_scratch_bytes(int in_channels, int m, int num_planes, int mode) {
   return mm3d_unet_topo_scratch_bytes(in_channels, m, num_planes, 1, 0, mode);
@@ -971,20 +924,19 @@ MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int 
                                     void* const* params, void* act, size_t act_bytes, void* scratch, size_t scratch_bytes,
                                     const mm3d_unet_mask* mask, mm3d_stream_t stream_) {
   MM3D_REQUIRE(level_desc, MM3D_ERR_INVALID, "unet forward: no level descriptors");
+  MM3D_REQUIRE(!mask || (mask->wb && (n_points == 0 || mask->s)), MM3D_ERR_INVALID, "unet forward: incomplete mask descriptor");
   Net net;
   int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points);
   if (rc) return rc;
-  Bump bp{(char*)act, 0, act_bytes, true};
-  carve(net, bp);
-  MM3D_REQUIRE(bp.ok, MM3D_ERR_WORKSPACE, "activation workspace too small: need %zu have %zu", bp.off, act_bytes);
-  Ctx c{&net, params, nullptr, scratch, scratch_bytes, (cudaStream_t)stream_, eps, momentum, training, 0, 0};
-  float* const wp_buf = (float*)((char*)scratch + scratch_bytes / 256 * 256 - mm3d_align(4 * (size_t)27 * net.cin_k * m));
-  rc = carve_tail(c, net);
-  if (rc) return rc;
+  const Sizes need = lay_out(net, act, nullptr, scratch);  // (no backward temporaries)
+  MM3D_REQUIRE(act_bytes >= need.act, MM3D_ERR_WORKSPACE, "activation workspace too small: need %zu have %zu", need.act, act_bytes);
+  MM3D_REQUIRE(scratch_bytes >= need.scratch, MM3D_ERR_WORKSPACE, "unet scratch too small: need %zu have %zu", need.scratch,
+               scratch_bytes);
+  Ctx c{&net, params, nullptr, (cudaStream_t)stream_, eps, momentum, training, 0};
+  MM3D_CUDA(cudaMemsetAsync(net.bn_ws, 0, net.bn_ws_bytes, c.stream));
   const int64_t n0 = net.lv[0].n;
   MARK("fwd start", -1);
   if (mask) {  // the RGB-mask prologue of Net3DSeg.forward folded into the point -> voxel scatter
-    MM3D_REQUIRE(mask->wb && (n_points == 0 || mask->s), MM3D_ERR_INVALID, "unet forward: incomplete mask descriptor");
     EX(mm3d_input_masked_fwd(feats, p2v, npts, n_points, n0, in_channels, 4, mask->wb, net.V, mask->s, c.stream));
   } else {
     EX(mm3d_input_fwd(feats, p2v, npts, n_points, n0, in_channels, 4, net.V, c.stream));
@@ -999,9 +951,8 @@ MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int 
     mm3d_count_launches(1);
   }
   if (net.cin_k != net.cin) {  // zero input channels for the stem weight too
-    float* wp = wp_buf;
-    launch_pad_cols(c, w_stem, 27, net.cin * m, wp, net.cin_k * m);
-    w_stem = wp;
+    launch_pad_cols(c, w_stem, 27, net.cin * m, net.wp, net.cin_k * m);
+    w_stem = net.wp;
   }
   EX(build_images(c, false, w_stem));
   build_identity_plans(c);  // (kept in `act`: the backward reuses them)
@@ -1009,8 +960,7 @@ MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int 
   conv_fwd(c, SMC, 0, net.Vp, net.cin_k, net.b[0].X, m, w_stem);
   MARK("stem fwd", -1);
   level_fwd(c, 0);
-  const int head = 1 + level_slots(net, 0);
-  bn_fwd(c, head, net.b[0].R, net.Z, n0, m, net.s_head, nullptr, 0, /*to_conv=*/false);
+  bn_fwd(c, net.head, net.b[0].R, net.Z, n0, m, net.s_head, nullptr, 0, /*to_conv=*/false);
   MARK("bn_fwd head", -1);
   EX(mm3d_output_fwd(net.Z, p2v, n_points, m, out, c.stream));
   MARK("output_fwd", -1);
@@ -1033,36 +983,35 @@ MM3D_API int mm3d_unet_topo_backward(int in_channels, int m, int num_planes, int
                                      void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask,
                                      mm3d_stream_t stream_) {
   MM3D_REQUIRE(level_desc, MM3D_ERR_INVALID, "unet backward: no level descriptors");
+  MM3D_REQUIRE(!mask || (mask->wb && mask->d_wb && mask->ws && (n_points == 0 || (mask->s && mask->feats))), MM3D_ERR_INVALID,
+               "unet backward: incomplete mask descriptor");
   Net net;
   int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points);
   if (rc) return rc;
-  Bump bp{(char*)act, 0, act_bytes, true};
-  carve(net, bp);
-  MM3D_REQUIRE(bp.ok, MM3D_ERR_WORKSPACE, "activation workspace too small");
-  MM3D_REQUIRE(tmp_bytes >= bwd_temp_bytes(net), MM3D_ERR_WORKSPACE, "backward workspace too small");
-  Ctx c{&net, params, grads, scratch, scratch_bytes, (cudaStream_t)stream_, 0.f, 0.f, training, 0, 0};
+  const Sizes need = lay_out(net, act, tmp, scratch);
+  MM3D_REQUIRE(act_bytes >= need.act, MM3D_ERR_WORKSPACE, "activation workspace too small: need %zu have %zu", need.act, act_bytes);
+  MM3D_REQUIRE(tmp_bytes >= need.tmp, MM3D_ERR_WORKSPACE, "backward workspace too small: need %zu have %zu", need.tmp, tmp_bytes);
+  MM3D_REQUIRE(scratch_bytes >= need.scratch, MM3D_ERR_WORKSPACE, "unet scratch too small: need %zu have %zu", need.scratch,
+               scratch_bytes);
+  Ctx c{&net, params, grads, (cudaStream_t)stream_, 0.f, 0.f, training, 0};
   c.side = getenv("MM3D_NO_SIDE_STREAM") ? nullptr : side_stream();
-  float* const wp_buf = (float*)((char*)scratch + scratch_bytes / 256 * 256 - mm3d_align(4 * (size_t)27 * net.cin_k * m));
-  rc = carve_tail(c, net);
-  if (rc) return rc;
-  Bump g{(char*)tmp, 0, tmp_bytes, true};
+  MM3D_CUDA(cudaMemsetAsync(net.bn_ws, 0, net.bn_ws_bytes, c.stream));
   const int64_t n0 = net.lv[0].n;
-  const int head = 1 + level_slots(net, 0);
   {  // One memset instead of one per layer when the gradient buffers are one contiguous block (the shipped host
      // code hands out views of one flat tensor): slot sizes follow from the network shape.
     const char *lo = nullptr, *hi = nullptr;
     size_t bytes = 0;
     bool all = true;
-    for (const ConvInfo& x : all_convs(net, net.cin)) {
+    for (const ConvInfo& x : net.convs) {
       const char* g0 = (const char*)grads[x.pidx];
       if (!g0) { all = false; break; }
-      const size_t nb_ = sizeof(float) * (size_t)x.K * x.c_in * x.c_out;
+      const size_t nb_ = sizeof(float) * (size_t)x.K * (x.pidx ? x.c_in : net.cin) * x.c_out;  // (the stem: real channels)
       if (!lo || g0 < lo) lo = g0;
       if (!hi || g0 + nb_ > hi) hi = g0 + nb_;
       bytes += nb_;
     }
     // BatchNorm gradients (2 * channels each) may sit in between: allow the span to be at most their size larger
-    const size_t bn_bytes = sizeof(float) * 2 * bn_channels(net);
+    const size_t bn_bytes = sizeof(float) * 2 * net.bn_channels;
     if (all && lo && (size_t)(hi - lo) <= bytes + bn_bytes) {
       MM3D_CUDA(cudaMemsetAsync((void*)lo, 0, (size_t)(hi - lo), c.stream));
       c.grad_lo = lo; c.grad_hi = hi; c.wgrad_acc = 1;
@@ -1071,28 +1020,22 @@ MM3D_API int mm3d_unet_topo_backward(int in_channels, int m, int num_planes, int
   {  // stem weight as the kernels see it (zero-padded input channels), then every layer's dgrad weight image
     const float* w_stem_k = P(c, 0);
     if (net.cin_k != net.cin) {
-      launch_pad_cols(c, w_stem_k, 27, net.cin * m, wp_buf, net.cin_k * m);
-      w_stem_k = wp_buf;
+      launch_pad_cols(c, w_stem_k, 27, net.cin * m, net.wp, net.cin_k * m);
+      w_stem_k = net.wp;
     }
     EX(build_images(c, true, w_stem_k));
   }
   MARK("bwd start (memset, images)", -1);
-  float* d_Z = g.f(n0, m);
-  EX(mm3d_output_bwd(d_out, p2v, n_points, n0, m, d_Z, c.stream));
+  EX(mm3d_output_bwd(d_out, p2v, n_points, n0, m, net.d_Z, c.stream));
   MARK("output_bwd", -1);
-  float* d_R0 = g.f(n0, (int64_t)m * net.pl());
-  bn_bwd(c, head, net.b[0].R, d_Z, d_R0, n0, m, net.s_head, 1);
+  bn_bwd(c, net.head, net.b[0].R, net.d_Z, net.d_R0, n0, m, net.s_head, 1);
   MARK("bn_bwd head", -1);
-  float* d_X0 = g.f(n0, (int64_t)m * net.pl());
-  level_bwd(c, g, 0, d_R0, d_X0);
+  level_bwd(c, 0, net.d_R0);
   // stem
   const float* w_stem = P(c, 0);
   float* d_w = Gp(c, 0);
-  if (mask)
-    MM3D_REQUIRE(mask->wb && mask->d_wb && mask->ws && (n_points == 0 || (mask->s && mask->feats)), MM3D_ERR_INVALID,
-                 "unet backward: incomplete mask descriptor");
   const bool need_dv = d_feats || mask;  // (the mask parameters get their gradient through the InputLayer)
-  float* d_Vp = need_dv ? g.f(n0, net.cin_k) : nullptr;
+  float* d_Vp = need_dv ? net.d_Vp : nullptr;
   auto input_bwd = [&](const float* d_v) {
     if (mask)
       EX(mm3d_input_masked_bwd(d_v, mask->feats, mask->s, p2v, npts, n_points, net.cin, 4, mask->wb, d_feats, mask->d_wb,
@@ -1101,24 +1044,21 @@ MM3D_API int mm3d_unet_topo_backward(int in_channels, int m, int num_planes, int
       EX(mm3d_input_bwd(d_v, p2v, npts, n_points, net.cin, 4, d_feats, c.stream));
   };
   if (net.cin_k != net.cin) {
-    float* wp = wp_buf;  // padded at the start of this call
-    float* d_wp = d_w ? g.f(27, (int64_t)net.cin_k * m) : nullptr;  // (frozen stem weight: no gradient)
-    conv_bwd(c, SMC, 0, net.Vp, net.cin_k, d_X0, m, wp, d_Vp, d_wp);
+    // (net.wp: padded at the start of this call; frozen stem weight: no gradient)
+    conv_bwd(c, SMC, 0, net.Vp, net.cin_k, net.d_X0, m, net.wp, d_Vp, d_w ? net.d_wp : nullptr);
     join_side(c);  // d_wp comes from the side stream
-    if (d_w) launch_pad_cols(c, d_wp, 27, net.cin_k * m, d_w, net.cin * m);  // slice the real channels back out
+    if (d_w) launch_pad_cols(c, net.d_wp, 27, net.cin_k * m, d_w, net.cin * m);  // slice the real channels back out
     if (need_dv) {
-      float* d_V = g.f(n0, net.cin);
-      launch_pad_cols(c, d_Vp, n0, net.cin_k, d_V, net.cin);
-      input_bwd(d_V);
+      launch_pad_cols(c, d_Vp, n0, net.cin_k, net.d_V, net.cin);
+      input_bwd(net.d_V);
     }
   } else {
-    conv_bwd(c, SMC, 0, net.Vp, net.cin, d_X0, m, w_stem, d_Vp, d_w);
+    conv_bwd(c, SMC, 0, net.Vp, net.cin, net.d_X0, m, w_stem, d_Vp, d_w);
     if (need_dv) input_bwd(d_Vp);
   }
   MARK("stem bwd + input_bwd", -1);
   join_side(c);  // everything after this call on `stream` sees the weight gradients
   MARK("join wgrad stream", -1);
-  MM3D_REQUIRE(g.ok, MM3D_ERR_WORKSPACE, "backward workspace overflow");
   return c.rc;
 }
 
