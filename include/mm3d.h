@@ -249,6 +249,18 @@ MM3D_API int mm3d_conv_wgrad(const float* in, int64_t n_in, int c_in, const floa
                     int c_out, float* d_weight, int K, const int32_t* tbl, int64_t tbl_stride,
                     const uint8_t* onehot_off, const void* plan, int64_t plan_cap, int accumulate, int mode,
                     void* ws, size_t ws_bytes, mm3d_stream_t stream);
+/* flags 0 = mm3d_conv_wgrad (ws unused).  MM3D_DETERMINISTIC (tensor-core modes, shapes the tcgen05 kernels take; else
+ * MM3D_ERR_UNSUPPORTED -- the FP32 mode and an unpadded stem run the SIMT kernel, which has no such form): every CTA
+ * stores its accumulators into its own slab of ws with plain stores, and a second launch adds the slabs of the CTAs
+ * of each offset to d_weight in ascending CTA order.  Which CTAs those are depends on the row plan, the shapes and the
+ * device's SM count, so the bits are the same on every run on one device model.  ws: mm3d_conv_wgrad_workspace_bytes
+ * -- 0 with flags 0, and also 0 (no deterministic form) for the FP32 mode and shapes the tcgen05 kernels do not take;
+ * otherwise at most (SM count) x 256 KB, whatever n_out. */
+MM3D_API size_t mm3d_conv_wgrad_workspace_bytes(int64_t n_out, int c_in, int c_out, int K, int mode, int flags);
+MM3D_API int mm3d_conv_wgrad_ex(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out,
+                       int c_out, float* d_weight, int K, const int32_t* tbl, int64_t tbl_stride,
+                       const uint8_t* onehot_off, const void* plan, int64_t plan_cap, int accumulate, int mode,
+                       void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags);
 
 /* ------------------------------------------------------------------------------------------
  * BatchNorm + (leaky) ReLU over active rows (replaces BatchNormalization_updateOutput/_backward).
@@ -263,6 +275,21 @@ MM3D_API int mm3d_bnrelu_bwd(const float* x, const float* dy, float* dx, int64_t
                     const float* beta, const float* save_mean, const float* save_invstd,
                     float* d_gamma, float* d_beta, float leakiness, int training,
                     void* ws, size_t ws_bytes, mm3d_stream_t stream);
+/* flags 0 = the functions above.  MM3D_DETERMINISTIC: the reductions over rows (batch statistics of the training
+ * forward; d_beta / d_gamma and the terms of dx of every backward) store one FP64 partial row per CTA, and the totals
+ * are summed in a fixed order, so save_mean / save_invstd, the running statistics, y, dx, d_gamma and d_beta are the
+ * same bits on every run.  The grid comes from the occupancy API, the SM count and MM3D_BN_PER_SM: the bits are per
+ * device model and per setting.  ws: mm3d_bnrelu_workspace_bytes_ex(c, flags), sized for the largest grid the current
+ * device can get (flags 0: mm3d_bnrelu_workspace_bytes). */
+MM3D_API size_t mm3d_bnrelu_workspace_bytes_ex(int c, int flags);
+MM3D_API int mm3d_bnrelu_fwd_ex(const float* x, float* y, int64_t n, int c, const float* gamma, const float* beta,
+                       float* running_mean, float* running_var, float* save_mean, float* save_invstd,
+                       float eps, float momentum, float leakiness, int training,
+                       void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags);
+MM3D_API int mm3d_bnrelu_bwd_ex(const float* x, const float* dy, float* dx, int64_t n, int c, const float* gamma,
+                       const float* beta, const float* save_mean, const float* save_invstd,
+                       float* d_gamma, float* d_beta, float leakiness, int training,
+                       void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags);
 
 /* ------------------------------------------------------------------------------------------
  * 2D->3D lift (replaces the per-sample advanced indexing of 2d_net/model.py:131-137):

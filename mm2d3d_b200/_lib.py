@@ -68,9 +68,14 @@ SIGNATURES = {
     "mm3d_split_tf32": (_i, [_p, _p, _i64, _p]),
     "mm3d_split_bf16": (_i, [_p, _p, _i64, _p]),
     "mm3d_conv_wgrad": (_i, [_p, _i64, _i, _p, _i64, _i, _p, _i, _p, _i64, _p, _p, _i64, _i, _i, _p, _sz, _p]),
+    "mm3d_conv_wgrad_workspace_bytes": (_sz, [_i64, _i, _i, _i, _i, _i]),
+    "mm3d_conv_wgrad_ex": (_i, [_p, _i64, _i, _p, _i64, _i, _p, _i, _p, _i64, _p, _p, _i64, _i, _i, _p, _sz, _p, _i]),
     "mm3d_bnrelu_workspace_bytes": (_sz, [_i]),
     "mm3d_bnrelu_fwd": (_i, [_p, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _f, _f, _f, _i, _p, _sz, _p]),
     "mm3d_bnrelu_bwd": (_i, [_p, _p, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _f, _i, _p, _sz, _p]),
+    "mm3d_bnrelu_workspace_bytes_ex": (_sz, [_i, _i]),
+    "mm3d_bnrelu_fwd_ex": (_i, [_p, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _f, _f, _f, _i, _p, _sz, _p, _i]),
+    "mm3d_bnrelu_bwd_ex": (_i, [_p, _p, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _f, _i, _p, _sz, _p, _i]),
     "mm3d_lift2d_fwd": (_i, [_p, _i, _i, _i, _i, _i, _i64, _i64, _i64, _i64, _p, _p, _i64, _p, _p]),
     "mm3d_lift2d_bwd": (_i, [_p, _i, _i, _i, _i, _i, _i64, _i64, _i64, _i64, _p, _p, _i64, _p, _p]),
     "mm3d_lift2d_bilinear_fwd": (_i, [_p, _i, _i, _i, _i, _i, _i64, _i64, _i64, _i64, _p, _p, _i64, _p, _p]),

@@ -78,8 +78,9 @@ extern __shared__ double s_acc[];
 
 // Block reduction of per-thread FP32 partials (VEC channels each, thread layout rows_pass x cv):
 // partials go to shared memory, then one thread per channel sums the rows_pass values in FP64 and
-// issues ONE global FP64 atomic per channel and CTA.
-template <int VEC>
+// issues ONE global FP64 atomic per channel and CTA -- or, deterministic (DET), stores it into this CTA's own row
+// sums[blockIdx.x][2 c].
+template <int VEC, bool DET = false>
 __device__ __forceinline__ void block_flush(const float (&s)[VEC], const float (&q)[VEC], int c, int cv, int rows_pass,
                                             int r, int v, double* __restrict__ sums) {
   float* part = reinterpret_cast<float*>(s_acc);  // [2][rows_pass][c]
@@ -95,7 +96,8 @@ __device__ __forceinline__ void block_flush(const float (&s)[VEC], const float (
     const int which = i >= c, ch = i - which * c;
     double acc = 0.0;
     for (int rr = 0; rr < rows_pass; ++rr) acc += (double)part[(which * rows_pass + rr) * c + ch];
-    atomicAdd(sums + i, acc);
+    if (DET) sums[(int64_t)blockIdx.x * 2 * c + i] = acc;
+    else atomicAdd(sums + i, acc);
   }
 }
 
@@ -195,15 +197,35 @@ __device__ __forceinline__ double slot_total(const double* sums, int c2, int i) 
   return t;
 }
 
+// Deterministic totals, between two grid barriers: the CTAs' partial rows [grid][c2] -> tot[c2] in a fixed order.
+// Warp w of the grid totals accumulators w, w + 8 grid, ...: lane l sums the rows of CTAs l, l + 32, ... in ascending
+// order, then a butterfly over the lanes (the same on every run) combines the 32 sums.  Each row is read once, by one
+// CTA, instead of every CTA reading all of them (grid^2 x c2 doubles).
+__device__ __forceinline__ void det_totals(const double* rows, double* tot, int c2) {
+  const int lane = threadIdx.x & 31, nw = kThreads / 32;
+#pragma unroll 1
+  for (int i = blockIdx.x * nw + (threadIdx.x >> 5); i < c2; i += gridDim.x * nw) {
+    double t = 0.0;
+    const double* src = rows + (size_t)lane * c2 + i;
+#pragma unroll 4
+    for (int b = lane; b < (int)gridDim.x; b += 32, src += 32 * c2) t += __ldcg(src);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+    if (lane == 0) tot[i] = t;
+  }
+}
+
 // ---- training forward in ONE launch: statistics, grid barrier, normalise + ReLU.  A CTA re-reads exactly the
 // rows it summed, so the second read comes from L2 / L1 instead of HBM.
-template <int VEC>
+// DET: the deterministic variant -- `rows` [grid][2 c] takes the CTAs' partials, `sums` [2 c] the totals (det_totals
+// between the barrier on `sync` and a second one on sync + kSlots + 1)
+template <int VEC, bool DET>
 __global__ void __launch_bounds__(kThreads)
 k_bn_fwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int c_lo, float* __restrict__ y, int64_t n, int c,
                const float* __restrict__ gamma, const float* __restrict__ beta,
                float* running_mean, float* running_var, float* save_mean, float* save_invstd,
-               double* sums, unsigned int* sync, double* other, int other_words, float eps, float momentum, float leak,
-               int round_tf32, int* err) {
+               double* sums, unsigned int* sync, double* rows, double* other, int other_words, float eps, float momentum,
+               float leak, int round_tf32, int* err) {
   mm3d_griddep_launch();
   mm3d_griddep_wait();
   zero_other(other, other_words);
@@ -238,15 +260,20 @@ k_bn_fwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
         for (int j = 0; j < VEC; ++j) { s[j] += t[j]; q[j] = fmaf(t[j], t[j], q[j]); }
       }
     }
-    block_flush<VEC>(s, q, c, cv, rows_pass, r, v, sums + (blockIdx.x % kSlots) * 2 * c);
+    if (DET) block_flush<VEC, true>(s, q, c, cv, rows_pass, r, v, rows);
+    else block_flush<VEC>(s, q, c, cv, rows_pass, r, v, sums + (blockIdx.x % kSlots) * 2 * c);
   }
   grid_arrive_and_wait(sync, err);
+  if (DET) {
+    det_totals(rows, sums, 2 * c);
+    grid_arrive_and_wait(sync + kSlots + 1, err);
+  }
   float* s_mean = reinterpret_cast<float*>(s_acc);
   float* s_scale = s_mean + c;
   __syncthreads();  // block_flush's use of the shared buffer is over
   for (int i = threadIdx.x; i < c; i += kThreads) {
-    const double m = slot_total(sums, 2 * c, i) / (double)n;
-    double var = slot_total(sums, 2 * c, c + i) / (double)n - m * m;
+    const double m = (DET ? __ldcg(sums + i) : slot_total(sums, 2 * c, i)) / (double)n;
+    double var = (DET ? __ldcg(sums + c + i) : slot_total(sums, 2 * c, c + i)) / (double)n - m * m;
     if (var < 0.0) var = 0.0;
     const float mean = (float)m, invstd = (float)(1.0 / sqrt(var + (double)eps));
     if (blockIdx.x == 0) {
@@ -296,13 +323,15 @@ k_bn_fwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
 }
 
 // ---- backward in ONE launch: reductions, grid barrier, dx (+ d_gamma / d_beta by CTA 0)
-template <int VEC>
+// (DET: as in k_bn_fwd_fused)
+template <int VEC, bool DET>
 __global__ void __launch_bounds__(kThreads)
 k_bn_bwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int c_lo, const float* __restrict__ dy,
                float* __restrict__ dx, float* __restrict__ dx_hi, int64_t n, int c,
                const float* __restrict__ gamma, const float* __restrict__ beta,
                const float* __restrict__ save_mean, const float* __restrict__ save_invstd, float leak,
-               double* sums, unsigned int* sync, double* other, int other_words, float* d_gamma, float* d_beta, int training,
+               double* sums, unsigned int* sync, double* rows, double* other, int other_words, float* d_gamma, float* d_beta,
+               int training,
                int round_flags, const float* __restrict__ add, int64_t add_ld, int* err) {
   mm3d_griddep_launch();
   mm3d_griddep_wait();
@@ -368,13 +397,18 @@ k_bn_bwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
         }
       }
     }
-    block_flush<VEC>(s, q, c, cv, rows_pass, r, v, sums + (blockIdx.x % kSlots) * 2 * c);
+    if (DET) block_flush<VEC, true>(s, q, c, cv, rows_pass, r, v, rows);
+    else block_flush<VEC>(s, q, c, cv, rows_pass, r, v, sums + (blockIdx.x % kSlots) * 2 * c);
   }
   grid_arrive_and_wait(sync, err);
+  if (DET) {
+    det_totals(rows, sums, 2 * c);
+    grid_arrive_and_wait(sync + kSlots + 1, err);
+  }
   // totals over the slot copies -> shared memory (block_flush's use of the buffer is over)
   double* s_tot = s_acc;
   __syncthreads();
-  for (int i = threadIdx.x; i < 2 * c; i += kThreads) s_tot[i] = slot_total(sums, 2 * c, i);
+  for (int i = threadIdx.x; i < 2 * c; i += kThreads) s_tot[i] = DET ? __ldcg(sums + i) : slot_total(sums, 2 * c, i);
   __syncthreads();
   if (blockIdx.x == 0)  // (frozen affine parameters: NULL gradient pointers)
     for (int i = threadIdx.x; i < c; i += kThreads) {
@@ -460,7 +494,7 @@ static int bn_per_sm_cap() {
   return v >= 1 && v <= 8 ? v : 2;
 }
 
-template <typename Kernel>
+template <bool DET, typename Kernel>
 int bn_grid(Kernel kernel, int64_t n, int cv, size_t smem) {
   const int rows_pass = kThreads / cv;
   int64_t g = mm3d_cdiv(n, (int64_t)rows_pass * 4);  // >= 4 rows per thread when there is enough work
@@ -468,7 +502,7 @@ int bn_grid(Kernel kernel, int64_t n, int cv, size_t smem) {
   // the query is cached per device and kernel instantiation for the 16 KB upper bound of these kernels' dynamic
   // shared memory (2 * rows_pass * c floats <= 8 KB for every supported c); larger requests are queried directly
   constexpr size_t kSmemBound = 16 * 1024;
-  static int cached[64] = {0};
+  static int cached[64] = {0};  // (DET is a template parameter: both variants of a kernel have the same type)
   int& slot = cached[mm3d_device_slot()];
   int per_sm = smem <= kSmemBound ? slot : 0;
   if (per_sm == 0) {
@@ -490,6 +524,16 @@ int* mm3d_device_err_flag();  // conv_tc.cu
 // workspace: two regions of [kSlots copies of 2*c doubles of totals | kSlots + 1 barrier counters]
 static size_t bn_region_bytes(int c) { return mm3d_align(sizeof(double) * (kSlots * 2 * (size_t)c + 8)); }
 extern "C" size_t mm3d_bnrelu_workspace_bytes(int c) { return 2 * bn_region_bytes(c); }
+// deterministic variant: two regions of [2*c doubles of totals | two sets of kSlots + 1 barrier counters], then the
+// partial rows [grid][2*c] doubles for the largest grid this device can get (every launch overwrites the rows it uses)
+static size_t bn_det_region_bytes(int c) {
+  return mm3d_align(sizeof(double) * 2 * (size_t)c + sizeof(unsigned int) * 2 * (kSlots + 1));
+}
+static int64_t bn_max_grid() { return (int64_t)mm3d_sm_count() * bn_per_sm_cap(); }
+extern "C" size_t mm3d_bnrelu_workspace_bytes_ex(int c, int flags) {
+  if (!(flags & MM3D_DETERMINISTIC)) return mm3d_bnrelu_workspace_bytes(c);
+  return 2 * bn_det_region_bytes(c) + sizeof(double) * 2 * (size_t)c * (size_t)bn_max_grid();
+}
 
 #define BN_DISPATCH(KERNEL, ...)                                                        \
   do {                                                                                  \
@@ -497,45 +541,54 @@ extern "C" size_t mm3d_bnrelu_workspace_bytes(int c) { return 2 * bn_region_byte
     if (vec4) KERNEL<4><<<grid, kThreads, smem, stream>>>(__VA_ARGS__);                 \
     else      KERNEL<1><<<grid, kThreads, smem, stream>>>(__VA_ARGS__);                 \
   } while (0)
-#define BN_DISPATCH_PDL(KERNEL, ...)                                                                        \
-  do {                                                                                                      \
-    if (vec4) { const int grid = bn_grid(KERNEL<4>, n, cv, smem);                                           \
-                MM3D_CUDA(mm3d_launch_pdl(KERNEL<4>, dim3(grid), dim3(kThreads), smem, stream, __VA_ARGS__)); } \
-    else      { const int grid = bn_grid(KERNEL<1>, n, cv, smem);                                           \
-                MM3D_CUDA(mm3d_launch_pdl(KERNEL<1>, dim3(grid), dim3(kThreads), smem, stream, __VA_ARGS__)); } \
+#define BN_DISPATCH_PDL(KERNEL, DET, ...)                                                                        \
+  do {                                                                                                           \
+    if (vec4) { const int grid = bn_grid<DET>(KERNEL<4, DET>, n, cv, smem);                                      \
+                MM3D_CUDA(mm3d_launch_pdl(KERNEL<4, DET>, dim3(grid), dim3(kThreads), smem, stream, __VA_ARGS__)); } \
+    else      { const int grid = bn_grid<DET>(KERNEL<1, DET>, n, cv, smem);                                      \
+                MM3D_CUDA(mm3d_launch_pdl(KERNEL<1, DET>, dim3(grid), dim3(kThreads), smem, stream, __VA_ARGS__)); } \
   } while (0)
 
 // parity == NULL: the workspace is not known to be clean: zero it, use region 0.  Otherwise it is all zero (the kernels
 // leave it that way, no memset), and the launches that use it alternate between its two regions by toggling *parity,
 // which the caller keeps with the workspace.
-int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, int64_t n, int c, const float* gamma,
-                         const float* beta,
-                         float* running_mean, float* running_var, float* save_mean, float* save_invstd,
-                         float eps, float momentum, float leakiness, int training,
-                         void* ws, size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream) {
+// det: the deterministic kernels, workspace mm3d_bnrelu_workspace_bytes_ex(c, MM3D_DETERMINISTIC), parity NULL
+static int bn_fwd(const float* x, const float* x_hi, int c_lo, float* y, int64_t n, int c, const float* gamma,
+                  const float* beta,
+                  float* running_mean, float* running_var, float* save_mean, float* save_invstd,
+                  float eps, float momentum, float leakiness, int training,
+                  void* ws, size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream, bool det) {
   MM3D_REQUIRE(c > 0 && n >= 0, MM3D_ERR_INVALID, "bad sizes");
   const bool vec4 = (c % 4 == 0) && (c_lo % 4 == 0) && ((((uintptr_t)x | (uintptr_t)x_hi | (uintptr_t)y) & 15) == 0);
   const int cv = vec4 ? c / 4 : c;
   MM3D_REQUIRE(cv <= kThreads, MM3D_ERR_UNSUPPORTED, "BatchNorm with %d channels not supported", c);
-  MM3D_REQUIRE(ws_bytes >= mm3d_bnrelu_workspace_bytes(c) && ws, MM3D_ERR_WORKSPACE, "bnrelu workspace too small");
+  MM3D_REQUIRE(ws_bytes >= mm3d_bnrelu_workspace_bytes_ex(c, det ? MM3D_DETERMINISTIC : 0) && ws, MM3D_ERR_WORKSPACE,
+               "bnrelu workspace too small");
   MM3D_REQUIRE(!x_hi || (training && c_lo > 0 && c_lo < c), MM3D_ERR_INVALID, "split input needs training mode and 0 < c_lo < c");
   if (n == 0) return MM3D_OK;
   // region `half` is this launch's (all zero: memset below, or zeroed by the previous launch), the other one is
   // zeroed by this launch for the next.  Region size follows the workspace size (the executor shares one workspace
   // among layers of different widths), so consecutive launches agree on where the regions are.
-  const size_t region = ws_bytes / 2 / 256 * 256;
+  const size_t region = det ? bn_det_region_bytes(c) : ws_bytes / 2 / 256 * 256;
   const int half = (parity && training) ? (*parity ^= 1) : 0;  // (only launches that use the workspace alternate)
   double* sums = (double*)((char*)ws + (size_t)half * region);
   double* other = (double*)((char*)ws + (size_t)(half ^ 1) * region);
-  unsigned int* sync = (unsigned int*)(sums + kSlots * 2 * c);
+  unsigned int* sync = (unsigned int*)(sums + (det ? 2 : kSlots * 2) * c);
+  double* rows = det ? (double*)((char*)ws + 2 * region) : nullptr;
   const int other_words = (int)(region / 8);
   const size_t smem = sizeof(double) * 2 * c > sizeof(float) * 2 * (kThreads / cv) * (size_t)c
                           ? sizeof(double) * 2 * c : sizeof(float) * 2 * (kThreads / cv) * (size_t)c;
   if (training) {
     MM3D_REQUIRE(save_mean && save_invstd && running_mean && running_var, MM3D_ERR_INVALID, "training needs stat buffers");
     if (!parity) MM3D_CUDA(cudaMemsetAsync(ws, 0, 2 * region, stream));
-    BN_DISPATCH_PDL(k_bn_fwd_fused, x, x_hi, c_lo, y, n, c, gamma, beta, running_mean, running_var, save_mean, save_invstd, sums, sync,
-                other, other_words, eps, momentum, leakiness, round_tf32, mm3d_device_err_flag());
+    if (det)
+      BN_DISPATCH_PDL(k_bn_fwd_fused, true, x, x_hi, c_lo, y, n, c, gamma, beta, running_mean, running_var, save_mean,
+                      save_invstd, sums, sync, rows, other, other_words, eps, momentum, leakiness, round_tf32,
+                      mm3d_device_err_flag());
+    else
+      BN_DISPATCH_PDL(k_bn_fwd_fused, false, x, x_hi, c_lo, y, n, c, gamma, beta, running_mean, running_var, save_mean,
+                      save_invstd, sums, sync, rows, other, other_words, eps, momentum, leakiness, round_tf32,
+                      mm3d_device_err_flag());
   } else {
     BN_DISPATCH(k_bn_apply, x, y, n, c, gamma, beta, running_mean, running_var, save_mean, save_invstd, sums, eps,
                 momentum, leakiness, training, round_tf32);
@@ -545,50 +598,94 @@ int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, 
   return MM3D_OK;
 }
 
-int mm3d_bnrelu_bwd_impl(const float* x, const float* x_hi, int c_lo, const float* dy, float* dx, float* dx_hi,
-                         int64_t n, int c, const float* gamma, const float* beta, const float* save_mean, const float* save_invstd,
-                         float* d_gamma, float* d_beta, float leakiness, int training,
-                         void* ws, size_t ws_bytes, int* parity, int round_flags, const float* add, int64_t add_ld,
-                         cudaStream_t stream) {
+int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, int64_t n, int c, const float* gamma,
+                         const float* beta,
+                         float* running_mean, float* running_var, float* save_mean, float* save_invstd,
+                         float eps, float momentum, float leakiness, int training,
+                         void* ws, size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream) {
+  return bn_fwd(x, x_hi, c_lo, y, n, c, gamma, beta, running_mean, running_var, save_mean, save_invstd, eps, momentum,
+                leakiness, training, ws, ws_bytes, parity, round_tf32, stream, false);
+}
+
+static int bn_bwd(const float* x, const float* x_hi, int c_lo, const float* dy, float* dx, float* dx_hi,
+                  int64_t n, int c, const float* gamma, const float* beta, const float* save_mean, const float* save_invstd,
+                  float* d_gamma, float* d_beta, float leakiness, int training,
+                  void* ws, size_t ws_bytes, int* parity, int round_flags, const float* add, int64_t add_ld,
+                  cudaStream_t stream, bool det) {
   MM3D_REQUIRE(c > 0 && n >= 0, MM3D_ERR_INVALID, "bad sizes");
   const bool vec4 = (c % 4 == 0) && (c_lo % 4 == 0) && (!add || add_ld % 4 == 0) &&
                     ((((uintptr_t)x | (uintptr_t)x_hi | (uintptr_t)dy | (uintptr_t)dx | (uintptr_t)dx_hi | (uintptr_t)add) & 15) == 0);
   const int cv = vec4 ? c / 4 : c;
   MM3D_REQUIRE(cv <= kThreads, MM3D_ERR_UNSUPPORTED, "BatchNorm with %d channels not supported", c);
-  MM3D_REQUIRE(ws_bytes >= mm3d_bnrelu_workspace_bytes(c) && ws, MM3D_ERR_WORKSPACE, "bnrelu workspace too small");
+  MM3D_REQUIRE(ws_bytes >= mm3d_bnrelu_workspace_bytes_ex(c, det ? MM3D_DETERMINISTIC : 0) && ws, MM3D_ERR_WORKSPACE,
+               "bnrelu workspace too small");
   if (n == 0) {
     if (d_gamma) MM3D_CUDA(cudaMemsetAsync(d_gamma, 0, sizeof(float) * c, stream));
     if (d_beta) MM3D_CUDA(cudaMemsetAsync(d_beta, 0, sizeof(float) * c, stream));
     return MM3D_OK;
   }
-  const size_t region = ws_bytes / 2 / 256 * 256;
+  const size_t region = det ? bn_det_region_bytes(c) : ws_bytes / 2 / 256 * 256;
   const int half = parity ? (*parity ^= 1) : 0;
   double* sums = (double*)((char*)ws + (size_t)half * region);
   double* other = (double*)((char*)ws + (size_t)(half ^ 1) * region);
-  unsigned int* sync = (unsigned int*)(sums + kSlots * 2 * c);
+  unsigned int* sync = (unsigned int*)(sums + (det ? 2 : kSlots * 2) * c);
+  double* rows = det ? (double*)((char*)ws + 2 * region) : nullptr;
   const int other_words = (int)(region / 8);
   if (!parity) MM3D_CUDA(cudaMemsetAsync(ws, 0, 2 * region, stream));
   const size_t smem = sizeof(double) * 2 * c > sizeof(float) * 2 * (kThreads / cv) * (size_t)c
                           ? sizeof(double) * 2 * c : sizeof(float) * 2 * (kThreads / cv) * (size_t)c;
-  BN_DISPATCH_PDL(k_bn_bwd_fused, x, x_hi, c_lo, dy, dx, dx_hi, n, c, gamma, beta, save_mean, save_invstd, leakiness, sums, sync, other, other_words, d_gamma,
-              d_beta, training, round_flags, add, add_ld, mm3d_device_err_flag());
+  if (det)
+    BN_DISPATCH_PDL(k_bn_bwd_fused, true, x, x_hi, c_lo, dy, dx, dx_hi, n, c, gamma, beta, save_mean, save_invstd, leakiness,
+                    sums, sync, rows, other, other_words, d_gamma, d_beta, training, round_flags, add, add_ld,
+                    mm3d_device_err_flag());
+  else
+    BN_DISPATCH_PDL(k_bn_bwd_fused, false, x, x_hi, c_lo, dy, dx, dx_hi, n, c, gamma, beta, save_mean, save_invstd, leakiness,
+                    sums, sync, rows, other, other_words, d_gamma, d_beta, training, round_flags, add, add_ld,
+                    mm3d_device_err_flag());
   mm3d_count_launches(1);
   MM3D_CHECK_LAUNCH("mm3d_bnrelu_bwd");
   return MM3D_OK;
+}
+
+int mm3d_bnrelu_bwd_impl(const float* x, const float* x_hi, int c_lo, const float* dy, float* dx, float* dx_hi,
+                         int64_t n, int c, const float* gamma, const float* beta, const float* save_mean, const float* save_invstd,
+                         float* d_gamma, float* d_beta, float leakiness, int training,
+                         void* ws, size_t ws_bytes, int* parity, int round_flags, const float* add, int64_t add_ld,
+                         cudaStream_t stream) {
+  return bn_bwd(x, x_hi, c_lo, dy, dx, dx_hi, n, c, gamma, beta, save_mean, save_invstd, d_gamma, d_beta, leakiness,
+                training, ws, ws_bytes, parity, round_flags, add, add_ld, stream, false);
+}
+
+extern "C" int mm3d_bnrelu_fwd_ex(const float* x, float* y, int64_t n, int c, const float* gamma, const float* beta,
+                                  float* running_mean, float* running_var, float* save_mean, float* save_invstd,
+                                  float eps, float momentum, float leakiness, int training,
+                                  void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags) {
+  MM3D_REQUIRE((flags & ~MM3D_DETERMINISTIC) == 0, MM3D_ERR_INVALID, "bnrelu_fwd: unknown flags %#x", flags);
+  return bn_fwd(x, nullptr, 0, y, n, c, gamma, beta, running_mean, running_var, save_mean, save_invstd, eps, momentum,
+                leakiness, training, ws, ws_bytes, nullptr, 0, (cudaStream_t)stream, (flags & MM3D_DETERMINISTIC) != 0);
+}
+
+extern "C" int mm3d_bnrelu_bwd_ex(const float* x, const float* dy, float* dx, int64_t n, int c, const float* gamma,
+                                  const float* beta, const float* save_mean, const float* save_invstd,
+                                  float* d_gamma, float* d_beta, float leakiness, int training,
+                                  void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags) {
+  MM3D_REQUIRE((flags & ~MM3D_DETERMINISTIC) == 0, MM3D_ERR_INVALID, "bnrelu_bwd: unknown flags %#x", flags);
+  return bn_bwd(x, nullptr, 0, dy, dx, nullptr, n, c, gamma, beta, save_mean, save_invstd, d_gamma, d_beta, leakiness,
+                training, ws, ws_bytes, nullptr, 0, nullptr, 0, (cudaStream_t)stream, (flags & MM3D_DETERMINISTIC) != 0);
 }
 
 extern "C" int mm3d_bnrelu_fwd(const float* x, float* y, int64_t n, int c, const float* gamma, const float* beta,
                                float* running_mean, float* running_var, float* save_mean, float* save_invstd,
                                float eps, float momentum, float leakiness, int training,
                                void* ws, size_t ws_bytes, mm3d_stream_t stream) {
-  return mm3d_bnrelu_fwd_impl(x, nullptr, 0, y, n, c, gamma, beta, running_mean, running_var, save_mean, save_invstd, eps, momentum,
-                              leakiness, training, ws, ws_bytes, nullptr, 0, (cudaStream_t)stream);
+  return mm3d_bnrelu_fwd_ex(x, y, n, c, gamma, beta, running_mean, running_var, save_mean, save_invstd, eps, momentum,
+                            leakiness, training, ws, ws_bytes, stream, 0);
 }
 
 extern "C" int mm3d_bnrelu_bwd(const float* x, const float* dy, float* dx, int64_t n, int c, const float* gamma,
                                const float* beta, const float* save_mean, const float* save_invstd,
                                float* d_gamma, float* d_beta, float leakiness, int training,
                                void* ws, size_t ws_bytes, mm3d_stream_t stream) {
-  return mm3d_bnrelu_bwd_impl(x, nullptr, 0, dy, dx, nullptr, n, c, gamma, beta, save_mean, save_invstd, d_gamma, d_beta, leakiness, training,
-                              ws, ws_bytes, nullptr, 0, nullptr, 0, (cudaStream_t)stream);
+  return mm3d_bnrelu_bwd_ex(x, dy, dx, n, c, gamma, beta, save_mean, save_invstd, d_gamma, d_beta, leakiness, training,
+                            ws, ws_bytes, stream, 0);
 }

@@ -51,7 +51,8 @@ int mm3d_conv_tc_supported(int c_in, int c_out, int K);
 int mm3d_conv_wgrad_tc_supported(int c_in, int c_out, int K);
 int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out, int c_out,
                        float* d_weight, int K, const void* plan, int64_t plan_cap, int accumulate,
-                       cudaStream_t stream, int bf16 = 0);
+                       cudaStream_t stream, int bf16 = 0, void* slab = nullptr, size_t slab_bytes = 0);
+size_t mm3d_conv_wgrad_tc_slab_bytes(int c_in, int c_out, int K);
 int mm3d_conv_fwd_tc(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
                      const float* weight, int K, const void* plan, int64_t plan_cap, int flags, void* ws,
                      size_t ws_bytes, cudaStream_t stream);
@@ -111,13 +112,27 @@ extern "C" int mm3d_conv_fwd(const float* in, int64_t n_in, int c_in, float* out
   }
 }
 
-extern "C" int mm3d_conv_wgrad(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out,
-                               int c_out, float* d_weight, int K, const int32_t* tbl, int64_t tbl_stride,
-                               const uint8_t* onehot_off, const void* plan, int64_t plan_cap, int accumulate, int mode,
-                               void* ws, size_t ws_bytes, mm3d_stream_t stream) {
-  (void)ws; (void)ws_bytes;
+extern "C" size_t mm3d_conv_wgrad_workspace_bytes(int64_t n_out, int c_in, int c_out, int K, int mode, int flags) {
+  (void)n_out;
+  if (!(flags & MM3D_DETERMINISTIC) || mode == MM3D_MODE_FP32) return 0;
+  return mm3d_conv_wgrad_tc_slab_bytes(c_in, c_out, K);  // (0 for the shapes only the SIMT kernel takes)
+}
+
+extern "C" int mm3d_conv_wgrad_ex(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out,
+                                  int c_out, float* d_weight, int K, const int32_t* tbl, int64_t tbl_stride,
+                                  const uint8_t* onehot_off, const void* plan, int64_t plan_cap, int accumulate, int mode,
+                                  void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags) {
+  MM3D_REQUIRE((flags & ~MM3D_DETERMINISTIC) == 0, MM3D_ERR_INVALID, "conv_wgrad: unknown flags %#x", flags);
+  const bool det = flags & MM3D_DETERMINISTIC;
   int rc = check_conv_args(in, d_out, d_weight, tbl, n_in, n_out, c_in, c_out, K, tbl_stride, onehot_off);
   if (rc) return rc;
+  // deterministic: the tcgen05 kernels with per-CTA slabs in `ws`; the SIMT kernel has no such form
+  MM3D_REQUIRE(!det || (mode != MM3D_MODE_FP32 && mm3d_conv_wgrad_tc_supported(c_in, c_out, K)), MM3D_ERR_UNSUPPORTED,
+               "conv_wgrad: no deterministic form for %s (c_in %d c_out %d K %d): only the tensor-core modes on shapes "
+               "the tcgen05 kernel takes (pad the channels to a multiple of 16)",
+               mode == MM3D_MODE_FP32 ? "the fp32 mode" : "this shape", c_in, c_out, K);
+  void* slab = det ? ws : nullptr;
+  const size_t slab_bytes = det ? ws_bytes : 0;
   switch (mode) {
     case MM3D_MODE_TF32X3: {
       // d_weight = in_hi^T d_out_hi + in_lo^T d_out_hi + in_hi^T d_out_lo: three launches of the TF32 kernel that
@@ -127,9 +142,12 @@ extern "C" int mm3d_conv_wgrad(const float* in, int64_t n_in, int c_in, const fl
       MM3D_REQUIRE(plan, MM3D_ERR_INVALID, "mm3d_conv_wgrad: tf32x3 mode needs the table's row plan (mm3d_build_plan)");
       const float* in_lo = in + n_in * (int64_t)c_in;
       const float* dout_lo = d_out + n_out * (int64_t)c_out;
-      rc = mm3d_conv_wgrad_tc(in, n_in, c_in, d_out, n_out, c_out, d_weight, K, plan, plan_cap, accumulate, (cudaStream_t)stream);
-      if (!rc) rc = mm3d_conv_wgrad_tc(in_lo, n_in, c_in, d_out, n_out, c_out, d_weight, K, plan, plan_cap, 1, (cudaStream_t)stream);
-      if (!rc) rc = mm3d_conv_wgrad_tc(in, n_in, c_in, dout_lo, n_out, c_out, d_weight, K, plan, plan_cap, 1, (cudaStream_t)stream);
+      rc = mm3d_conv_wgrad_tc(in, n_in, c_in, d_out, n_out, c_out, d_weight, K, plan, plan_cap, accumulate, (cudaStream_t)stream,
+                              0, slab, slab_bytes);
+      if (!rc) rc = mm3d_conv_wgrad_tc(in_lo, n_in, c_in, d_out, n_out, c_out, d_weight, K, plan, plan_cap, 1, (cudaStream_t)stream,
+                                       0, slab, slab_bytes);
+      if (!rc) rc = mm3d_conv_wgrad_tc(in, n_in, c_in, dout_lo, n_out, c_out, d_weight, K, plan, plan_cap, 1, (cudaStream_t)stream,
+                                       0, slab, slab_bytes);
       return rc;
     }
     case MM3D_MODE_BF16:
@@ -137,7 +155,7 @@ extern "C" int mm3d_conv_wgrad(const float* in, int64_t n_in, int c_in, const fl
       // otherwise the TF32 kernel on the FP32 planes
       if (plan && mm3d_conv_wgrad_tc_supported(c_in, c_out, K) && n_out > 0) {
         rc = mm3d_conv_wgrad_tc(in + n_in * (int64_t)c_in, n_in, c_in, d_out + n_out * (int64_t)c_out, n_out, c_out, d_weight, K,
-                                plan, plan_cap, accumulate, (cudaStream_t)stream, 1);
+                                plan, plan_cap, accumulate, (cudaStream_t)stream, 1, slab, slab_bytes);
         if (rc != MM3D_ERR_UNSUPPORTED) return rc;
       }
       // fall through
@@ -145,7 +163,7 @@ extern "C" int mm3d_conv_wgrad(const float* in, int64_t n_in, int c_in, const fl
       if (mm3d_conv_wgrad_tc_supported(c_in, c_out, K)) {
         MM3D_REQUIRE(plan, MM3D_ERR_INVALID, "mm3d_conv_wgrad: tf32 mode needs the table's row plan (mm3d_build_plan)");
         return mm3d_conv_wgrad_tc(in, n_in, c_in, d_out, n_out, c_out, d_weight, K, plan, plan_cap, accumulate,
-                                  (cudaStream_t)stream);
+                                  (cudaStream_t)stream, 0, slab, slab_bytes);
       }
       // fall through: shapes the tcgen05 kernel does not take (the 3-channel stem) use the FP32 kernel
     case MM3D_MODE_FP32:
@@ -154,4 +172,12 @@ extern "C" int mm3d_conv_wgrad(const float* in, int64_t n_in, int c_in, const fl
     default:
       MM3D_REQUIRE(false, MM3D_ERR_UNSUPPORTED, "wgrad mode %d not implemented in this build", mode);
   }
+}
+
+extern "C" int mm3d_conv_wgrad(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out,
+                               int c_out, float* d_weight, int K, const int32_t* tbl, int64_t tbl_stride,
+                               const uint8_t* onehot_off, const void* plan, int64_t plan_cap, int accumulate, int mode,
+                               void* ws, size_t ws_bytes, mm3d_stream_t stream) {
+  return mm3d_conv_wgrad_ex(in, n_in, c_in, d_out, n_out, c_out, d_weight, K, tbl, tbl_stride, onehot_off, plan, plan_cap,
+                            accumulate, mode, ws, ws_bytes, stream, 0);
 }

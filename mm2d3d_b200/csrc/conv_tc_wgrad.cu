@@ -62,6 +62,11 @@ struct WgParams {
   int groups;       // offset groups; group g owns the offsets of gmask[g]; its CTAs are decided in the kernel
   uint32_t gmask[32];
   int* err;
+  // deterministic variant: CTA b stores its accumulators to slab + b * slab_cta ([gk][c_in][c_out] floats), CTA 0 the
+  // group -> first-CTA table to slab_cta0 [groups + 1]; k_wgrad_reduce sums them
+  float* slab;
+  int* slab_cta0;
+  int64_t slab_cta;
 #ifdef MM3D_TRACE
   long long* trace;  // development builds: clock64 stamps of CTA 0's roles, [role][64 records][4]
 #endif
@@ -165,6 +170,79 @@ __device__ __forceinline__ void red_add_v4(float* dst, float a, float b, float c
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 
+// Deterministic epilogue (epilogue warp ew): this CTA's accumulators of EVERY offset of its group -> its own slab with
+// plain stores, zeros for the offsets it never touched (their TMEM columns were never written), so that the reduction
+// can sum a fixed set of CTAs without knowing which of them saw which offset.  Slab row = kidx (the offset's rank in
+// the group), then the dW[k] layout [c_in][c_out].
+__device__ __forceinline__ void flush_to_slab(const WgParams& p, uint32_t tmem_base, int ew, int lane, uint32_t gmask,
+                                              uint32_t seen) {
+  const int ci = p.mm == 128 ? ew * 32 + lane : ew * 16 + lane;
+  const bool lane_ok = (p.mm == 128 || lane < 16) && ci < p.cm;
+  float* slab = p.slab + (int64_t)blockIdx.x * p.slab_cta;
+  int kidx = 0;
+  for (uint32_t rem = gmask; rem; rem &= rem - 1, ++kidx) {
+    const bool touched = (seen >> (__ffs(rem) - 1)) & 1u;
+    for (int h = 0; h < p.nmb; ++h) {
+      const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + (uint32_t)((kidx * p.nmb + h) * p.c_out);
+      float* dst = slab + ((int64_t)kidx * p.c_in + h * p.cm + ci) * p.c_out;
+      for (int c0 = 0; c0 < p.c_out; c0 += 16) {
+        float acc[16];
+        if (touched) tmem_ld16(taddr + (uint32_t)c0, acc);  // (warp-uniform: every lane takes part)
+        else {
+#pragma unroll
+          for (int q = 0; q < 16; ++q) acc[q] = 0.f;
+        }
+        if (lane_ok) {
+#pragma unroll
+          for (int q = 0; q < 16; q += 4)
+            *reinterpret_cast<float4*>(dst + c0 + q) = make_float4(acc[q], acc[q + 1], acc[q + 2], acc[q + 3]);
+        }
+      }
+    }
+  }
+}
+
+// Deterministic variant, second launch: dW[k] = (accumulate ? dW[k] : 0) + sum of the slabs of the CTAs of the group
+// that owns k, in ascending CTA index, in FP32.  Which CTAs those are comes from the plan, the shapes and the SM count
+// only (the table the first launch's CTA 0 wrote), never from timing.
+struct WgReduceParams {
+  const float* slab;
+  const int* cta0;
+  float* dw;
+  int64_t slab_cta;
+  int c_in, c_out, K, accumulate, groups;
+  uint32_t gmask[32];  // as WgParams::gmask
+};
+
+__global__ void __launch_bounds__(256)
+k_wgrad_reduce(const WgReduceParams r) {
+  const int64_t per_k = (int64_t)r.c_in * r.c_out;  // (a multiple of 256: float4 pieces never straddle an offset)
+  const int64_t n4 = (int64_t)r.K * per_k / 4;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+    const int k = (int)(4 * i / per_k);
+    const int64_t e = 4 * i - k * per_k;
+    int g = 0;  // the group that owns k, and k's rank in it (constant indices: the table stays in parameter space)
+    uint32_t gm = 0;
+#pragma unroll
+    for (int j = 0; j < 32; ++j)
+      if (j < r.groups && ((r.gmask[j] >> k) & 1u)) { g = j; gm = r.gmask[j]; }
+    const int b0 = __ldg(r.cta0 + g), b1 = __ldg(r.cta0 + g + 1);
+    const float* src = r.slab + (int64_t)__popc(gm & ((1u << k) - 1u)) * per_k + e;
+    float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int b = b0; b < b1; ++b) {
+      const float4 v = __ldcs(reinterpret_cast<const float4*>(src + (int64_t)b * r.slab_cta));
+      s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+    }
+    float4* d = reinterpret_cast<float4*>(r.dw + 4 * i);
+    if (r.accumulate) {
+      const float4 o = *d;
+      s = make_float4(o.x + s.x, o.y + s.y, o.z + s.z, o.w + s.w);
+    }
+    *d = s;
+  }
+}
+
+template <bool kDet>
 __global__ void __launch_bounds__(kThreads, 1)
 k_wgrad_tc(const WgParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -246,6 +324,7 @@ k_wgrad_tc(const WgParams p) {
     if (lane == 0) s_cta0[0] = 0;
   }
   __syncthreads();
+  if (kDet && blockIdx.x == 0 && threadIdx.x <= p.groups) p.slab_cta0[threadIdx.x] = s_cta0[threadIdx.x];
   int grp = 0;  // this CTA's offset group, its index among the group's CTAs and their number
   while (grp + 1 < p.groups && (int)blockIdx.x >= s_cta0[grp + 1]) ++grp;
   const uint32_t gmask = p.gmask[grp];
@@ -329,10 +408,18 @@ k_wgrad_tc(const WgParams p) {
     for (int i = lane; i < n_local; i += 32) seen |= lmask[i];
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) seen |= __shfl_xor_sync(0xffffffffu, seen, o);
-    if (seen == 0) goto done;
+    if (seen == 0) {
+      if constexpr (kDet) flush_to_slab(p, tmem_base, ew, lane, gmask, 0u);
+      goto done;
+    }
     if (!mbar_wait_sleep(acc_full, 0u, abort_flag, 1000)) goto done;
     if (ew == 0) TRACE(kProducers + 2, 0, 0);
     tc_fence_after();
+    if constexpr (kDet) {
+      flush_to_slab(p, tmem_base, ew, lane, gmask, seen);
+      tc_fence_before();
+      goto done;
+    }
     // accumulator row (= input channel of the M-block) of this thread: M=128 -> lane i holds row i; M=64 -> row m
     // sits in lane 32*(m/16) + m%16 (16 lanes per sub-partition)
     const int ci = p.mm == 128 ? ew * 32 + lane : ew * 16 + lane;
@@ -434,6 +521,7 @@ constexpr int kRingStages = 6;
 constexpr int kRingThreads = 14 * 32;
 constexpr int kRingEntBytes = kTileM * 4;
 
+template <bool kDet>
 __global__ void __launch_bounds__(kRingThreads, 1)
 k_wgrad_tc_rings(const WgParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -546,6 +634,7 @@ k_wgrad_tc_rings(const WgParams p) {
     if (lane == 0) s_cta0[0] = 0;
   }
   __syncthreads();
+  if (kDet && blockIdx.x == 0 && threadIdx.x <= p.groups) p.slab_cta0[threadIdx.x] = s_cta0[threadIdx.x];
   int grp = 0;
   while (grp + 1 < p.groups && (int)blockIdx.x >= s_cta0[grp + 1]) ++grp;
   const uint32_t gmask = p.gmask[grp], ring1 = s_ring1[grp];
@@ -709,10 +798,18 @@ k_wgrad_tc_rings(const WgParams p) {
     for (int i = lane; i < ne; i += 32) seen |= cmask[i];
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) seen |= __shfl_xor_sync(0xffffffffu, seen, o);
-    if (seen == 0) goto done;
+    if (seen == 0) {
+      if constexpr (kDet) flush_to_slab(p, tmem_base, ew, lane, gmask, 0u);
+      goto done;
+    }
     if (!mbar_wait_sleep(acc_full, 0u, abort_flag, 1000)) goto done;
     if (ew == 0) TRACE(kProducers + 2, 0, 0);
     tc_fence_after();
+    if constexpr (kDet) {
+      flush_to_slab(p, tmem_base, ew, lane, gmask, seen);
+      tc_fence_before();
+      goto done;
+    }
     const int ci = p.mm == 128 ? ew * 32 + lane : ew * 16 + lane;
     const bool lane_ok = (p.mm == 128 || lane < 16) && ci < p.cm;
     const int rot = (int)((unsigned)split * 5u % 32u);
@@ -815,11 +912,34 @@ int mm3d_conv_wgrad_tc_supported(int c_in, int c_out, int K) {
   return nmb * c_out <= 512;
 }
 
+// offsets per group: as many (offset, M-block) accumulators of c_out TMEM columns as fit the 512 columns
+static int wgrad_group_size(int c_in, int c_out, int K) {
+  const int gk = 512 / (c_out * (c_in > 128 ? 2 : 1));
+  return gk < K ? gk : K;
+}
+
+// Launch grid of both kernels: one CTA per SM, at least one per offset group
+static int wgrad_ctas(int c_in, int c_out, int K) {
+  const int gk = wgrad_group_size(c_in, c_out, K), groups = (K + gk - 1) / gk;
+  const int sms = mm3d_sm_count();
+  return sms < groups ? groups : sms;
+}
+
+// Deterministic variant's workspace: the group -> first-CTA table (256 bytes), then one slab of gk * c_in * c_out floats
+// per CTA (at most 512 TMEM columns x 128 lanes = 256 KB).  Independent of the row count; 0 for shapes the kernels do
+// not take.
+size_t mm3d_conv_wgrad_tc_slab_bytes(int c_in, int c_out, int K) {
+  if (!mm3d_conv_wgrad_tc_supported(c_in, c_out, K)) return 0;
+  return 256 + (size_t)wgrad_ctas(c_in, c_out, K) * wgrad_group_size(c_in, c_out, K) * c_in * c_out * sizeof(float);
+}
+
 // bf16 != 0: `in` / `d_out` point at BF16 planes ([rows, c] bfloat16); only shapes the two-ring kernel takes
 // (c_in <= 128), MM3D_ERR_UNSUPPORTED otherwise (the caller then runs the TF32 kernel on the FP32 planes)
+// slab != NULL: the deterministic variant (slab_bytes >= mm3d_conv_wgrad_tc_slab_bytes): every launch is followed by
+// k_wgrad_reduce, which adds that launch's slabs into d_weight, so the pieces of a long tile list reduce in piece order
 int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out, int c_out,
                        float* d_weight, int K, const void* plan, int64_t plan_cap, int accumulate,
-                       cudaStream_t stream, int bf16) {
+                       cudaStream_t stream, int bf16, void* slab, size_t slab_bytes) {
   MM3D_REQUIRE(mm3d_conv_wgrad_tc_supported(c_in, c_out, K), MM3D_ERR_UNSUPPORTED,
                "tcgen05 wgrad: unsupported shape c_in %d c_out %d K %d", c_in, c_out, K);
   MM3D_REQUIRE(n_out < (1ll << 31) && n_in * (int64_t)c_in < (1ll << 32) && n_out * (int64_t)c_out < (1ll << 32),
@@ -827,7 +947,14 @@ int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_o
   MM3D_REQUIRE(plan && plan_cap >= n_out, MM3D_ERR_INVALID, "tcgen05 wgrad: needs a row plan covering n_out rows");
   MM3D_REQUIRE((((uintptr_t)in | (uintptr_t)d_out | (uintptr_t)d_weight) & 15) == 0, MM3D_ERR_INVALID,
                "tcgen05 wgrad: pointers must be 16-byte aligned");
-  if (!accumulate) MM3D_CUDA(cudaMemsetAsync(d_weight, 0, sizeof(float) * (size_t)K * c_in * c_out, stream));
+  const bool det = slab != nullptr;
+  MM3D_REQUIRE(!det || slab_bytes >= mm3d_conv_wgrad_tc_slab_bytes(c_in, c_out, K), MM3D_ERR_WORKSPACE,
+               "deterministic wgrad: workspace %zu bytes < %zu (mm3d_conv_wgrad_workspace_bytes)", slab_bytes,
+               mm3d_conv_wgrad_tc_slab_bytes(c_in, c_out, K));
+  MM3D_REQUIRE(((uintptr_t)slab & 15) == 0, MM3D_ERR_INVALID, "deterministic wgrad: workspace must be 16-byte aligned");
+  // (the deterministic variant's reduction overwrites d_weight itself when !accumulate)
+  if (!accumulate && (!det || n_out == 0))
+    MM3D_CUDA(cudaMemsetAsync(d_weight, 0, sizeof(float) * (size_t)K * c_in * c_out, stream));
   if (n_out == 0) return MM3D_OK;
   const Mm3dPlanView pv = mm3d_plan_view(plan, plan_cap);
   WgParams p;
@@ -852,8 +979,7 @@ int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_o
   }
   p.mm = p.cm <= 64 ? 64 : 128;
   p.num_tiles = (int)mm3d_cdiv(n_out, kTileM);
-  int gk = 512 / (c_out * p.nmb);  // TMEM: c_out accumulator columns per (offset, M-block)
-  if (gk > K) gk = K;
+  const int gk = wgrad_group_size(c_in, c_out, K);  // TMEM: c_out accumulator columns per (offset, M-block)
   const int groups = (K + gk - 1) / gk;
   int cols = 32;
   while (cols < gk * p.nmb * c_out) cols <<= 1;
@@ -874,6 +1000,9 @@ int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_o
   while (p.gbufs < kMaxGBufs && (size_t)p.S * a_bytes + (size_t)(p.gbufs + 1) * g_bytes <= budget) ++p.gbufs;
   const size_t smem_fixed = fixed + (size_t)p.S * a_bytes + (size_t)p.gbufs * g_bytes;
   p.err = mm3d_device_err_flag();
+  p.slab_cta0 = det ? (int*)slab : nullptr;
+  p.slab = det ? (float*)((char*)slab + 256) : nullptr;
+  p.slab_cta = (int64_t)gk * c_in * c_out;
 #ifdef MM3D_TRACE
   p.trace = mm3d_debug_trace_ptr();
 #endif
@@ -910,16 +1039,30 @@ int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_o
   }
   // CTA shares of the groups are computed in the kernel from measured offset frequencies; here only the bound
   // on tiles per CTA (size of the shared-memory tile list): every group gets >= ceil(num_tiles / n_local) CTAs
-  int total_ctas = mm3d_sm_count();
-  if (total_ctas < groups) total_ctas = groups;
+  const int total_ctas = wgrad_ctas(c_in, c_out, K);
   int per_group_min = total_ctas / groups / 3;
   if (per_group_min < 1) per_group_min = 1;
   MM3D_REQUIRE(smem_fixed + 1024 <= 226 * 1024, MM3D_ERR_UNSUPPORTED, "tcgen05 wgrad: shared memory budget exceeded");
-  static bool once_dev[64] = {false};
-  bool& once = once_dev[mm3d_device_slot()];
+  // deterministic variant: after each launch, its slabs -> d_weight (the first piece honours `accumulate`, later
+  // pieces add to it)
+  WgReduceParams rp;
+  if (det) {
+    rp.slab = p.slab; rp.cta0 = p.slab_cta0; rp.dw = d_weight; rp.slab_cta = p.slab_cta;
+    rp.c_in = c_in; rp.c_out = c_out; rp.K = K; rp.groups = groups;
+    for (int g = 0; g < 32; ++g) rp.gmask[g] = g < groups ? p.gmask[g] : 0u;
+  }
+  const int reduce_grid = (int)mm3d_cdiv((int64_t)K * c_in * c_out / 4, 256);
+  auto reduce = [&](bool first) {
+    rp.accumulate = first ? accumulate : 1;
+    k_wgrad_reduce<<<reduce_grid < 4 * MM3D_NUM_SMS ? reduce_grid : 4 * MM3D_NUM_SMS, 256, 0, stream>>>(rp);
+    mm3d_count_launches(1);
+  };
+  static bool once_dev[2][64] = {{false}};
+  bool& once = once_dev[det][mm3d_device_slot()];
+  auto* const k_tc = det ? k_wgrad_tc<true> : k_wgrad_tc<false>;
   if (!once) {
-    MM3D_CUDA(cudaFuncSetAttribute(k_wgrad_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
-    MM3D_CUDA(cudaFuncSetAttribute(k_wgrad_tc, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    MM3D_CUDA(cudaFuncSetAttribute(k_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+    MM3D_CUDA(cudaFuncSetAttribute(k_tc, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     once = true;
   }
   // Narrow layers (one 32-channel block per item): the two-ring kernel.  MM3D_WGRAD_RINGS_NBI overrides the widest
@@ -929,11 +1072,12 @@ int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_o
   const int all_tiles = p.num_tiles;
   if (bf16) ring_nbi = 2;
   if (p.nmb == 1 && p.nbi <= ring_nbi) {
-    static bool once_r[64] = {false};
-    bool& once2 = once_r[mm3d_device_slot()];
+    static bool once_r[2][64] = {{false}};
+    bool& once2 = once_r[det][mm3d_device_slot()];
+    auto* const k_rings = det ? k_wgrad_tc_rings<true> : k_wgrad_tc_rings<false>;
     if (!once2) {
-      MM3D_CUDA(cudaFuncSetAttribute(k_wgrad_tc_rings, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
-      MM3D_CUDA(cudaFuncSetAttribute(k_wgrad_tc_rings, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+      MM3D_CUDA(cudaFuncSetAttribute(k_rings, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+      MM3D_CUDA(cudaFuncSetAttribute(k_rings, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
       once2 = true;
     }
     int gbufs = 4;
@@ -960,8 +1104,9 @@ int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_o
         p.max_items = p.n_local * gk;
         const size_t smem = fixed_r + (size_t)p.n_local * 8 + (size_t)(p.n_local + 1) * 8 + (size_t)p.max_items * 4 + 32;
         MM3D_REQUIRE(smem <= 226 * 1024, MM3D_ERR_UNSUPPORTED, "tcgen05 wgrad: shared memory budget exceeded");
-        MM3D_CUDA(mm3d_launch_pdl(k_wgrad_tc_rings, dim3((unsigned)total_ctas), dim3(kRingThreads), smem, stream, p));
+        MM3D_CUDA(mm3d_launch_pdl(k_rings, dim3((unsigned)total_ctas), dim3(kRingThreads), smem, stream, p));
         mm3d_count_launches(1);
+        if (det) reduce(start == 0);
       }
       MM3D_CHECK_LAUNCH("mm3d_conv_wgrad_tc");
       return MM3D_OK;
@@ -983,8 +1128,9 @@ int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_o
     p.num_tiles = cnt;
     p.n_local = (cnt + per_group_min - 1) / per_group_min;
     const size_t smem = smem_fixed + ((size_t)p.n_local * 8 + 15) / 16 * 16;
-    MM3D_CUDA(mm3d_launch_pdl(k_wgrad_tc, dim3((unsigned)total_ctas), dim3(kThreads), smem, stream, p));
+    MM3D_CUDA(mm3d_launch_pdl(k_tc, dim3((unsigned)total_ctas), dim3(kThreads), smem, stream, p));
     mm3d_count_launches(1);
+    if (det) reduce(start == 0);
   }
   MM3D_CHECK_LAUNCH("mm3d_conv_wgrad_tc");
   return MM3D_OK;

@@ -117,7 +117,8 @@ class UNetSCNFn(torch.autograd.Function):
         in_ch, m, L, mode, training, eps, momentum, spatial0, reps, res = cfg
         if F.deterministic():
             F.alert_not_deterministic("the whole-network UNetSCN executor (weight gradients, BatchNorm statistics, "
-                                      "point->voxel sums)")
+                                      "point->voxel sums; net.fused = False runs the module path, whose training step "
+                                      "is reproducible in the tf32, tf32x3 and bf16 modes)")
         feats = feats.float().contiguous()
         dev = feats.device
         # optional RGB mask of Net3DSeg.forward (3d_net/model.py:46-48), folded into the InputLayer scatter

@@ -250,12 +250,21 @@ class TableConvFn(torch.autograd.Function):
                                         bwd_t.tbl, bwd_t.stride, bwd_t.onehot, bwd_t.plan, bwd_t.plan_cap, bwd_flags, m,
                                         ptr(ws), ws.numel(), stream), "mm3d_conv_fwd(dgrad)")
             if ctx.needs_input_grad[1]:
-                if ctx.det:
-                    alert_not_deterministic("the sparse-convolution weight gradient")
                 d_w = torch.empty(w.shape, dtype=torch.float32, device=x.device)
-                check(lib.mm3d_conv_wgrad(ptr(x), fwd_t.n_in, c_in, ptr(d_out), fwd_t.n_out, c_out, ptr(d_w), K,
-                                          fwd_t.tbl, fwd_t.stride, fwd_t.onehot, fwd_t.plan, fwd_t.plan_cap, 0, m, ptr(ws),
-                                          ws.numel(), stream), "mm3d_conv_wgrad")
+                # deterministic form: per-CTA slabs summed in CTA order (0 bytes = none: the fp32 mode's SIMT kernel)
+                det_wsb = (lib.mm3d_conv_wgrad_workspace_bytes(fwd_t.n_out, c_in, c_out, K, m, _lib.DETERMINISTIC)
+                           if ctx.det else 0)
+                if ctx.det and not det_wsb:
+                    alert_not_deterministic("the sparse-convolution weight gradient in the fp32 mode")
+                if det_wsb:
+                    ws = scratch(max(wsb, det_wsb), x.device)
+                    check(lib.mm3d_conv_wgrad_ex(ptr(x), fwd_t.n_in, c_in, ptr(d_out), fwd_t.n_out, c_out, ptr(d_w), K,
+                                                 fwd_t.tbl, fwd_t.stride, fwd_t.onehot, fwd_t.plan, fwd_t.plan_cap, 0, m,
+                                                 ptr(ws), ws.numel(), stream, _lib.DETERMINISTIC), "mm3d_conv_wgrad_ex")
+                else:
+                    check(lib.mm3d_conv_wgrad(ptr(x), fwd_t.n_in, c_in, ptr(d_out), fwd_t.n_out, c_out, ptr(d_w), K,
+                                              fwd_t.tbl, fwd_t.stride, fwd_t.onehot, fwd_t.plan, fwd_t.plan_cap, 0, m, ptr(ws),
+                                              ws.numel(), stream), "mm3d_conv_wgrad")
         if ctx.pad:
             d_x = d_x[:, :c_in - ctx.pad] if d_x is not None else None
             d_w = d_w[..., :c_in - ctx.pad, :] if d_w is not None else None
@@ -268,20 +277,27 @@ class BatchNormReLUFn(torch.autograd.Function):
     @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
     def forward(ctx, x, gamma, beta, running_mean, running_var, eps, momentum, leakiness, training):
         _require_cuda(x, "BatchNormReLU")
-        if training and deterministic():
-            alert_not_deterministic("BatchNorm in training mode (batch statistics, gamma / beta gradients)")
         x = _f32c(x)
         n, c = x.shape
         y = torch.empty_like(x)
         save = torch.empty(2, c, dtype=torch.float32, device=x.device)
+        # deterministic: every reduction over rows (the training forward's statistics, and every backward: d_gamma /
+        # d_beta are row sums in eval mode too) in its fixed-order form
+        det = deterministic()
         with torch.cuda.device(x.device):
-            wsb = lib.mm3d_bnrelu_workspace_bytes(c)
-            ws = scratch(wsb, x.device)
-            check(lib.mm3d_bnrelu_fwd(ptr(x), ptr(y), n, c, ptr(gamma), ptr(beta), ptr(running_mean), ptr(running_var),
-                                      ptr(save[0]), ptr(save[1]), eps, momentum, leakiness, int(training), ptr(ws),
-                                      ws.numel(), _lib.stream_ptr()), "mm3d_bnrelu_fwd")
+            if det and training:
+                ws = scratch(lib.mm3d_bnrelu_workspace_bytes_ex(c, _lib.DETERMINISTIC), x.device)
+                check(lib.mm3d_bnrelu_fwd_ex(ptr(x), ptr(y), n, c, ptr(gamma), ptr(beta), ptr(running_mean),
+                                             ptr(running_var), ptr(save[0]), ptr(save[1]), eps, momentum, leakiness, 1,
+                                             ptr(ws), ws.numel(), _lib.stream_ptr(), _lib.DETERMINISTIC), "mm3d_bnrelu_fwd_ex")
+            else:
+                wsb = lib.mm3d_bnrelu_workspace_bytes(c)
+                ws = scratch(wsb, x.device)
+                check(lib.mm3d_bnrelu_fwd(ptr(x), ptr(y), n, c, ptr(gamma), ptr(beta), ptr(running_mean), ptr(running_var),
+                                          ptr(save[0]), ptr(save[1]), eps, momentum, leakiness, int(training), ptr(ws),
+                                          ws.numel(), _lib.stream_ptr()), "mm3d_bnrelu_fwd")
         ctx.save_for_backward(x, gamma, beta, save)
-        ctx.leak, ctx.training = leakiness, bool(training)
+        ctx.leak, ctx.training, ctx.det = leakiness, bool(training), det
         return y
 
     @staticmethod
@@ -293,11 +309,17 @@ class BatchNormReLUFn(torch.autograd.Function):
         dx = torch.empty_like(x)
         dgb = torch.empty(2, c, dtype=torch.float32, device=x.device)
         with torch.cuda.device(x.device):
-            wsb = lib.mm3d_bnrelu_workspace_bytes(c)
-            ws = scratch(wsb, x.device)
-            check(lib.mm3d_bnrelu_bwd(ptr(x), ptr(dy), ptr(dx), n, c, ptr(gamma), ptr(beta), ptr(save[0]), ptr(save[1]),
-                                      ptr(dgb[0]), ptr(dgb[1]), ctx.leak, int(ctx.training), ptr(ws), ws.numel(),
-                                      _lib.stream_ptr()), "mm3d_bnrelu_bwd")
+            if ctx.det:
+                ws = scratch(lib.mm3d_bnrelu_workspace_bytes_ex(c, _lib.DETERMINISTIC), x.device)
+                check(lib.mm3d_bnrelu_bwd_ex(ptr(x), ptr(dy), ptr(dx), n, c, ptr(gamma), ptr(beta), ptr(save[0]),
+                                             ptr(save[1]), ptr(dgb[0]), ptr(dgb[1]), ctx.leak, int(ctx.training), ptr(ws),
+                                             ws.numel(), _lib.stream_ptr(), _lib.DETERMINISTIC), "mm3d_bnrelu_bwd_ex")
+            else:
+                wsb = lib.mm3d_bnrelu_workspace_bytes(c)
+                ws = scratch(wsb, x.device)
+                check(lib.mm3d_bnrelu_bwd(ptr(x), ptr(dy), ptr(dx), n, c, ptr(gamma), ptr(beta), ptr(save[0]), ptr(save[1]),
+                                          ptr(dgb[0]), ptr(dgb[1]), ctx.leak, int(ctx.training), ptr(ws), ws.numel(),
+                                          _lib.stream_ptr()), "mm3d_bnrelu_bwd")
         return dx, dgb[0], dgb[1], None, None, None, None, None, None
 
 
