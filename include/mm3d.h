@@ -217,6 +217,15 @@ MM3D_API int mm3d_input_fwd_csr(const float* feats, const int32_t* vox_start, co
                        int mode, float* out_vox, mm3d_stream_t stream);
 MM3D_API int mm3d_output_bwd_csr(const float* d_out, const int32_t* vox_start, const int32_t* vox_pts, int64_t n_vox, int c,
                         float* d_vox, mm3d_stream_t stream);
+/* The masked InputLayer over those lists: every voxel row and every point's gate s_out[p] written once (no memset, no
+ * atomics); a voxel of one point gets the bits of mm3d_input_masked_fwd. */
+MM3D_API int mm3d_input_masked_fwd_csr(const float* feats, const int32_t* vox_start, const int32_t* vox_pts, int64_t n_vox,
+                              int c, int mode, const float* wb, float* out_vox, float* s_out, mm3d_stream_t stream);
+/* flags 0 = mm3d_input_masked_bwd.  MM3D_DETERMINISTIC: d_feats as there (per point); d_wb from one FP64 row per CTA
+ * summed in CTA order instead of FP64 atomics -- ws: MM3D_DET_CTAS * (c + 1) doubles. */
+MM3D_API int mm3d_input_masked_bwd_ex(const float* d_vox, const float* feats, const float* s, const int32_t* p2v,
+                             const int32_t* npts, int64_t n_points, int c, int mode, const float* wb, float* d_feats,
+                             float* d_wb, void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags);
 
 /* ------------------------------------------------------------------------------------------
  * Rule-table convolution (replaces SubmanifoldConvolution_/Convolution_/Deconvolution_
@@ -422,7 +431,7 @@ typedef struct {
   float* s;           /* [n_points] gates */
   const float* feats; /* backward only */
   float* d_wb;        /* backward only: [in_channels + 1] gradient of wb, overwritten */
-  void* ws;           /* backward only: (in_channels + 1) doubles */
+  void* ws;           /* backward only: (in_channels + 1) doubles; MM3D_DETERMINISTIC: MM3D_DET_CTAS * (in_channels + 1) */
   size_t ws_bytes;
 } mm3d_unet_mask;
 MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
@@ -444,6 +453,29 @@ MM3D_API int mm3d_unet_backward(int in_channels, int m, int num_planes, int mode
                        const float* d_out, float* d_feats, void* const* params, void* const* grads,
                        void* act, size_t act_bytes, void* tmp, size_t tmp_bytes, void* scratch,
                        size_t scratch_bytes, const mm3d_unet_mask* mask, mm3d_stream_t stream);
+/* flags 0 = the mm3d_unet_topo_* functions above (vox_start / vox_pts unused).  MM3D_DETERMINISTIC: a training step
+ * whose outputs, gradients and running statistics are the same bits on every run on one device model --
+ *   InputLayer forward and OutputLayer backward over the voxels' point lists vox_start / vox_pts (mm3d_point_csr,
+ *   required), the masked InputLayer backward's mask gradient in CTA order (mask->ws as documented there), every
+ *   BatchNorm in its deterministic form, and every weight gradient through mm3d_conv_wgrad_ex's fixed-order form with
+ *   slabs in the scratch buffer (mm3d_unet_topo_scratch_bytes_ex with the same flags).
+ * A weight gradient without such a form (mm3d_conv_wgrad_workspace_bytes(..., MM3D_DETERMINISTIC) == 0: every one of
+ * the fp32 mode, and channel counts the tcgen05 kernels do not take) runs its default kernel; the caller decides
+ * beforehand whether that is acceptable. */
+MM3D_API size_t mm3d_unet_topo_scratch_bytes_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                       int flags);
+MM3D_API int mm3d_unet_topo_forward_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                              int training, float eps, float momentum, const int64_t* level_desc, int64_t n_points,
+                              const int32_t* p2v, const int32_t* npts, const int32_t* vox_start, const int32_t* vox_pts,
+                              const float* feats, float* out, void* const* params, void* act, size_t act_bytes,
+                              void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask, mm3d_stream_t stream,
+                              int flags);
+MM3D_API int mm3d_unet_topo_backward_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                               int training, const int64_t* level_desc, int64_t n_points, const int32_t* p2v,
+                               const int32_t* npts, const int32_t* vox_start, const int32_t* vox_pts, const float* d_out,
+                               float* d_feats, void* const* params, void* const* grads, void* act, size_t act_bytes,
+                               void* tmp, size_t tmp_bytes, void* scratch, size_t scratch_bytes,
+                               const mm3d_unet_mask* mask, mm3d_stream_t stream, int flags);
 
 #ifdef __cplusplus
 }

@@ -114,6 +114,13 @@ SIGNATURES = {
     "mm3d_kl_logits_fwd_ex": (_i, [_p, _p, _i64, _i, _p, _p, _sz, _p, _i]),
     "mm3d_heads3d_fwd_ex": (_i, [_p, _i64, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _i]),
     "mm3d_heads3d_bwd_ex": (_i, [_p, _i64, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _i]),
+    "mm3d_input_masked_fwd_csr": (_i, [_p, _p, _p, _i64, _i, _i, _p, _p, _p, _p]),
+    "mm3d_input_masked_bwd_ex": (_i, [_p, _p, _p, _p, _p, _i64, _i, _i, _p, _p, _p, _p, _sz, _p, _i]),
+    "mm3d_unet_topo_scratch_bytes_ex": (_sz, [_i, _i, _i, _i, _i, _i, _i]),
+    "mm3d_unet_topo_forward_ex": (_i, [_i, _i, _i, _i, _i, _i, _i, _f, _f, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _sz,
+                                       _p, _p, _i]),
+    "mm3d_unet_topo_backward_ex": (_i, [_i, _i, _i, _i, _i, _i, _i, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _sz,
+                                        _p, _sz, _p, _p, _i]),
 }
 
 class PlanDesc(C.Structure):

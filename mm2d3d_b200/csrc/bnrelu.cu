@@ -534,6 +534,13 @@ extern "C" size_t mm3d_bnrelu_workspace_bytes_ex(int c, int flags) {
   if (!(flags & MM3D_DETERMINISTIC)) return mm3d_bnrelu_workspace_bytes(c);
   return 2 * bn_det_region_bytes(c) + sizeof(double) * 2 * (size_t)c * (size_t)bn_max_grid();
 }
+// the most channels a deterministic workspace of ws_bytes serves: a workspace shared by launches of different widths
+// (parity != NULL) lays its two regions out for this many, so that every launch agrees on where the other region is
+static int bn_det_capacity(size_t ws_bytes) {
+  int64_t c = (int64_t)(ws_bytes / (2 * sizeof(double) * (2 + (size_t)bn_max_grid())));  // (an upper bound)
+  while (c > 0 && mm3d_bnrelu_workspace_bytes_ex((int)c, MM3D_DETERMINISTIC) > ws_bytes) --c;
+  return (int)c;
+}
 
 #define BN_DISPATCH(KERNEL, ...)                                                        \
   do {                                                                                  \
@@ -552,7 +559,8 @@ extern "C" size_t mm3d_bnrelu_workspace_bytes_ex(int c, int flags) {
 // parity == NULL: the workspace is not known to be clean: zero it, use region 0.  Otherwise it is all zero (the kernels
 // leave it that way, no memset), and the launches that use it alternate between its two regions by toggling *parity,
 // which the caller keeps with the workspace.
-// det: the deterministic kernels, workspace mm3d_bnrelu_workspace_bytes_ex(c, MM3D_DETERMINISTIC), parity NULL
+// det: the deterministic kernels, workspace mm3d_bnrelu_workspace_bytes_ex(c, MM3D_DETERMINISTIC); with a parity, their
+// regions are laid out for the workspace's channel capacity (bn_det_capacity), not for this launch's c
 static int bn_fwd(const float* x, const float* x_hi, int c_lo, float* y, int64_t n, int c, const float* gamma,
                   const float* beta,
                   float* running_mean, float* running_var, float* save_mean, float* save_invstd,
@@ -568,8 +576,9 @@ static int bn_fwd(const float* x, const float* x_hi, int c_lo, float* y, int64_t
   if (n == 0) return MM3D_OK;
   // region `half` is this launch's (all zero: memset below, or zeroed by the previous launch), the other one is
   // zeroed by this launch for the next.  Region size follows the workspace size (the executor shares one workspace
-  // among layers of different widths), so consecutive launches agree on where the regions are.
-  const size_t region = det ? bn_det_region_bytes(c) : ws_bytes / 2 / 256 * 256;
+  // among layers of different widths), so consecutive launches agree on where the regions are -- in the deterministic
+  // variant through the workspace's channel capacity.
+  const size_t region = det ? bn_det_region_bytes(parity ? bn_det_capacity(ws_bytes) : c) : ws_bytes / 2 / 256 * 256;
   const int half = (parity && training) ? (*parity ^= 1) : 0;  // (only launches that use the workspace alternate)
   double* sums = (double*)((char*)ws + (size_t)half * region);
   double* other = (double*)((char*)ws + (size_t)(half ^ 1) * region);
@@ -602,9 +611,9 @@ int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, 
                          const float* beta,
                          float* running_mean, float* running_var, float* save_mean, float* save_invstd,
                          float eps, float momentum, float leakiness, int training,
-                         void* ws, size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream) {
+                         void* ws, size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream, int det) {
   return bn_fwd(x, x_hi, c_lo, y, n, c, gamma, beta, running_mean, running_var, save_mean, save_invstd, eps, momentum,
-                leakiness, training, ws, ws_bytes, parity, round_tf32, stream, false);
+                leakiness, training, ws, ws_bytes, parity, round_tf32, stream, det != 0);
 }
 
 static int bn_bwd(const float* x, const float* x_hi, int c_lo, const float* dy, float* dx, float* dx_hi,
@@ -624,7 +633,7 @@ static int bn_bwd(const float* x, const float* x_hi, int c_lo, const float* dy, 
     if (d_beta) MM3D_CUDA(cudaMemsetAsync(d_beta, 0, sizeof(float) * c, stream));
     return MM3D_OK;
   }
-  const size_t region = det ? bn_det_region_bytes(c) : ws_bytes / 2 / 256 * 256;
+  const size_t region = det ? bn_det_region_bytes(parity ? bn_det_capacity(ws_bytes) : c) : ws_bytes / 2 / 256 * 256;
   const int half = parity ? (*parity ^= 1) : 0;
   double* sums = (double*)((char*)ws + (size_t)half * region);
   double* other = (double*)((char*)ws + (size_t)(half ^ 1) * region);
@@ -651,9 +660,9 @@ int mm3d_bnrelu_bwd_impl(const float* x, const float* x_hi, int c_lo, const floa
                          int64_t n, int c, const float* gamma, const float* beta, const float* save_mean, const float* save_invstd,
                          float* d_gamma, float* d_beta, float leakiness, int training,
                          void* ws, size_t ws_bytes, int* parity, int round_flags, const float* add, int64_t add_ld,
-                         cudaStream_t stream) {
+                         cudaStream_t stream, int det) {
   return bn_bwd(x, x_hi, c_lo, dy, dx, dx_hi, n, c, gamma, beta, save_mean, save_invstd, d_gamma, d_beta, leakiness,
-                training, ws, ws_bytes, parity, round_flags, add, add_ld, stream, false);
+                training, ws, ws_bytes, parity, round_flags, add, add_ld, stream, det != 0);
 }
 
 extern "C" int mm3d_bnrelu_fwd_ex(const float* x, float* y, int64_t n, int c, const float* gamma, const float* beta,

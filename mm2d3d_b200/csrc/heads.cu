@@ -362,6 +362,16 @@ k_heads3d_bwd(const float* __restrict__ feat, int64_t n, int f, int C, const flo
 
 }  // namespace
 
+// The finalize launch of the deterministic reductions, for other files' kernels that store one row of `words` doubles per
+// CTA (the masked InputLayer backward, io_layers.cu): dst[j] = (float) sum of part[b][j] over b < nparts, in CTA order
+int mm3d_det_sum_parts(const double* part, int nparts, int words, float* dst, cudaStream_t stream) {
+  MM3D_REQUIRE(words > 0 && nparts >= 0 && nparts <= MM3D_DET_CTAS && dst, MM3D_ERR_INVALID, "det_sum_parts: bad arguments");
+  const PartOuts o = {{dst, nullptr, nullptr, nullptr}, {words, 0, 0, 0}};
+  MM3D_CUDA(mm3d_launch_pdl(k_sum_parts, dim3(1), dim3(32), 0, stream, part, nparts, words, 1.0, o));
+  mm3d_count_launches(1);
+  return MM3D_OK;
+}
+
 extern "C" {
 
 // y = x * sigmoid(x . w + b) row-wise; s_out [n] keeps the gate for the backward pass.  y may be x (in place,

@@ -11,6 +11,7 @@
 #include "common.cuh"
 
 int* mm3d_device_err_flag();  // conv_tc.cu
+int mm3d_det_sum_parts(const double* part, int nparts, int words, float* dst, cudaStream_t stream);  // heads.cu
 
 namespace {
 
@@ -107,14 +108,16 @@ k_input_masked_fwd(const float* __restrict__ feats, const int32_t* __restrict__ 
 }
 
 // backward of the above: g = d_vox[voxel] (/ count); t = (g . x) s (1 - s); d_feats = g s + t w; d_w += t x; d_b += t
-// (FP64 totals, one atomic per CTA and value, as in heads.cu)
-template <int C>
+// (FP64 totals, one atomic per CTA and value, as in heads.cu).  DET: no atomics -- the CTA's totals, its warps summed
+// in warp order, go to its own row dwb[blockIdx.x][C + 1], which mm3d_det_sum_parts (heads.cu) sums in CTA order.
+template <int C, bool DET>
 __global__ void __launch_bounds__(256)
 k_input_masked_bwd(const float* __restrict__ d_vox, const float* __restrict__ feats, const float* __restrict__ s_in,
                    const int32_t* __restrict__ p2v, const int32_t* __restrict__ npts, int64_t n_points, int mode,
                    const float* __restrict__ wb, float* __restrict__ d_feats, double* __restrict__ dwb) {
   mm3d_griddep_wait();
   __shared__ double red[C + 1];
+  __shared__ double wred[DET ? 8 : 1][C + 1];
   if (threadIdx.x <= C) red[threadIdx.x] = 0.0;
   __syncthreads();
   float w[C];
@@ -148,10 +151,21 @@ k_input_masked_bwd(const float* __restrict__ d_vox, const float* __restrict__ fe
   for (int j = 0; j <= C; ++j) {
     double vv = loc[j];
     for (int o = 16; o; o >>= 1) vv += __shfl_xor_sync(0xffffffffu, vv, o);
-    if ((threadIdx.x & 31) == 0) atomicAdd(&red[j], vv);
+    if ((threadIdx.x & 31) == 0) {
+      if (DET) wred[threadIdx.x >> 5][j] = vv;
+      else atomicAdd(&red[j], vv);
+    }
   }
   __syncthreads();
-  if (threadIdx.x <= C) atomicAdd(dwb + threadIdx.x, red[threadIdx.x]);
+  if (threadIdx.x <= C) {
+    if (DET) {  // 256 threads = 8 warps
+      double t = 0.0;
+      for (int w = 0; w < 8; ++w) t += wred[w][threadIdx.x];
+      dwb[(int64_t)blockIdx.x * (C + 1) + threadIdx.x] = t;
+    } else {
+      atomicAdd(dwb + threadIdx.x, red[threadIdx.x]);
+    }
+  }
 }
 
 __global__ void k_f64_to_f32_io(const double* __restrict__ src, float* __restrict__ dst, int n) {
@@ -410,6 +424,45 @@ k_input_fwd_csr(const float* __restrict__ feats, const int32_t* __restrict__ vst
   }
 }
 
+// InputLayer forward with the RGB mask folded in (k_input_masked_fwd): one thread per voxel writes its row and the gates
+// of its points (every point is in exactly one list).  The gate and the terms y / cnt are computed as there and summed in
+// point order, so a voxel of one point gets exactly the bits of the default path.
+template <int C>
+__global__ void __launch_bounds__(256)
+k_input_masked_fwd_csr(const float* __restrict__ feats, const int32_t* __restrict__ vstart, const int32_t* __restrict__ vpts,
+                       int64_t n_vox, int mode, const float* __restrict__ wb, float* __restrict__ out,
+                       float* __restrict__ s_out) {
+  mm3d_griddep_wait();
+  float w[C + 1];
+#pragma unroll
+  for (int j = 0; j <= C; ++j) w[j] = __ldg(wb + j);
+  for (int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; v < n_vox; v += (int64_t)gridDim.x * blockDim.x) {
+    const int32_t b = __ldg(vstart + v), e = __ldg(vstart + v + 1), cnt = e - b;
+    float acc[C];
+#pragma unroll
+    for (int j = 0; j < C; ++j) acc[j] = 0.f;
+    for (int32_t q = b; q < e; ++q) {
+      const int64_t p = __ldg(vpts + q);
+      float f[C], a = w[C];
+#pragma unroll
+      for (int j = 0; j < C; ++j) {
+        f[j] = __ldg(feats + p * C + j);
+        a = fmaf(f[j], w[j], a);
+      }
+      const float sg = 1.f / (1.f + expf(-a));
+      s_out[p] = sg;
+#pragma unroll
+      for (int j = 0; j < C; ++j) {
+        const float y = f[j] * sg;
+        if (cnt == 1) acc[j] = y;
+        else acc[j] += mode == 4 ? y / (float)cnt : y;
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < C; ++j) out[v * C + j] = acc[j];
+  }
+}
+
 // OutputLayer backward: a voxel's gradient = the sum of its points' gradients, in point order
 __global__ void __launch_bounds__(256)
 k_output_bwd_csr(const float* __restrict__ d_out, const int32_t* __restrict__ vstart, const int32_t* __restrict__ vpts,
@@ -558,17 +611,35 @@ extern "C" int mm3d_input_masked_fwd(const float* feats, const int32_t* p2v, con
 
 // ... and its backward: d_feats [n_points, c] (may be NULL: the features are data), d_wb [c + 1] = d_w, d_b
 // (overwritten); feats = the UNMASKED features, s = the gates of the forward; ws: (c + 1) doubles
-extern "C" int mm3d_input_masked_bwd(const float* d_vox, const float* feats, const float* s, const int32_t* p2v,
-                                     const int32_t* npts, int64_t n_points, int c, int mode, const float* wb, float* d_feats,
-                                     float* d_wb, void* ws, size_t ws_bytes, mm3d_stream_t stream_) {
+// (flags MM3D_DETERMINISTIC: MM3D_DET_CTAS * (c + 1) doubles, one row per CTA, summed in CTA order by a second launch)
+extern "C" int mm3d_input_masked_bwd_ex(const float* d_vox, const float* feats, const float* s, const int32_t* p2v,
+                                        const int32_t* npts, int64_t n_points, int c, int mode, const float* wb, float* d_feats,
+                                        float* d_wb, void* ws, size_t ws_bytes, mm3d_stream_t stream_, int flags) {
   cudaStream_t stream = (cudaStream_t)stream_;
   MM3D_REQUIRE(mode == 3 || mode == 4, MM3D_ERR_UNSUPPORTED, "InputLayer mode %d not implemented", mode);
   MM3D_REQUIRE(c == 3, MM3D_ERR_UNSUPPORTED, "masked InputLayer: 3 feature channels supported, got %d", c);
-  MM3D_REQUIRE(d_wb && wb && ws && ws_bytes >= sizeof(double) * (size_t)(c + 1), MM3D_ERR_WORKSPACE, "masked InputLayer: workspace too small");
+  MM3D_REQUIRE((flags & ~MM3D_DETERMINISTIC) == 0, MM3D_ERR_INVALID, "masked InputLayer: unknown flags %#x", flags);
+  const bool det = flags & MM3D_DETERMINISTIC;
+  MM3D_REQUIRE(d_wb && wb && ws && ws_bytes >= sizeof(double) * (size_t)(c + 1) * (det ? MM3D_DET_CTAS : 1), MM3D_ERR_WORKSPACE,
+               "masked InputLayer: workspace too small");
+  if (det) {
+    const int64_t g = mm3d_grid(n_points, 256, 8);
+    const int grid = n_points > 0 ? (int)(g < MM3D_DET_CTAS ? g : MM3D_DET_CTAS) : 0;
+    if (n_points > 0) {
+      MM3D_REQUIRE(d_vox && feats && s, MM3D_ERR_INVALID, "masked InputLayer: null pointer");
+      MM3D_CUDA(mm3d_launch_pdl(k_input_masked_bwd<3, true>, dim3(grid), dim3(256), 0, stream, d_vox, feats, s, p2v, npts,
+                                n_points, mode, wb, d_feats, (double*)ws));
+      mm3d_count_launches(1);
+    }
+    const int rc = mm3d_det_sum_parts((const double*)ws, grid, c + 1, d_wb, stream);
+    if (rc) return rc;
+    MM3D_CHECK_LAUNCH("mm3d_input_masked_bwd_ex");
+    return MM3D_OK;
+  }
   MM3D_CUDA(cudaMemsetAsync(ws, 0, sizeof(double) * (size_t)(c + 1), stream));
   if (n_points > 0) {
     MM3D_REQUIRE(d_vox && feats && s, MM3D_ERR_INVALID, "masked InputLayer: null pointer");
-    MM3D_CUDA(mm3d_launch_pdl(k_input_masked_bwd<3>, dim3(mm3d_grid(n_points, 256, 8)), dim3(256), 0, stream, d_vox, feats, s, p2v, npts,
+    MM3D_CUDA(mm3d_launch_pdl(k_input_masked_bwd<3, false>, dim3(mm3d_grid(n_points, 256, 8)), dim3(256), 0, stream, d_vox, feats, s, p2v, npts,
                               n_points, mode, wb, d_feats, (double*)ws));
     mm3d_count_launches(1);
   }
@@ -576,6 +647,12 @@ extern "C" int mm3d_input_masked_bwd(const float* d_vox, const float* feats, con
   mm3d_count_launches(1);
   MM3D_CHECK_LAUNCH("mm3d_input_masked_bwd");
   return MM3D_OK;
+}
+
+extern "C" int mm3d_input_masked_bwd(const float* d_vox, const float* feats, const float* s, const int32_t* p2v,
+                                     const int32_t* npts, int64_t n_points, int c, int mode, const float* wb, float* d_feats,
+                                     float* d_wb, void* ws, size_t ws_bytes, mm3d_stream_t stream) {
+  return mm3d_input_masked_bwd_ex(d_vox, feats, s, p2v, npts, n_points, c, mode, wb, d_feats, d_wb, ws, ws_bytes, stream, 0);
 }
 
 extern "C" int mm3d_output_fwd(const float* vox, const int32_t* p2v, int64_t n_points, int c, float* out,
@@ -708,6 +785,22 @@ extern "C" int mm3d_input_fwd_csr(const float* feats, const int32_t* vox_start, 
                             vox_pts, n_vox, c, mode, out_vox));
   mm3d_count_launches(1);
   MM3D_CHECK_LAUNCH("mm3d_input_fwd_csr");
+  return MM3D_OK;
+}
+
+// mm3d_input_masked_fwd over the voxel point lists: one thread per voxel row, no memset, no atomics
+extern "C" int mm3d_input_masked_fwd_csr(const float* feats, const int32_t* vox_start, const int32_t* vox_pts, int64_t n_vox,
+                                         int c, int mode, const float* wb, float* out_vox, float* s_out, mm3d_stream_t stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  MM3D_REQUIRE(mode == 3 || mode == 4, MM3D_ERR_UNSUPPORTED, "InputLayer mode %d not implemented (3=sum, 4=mean)", mode);
+  MM3D_REQUIRE(c == 3, MM3D_ERR_UNSUPPORTED, "masked InputLayer: 3 feature channels supported, got %d", c);
+  MM3D_REQUIRE(n_vox >= 0 && wb, MM3D_ERR_INVALID, "masked input_fwd_csr: bad arguments");
+  if (n_vox == 0) return MM3D_OK;
+  MM3D_REQUIRE(feats && vox_start && vox_pts && out_vox && s_out, MM3D_ERR_INVALID, "masked input_fwd_csr: null pointer");
+  MM3D_CUDA(mm3d_launch_pdl(k_input_masked_fwd_csr<3>, dim3(mm3d_grid(n_vox, 256, 16)), dim3(256), 0, stream, feats, vox_start,
+                            vox_pts, n_vox, mode, wb, out_vox, s_out));
+  mm3d_count_launches(1);
+  MM3D_CHECK_LAUNCH("mm3d_input_masked_fwd_csr");
   return MM3D_OK;
 }
 

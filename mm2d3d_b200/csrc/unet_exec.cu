@@ -34,12 +34,12 @@
 int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, int64_t n, int c, const float* gamma,
                          const float* beta, float* running_mean, float* running_var, float* save_mean,
                          float* save_invstd, float eps, float momentum, float leakiness, int training, void* ws,
-                         size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream);
+                         size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream, int det);
 int mm3d_bnrelu_bwd_impl(const float* x, const float* x_hi, int c_lo, const float* dy, float* dx, float* dx_hi,
                          int64_t n, int c, const float* gamma, const float* beta, const float* save_mean,
                          const float* save_invstd, float* d_gamma, float* d_beta, float leakiness, int training,
                          void* ws, size_t ws_bytes, int* parity, int round_flags, const float* add, int64_t add_ld,
-                         cudaStream_t stream);
+                         cudaStream_t stream, int det);
 
 // conv_tc.cu
 size_t mm3d_conv_tc_workspace_bytes(int c_in, int c_out, int K);
@@ -114,6 +114,7 @@ struct Net {
   int L, m, cin, cin_k;  // cin_k = stem input channels as seen by the kernels (padded to 16 in TC modes)
   int reps, res;         // blocks per pre / post group; residual blocks
   int mode;
+  int flags;  // MM3D_DETERMINISTIC or 0
   std::vector<LevelMeta> lv;
   std::vector<LevelBufs> b;
   float *V, *Vp, *Z, *s_head;
@@ -122,13 +123,16 @@ struct Net {
   int head, n_params;                     // the head BatchNorm's first parameter slot; the number of slots
   std::vector<ConvInfo> convs;            // every convolution, in slot order
   size_t bn_channels = 0;                 // of all BatchNorms (each has a gamma and a beta gradient)
-  // The scratch buffer: [convolution workspace | weight images | BatchNorm workspace | padded stem weight].  Weight
-  // images (tensor-core modes): every layer's, for this call's direction, built by one launch up front.  BatchNorm
-  // workspace: totals and barrier counters, zeroed at the start of each call; the kernels keep it clean.
-  void *conv_ws, *img_ws, *bn_ws;
-  size_t conv_ws_bytes, img_ws_bytes, bn_ws_bytes;
+  // The scratch buffer: [convolution workspace | weight images | BatchNorm workspace | padded stem weight], and in the
+  // deterministic mode behind that [deterministic BatchNorm workspace | weight-gradient slabs].  Weight images
+  // (tensor-core modes): every layer's, for this call's direction, built by one launch up front.  BatchNorm workspace:
+  // totals and barrier counters, zeroed at the start of each call; the kernels keep it clean.  Weight-gradient slabs:
+  // one region for the largest convolution -- every weight gradient runs on one stream, one after the other.
+  void *conv_ws, *img_ws, *bn_ws, *wg_ws = nullptr;
+  size_t conv_ws_bytes, img_ws_bytes, bn_ws_bytes, wg_ws_bytes = 0;
   float* wp;  // the stem weight with zeros for the padded input channels (cin_k != cin only)
   int64_t n_points;
+  bool det() const { return (flags & MM3D_DETERMINISTIC) != 0; }
   int planes(int l) const { return m * (l + 1); }
   // TF32x3 mode: every tensor a convolution gathers carries a hi and a lo plane ([rows, c] floats each)
   // BF16 mode: an FP32 plane (TF32-rounded: the weight-gradient operand) and a BF16 plane behind it (what forward and
@@ -278,6 +282,17 @@ void carve_scratch(Net& net, Bump& bp) {
   net.bn_ws_bytes = mm3d_bnrelu_workspace_bytes(2 * net.m * net.L);
   net.bn_ws = bp.bytes(net.bn_ws_bytes);
   net.wp = net.cin_k != net.cin ? bp.f(27, (int64_t)net.cin_k * net.m) : nullptr;
+  if (!net.det()) return;
+  // (behind the default layout, which stays as it is; the default BatchNorm workspace is then unused)
+  net.bn_ws_bytes = mm3d_bnrelu_workspace_bytes_ex(2 * net.m * net.L, MM3D_DETERMINISTIC);
+  net.bn_ws = bp.bytes(net.bn_ws_bytes);
+  size_t wg = 0;
+  for (const ConvInfo& ci : net.convs) {  // (0 for a convolution without a deterministic form: it keeps the default)
+    const size_t s = mm3d_conv_wgrad_workspace_bytes(0, ci.c_in, ci.c_out, ci.K, net.mode, MM3D_DETERMINISTIC);
+    if (s > wg) wg = s;
+  }
+  net.wg_ws_bytes = wg;
+  net.wg_ws = bp.bytes(wg);
 }
 
 // Identity row plans (NetworkInNetwork as a K = 1 rule-table convolution): perm = iota (-1 past the rows), one
@@ -487,7 +502,7 @@ void bn_fwd(Ctx& c, int pidx, const float* x, float* y, int64_t n, int ch, float
   if (abl_skip("bn")) return;
   EX(mm3d_bnrelu_fwd_impl(x, x_hi, c_lo, y, n, ch, P(c, pidx), P(c, pidx + 1), (float*)c.params[pidx + 2], (float*)c.params[pidx + 3],
                           save, save + ch, c.eps, c.momentum, 0.f, c.training, c.net->bn_ws, c.net->bn_ws_bytes, &c.bn_parity,
-                          tc_mode(c) && to_conv ? c.net->rmode() : 0, c.stream));
+                          tc_mode(c) && to_conv ? c.net->rmode() : 0, c.stream, c.net->det()));
 }
 // round: bit 0 = dx (its low column block when split) feeds a convolution as d_out, bit 1 = dx_hi does
 // add (rows add_ld floats apart): another gradient of the same tensor, summed into dx before it is stored;
@@ -498,7 +513,7 @@ void bn_bwd(Ctx& c, int pidx, const float* x, const float* dy, float* dx, int64_
   if (abl_skip("bn")) return;
   const int flags = tc_mode(c) ? (round | (c.net->x3() ? 4 : c.net->bf16() ? 8 : 0) | (add_lo ? 16 : 0)) : 0;
   EX(mm3d_bnrelu_bwd_impl(x, x_hi, c_lo, dy, dx, dx_hi, n, ch, P(c, pidx), P(c, pidx + 1), save, save + ch, Gp(c, pidx), Gp(c, pidx + 1), 0.f,
-                          c.training, c.net->bn_ws, c.net->bn_ws_bytes, &c.bn_parity, flags, add, add_ld, c.stream));
+                          c.training, c.net->bn_ws, c.net->bn_ws_bytes, &c.bn_parity, flags, add, add_ld, c.stream, c.net->det()));
 }
 // NIN: NetworkInNetwork, a K = 1 convolution over the level's identity row plan
 enum Kind { SMC, DOWN, UP, NIN };
@@ -588,7 +603,13 @@ void conv_bwd(Ctx& c, Kind kind, int l, const float* in, int c_in, const float* 
   // The weight gradient (side stream) is enqueued before the data gradient.  (Measured with the in-process A/B of
   // bench.py on the final kernels: the order makes no difference, 2.959 vs 2.958 ms per step -- the step is bound by
   // the total work of both streams, not by which kernel gets the SMs first.)
-  if (do_wg)
+  // Deterministic mode: the fixed-order form through the slab region wherever the shape has one (the caller learns
+  // beforehand which do not: the fp32 mode, channels that are not multiples of 16); the others keep the default.
+  const bool det_wg = c.net->det() && mm3d_conv_wgrad_workspace_bytes(t.n_out, c_in, c_out, t.K, md, MM3D_DETERMINISTIC) > 0;
+  if (do_wg && det_wg)
+    EX(mm3d_conv_wgrad_ex(in, t.n_in, c_in, d_out, t.n_out, c_out, d_w, t.K, t.tbl, t.stride, t.onehot, t.plan, t.cap, acc,
+                          md, c.net->wg_ws, c.net->wg_ws_bytes, ws, MM3D_DETERMINISTIC));
+  else if (do_wg)
     EX(mm3d_conv_wgrad(in, t.n_in, c_in, d_out, t.n_out, c_out, d_w, t.K, t.tbl, t.stride, t.onehot, t.plan, t.cap, acc,
                        md, nullptr, 0, ws));
   if (im && do_dg)
@@ -842,14 +863,15 @@ void level_bwd(Ctx& c, int l, const float* d_R) {
 }
 
 int fill_net(Net& net, int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
-             const int64_t* level_desc, int64_t n_points) {
+             const int64_t* level_desc, int64_t n_points, int flags = 0) {
+  MM3D_REQUIRE((flags & ~MM3D_DETERMINISTIC) == 0, MM3D_ERR_INVALID, "unet: unknown flags %#x", flags);
   MM3D_REQUIRE(num_planes >= 1 && num_planes <= 16 && m > 0 && in_channels > 0, MM3D_ERR_INVALID, "bad network shape");
   MM3D_REQUIRE(block_reps >= 1 && block_reps <= 16 && (residual == 0 || residual == 1), MM3D_ERR_INVALID,
                "bad block topology: block_reps %d residual %d", block_reps, residual);
   MM3D_REQUIRE(mode == MM3D_MODE_FP32 || mode == MM3D_MODE_TF32 || mode == MM3D_MODE_TF32X3 || mode == MM3D_MODE_BF16, MM3D_ERR_UNSUPPORTED,
                "conv mode %d not implemented in this build", mode);
   net.L = num_planes; net.m = m; net.cin = in_channels; net.mode = mode; net.n_points = n_points;
-  net.reps = block_reps; net.res = residual;
+  net.reps = block_reps; net.res = residual; net.flags = flags;
   // tensor-core kernels gather rows in 64-byte pieces: pad the stem input to a multiple of 16 channels
   net.cin_k = in_channels;
   if (mode != MM3D_MODE_FP32) net.cin_k = (in_channels + 15) / 16 * 16;
@@ -909,24 +931,31 @@ MM3D_API size_t mm3d_unet_bwd_bytes(int in_channels, int m, int num_planes, int 
   return mm3d_unet_topo_bwd_bytes(in_channels, m, num_planes, 1, 0, mode, level_desc, n_points);
 }
 
-MM3D_API size_t mm3d_unet_topo_scratch_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode) {
+MM3D_API size_t mm3d_unet_topo_scratch_bytes_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                               int flags) {
   Net net;
-  if (fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, nullptr, 0)) return 0;
+  if (fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, nullptr, 0, flags)) return 0;
   return lay_out(net, nullptr, nullptr, nullptr).scratch;  // (independent of the row counts)
+}
+MM3D_API size_t mm3d_unet_topo_scratch_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode) {
+  return mm3d_unet_topo_scratch_bytes_ex(in_channels, m, num_planes, block_reps, residual, mode, 0);
 }
 MM3D_API size_t mm3d_unet_scratch_bytes(int in_channels, int m, int num_planes, int mode) {
   return mm3d_unet_topo_scratch_bytes(in_channels, m, num_planes, 1, 0, mode);
 }
 
-MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
-                                    int training, float eps, float momentum, const int64_t* level_desc, int64_t n_points,
-                                    const int32_t* p2v, const int32_t* npts, const float* feats, float* out,
-                                    void* const* params, void* act, size_t act_bytes, void* scratch, size_t scratch_bytes,
-                                    const mm3d_unet_mask* mask, mm3d_stream_t stream_) {
+MM3D_API int mm3d_unet_topo_forward_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                       int training, float eps, float momentum, const int64_t* level_desc, int64_t n_points,
+                                       const int32_t* p2v, const int32_t* npts, const int32_t* vox_start,
+                                       const int32_t* vox_pts, const float* feats, float* out, void* const* params, void* act,
+                                       size_t act_bytes, void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask,
+                                       mm3d_stream_t stream_, int flags) {
   MM3D_REQUIRE(level_desc, MM3D_ERR_INVALID, "unet forward: no level descriptors");
   MM3D_REQUIRE(!mask || (mask->wb && (n_points == 0 || mask->s)), MM3D_ERR_INVALID, "unet forward: incomplete mask descriptor");
+  MM3D_REQUIRE(!(flags & MM3D_DETERMINISTIC) || (vox_start && vox_pts), MM3D_ERR_INVALID,
+               "unet forward: the deterministic mode needs the voxels' point lists (mm3d_point_csr)");
   Net net;
-  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points);
+  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points, flags);
   if (rc) return rc;
   const Sizes need = lay_out(net, act, nullptr, scratch);  // (no backward temporaries)
   MM3D_REQUIRE(act_bytes >= need.act, MM3D_ERR_WORKSPACE, "activation workspace too small: need %zu have %zu", need.act, act_bytes);
@@ -937,7 +966,12 @@ MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int 
   const int64_t n0 = net.lv[0].n;
   MARK("fwd start", -1);
   if (mask) {  // the RGB-mask prologue of Net3DSeg.forward folded into the point -> voxel scatter
-    EX(mm3d_input_masked_fwd(feats, p2v, npts, n_points, n0, in_channels, 4, mask->wb, net.V, mask->s, c.stream));
+    if (net.det())
+      EX(mm3d_input_masked_fwd_csr(feats, vox_start, vox_pts, n0, in_channels, 4, mask->wb, net.V, mask->s, c.stream));
+    else
+      EX(mm3d_input_masked_fwd(feats, p2v, npts, n_points, n0, in_channels, 4, mask->wb, net.V, mask->s, c.stream));
+  } else if (net.det()) {
+    EX(mm3d_input_fwd_csr(feats, vox_start, vox_pts, n0, in_channels, 4, net.V, c.stream));
   } else {
     EX(mm3d_input_fwd(feats, p2v, npts, n_points, n0, in_channels, 4, net.V, c.stream));
   }
@@ -967,6 +1001,16 @@ MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int 
   return c.rc;
 }
 
+MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                    int training, float eps, float momentum, const int64_t* level_desc, int64_t n_points,
+                                    const int32_t* p2v, const int32_t* npts, const float* feats, float* out,
+                                    void* const* params, void* act, size_t act_bytes, void* scratch, size_t scratch_bytes,
+                                    const mm3d_unet_mask* mask, mm3d_stream_t stream_) {
+  return mm3d_unet_topo_forward_ex(in_channels, m, num_planes, block_reps, residual, mode, training, eps, momentum, level_desc,
+                                   n_points, p2v, npts, nullptr, nullptr, feats, out, params, act, act_bytes, scratch,
+                                   scratch_bytes, mask, stream_, 0);
+}
+
 MM3D_API int mm3d_unet_forward(int in_channels, int m, int num_planes, int mode, int training, float eps, float momentum,
                                const int64_t* level_desc, int64_t n_points, const int32_t* p2v, const int32_t* npts,
                                const float* feats, float* out, void* const* params, void* act, size_t act_bytes,
@@ -976,17 +1020,22 @@ MM3D_API int mm3d_unet_forward(int in_channels, int m, int num_planes, int mode,
 }
 
 // grads: same slot order as params (running-stat slots ignored); d_feats may be NULL.
-MM3D_API int mm3d_unet_topo_backward(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
-                                     int training, const int64_t* level_desc, int64_t n_points, const int32_t* p2v,
-                                     const int32_t* npts, const float* d_out, float* d_feats, void* const* params,
-                                     void* const* grads, void* act, size_t act_bytes, void* tmp, size_t tmp_bytes,
-                                     void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask,
-                                     mm3d_stream_t stream_) {
+MM3D_API int mm3d_unet_topo_backward_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                        int training, const int64_t* level_desc, int64_t n_points, const int32_t* p2v,
+                                        const int32_t* npts, const int32_t* vox_start, const int32_t* vox_pts,
+                                        const float* d_out, float* d_feats, void* const* params, void* const* grads, void* act,
+                                        size_t act_bytes, void* tmp, size_t tmp_bytes, void* scratch, size_t scratch_bytes,
+                                        const mm3d_unet_mask* mask, mm3d_stream_t stream_, int flags) {
   MM3D_REQUIRE(level_desc, MM3D_ERR_INVALID, "unet backward: no level descriptors");
   MM3D_REQUIRE(!mask || (mask->wb && mask->d_wb && mask->ws && (n_points == 0 || (mask->s && mask->feats))), MM3D_ERR_INVALID,
                "unet backward: incomplete mask descriptor");
+  MM3D_REQUIRE(!(flags & MM3D_DETERMINISTIC) || (vox_start && vox_pts), MM3D_ERR_INVALID,
+               "unet backward: the deterministic mode needs the voxels' point lists (mm3d_point_csr)");
+  MM3D_REQUIRE(!(flags & MM3D_DETERMINISTIC) || !mask || mask->ws_bytes >= sizeof(double) * MM3D_DET_CTAS * (in_channels + 1),
+               MM3D_ERR_WORKSPACE, "unet backward: the deterministic mode's mask workspace needs %d doubles",
+               MM3D_DET_CTAS * (in_channels + 1));
   Net net;
-  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points);
+  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points, flags);
   if (rc) return rc;
   const Sizes need = lay_out(net, act, tmp, scratch);
   MM3D_REQUIRE(act_bytes >= need.act, MM3D_ERR_WORKSPACE, "activation workspace too small: need %zu have %zu", need.act, act_bytes);
@@ -1026,7 +1075,10 @@ MM3D_API int mm3d_unet_topo_backward(int in_channels, int m, int num_planes, int
     EX(build_images(c, true, w_stem_k));
   }
   MARK("bwd start (memset, images)", -1);
-  EX(mm3d_output_bwd(d_out, p2v, n_points, n0, m, net.d_Z, c.stream));
+  if (net.det())
+    EX(mm3d_output_bwd_csr(d_out, vox_start, vox_pts, n0, m, net.d_Z, c.stream));
+  else
+    EX(mm3d_output_bwd(d_out, p2v, n_points, n0, m, net.d_Z, c.stream));
   MARK("output_bwd", -1);
   bn_bwd(c, net.head, net.b[0].R, net.d_Z, net.d_R0, n0, m, net.s_head, 1);
   MARK("bn_bwd head", -1);
@@ -1038,8 +1090,8 @@ MM3D_API int mm3d_unet_topo_backward(int in_channels, int m, int num_planes, int
   float* d_Vp = need_dv ? net.d_Vp : nullptr;
   auto input_bwd = [&](const float* d_v) {
     if (mask)
-      EX(mm3d_input_masked_bwd(d_v, mask->feats, mask->s, p2v, npts, n_points, net.cin, 4, mask->wb, d_feats, mask->d_wb,
-                               mask->ws, mask->ws_bytes, c.stream));
+      EX(mm3d_input_masked_bwd_ex(d_v, mask->feats, mask->s, p2v, npts, n_points, net.cin, 4, mask->wb, d_feats, mask->d_wb,
+                                  mask->ws, mask->ws_bytes, c.stream, net.flags));
     else
       EX(mm3d_input_bwd(d_v, p2v, npts, n_points, net.cin, 4, d_feats, c.stream));
   };
@@ -1060,6 +1112,17 @@ MM3D_API int mm3d_unet_topo_backward(int in_channels, int m, int num_planes, int
   join_side(c);  // everything after this call on `stream` sees the weight gradients
   MARK("join wgrad stream", -1);
   return c.rc;
+}
+
+MM3D_API int mm3d_unet_topo_backward(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                     int training, const int64_t* level_desc, int64_t n_points, const int32_t* p2v,
+                                     const int32_t* npts, const float* d_out, float* d_feats, void* const* params,
+                                     void* const* grads, void* act, size_t act_bytes, void* tmp, size_t tmp_bytes,
+                                     void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask,
+                                     mm3d_stream_t stream_) {
+  return mm3d_unet_topo_backward_ex(in_channels, m, num_planes, block_reps, residual, mode, training, level_desc, n_points,
+                                    p2v, npts, nullptr, nullptr, d_out, d_feats, params, grads, act, act_bytes, tmp,
+                                    tmp_bytes, scratch, scratch_bytes, mask, stream_, 0);
 }
 
 MM3D_API int mm3d_unet_backward(int in_channels, int m, int num_planes, int mode, int training,

@@ -8,10 +8,17 @@ not implement (per-layer conv modes, conv or NetworkInNetwork bias, leaky ReLU) 
 Results are the same kernels in the same order, so parity is unchanged; the one exception is the
 residual blocks' NetworkInNetwork, which the module path runs as an FP32 torch matmul and the executor
 as this library's K = 1 rule-table convolution in the network's convolution mode.
+
+Deterministic mode (``scn.set_deterministic``, or ``torch.use_deterministic_algorithms``), read at the forward and
+kept by its backward: the executor then sums the InputLayer and OutputLayer over the voxels' point lists, runs every
+BatchNorm and the masked InputLayer's mask gradient in their fixed-order forms and every weight gradient through the
+fixed-order tcgen05 form, so a training step in the ``tf32``, ``tf32x3`` and ``bf16`` modes is the same bits on every
+run.  The ``fp32`` mode's weight gradients (the SIMT kernel) have no such form: there the step warns.
 """
 from __future__ import annotations
 
 import ctypes as C
+import functools
 
 import torch
 
@@ -80,6 +87,26 @@ def _fusable(net) -> bool:
     return True
 
 
+@functools.lru_cache(maxsize=None)
+def wgrad_covered(in_ch: int, m: int, L: int, residual: int, mode: int) -> bool:
+    """Whether every weight gradient of this network shape has a deterministic form (the tcgen05 kernel takes it):
+    never in the fp32 mode; in the tensor-core modes for the usual widths (multiples of 16).  The executor runs the
+    default kernel for a shape without one, so the caller warns."""
+    if mode == _lib.MODE_FP32:
+        return False
+    cin_k = (in_ch + 15) // 16 * 16  # the stem input as the kernels see it (padded)
+    shapes = {(cin_k, m, 27)}
+    for l in range(L):
+        p = m * (l + 1)
+        shapes.add((p, p, 27))
+        if l + 1 < L:
+            q = m * (l + 2)
+            shapes |= {(p, q, 8), (q, p, 8), (2 * p, p, 27)}
+            if residual:
+                shapes.add((2 * p, p, 1))  # NetworkInNetwork of the first post block
+    return all(lib.mm3d_conv_wgrad_workspace_bytes(0, ci, co, K, mode, _lib.DETERMINISTIC) > 0 for ci, co, K in shapes)
+
+
 def _level_desc(meta: Metadata, num_planes: int, spatial0: int, plans: bool):
     W = _lib.LEVEL_DESC_WORDS
     desc = (C.c_int64 * (W * num_planes))()
@@ -115,10 +142,12 @@ class UNetSCNFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, feats, meta, cfg, mask_w, mask_b, *slots):
         in_ch, m, L, mode, training, eps, momentum, spatial0, reps, res = cfg
-        if F.deterministic():
-            F.alert_not_deterministic("the whole-network UNetSCN executor (weight gradients, BatchNorm statistics, "
-                                      "point->voxel sums; net.fused = False runs the module path, whose training step "
-                                      "is reproducible in the tf32, tf32x3 and bf16 modes)")
+        det = F.deterministic()
+        if det and not wgrad_covered(in_ch, m, L, res, mode):
+            F.alert_not_deterministic("the sparse-convolution weight gradient in the fp32 mode" if mode == _lib.MODE_FP32
+                                      else f"the sparse-convolution weight gradient with m = {m} (channel counts that "
+                                           "are not multiples of 16)")
+        flags = _lib.DETERMINISTIC if det else 0
         feats = feats.float().contiguous()
         dev = feats.device
         # optional RGB mask of Net3DSeg.forward (3d_net/model.py:46-48), folded into the InputLayer scatter
@@ -133,18 +162,28 @@ class UNetSCNFn(torch.autograd.Function):
             _lib.raise_device_errors("UNetSCN.forward")
             act_bytes = lib.mm3d_unet_topo_act_bytes(in_ch, m, L, reps, res, mode, desc, n_points)
             act = torch.empty(act_bytes, dtype=torch.uint8, device=dev)
-            scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes(in_ch, m, L, reps, res, mode), dev)
+            scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes_ex(in_ch, m, L, reps, res, mode, flags), dev)
             out = torch.empty(n_points, m, dtype=torch.float32, device=dev)
+            vox_start, vox_pts = meta.point_csr() if det else (None, None)
             params = (C.c_void_p * len(slots))(*[t.data_ptr() for t in slots])
             mask, wb, gate = None, None, None
             if masked:
                 wb = torch.cat([mask_w.detach().reshape(-1), mask_b.detach().reshape(-1)]).float().contiguous()
                 gate = torch.empty(max(n_points, 1), dtype=torch.float32, device=dev)
                 mask = C.byref(_lib.UnetMask(wb.data_ptr(), gate.data_ptr(), None, None, None, 0))
-            check(lib.mm3d_unet_topo_forward(in_ch, m, L, reps, res, mode, int(training), eps, momentum, desc, n_points, meta.p2v_ptr,
-                                        meta.npts_ptr, feats.data_ptr(), out.data_ptr(), params, act.data_ptr(), act_bytes,
-                                        scr.data_ptr(), scr.numel(), mask, _lib.stream_ptr()), "mm3d_unet_topo_forward")
+            if det:
+                check(lib.mm3d_unet_topo_forward_ex(in_ch, m, L, reps, res, mode, int(training), eps, momentum, desc, n_points,
+                                                    meta.p2v_ptr, meta.npts_ptr, vox_start.data_ptr(), vox_pts.data_ptr(),
+                                                    feats.data_ptr(), out.data_ptr(), params, act.data_ptr(), act_bytes,
+                                                    scr.data_ptr(), scr.numel(), mask, _lib.stream_ptr(), flags),
+                      "mm3d_unet_topo_forward_ex")
+            else:
+                check(lib.mm3d_unet_topo_forward(in_ch, m, L, reps, res, mode, int(training), eps, momentum, desc, n_points,
+                                                 meta.p2v_ptr, meta.npts_ptr, feats.data_ptr(), out.data_ptr(), params,
+                                                 act.data_ptr(), act_bytes, scr.data_ptr(), scr.numel(), mask,
+                                                 _lib.stream_ptr()), "mm3d_unet_topo_forward")
         ctx.meta, ctx.cfg, ctx.desc, ctx.act, ctx.slots = meta, cfg, desc, act, slots
+        ctx.flags = flags  # the backward keeps the forward's choice
         ctx.feats_shape = feats.shape
         ctx.mask = (feats, wb, gate, mask_w.shape, mask_b.shape) if masked else None
         return out
@@ -157,6 +196,7 @@ class UNetSCNFn(torch.autograd.Function):
         dev = d_out.device
         n_points = meta.n_points
         need_feats = ctx.needs_input_grad[0]
+        flags = ctx.flags
         with torch.cuda.device(dev):
             _lib.raise_device_errors("UNetSCN.backward")
             # one flat buffer for every parameter gradient; the returned grads are views into it
@@ -178,21 +218,31 @@ class UNetSCNFn(torch.autograd.Function):
                 d_feats.zero_()
             tmp_bytes = lib.mm3d_unet_topo_bwd_bytes(in_ch, m, L, reps, res, mode, desc, n_points)
             tmp = torch.empty(tmp_bytes, dtype=torch.uint8, device=dev)
-            scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes(in_ch, m, L, reps, res, mode), dev)
+            scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes_ex(in_ch, m, L, reps, res, mode, flags), dev)
             params = (C.c_void_p * len(slots))(*[t.data_ptr() for t in slots])
             gp = (C.c_void_p * len(slots))(*gptrs)
             mask, d_mw, d_mb = None, None, None
             if ctx.mask is not None:
                 feats, wb, gate, w_shape, b_shape = ctx.mask
                 d_wb = torch.empty(in_ch + 1, dtype=torch.float32, device=dev)
-                mws = torch.empty(in_ch + 1, dtype=torch.float64, device=dev)
+                # (deterministic: one row of partial sums per CTA)
+                mws = torch.empty((in_ch + 1) * (_lib.DET_CTAS if flags else 1), dtype=torch.float64, device=dev)
                 mask = C.byref(_lib.UnetMask(wb.data_ptr(), gate.data_ptr(), feats.data_ptr(), d_wb.data_ptr(), mws.data_ptr(),
                                              mws.numel() * 8))
                 d_mw, d_mb = d_wb[:in_ch].reshape(w_shape), d_wb[in_ch:].reshape(b_shape)
-            check(lib.mm3d_unet_topo_backward(in_ch, m, L, reps, res, mode, int(training), desc, n_points, meta.p2v_ptr, meta.npts_ptr,
-                                         d_out.data_ptr(), d_feats.data_ptr() if need_feats else None, params, gp,
-                                         act.data_ptr(), act.numel(), tmp.data_ptr(), tmp_bytes, scr.data_ptr(),
-                                         scr.numel(), mask, _lib.stream_ptr()), "mm3d_unet_topo_backward")
+            d_feats_ptr = d_feats.data_ptr() if need_feats else None
+            if flags:
+                vox_start, vox_pts = meta.point_csr()
+                check(lib.mm3d_unet_topo_backward_ex(in_ch, m, L, reps, res, mode, int(training), desc, n_points, meta.p2v_ptr,
+                                                     meta.npts_ptr, vox_start.data_ptr(), vox_pts.data_ptr(), d_out.data_ptr(),
+                                                     d_feats_ptr, params, gp, act.data_ptr(), act.numel(), tmp.data_ptr(),
+                                                     tmp_bytes, scr.data_ptr(), scr.numel(), mask, _lib.stream_ptr(), flags),
+                      "mm3d_unet_topo_backward_ex")
+            else:
+                check(lib.mm3d_unet_topo_backward(in_ch, m, L, reps, res, mode, int(training), desc, n_points, meta.p2v_ptr,
+                                                  meta.npts_ptr, d_out.data_ptr(), d_feats_ptr, params, gp, act.data_ptr(),
+                                                  act.numel(), tmp.data_ptr(), tmp_bytes, scr.data_ptr(), scr.numel(), mask,
+                                                  _lib.stream_ptr()), "mm3d_unet_topo_backward")
         return (d_feats, None, None, d_mw, d_mb, *grads)
 
 
@@ -248,6 +298,8 @@ def prepare(net, coords, wait=False):
     L = net._num_planes
     with torch.cuda.device(coords.device):
         meta = Metadata(coords, spatial0, L, plans=F.DEFAULT_MODE != "fp32", defer_sync=not wait)
+        if F.deterministic():  # the voxels' point lists too, one step ahead like the rest of the structure
+            meta.point_csr()
         return PreparedScans(meta, F.DEFAULT_MODE, spatial0, L)
 
 
@@ -262,6 +314,8 @@ def prepare_points(net, points, sample_offsets, rot, transl_u, scale, wait=False
     ps = voxelize_points(points, sample_offsets, rot, transl_u, scale, spatial0, L, plans=F.DEFAULT_MODE != "fp32",
                          defer_sync=not wait)
     with torch.cuda.device(ps.meta.device):
+        if F.deterministic():  # (a structure rebuilt from the kept points builds its lists at the forward)
+            ps.meta.point_csr()
         prep = PreparedScans(ps.meta, F.DEFAULT_MODE, spatial0, L, points=ps)
     if wait:
         prep.kept()

@@ -227,9 +227,13 @@ class Metadata:
     def point_csr(self):
         """(vox_start int32 [n_voxels + 1], vox_pts int32 [n_points]): the points of every voxel in ascending point
         index, for the deterministic InputLayer forward and OutputLayer backward.  Built on the current stream at
-        first use and kept."""
+        first use and kept.  Called before a deferred build's row counts are known (``UNetSCN.prepare`` with the
+        deterministic mode on), it does not wait for them: the lists are built over the point count, a bound on the
+        voxel count (the build zeroes the per-voxel counts that far, so the voxels past the real ones are empty and
+        ``vox_start`` is longer than ``n_voxels + 1``, with the same first ``n_voxels + 1`` entries)."""
         if self._point_csr is None:
-            nv, n = self.n_voxels, self.n_points
+            n = self.n_points
+            nv = n if self._pending is not None else self.n_voxels
             start = torch.empty(nv + 1, dtype=torch.int32, device=self.device)
             pts = torch.empty(max(n, 1), dtype=torch.int32, device=self.device)
             with torch.cuda.device(self.device):
