@@ -32,19 +32,26 @@ def collect_slots(net):
     """Parameters and BN buffers of ``net`` in the executor's slot order, which is module-tree order: per
     BatchNorm ``weight, bias, running_mean, running_var``, per convolution or NetworkInNetwork ``weight``.
     For the reference configuration: stem.w | per level: pre_bn pre.w [dn_bn dn.w <deeper> up_bn up.w post_bn
-    post.w] | head_bn."""
+    post.w] | head_bn.
+
+    The module walk is cached as (parameter or buffer dict of the module, name) pairs and the slots are read through
+    them on every call, so a parameter or buffer replaced by a new object (``conv.weight = nn.Parameter(...)``,
+    ``bn.running_mean = torch.zeros(...)``, ``load_state_dict(..., assign=True)``, buffers moved by ``.to()``) is the
+    one the executor reads and writes the gradient of."""
     from . import scn
-    cached = getattr(net, "_exec_slots", None)
-    if cached is not None and cached[0] is net.layer2.weight and cached[-1] is net.layer4.running_var:
-        return cached  # (the module walk costs ~0.1 ms per call; parameters are updated in place by optimisers / .to())
-    slots = []
-    for mod in net.modules():
-        if isinstance(mod, scn.BatchNormLeakyReLU):
-            slots += [mod.weight, mod.bias, mod.running_mean, mod.running_var]
-        elif isinstance(mod, (scn._ConvBase, scn.NetworkInNetwork)):
-            slots.append(mod.weight)
-    net._exec_slots = slots
-    return slots
+    refs = getattr(net, "_exec_slot_refs", None)
+    # (host time per call, measured on an x86 CPU: the walk ~70 us for the reference configuration; reading its 130
+    # slots through the refs ~5 us, the 331 of block_reps = 2 with residual blocks ~11 us)
+    if refs is None:
+        refs = []
+        for mod in net.modules():
+            if isinstance(mod, scn.BatchNormLeakyReLU):
+                refs += [(mod._parameters, "weight"), (mod._parameters, "bias"), (mod._buffers, "running_mean"),
+                         (mod._buffers, "running_var")]
+            elif isinstance(mod, (scn._ConvBase, scn.NetworkInNetwork)):
+                refs.append((mod._parameters, "weight"))
+        net._exec_slot_refs = refs
+    return [d[k] for d, k in refs]
 
 
 def topology(net):
