@@ -476,6 +476,20 @@ MM3D_API int mm3d_unet_topo_backward_ex(int in_channels, int m, int num_planes, 
                                float* d_feats, void* const* params, void* const* grads, void* act, size_t act_bytes,
                                void* tmp, size_t tmp_bytes, void* scratch, size_t scratch_bytes,
                                const mm3d_unet_mask* mask, mm3d_stream_t stream, int flags);
+/* Inference forward: the eval-mode forward (BatchNorm with the running statistics, training = 0) without anything a
+ * backward would read.  Every BatchNorm+ReLU is applied in the epilogue of the convolution that produces its input and
+ * the JoinTable concatenations are never materialised; the output is the same bits as mm3d_unet_topo_forward_ex with
+ * training = 0 and the same flags.  ws: one device workspace of mm3d_unet_topo_infer_bytes (the exact need: the
+ * tensors this call writes, the forward weight images and the BatchNorm scales); a short one gives MM3D_ERR_WORKSPACE
+ * before any CUDA call.  flags: 0 or MM3D_DETERMINISTIC (InputLayer over the voxels' point lists vox_start / vox_pts).
+ * params as above (running statistics read, nothing written); mask: wb and s as in the forward. */
+MM3D_API size_t mm3d_unet_topo_infer_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                  const int64_t* level_desc, int64_t n_points, int flags);
+MM3D_API int mm3d_unet_topo_infer(int in_channels, int m, int num_planes, int block_reps, int residual, int mode, float eps,
+                         const int64_t* level_desc, int64_t n_points, const int32_t* p2v, const int32_t* npts,
+                         const int32_t* vox_start, const int32_t* vox_pts, const float* feats, float* out,
+                         void* const* params, void* ws, size_t ws_bytes, const mm3d_unet_mask* mask, mm3d_stream_t stream,
+                         int flags);
 
 #ifdef __cplusplus
 }

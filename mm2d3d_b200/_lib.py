@@ -121,6 +121,8 @@ SIGNATURES = {
                                        _p, _p, _i]),
     "mm3d_unet_topo_backward_ex": (_i, [_i, _i, _i, _i, _i, _i, _i, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _sz,
                                         _p, _sz, _p, _p, _i]),
+    "mm3d_unet_topo_infer_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _p, _i64, _i]),
+    "mm3d_unet_topo_infer": (_i, [_i, _i, _i, _i, _i, _i, _f, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _p, _i]),
 }
 
 class PlanDesc(C.Structure):

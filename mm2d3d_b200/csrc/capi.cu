@@ -35,11 +35,12 @@ extern "C" int mm3d_device_supports_tc(void) {
 }
 
 // conv_simt.cu
+struct ConvEpi;
 size_t mm3d_conv_simt_workspace_bytes(int c_in, int c_out, int K);
 int mm3d_conv_fwd_simt(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
                        const float* weight, int K, const int32_t* tbl, int64_t tbl_stride,
                        const uint8_t* onehot_off, int flags, void* ws, size_t ws_bytes, cudaStream_t stream,
-                       const float* add = nullptr);
+                       const float* add = nullptr, const ConvEpi* epi = nullptr);
 int mm3d_conv_wgrad_simt(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out, int c_out,
                          float* d_weight, int K, const int32_t* tbl, int64_t tbl_stride,
                          const uint8_t* onehot_off, int accumulate, cudaStream_t stream);

@@ -8,6 +8,7 @@
 // (SparseConvNet's kernels re-read and re-write the output rows once per offset), and the
 // result is bit-reproducible.  The tcgen05 kernels in conv_tc.cu share this contract.
 #include "common.cuh"
+#include "epilogue.cuh"
 
 namespace {
 
@@ -35,11 +36,12 @@ __global__ void k_weight_transpose(const float* __restrict__ w, float* __restric
   }
 }
 
-template <int CPL>
+// Epi: empty (the default kernel) or one ConvEpi (the inference form: the value goes to its destinations, not to `out`)
+template <int CPL, class... Epi>
 __global__ void __launch_bounds__(kFwdThreads)
 k_conv_fwd_simt(const float* __restrict__ in, float* __restrict__ out, const float* __restrict__ W,
                 const int32_t* __restrict__ tbl, int64_t tbl_stride, const uint8_t* __restrict__ onehot_off,
-                int64_t n_out, int c_in, int c_out, int K, const float* add) {
+                int64_t n_out, int c_in, int c_out, int K, const float* add, const __grid_constant__ Epi... epi) {
   extern __shared__ __align__(16) float s_rows[];  // [kWarps][kRows][c_in]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* a = s_rows + (size_t)warp * kRows * c_in;
@@ -126,7 +128,12 @@ k_conv_fwd_simt(const float* __restrict__ in, float* __restrict__ out, const flo
           const int co = lane + 32 * j;
           if (co < c_out) {
             const int64_t o = (j0 + r) * c_out + co;
-            out[o] = add ? add[o] + acc[r][j] : acc[r][j];  // (add may be `out`: each element is read, then written once)
+            if constexpr (sizeof...(Epi) > 0) {
+              const float v[1] = {add ? add[o] + acc[r][j] : acc[r][j]};
+              (epi_store<1>(epi, j0 + r, co, v), ...);
+            } else {
+              out[o] = add ? add[o] + acc[r][j] : acc[r][j];  // (add may be `out`: each element is read, then written once)
+            }
           }
         }
       }
@@ -274,7 +281,7 @@ size_t mm3d_conv_simt_workspace_bytes(int c_in, int c_out, int K) {
 int mm3d_conv_fwd_simt(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
                        const float* weight, int K, const int32_t* tbl, int64_t tbl_stride,
                        const uint8_t* onehot_off, int flags, void* ws, size_t ws_bytes, cudaStream_t stream,
-                       const float* add) {
+                       const float* add, const ConvEpi* epi) {
   (void)n_in;
   MM3D_REQUIRE(c_out <= 32 * 8, MM3D_ERR_UNSUPPORTED, "SIMT conv: c_out %d > 256", c_out);
   MM3D_REQUIRE(c_in <= 384, MM3D_ERR_UNSUPPORTED, "SIMT conv: c_in %d > 384", c_in);
@@ -294,8 +301,12 @@ int mm3d_conv_fwd_simt(const float* in, int64_t n_in, int c_in, float* out, int6
   const int grid = mm3d_grid(mm3d_cdiv(n_out, kRows) * 32, kFwdThreads, 16);
 #define FWD_CASE(CPL)                                                                                       \
   case CPL:                                                                                                 \
-    k_conv_fwd_simt<CPL><<<grid, kFwdThreads, smem, stream>>>(in, out, W, tbl, tbl_stride, onehot_off, n_out, \
-                                                             c_in, c_out, K, add);                               \
+    if (epi)                                                                                                \
+      k_conv_fwd_simt<CPL, ConvEpi><<<grid, kFwdThreads, smem, stream>>>(in, out, W, tbl, tbl_stride, onehot_off, \
+                                                                        n_out, c_in, c_out, K, add, *epi);       \
+    else                                                                                                    \
+      k_conv_fwd_simt<CPL><<<grid, kFwdThreads, smem, stream>>>(in, out, W, tbl, tbl_stride, onehot_off, n_out, \
+                                                               c_in, c_out, K, add);                             \
     break;
   switch (cpl) {
     FWD_CASE(1) FWD_CASE(2) FWD_CASE(3) FWD_CASE(4) FWD_CASE(5) FWD_CASE(6) FWD_CASE(7) FWD_CASE(8)

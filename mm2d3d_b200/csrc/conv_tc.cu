@@ -25,6 +25,9 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <type_traits>
+
+#include "epilogue.cuh"
 #include "plan.cuh"
 #include "tc_common.cuh"
 
@@ -71,6 +74,12 @@ struct TcParams {
                      // [4096 + 2 cta]: globaltimer at every CTA's start (after the dependency wait) and end
   int trace_cta;     // ... which CTA's roles (MM3D_TC_TRACE_CTA)
 #endif
+};
+
+// the inference form (mm3d_unet_topo_infer): the epilogue writes its value to the destinations of `epi` (epilogue.cuh)
+// instead of `out`.  The default kernel is the instantiation with TcParams, whose code the inference form leaves as it is.
+struct TcEpiParams : TcParams {
+  ConvEpi epi;
 };
 
 #ifdef MM3D_TRACE
@@ -166,8 +175,9 @@ __device__ __forceinline__ int item_tile(uint32_t it) { return (int)(it >> 8); }
 __device__ __forceinline__ int item_k(uint32_t it) { return (int)((it >> 3) & 31u); }
 __device__ __forceinline__ int item_j(uint32_t it) { return (int)(it & 7u); }
 
+template <class P>
 __global__ void __launch_bounds__(kThreads, 2)
-k_conv_tc(const __grid_constant__ TcParams p) {
+k_conv_tc(const __grid_constant__ P p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const int S = p.S;
   // carve: [A stages][B stages][entry rows (one per producer warp)][tile masks | tile indices | item0][items][barriers]
@@ -351,7 +361,30 @@ k_conv_tc(const __grid_constant__ TcParams p) {
 #pragma unroll
           for (int q = 0; q < 16; ++q) acc[q] += acc1[q];
         }
-        if (row >= 0) {
+        if constexpr (std::is_same<P, TcEpiParams>::value) {
+          if (row >= 0) {
+            const float* add = p.add ? p.add + (int64_t)row * p.c_out + c0 : nullptr;
+            if ((p.c_out & 3) == 0) {
+#pragma unroll
+              for (int jj = 0; jj < 16; jj += 4)
+                if (c0 + jj < p.c_out) {
+                  float v[4] = {acc[jj], acc[jj + 1], acc[jj + 2], acc[jj + 3]};
+                  if (add) {
+                    const float4 t = *reinterpret_cast<const float4*>(add + jj);
+                    v[0] += t.x; v[1] += t.y; v[2] += t.z; v[3] += t.w;
+                  }
+                  epi_store<4>(p.epi, row, c0 + jj, v);
+                }
+            } else {
+#pragma unroll
+              for (int jj = 0; jj < 16; ++jj)
+                if (c0 + jj < p.c_out) {
+                  const float v[1] = {add ? add[jj] + acc[jj] : acc[jj]};
+                  epi_store<1>(p.epi, row, c0 + jj, v);
+                }
+            }
+          }
+        } else if (row >= 0) {
           float* dst = p.out + (int64_t)row * p.c_out + c0;
           if ((p.c_out & 3) == 0) {
 #pragma unroll
@@ -594,7 +627,7 @@ int mm3d_conv_tc_build_images(const float* const* weights, float* const* images,
 
 int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
                          const float* wimg, int K, const void* plan, int64_t plan_cap, const float* add, cudaStream_t stream,
-                         const float* wimg_lo = nullptr, int bf16 = 0);
+                         const float* wimg_lo = nullptr, int bf16 = 0, const ConvEpi* epi = nullptr);
 
 int mm3d_conv_fwd_tc(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
                      const float* weight, int K, const void* plan, int64_t plan_cap, int flags, void* ws,
@@ -626,12 +659,25 @@ int mm3d_conv_fwd_tc(const float* in, int64_t n_in, int c_in, float* out, int64_
   return mm3d_conv_fwd_tc_img(in, n_in, c_in, out, n_out, c_out, wimg, K, plan, plan_cap, nullptr, stream, wimg_lo);
 }
 
+template <class P>
+static int set_conv_tc_attributes() {
+  static bool once_dev[64] = {false};
+  bool& once = once_dev[mm3d_device_slot()];
+  if (!once) {
+    MM3D_CUDA(cudaFuncSetAttribute(k_conv_tc<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+    MM3D_CUDA(cudaFuncSetAttribute(k_conv_tc<P>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    once = true;
+  }
+  return MM3D_OK;
+}
+
 // the convolution proper, from a prebuilt weight image
 // wimg_lo != NULL: the TF32x3 form -- `in` carries a lo plane n_in * c_in floats behind the hi one, wimg_lo is the image of
 // the weights' TF32 remainder, and every item is three products (one launch, one gather of both planes)
+// epi != NULL: the inference form -- the epilogue writes to epi's destinations; `out` is not written
 int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
                          const float* wimg, int K, const void* plan, int64_t plan_cap, const float* add, cudaStream_t stream,
-                         const float* wimg_lo, int bf16) {
+                         const float* wimg_lo, int bf16, const ConvEpi* epi) {
   int nb, n_pad;
   MM3D_REQUIRE(!(bf16 && wimg_lo), MM3D_ERR_INVALID, "tcgen05 conv: BF16 and TF32x3 exclude each other");
   MM3D_REQUIRE(tc_geometry(c_in, c_out, K, &nb, &n_pad, bf16) == 0, MM3D_ERR_UNSUPPORTED,
@@ -641,6 +687,15 @@ int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, in
   MM3D_REQUIRE(plan && plan_cap >= n_out, MM3D_ERR_INVALID, "tcgen05 conv: needs a row plan covering n_out rows");
   MM3D_REQUIRE((((uintptr_t)in | (uintptr_t)out | (uintptr_t)wimg | (uintptr_t)add) & 15) == 0, MM3D_ERR_INVALID,
                "tcgen05 conv: pointers must be 16-byte aligned");
+  if (epi && (c_out & 3) == 0) {  // the epilogue stores whole float4s (BF16 planes: 8-byte groups of four)
+    MM3D_REQUIRE(epi->n >= 1 && epi->n <= kEpiDsts, MM3D_ERR_INVALID, "tcgen05 conv: %d epilogue destinations", epi->n);
+    for (int i = 0; i < epi->n; ++i) {
+      const EpiDst& d = epi->d[i];
+      const uintptr_t a = (d.store == 4 ? 0 : (uintptr_t)d.p) | (d.store == 2 ? (uintptr_t)d.p2 : 0);
+      MM3D_REQUIRE((d.ld & 3) == 0 && (a & 15) == 0 && (d.store < 3 || ((uintptr_t)d.p2 & 7) == 0), MM3D_ERR_INVALID,
+                   "tcgen05 conv: epilogue destination %d not aligned for vector stores (ld %d)", i, d.ld);
+    }
+  }
   if (n_out == 0) return MM3D_OK;
   const Mm3dPlanView pv = mm3d_plan_view(plan, plan_cap);
   TcParams p;
@@ -673,13 +728,7 @@ int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, in
   }
   const uint32_t b_stride = ((uint32_t)n_pad * 128u + 1023u) & ~1023u;
   const size_t per_stage = ((size_t)kStageBytes + b_stride) * (wimg_lo ? 2 : 1);
-  static bool once_dev[64] = {false};
-  bool& once = once_dev[mm3d_device_slot()];
-  if (!once) {
-    MM3D_CUDA(cudaFuncSetAttribute(k_conv_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
-    MM3D_CUDA(cudaFuncSetAttribute(k_conv_tc, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    once = true;
-  }
+  if (int rc = epi ? set_conv_tc_attributes<TcEpiParams>() : set_conv_tc_attributes<TcParams>()) return rc;
   // Two issuer warps with their own accumulators (double buffered: 4 x n_pad TMEM columns) whenever they fit.
   // Two CTAs per SM when the layer has more tiles than SMs, each CTA's accumulators fit half the TMEM and half the
   // shared memory still holds a ring of >= 4 stages; one CTA per SM with a deeper ring otherwise.  S is even (ring
@@ -721,7 +770,14 @@ int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, in
     p.max_items = p.n_local * K * nb;
     const size_t smem = smem_fixed + (((size_t)(3 * p.n_local + 1) * 4 + 15) & ~(size_t)15) + (((size_t)p.max_items * 2 + 15) & ~(size_t)15);
     MM3D_REQUIRE(smem <= 226 * 1024, MM3D_ERR_UNSUPPORTED, "tcgen05 conv: shared memory budget exceeded");
-    MM3D_CUDA(mm3d_launch_pdl(k_conv_tc, dim3(grid), dim3(kThreads), smem, stream, p));
+    if (epi) {
+      TcEpiParams pe;
+      static_cast<TcParams&>(pe) = p;
+      pe.epi = *epi;
+      MM3D_CUDA(mm3d_launch_pdl(k_conv_tc<TcEpiParams>, dim3(grid), dim3(kThreads), smem, stream, pe));
+    } else {
+      MM3D_CUDA(mm3d_launch_pdl(k_conv_tc<TcParams>, dim3(grid), dim3(kThreads), smem, stream, p));
+    }
     mm3d_count_launches(1);
   }
   MM3D_CHECK_LAUNCH("mm3d_conv_fwd_tc");

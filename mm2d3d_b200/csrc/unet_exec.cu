@@ -28,6 +28,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "epilogue.cuh"
 #include "plan.cuh"
 
 // bnrelu.cu
@@ -48,12 +49,12 @@ int mm3d_conv_tc_build_images(const float* const* weights, float* const* images,
                               const int* c_out, const int* flags, int n, cudaStream_t stream);
 int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
                          const float* wimg, int K, const void* plan, int64_t plan_cap, const float* add, cudaStream_t stream,
-                         const float* wimg_lo = nullptr, int bf16 = 0);
+                         const float* wimg_lo = nullptr, int bf16 = 0, const ConvEpi* epi = nullptr);
 // conv_simt.cu
 int mm3d_conv_fwd_simt(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
                        const float* weight, int K, const int32_t* tbl, int64_t tbl_stride,
                        const uint8_t* onehot_off, int flags, void* ws, size_t ws_bytes, cudaStream_t stream,
-                       const float* add);
+                       const float* add, const ConvEpi* epi = nullptr);
 
 namespace {
 
@@ -122,6 +123,7 @@ struct Net {
   float *d_wp = nullptr, *d_V = nullptr;  // backward, padded stem input only: gradients w.r.t. wp and V
   int head, n_params;                     // the head BatchNorm's first parameter slot; the number of slots
   std::vector<ConvInfo> convs;            // every convolution, in slot order
+  std::vector<std::pair<int, int>> bns;   // every BatchNorm's first parameter slot and channels, in slot order
   size_t bn_channels = 0;                 // of all BatchNorms (each has a gamma and a beta gradient)
   // The scratch buffer: [convolution workspace | weight images | BatchNorm workspace | padded stem weight], and in the
   // deterministic mode behind that [deterministic BatchNorm workspace | weight-gradient slabs].  Weight images
@@ -155,6 +157,7 @@ struct Carve {
 
   int bn(int ch) {
     net.bn_channels += ch;
+    net.bns.push_back({pi, ch});
     pi += 4;  // gamma, beta, running mean, running var
     return pi - 4;
   }
@@ -256,13 +259,14 @@ struct Carve {
   }
 };
 
-// the region of the weight images: the larger direction's images, twice in TF32x3 mode (hi and lo)
-size_t img_region_bytes(const Net& net) {
+// the region of the weight images: the larger direction's images (the forward's alone without `backward`), twice in
+// TF32x3 mode (hi and lo)
+size_t img_region_bytes(const Net& net, bool backward = true) {
   if (net.mode == MM3D_MODE_FP32) return 0;
   size_t fwd = 0, bwd = 0;
   for (const ConvInfo& ci : net.convs) {  // (0 bytes for a shape the tensor cores do not take)
     fwd += mm3d_align(mm3d_conv_tc_workspace_bytes(ci.c_in, ci.c_out, ci.K));
-    bwd += mm3d_align(mm3d_conv_tc_workspace_bytes(ci.c_out, ci.c_in, ci.K));
+    if (backward) bwd += mm3d_align(mm3d_conv_tc_workspace_bytes(ci.c_out, ci.c_in, ci.K));
   }
   return (fwd > bwd ? fwd : bwd) * (net.x3() ? 2 : 1);
 }
@@ -530,13 +534,16 @@ const float* find_img_lo(const Ctx& c, const float* w) {
 }
 // One rule-table convolution from prebuilt weight images.  TF32x3 mode: hi.Whi + lo.Whi + hi.Wlo inside one launch (`in`
 // carries the lo plane n_in * c_in floats behind the hi one, both planes are gathered into every ring stage).
-// add != NULL: out = conv + add (add == out accumulates)
+// add != NULL: out = conv + add (add == out accumulates); epi != NULL: the value goes to epi's destinations instead of out
 int conv_img(const Ctx& c, const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out, const float* im,
-             const float* im_lo, int K, const void* plan, int64_t plan_cap, const float* add = nullptr) {
+             const float* im_lo, int K, const void* plan, int64_t plan_cap, const float* add = nullptr,
+             const ConvEpi* epi = nullptr) {
   if (c.net->x3() && !im_lo) { mm3d_set_error("tf32x3: missing lo weight image"); return MM3D_ERR_INVALID; }
   if (c.net->bf16())  // the BF16 plane sits n_in * c_in floats behind the FP32 one
-    return mm3d_conv_fwd_tc_img(in + n_in * (int64_t)c_in, n_in, c_in, out, n_out, c_out, im, K, plan, plan_cap, add, c.stream, nullptr, 1);
-  return mm3d_conv_fwd_tc_img(in, n_in, c_in, out, n_out, c_out, im, K, plan, plan_cap, add, c.stream, c.net->x3() ? im_lo : nullptr);
+    return mm3d_conv_fwd_tc_img(in + n_in * (int64_t)c_in, n_in, c_in, out, n_out, c_out, im, K, plan, plan_cap, add, c.stream, nullptr, 1,
+                                epi);
+  return mm3d_conv_fwd_tc_img(in, n_in, c_in, out, n_out, c_out, im, K, plan, plan_cap, add, c.stream, c.net->x3() ? im_lo : nullptr,
+                              0, epi);
 }
 
 // the rule table of a layer type at FINE level l, as the convolutions take it
@@ -895,6 +902,256 @@ Sizes lay_out(Net& net, void* act, void* tmp, void* scratch) {
   return {a.off, t.off, s.off};
 }
 
+// The InputLayer (+ the folded RGB mask) into net.V, the stem input in operand form (net.Vp) and the stem weight as the
+// kernels see it, which is returned
+const float* input_stage(Ctx& c, int64_t n_points, const int32_t* p2v, const int32_t* npts, const int32_t* vox_start,
+                         const int32_t* vox_pts, const float* feats, const mm3d_unet_mask* mask) {
+  Net& net = *c.net;
+  const int64_t n0 = net.lv[0].n;
+  if (mask) {  // the RGB-mask prologue of Net3DSeg.forward folded into the point -> voxel scatter
+    if (net.det())
+      EX(mm3d_input_masked_fwd_csr(feats, vox_start, vox_pts, n0, net.cin, 4, mask->wb, net.V, mask->s, c.stream));
+    else
+      EX(mm3d_input_masked_fwd(feats, p2v, npts, n_points, n0, net.cin, 4, mask->wb, net.V, mask->s, c.stream));
+  } else if (net.det()) {
+    EX(mm3d_input_fwd_csr(feats, vox_start, vox_pts, n0, net.cin, 4, net.V, c.stream));
+  } else {
+    EX(mm3d_input_fwd(feats, p2v, npts, n_points, n0, net.cin, 4, net.V, c.stream));
+  }
+  MARK("input_fwd", -1);
+  const float* w_stem = P(c, 0);
+  if (net.Vp != net.V)  // pad the stem input to whole 64-byte pieces; rounded to TF32 (+ lo plane in TF32x3 mode)
+    launch_pad_cols(c, net.V, n0, net.cin, net.Vp, net.cin_k, net.rmode());
+  else if (tc_mode(c) && n0 > 0 && !c.rc) {
+    // (stem input already a whole number of 64-byte pieces: round the InputLayer output in place)
+    if (mm3d_launch_pdl(k_round_tf32, dim3(mm3d_grid(n0 * net.cin / 4 + 1, 256)), dim3(256), 0, c.stream, (const float*)net.V, net.V, n0 * (int64_t)net.cin) != cudaSuccess) c.rc = MM3D_ERR_CUDA;
+    mm3d_count_launches(1);
+  }
+  if (net.cin_k != net.cin) {  // zero input channels for the stem weight too
+    launch_pad_cols(c, w_stem, 27, net.cin * net.m, net.wp, net.cin_k * net.m);
+    w_stem = net.wp;
+  }
+  return w_stem;
+}
+
+// ---- inference forward (eval-mode BatchNorm, nothing kept for a backward) ---------------------------------------------
+// Every BatchNorm+ReLU runs in the epilogue of the convolution that produces its input (epilogue.cuh): a tensor is
+// written straight into the normalised operand forms its consumers gather, and the JoinTable [Y | F] is never
+// materialised -- Y and F each write their column block of the first post block's normalised input (rows 2p floats
+// apart) and, with residual blocks, of J in operand form, which the NetworkInNetwork shortcut gathers.  Destinations
+// per tensor (at most kEpiDsts = 3):
+//   a block's input (stem / down output / previous block's output): the block's first BatchNorm -> A; residual:
+//     + raw (the identity shortcut's addend)
+//   Y (the last pre block's output, not the deepest level): down BatchNorm -> B, the first post block's BatchNorm ->
+//     AJ[:, :p]; residual: + J[:, :p] in operand form
+//   F (the deconvolution's output): AJ[:, p:]; residual: + J[:, p:] in operand form
+//   R (a level's output): the parent's up BatchNorm -> E, or at level 0 the head BatchNorm -> Z (FP32, for the
+//     OutputLayer)
+//   residual blocks: first SMC -> the second BatchNorm -> A2; NetworkInNetwork -> S (raw, the second SMC's addend)
+// No standalone BatchNorm or join launch remains, in any block topology.
+struct IBlock {
+  float *A, *xr, *A2, *S;  // normalised input (operand form), raw input, second normalised input, shortcut output
+};
+struct ILevel {
+  std::vector<IBlock> pre, post;
+  float *B, *E, *AJ, *Jop;  // down input, up input (the next level's rows), first post block's input [n, 2p], J (operand form)
+};
+struct InferLayout {
+  std::vector<ILevel> lv;
+  std::vector<float*> scale;  // per BatchNorm (at its first slot): rsqrtf(running_var + eps) * gamma
+};
+
+// The workspace walk: sizes (NULL ws) and lays out everything the inference forward writes -- the InputLayer output and
+// stem input, each convolution's destinations, the identity row plans, the forward weight images, the padded stem
+// weight and the BatchNorm scales.  Returns the bytes it needs.
+size_t infer_layout(Net& net, InferLayout& IL, void* ws) {
+  Bump none{nullptr, 0}, none2{nullptr, 0};
+  Carve{net, none, none2}.run();  // (parameter slots, the convolution and BatchNorm lists; no buffers)
+  Bump a{(char*)ws, 0};
+  const int pl = net.pl();
+  const int64_t n0 = net.lv[0].n;
+  net.V = a.f(n0, net.cin);
+  net.Vp = (net.cin_k != net.cin || pl == 2) ? a.f(n0, (int64_t)net.cin_k * pl) : net.V;
+  IL.lv.assign(net.L, ILevel());
+  auto block = [&](int64_t n, int a_ch, int b_ch) {
+    IBlock k{};
+    k.A = a.f(n, (int64_t)a_ch * pl);
+    if (net.res) {
+      if (a_ch == b_ch) k.xr = a.f(n, a_ch);
+      else k.S = a.f(n, b_ch);
+      k.A2 = a.f(n, (int64_t)b_ch * pl);
+    }
+    return k;
+  };
+  for (int l = 0; l < net.L; ++l) {
+    const int64_t n = net.lv[l].n;
+    const int p = net.planes(l);
+    ILevel& I = IL.lv[l];
+    for (int r = 0; r < net.reps; ++r) I.pre.push_back(block(n, p, p));
+    if (l + 1 == net.L) continue;
+    I.B = a.f(n, (int64_t)p * pl);
+    I.E = a.f(net.lv[l + 1].n, (int64_t)net.planes(l + 1) * pl);
+    for (int r = 0; r < net.reps; ++r) {
+      if (r == 0) {
+        IBlock k{};
+        k.A = I.AJ = a.f(n, (int64_t)2 * p * pl);
+        if (net.res) {
+          I.Jop = a.f(n, (int64_t)2 * p * pl);
+          net.b[l].id_plan = a.bytes(mm3d_plan_size(n, 1));
+          k.S = a.f(n, p);
+          k.A2 = a.f(n, (int64_t)p * pl);
+        }
+        I.post.push_back(k);
+      } else {
+        I.post.push_back(block(n, p, p));
+      }
+    }
+  }
+  net.Z = a.f(n0, net.m);
+  net.img_ws_bytes = img_region_bytes(net, false);
+  net.img_ws = a.bytes(net.img_ws_bytes);
+  net.wp = net.cin_k != net.cin ? a.f(27, (int64_t)net.cin_k * net.m) : nullptr;
+  IL.scale.assign(net.n_params, nullptr);
+  for (const auto& bn : net.bns) IL.scale[bn.first] = a.f(1, bn.second);
+  return a.off;
+}
+
+// the scales of every BatchNorm, one CTA each, in as few launches as the list takes (one for the usual networks)
+constexpr int kMaxBnScales = 128;
+struct BnScales {
+  const float* gamma[kMaxBnScales];
+  const float* var[kMaxBnScales];
+  float* scale[kMaxBnScales];
+  int c[kMaxBnScales];
+  float eps;
+};
+__global__ void k_bn_scales(const __grid_constant__ BnScales b) {
+  mm3d_griddep_launch();
+  mm3d_griddep_wait();
+  const int i = blockIdx.x;
+  for (int ch = threadIdx.x; ch < b.c[i]; ch += blockDim.x) b.scale[i][ch] = rsqrtf(b.var[i][ch] + b.eps) * b.gamma[i][ch];
+}
+void bn_scales(Ctx& c, const InferLayout& IL) {
+  const auto& bns = c.net->bns;
+  for (size_t first = 0; first < bns.size() && !c.rc; first += kMaxBnScales) {
+    BnScales b;
+    b.eps = c.eps;
+    int k = 0;
+    for (size_t i = first; i < bns.size() && k < kMaxBnScales; ++i, ++k) {
+      const int s = bns[i].first;
+      b.gamma[k] = P(c, s);
+      b.var[k] = P(c, s + 3);
+      b.scale[k] = IL.scale[s];
+      b.c[k] = bns[i].second;
+    }
+    if (mm3d_launch_pdl(k_bn_scales, dim3(k), dim3(128), 0, c.stream, b) != cudaSuccess) c.rc = MM3D_ERR_CUDA;
+    mm3d_count_launches(1);
+  }
+}
+
+struct Infer {
+  Ctx& c;
+  const InferLayout& IL;
+  Net& net;
+
+  // how a tensor that a convolution gathers is stored: the store_planes forms, except that the BF16 mode's FP32 plane
+  // (the weight gradients' operand) is not written
+  int op() const { return net.bf16() ? 4 : net.rmode(); }
+  // column block col0.. of the [rows, ld] tensor t (planes rows * ld floats apart), in store form `store`; bn >= 0:
+  // normalised with the BatchNorm of that first slot (its channels col0..)
+  EpiDst dst(float* t, int64_t rows, int ld, int col0, int store, int bn = -1) const {
+    EpiDst d{};
+    d.p = t + col0;
+    d.ld = ld;
+    d.store = store;
+    if (store == 2) d.p2 = t + rows * ld + col0;
+    if (store >= 3) d.p2 = reinterpret_cast<__nv_bfloat16*>(t + rows * ld) + col0;
+    if (bn >= 0) {
+      d.mean = P(c, bn + 2) + col0;
+      d.scale = IL.scale[bn] + col0;
+      d.beta = P(c, bn + 1) + col0;
+    }
+    return d;
+  }
+  int bn1(const BlockBufs& k) const { return k.pidx + (net.nin(k.a, k.b) ? 1 : 0); }
+  // the destinations of a block's input
+  ConvEpi input_of(int l, const BlockBufs& k, const IBlock& ib) const {
+    const int64_t n = net.lv[l].n;
+    ConvEpi e{};
+    e.d[e.n++] = dst(ib.A, n, k.a, 0, op(), bn1(k));
+    if (net.res) e.d[e.n++] = dst(ib.xr, n, k.a, 0, 0);
+    return e;
+  }
+  // R_l, the output of level l
+  ConvEpi level_output(int l) const {
+    ConvEpi e{};
+    if (l == 0) e.d[e.n++] = dst(net.Z, net.lv[0].n, net.m, 0, 0, net.head);
+    else e.d[e.n++] = dst(IL.lv[l - 1].E, net.lv[l].n, net.planes(l), 0, op(), net.b[l - 1].up);
+    return e;
+  }
+  // Y (pre = true) or F: their column block of the join
+  ConvEpi join_half(int l, bool pre) const {
+    const int64_t n = net.lv[l].n;
+    const int p = net.planes(l), col0 = pre ? 0 : p;
+    const ILevel& I = IL.lv[l];
+    ConvEpi e{};
+    if (pre) e.d[e.n++] = dst(I.B, n, p, 0, op(), net.b[l].dn);
+    e.d[e.n++] = dst(I.AJ, n, 2 * p, col0, op(), bn1(net.b[l].post[0]));
+    if (net.res) e.d[e.n++] = dst(I.Jop, n, 2 * p, col0, op());
+    return e;
+  }
+
+  void conv(Kind kind, int l, const float* in, int c_in, int c_out, const float* w, const float* add, const ConvEpi& e) {
+    if (abl_skip("conv")) return;
+    const Table t = table(c, kind, l);
+    if (const float* im = find_img(c, w)) {
+      EX(conv_img(c, in, t.n_in, c_in, nullptr, t.n_out, c_out, im, find_img_lo(c, w), t.K, t.plan, t.cap, add, &e));
+    } else if (net.x3() || net.bf16()) {
+      mm3d_set_error("unet: conv c_in %d c_out %d has no tensor-core weight image in this mode", c_in, c_out);
+      if (c.rc == 0) c.rc = MM3D_ERR_UNSUPPORTED;
+    } else {  // FP32 mode, or a TF32 shape the tensor cores do not take
+      EX(mm3d_conv_fwd_simt(in, t.n_in, c_in, nullptr, t.n_out, c_out, w, t.K, t.tbl, t.stride, t.onehot, 0, nullptr, 0,
+                            c.stream, add, &e));
+    }
+  }
+
+  void block(int l, const BlockBufs& k, const IBlock& ib, const ConvEpi& out) {
+    const int64_t n = net.lv[l].n;
+    if (!net.res) {
+      conv(SMC, l, ib.A, k.a, k.b, P(c, k.pidx + 4), nullptr, out);
+      return;
+    }
+    const int b1 = bn1(k);
+    ConvEpi e{};
+    e.d[e.n++] = dst(ib.A2, n, k.b, 0, op(), b1 + 5);
+    conv(SMC, l, ib.A, k.a, k.b, P(c, b1 + 4), nullptr, e);
+    if (net.nin(k.a, k.b)) {
+      ConvEpi s{};
+      s.d[s.n++] = dst(ib.S, n, k.b, 0, 0);
+      conv(NIN, l, IL.lv[l].Jop, k.a, k.b, P(c, k.pidx), nullptr, s);
+    }
+    conv(SMC, l, ib.A2, k.b, k.b, P(c, b1 + 9), net.nin(k.a, k.b) ? ib.S : ib.xr, out);
+  }
+
+  void level(int l) {
+    const LevelBufs& B = net.b[l];
+    const ILevel& I = IL.lv[l];
+    const bool deepest = l + 1 == net.L;
+    for (int r = 0; r < net.reps; ++r)
+      block(l, B.pre[r], I.pre[r],
+            r + 1 < net.reps ? input_of(l, B.pre[r + 1], I.pre[r + 1]) : deepest ? level_output(l) : join_half(l, true));
+    MARK("pre blocks (infer)", l);
+    if (deepest) return;
+    const int p = net.planes(l), q = net.planes(l + 1);
+    conv(DOWN, l, I.B, p, q, P(c, B.dn + 4), nullptr, input_of(l + 1, net.b[l + 1].pre[0], IL.lv[l + 1].pre[0]));
+    level(l + 1);
+    conv(UP, l, I.E, q, p, P(c, B.up + 4), nullptr, join_half(l, false));
+    for (int r = 0; r < net.reps; ++r)
+      block(l, B.post[r], I.post[r], r + 1 < net.reps ? input_of(l, B.post[r + 1], I.post[r + 1]) : level_output(l));
+    MARK("post blocks (infer)", l);
+  }
+};
+
 }  // namespace
 
 extern "C" {
@@ -965,29 +1222,7 @@ MM3D_API int mm3d_unet_topo_forward_ex(int in_channels, int m, int num_planes, i
   MM3D_CUDA(cudaMemsetAsync(net.bn_ws, 0, net.bn_ws_bytes, c.stream));
   const int64_t n0 = net.lv[0].n;
   MARK("fwd start", -1);
-  if (mask) {  // the RGB-mask prologue of Net3DSeg.forward folded into the point -> voxel scatter
-    if (net.det())
-      EX(mm3d_input_masked_fwd_csr(feats, vox_start, vox_pts, n0, in_channels, 4, mask->wb, net.V, mask->s, c.stream));
-    else
-      EX(mm3d_input_masked_fwd(feats, p2v, npts, n_points, n0, in_channels, 4, mask->wb, net.V, mask->s, c.stream));
-  } else if (net.det()) {
-    EX(mm3d_input_fwd_csr(feats, vox_start, vox_pts, n0, in_channels, 4, net.V, c.stream));
-  } else {
-    EX(mm3d_input_fwd(feats, p2v, npts, n_points, n0, in_channels, 4, net.V, c.stream));
-  }
-  MARK("input_fwd", -1);
-  const float* w_stem = P(c, 0);
-  if (net.Vp != net.V)  // pad the stem input to whole 64-byte pieces; rounded to TF32 (+ lo plane in TF32x3 mode)
-    launch_pad_cols(c, net.V, n0, net.cin, net.Vp, net.cin_k, net.rmode());
-  else if (tc_mode(c) && n0 > 0 && !c.rc) {
-    // (stem input already a whole number of 64-byte pieces: round the InputLayer output in place)
-    if (mm3d_launch_pdl(k_round_tf32, dim3(mm3d_grid(n0 * net.cin / 4 + 1, 256)), dim3(256), 0, c.stream, (const float*)net.V, net.V, n0 * (int64_t)net.cin) != cudaSuccess) c.rc = MM3D_ERR_CUDA;
-    mm3d_count_launches(1);
-  }
-  if (net.cin_k != net.cin) {  // zero input channels for the stem weight too
-    launch_pad_cols(c, w_stem, 27, net.cin * m, net.wp, net.cin_k * m);
-    w_stem = net.wp;
-  }
+  const float* w_stem = input_stage(c, n_points, p2v, npts, vox_start, vox_pts, feats, mask);
   EX(build_images(c, false, w_stem));
   build_identity_plans(c);  // (kept in `act`: the backward reuses them)
   MARK("pad + weight images", -1);
@@ -1111,6 +1346,45 @@ MM3D_API int mm3d_unet_topo_backward_ex(int in_channels, int m, int num_planes, 
   MARK("stem bwd + input_bwd", -1);
   join_side(c);  // everything after this call on `stream` sees the weight gradients
   MARK("join wgrad stream", -1);
+  return c.rc;
+}
+
+MM3D_API size_t mm3d_unet_topo_infer_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                           const int64_t* level_desc, int64_t n_points, int flags) {
+  Net net;
+  InferLayout IL;
+  if (!level_desc || fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points, flags)) return 0;
+  return infer_layout(net, IL, nullptr);
+}
+
+MM3D_API int mm3d_unet_topo_infer(int in_channels, int m, int num_planes, int block_reps, int residual, int mode, float eps,
+                                  const int64_t* level_desc, int64_t n_points, const int32_t* p2v, const int32_t* npts,
+                                  const int32_t* vox_start, const int32_t* vox_pts, const float* feats, float* out,
+                                  void* const* params, void* ws, size_t ws_bytes, const mm3d_unet_mask* mask,
+                                  mm3d_stream_t stream_, int flags) {
+  MM3D_REQUIRE(level_desc, MM3D_ERR_INVALID, "unet infer: no level descriptors");
+  MM3D_REQUIRE(!mask || (mask->wb && (n_points == 0 || mask->s)), MM3D_ERR_INVALID, "unet infer: incomplete mask descriptor");
+  MM3D_REQUIRE(!(flags & MM3D_DETERMINISTIC) || (vox_start && vox_pts), MM3D_ERR_INVALID,
+               "unet infer: the deterministic mode needs the voxels' point lists (mm3d_point_csr)");
+  Net net;
+  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points, flags);
+  if (rc) return rc;
+  InferLayout IL;
+  const size_t need = infer_layout(net, IL, ws);
+  MM3D_REQUIRE(ws && ws_bytes >= need, MM3D_ERR_WORKSPACE, "inference workspace too small: need %zu have %zu", need, ws_bytes);
+  Ctx c{&net, params, nullptr, (cudaStream_t)stream_, eps, 0.f, 0, 0};
+  MARK("infer start", -1);
+  const float* w_stem = input_stage(c, n_points, p2v, npts, vox_start, vox_pts, feats, mask);
+  EX(build_images(c, false, w_stem));
+  build_identity_plans(c);
+  bn_scales(c, IL);
+  MARK("pad + weight images + BatchNorm scales", -1);
+  Infer f{c, IL, net};
+  f.conv(SMC, 0, net.Vp, net.cin_k, m, w_stem, nullptr, f.input_of(0, net.b[0].pre[0], IL.lv[0].pre[0]));
+  MARK("stem (infer)", -1);
+  f.level(0);
+  EX(mm3d_output_fwd(net.Z, p2v, n_points, m, out, c.stream));
+  MARK("output_fwd", -1);
   return c.rc;
 }
 

@@ -14,6 +14,12 @@ kept by its backward: the executor then sums the InputLayer and OutputLayer over
 BatchNorm and the masked InputLayer's mask gradient in their fixed-order forms and every weight gradient through the
 fixed-order tcgen05 form, so a training step in the ``tf32``, ``tf32x3`` and ``bf16`` modes is the same bits on every
 run.  The ``fp32`` mode's weight gradients (the SIMT kernel) have no such form: there the step warns.
+
+Inference (validation, test, deployment): in the bf16 mode (``INFER_MODES``), a network in eval mode whose forward
+autograd would not record -- grad mode off, or no input of the call (features, RGB-mask weight and bias, parameters)
+requiring a gradient -- runs ``mm3d_unet_topo_infer`` instead: every BatchNorm+ReLU in the epilogue of the convolution that produces its input, no
+JoinTable copies, a workspace of only what the forward writes, no autograd node.  The output is the same bits as the
+eval forward through ``UNetSCNFn`` (which ``net(x).detach()`` with grad mode on still runs).
 """
 from __future__ import annotations
 
@@ -159,8 +165,7 @@ class UNetSCNFn(torch.autograd.Function):
         dev = feats.device
         # optional RGB mask of Net3DSeg.forward (3d_net/model.py:46-48), folded into the InputLayer scatter
         masked = mask_w is not None
-        if masked and (mask_w.numel() != in_ch or mask_b is None or mask_b.numel() != 1):
-            raise ValueError("UNetSCN: rgb_mask must be the weight [1, C] and bias [1] of an nn.Linear(C, 1)")
+        wb = _mask_wb(in_ch, mask_w, mask_b) if masked else None  # (checked before anything is allocated)
         n_points = meta.n_points
         desc = _level_desc(meta, L, spatial0, plans=mode != _lib.MODE_FP32)
         with torch.cuda.device(dev):
@@ -173,9 +178,8 @@ class UNetSCNFn(torch.autograd.Function):
             out = torch.empty(n_points, m, dtype=torch.float32, device=dev)
             vox_start, vox_pts = meta.point_csr() if det else (None, None)
             params = (C.c_void_p * len(slots))(*[t.data_ptr() for t in slots])
-            mask, wb, gate = None, None, None
+            mask, gate = None, None
             if masked:
-                wb = torch.cat([mask_w.detach().reshape(-1), mask_b.detach().reshape(-1)]).float().contiguous()
                 gate = torch.empty(max(n_points, 1), dtype=torch.float32, device=dev)
                 mask = C.byref(_lib.UnetMask(wb.data_ptr(), gate.data_ptr(), None, None, None, 0))
             if det:
@@ -329,6 +333,57 @@ def prepare_points(net, points, sample_offsets, rot, transl_u, scale, wait=False
     return prep
 
 
+# Convolution modes that take the inference path: those where it measured faster than the eval forward through
+# UNetSCNFn on a batch of 8 nuScenes-shaped scans (tools/infer_bench.py, profiles/r4_infer_bench.txt, B200).  In the
+# fp32, tf32 and tf32x3 modes the BatchNorm arithmetic and the extra row stores in the convolution epilogues cost more
+# than the passes they remove, so there the eval forward stays on UNetSCNFn.
+INFER_MODES = frozenset({_lib.MODE_BF16})
+
+
+def inference_path(training: bool, inputs) -> bool:
+    """Whether a forward takes the inference path: the network is in eval mode and autograd would record nothing --
+    grad mode is off, or none of ``inputs`` (the call's tensors; ``None`` entries ignored) requires a gradient."""
+    if training:
+        return False
+    if not torch.is_grad_enabled():
+        return True
+    return not any(t is not None and t.requires_grad for t in inputs)
+
+
+def _mask_wb(in_ch, mask_w, mask_b):
+    """The RGB mask of Net3DSeg.forward (3d_net/model.py:46-48) as the executor takes it: [weight | bias], FP32."""
+    if mask_w.numel() != in_ch or mask_b is None or mask_b.numel() != 1:
+        raise ValueError("UNetSCN: rgb_mask must be the weight [1, C] and bias [1] of an nn.Linear(C, 1)")
+    return torch.cat([mask_w.detach().reshape(-1), mask_b.detach().reshape(-1)]).float().contiguous()
+
+
+def infer(feats, meta, cfg, mask_w, mask_b, slots):
+    """The inference forward (``mm3d_unet_topo_infer``): plain tensors in, a plain ``[n_points, m]`` tensor out, nothing
+    kept.  ``cfg`` as for :class:`UNetSCNFn` (its training flag and momentum unused)."""
+    in_ch, m, L, mode, _, eps, _, spatial0, reps, res = cfg
+    flags = _lib.DETERMINISTIC if F.deterministic() else 0
+    feats = feats.detach().float().contiguous()
+    dev = feats.device
+    wb = _mask_wb(in_ch, mask_w, mask_b) if mask_w is not None else None
+    n_points = meta.n_points
+    desc = _level_desc(meta, L, spatial0, plans=mode != _lib.MODE_FP32)
+    with torch.cuda.device(dev):
+        _lib.raise_device_errors("UNetSCN.forward")
+        ws_bytes = lib.mm3d_unet_topo_infer_bytes(in_ch, m, L, reps, res, mode, desc, n_points, flags)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        out = torch.empty(n_points, m, dtype=torch.float32, device=dev)
+        vox_start, vox_pts = meta.point_csr() if flags else (None, None)
+        params = (C.c_void_p * len(slots))(*[t.data_ptr() for t in slots])
+        mask = None
+        if wb is not None:
+            gate = torch.empty(max(n_points, 1), dtype=torch.float32, device=dev)
+            mask = C.byref(_lib.UnetMask(wb.data_ptr(), gate.data_ptr(), None, None, None, 0))
+        check(lib.mm3d_unet_topo_infer(in_ch, m, L, reps, res, mode, eps, desc, n_points, meta.p2v_ptr, meta.npts_ptr,
+                                       _lib.ptr(vox_start), _lib.ptr(vox_pts), feats.data_ptr(), out.data_ptr(), params,
+                                       ws.data_ptr(), ws_bytes, mask, _lib.stream_ptr(), flags), "mm3d_unet_topo_infer")
+    return out
+
+
 def run(net, coords, feats, rgb_mask=None):
     if not feats.is_cuda:
         raise RuntimeError("UNetSCN: features must be a CUDA tensor -- mm2d3d_b200 has no CPU path")
@@ -354,5 +409,8 @@ def run(net, coords, feats, rgb_mask=None):
     cfg = (net.in_channels, net.out_channels, L, _lib.MODES[F.DEFAULT_MODE], bool(net.training), float(bn0.eps),
            float(bn0.momentum), spatial0, *topology(net))
     mask_w, mask_b = rgb_mask if rgb_mask is not None else (None, None)
+    slots = collect_slots(net)
+    if cfg[3] in INFER_MODES and inference_path(net.training, (feats, mask_w, mask_b, *slots)):
+        return infer(feats, meta, cfg, mask_w, mask_b, slots)
     with torch.autocast("cuda", enabled=False):
-        return UNetSCNFn.apply(feats, meta, cfg, mask_w, mask_b, *collect_slots(net))
+        return UNetSCNFn.apply(feats, meta, cfg, mask_w, mask_b, *slots)

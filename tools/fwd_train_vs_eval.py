@@ -1,3 +1,7 @@
+"""Training-mode against eval-mode forward of UNetSCN (tf32, batch of 8 nuScenes-shaped scans, structures reused),
+both under torch.no_grad().  A no_grad eval forward takes the inference path (mm3d_unet_topo_infer) in the modes of
+executor.INFER_MODES (bf16); in the tf32 mode timed here it runs the eval forward through UNetSCNFn, where the
+inference path measured slower (tools/infer_bench.py)."""
 import os, sys
 sys.path.insert(0, "/root/repo")
 import numpy as np, torch
