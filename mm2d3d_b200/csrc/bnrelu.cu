@@ -4,7 +4,8 @@
 // HBM-bound: forward = read x (stats) + read x again (L2) + write y; backward = read x, dy + again (L2) +
 // write dx.  Training forward and backward are ONE launch each: per-CTA partial sums -> FP64 atomics ->
 // grid-wide barrier (all CTAs co-resident) -> every CTA normalises the rows it summed.
-// Layout: a CTA's 256 threads tile (rows_pass x CV) where CV = C / VEC channel vectors, so a
+// Layout: a CTA's 256 threads (512 for 257..512 channels that are not multiples of 4) tile (rows_pass x CV) where
+// CV = C / VEC channel vectors, so a
 // warp reads consecutive float4s of consecutive rows (fully coalesced) and every thread keeps
 // one fixed channel vector; per-thread FP32 partials are combined in FP64 (shared, then global
 // atomics into 2*C doubles), which makes var = E[x^2] - mean^2 safe.
@@ -15,6 +16,9 @@
 namespace {
 
 constexpr int kThreads = 256;
+// Channel counts that are not multiples of 4 take one thread per channel: CTAs of kWideThreads for 257..512 of them
+// (the kernels' NT; everything else keeps kThreads)
+constexpr int kWideThreads = 512;
 // Same-address atomics from ~300 CTAs serialise in L2 (~27 cycles each): the per-channel totals therefore go to one
 // of kSlots copies (CTA b adds into copy b % kSlots, every CTA sums the copies after the barrier), the barrier has
 // one counter per slot plus a top counter for the slots' last arrivers, and nobody cleans up behind a launch:
@@ -80,7 +84,7 @@ extern __shared__ double s_acc[];
 // partials go to shared memory, then one thread per channel sums the rows_pass values in FP64 and
 // issues ONE global FP64 atomic per channel and CTA -- or, deterministic (DET), stores it into this CTA's own row
 // sums[blockIdx.x][2 c].
-template <int VEC, bool DET = false>
+template <int VEC, bool DET = false, int NT = kThreads>
 __device__ __forceinline__ void block_flush(const float (&s)[VEC], const float (&q)[VEC], int c, int cv, int rows_pass,
                                             int r, int v, double* __restrict__ sums) {
   float* part = reinterpret_cast<float*>(s_acc);  // [2][rows_pass][c]
@@ -92,7 +96,7 @@ __device__ __forceinline__ void block_flush(const float (&s)[VEC], const float (
     }
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < 2 * c; i += kThreads) {
+  for (int i = threadIdx.x; i < 2 * c; i += NT) {
     const int which = i >= c, ch = i - which * c;
     double acc = 0.0;
     for (int rr = 0; rr < rows_pass; ++rr) acc += (double)part[(which * rows_pass + rr) * c + ch];
@@ -102,15 +106,15 @@ __device__ __forceinline__ void block_flush(const float (&s)[VEC], const float (
 }
 
 // ---- inference forward: normalise with the running statistics (+ optional copy of them to save_*)
-template <int VEC>
-__global__ void __launch_bounds__(kThreads)
+template <int VEC, int NT = kThreads>
+__global__ void __launch_bounds__(NT)
 k_bn_apply(const float* __restrict__ x, float* __restrict__ y, int64_t n, int c,
            const float* __restrict__ gamma, const float* __restrict__ beta,
            float* running_mean, float* running_var, float* save_mean, float* save_invstd,
            const double* __restrict__ sums, float eps, float momentum, float leak, int training, int round_tf32) {
   float* s_mean = reinterpret_cast<float*>(s_acc);
   float* s_scale = s_mean + c;
-  for (int i = threadIdx.x; i < c; i += kThreads) {
+  for (int i = threadIdx.x; i < c; i += NT) {
     float mean, invstd;
     if (training) {
       const double m = sums[i] / (double)n;
@@ -135,7 +139,7 @@ k_bn_apply(const float* __restrict__ x, float* __restrict__ y, int64_t n, int c,
   }
   __syncthreads();
   const int cv = c / VEC;
-  const int rows_pass = kThreads / cv;
+  const int rows_pass = NT / cv;
   const int r = threadIdx.x / cv, v = threadIdx.x - r * cv;
   if (r >= rows_pass) return;
   float mean[VEC], scale[VEC], bet[VEC];
@@ -186,8 +190,9 @@ __device__ __forceinline__ bool grid_arrive_and_wait(unsigned int* sync, int* er
   return s_ok != 0;
 }
 // zero the workspace region the NEXT launch will use (this launch does not touch it otherwise)
+template <int NT = kThreads>
 __device__ __forceinline__ void zero_other(double* other, int words) {
-  for (int i = blockIdx.x * kThreads + threadIdx.x; i < words; i += gridDim.x * kThreads) other[i] = 0.0;
+  for (int i = blockIdx.x * NT + threadIdx.x; i < words; i += gridDim.x * NT) other[i] = 0.0;
 }
 // total of one accumulator over the slot copies
 __device__ __forceinline__ double slot_total(const double* sums, int c2, int i) {
@@ -201,8 +206,9 @@ __device__ __forceinline__ double slot_total(const double* sums, int c2, int i) 
 // Warp w of the grid totals accumulators w, w + 8 grid, ...: lane l sums the rows of CTAs l, l + 32, ... in ascending
 // order, then a butterfly over the lanes (the same on every run) combines the 32 sums.  Each row is read once, by one
 // CTA, instead of every CTA reading all of them (grid^2 x c2 doubles).
+template <int NT = kThreads>
 __device__ __forceinline__ void det_totals(const double* rows, double* tot, int c2) {
-  const int lane = threadIdx.x & 31, nw = kThreads / 32;
+  const int lane = threadIdx.x & 31, nw = NT / 32;
 #pragma unroll 1
   for (int i = blockIdx.x * nw + (threadIdx.x >> 5); i < c2; i += gridDim.x * nw) {
     double t = 0.0;
@@ -219,8 +225,8 @@ __device__ __forceinline__ void det_totals(const double* rows, double* tot, int 
 // rows it summed, so the second read comes from L2 / L1 instead of HBM.
 // DET: the deterministic variant -- `rows` [grid][2 c] takes the CTAs' partials, `sums` [2 c] the totals (det_totals
 // between the barrier on `sync` and a second one on sync + kSlots + 1)
-template <int VEC, bool DET>
-__global__ void __launch_bounds__(kThreads)
+template <int VEC, bool DET, int NT = kThreads>
+__global__ void __launch_bounds__(NT)
 k_bn_fwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int c_lo, float* __restrict__ y, int64_t n, int c,
                const float* __restrict__ gamma, const float* __restrict__ beta,
                float* running_mean, float* running_var, float* save_mean, float* save_invstd,
@@ -228,9 +234,9 @@ k_bn_fwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
                float leak, int round_tf32, int* err) {
   mm3d_griddep_launch();
   mm3d_griddep_wait();
-  zero_other(other, other_words);
+  zero_other<NT>(other, other_words);
   const int cv = c / VEC;
-  const int rows_pass = kThreads / cv;
+  const int rows_pass = NT / cv;
   const int r = threadIdx.x / cv, v = threadIdx.x - r * cv;
   const int64_t stride = (int64_t)gridDim.x * rows_pass;
   // x may be given as two column blocks [x | x_hi] (JoinTable without materialising the concatenation): this
@@ -260,18 +266,18 @@ k_bn_fwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
         for (int j = 0; j < VEC; ++j) { s[j] += t[j]; q[j] = fmaf(t[j], t[j], q[j]); }
       }
     }
-    if (DET) block_flush<VEC, true>(s, q, c, cv, rows_pass, r, v, rows);
-    else block_flush<VEC>(s, q, c, cv, rows_pass, r, v, sums + (blockIdx.x % kSlots) * 2 * c);
+    if (DET) block_flush<VEC, true, NT>(s, q, c, cv, rows_pass, r, v, rows);
+    else block_flush<VEC, false, NT>(s, q, c, cv, rows_pass, r, v, sums + (blockIdx.x % kSlots) * 2 * c);
   }
   grid_arrive_and_wait(sync, err);
   if (DET) {
-    det_totals(rows, sums, 2 * c);
+    det_totals<NT>(rows, sums, 2 * c);
     grid_arrive_and_wait(sync + kSlots + 1, err);
   }
   float* s_mean = reinterpret_cast<float*>(s_acc);
   float* s_scale = s_mean + c;
   __syncthreads();  // block_flush's use of the shared buffer is over
-  for (int i = threadIdx.x; i < c; i += kThreads) {
+  for (int i = threadIdx.x; i < c; i += NT) {
     const double m = (DET ? __ldcg(sums + i) : slot_total(sums, 2 * c, i)) / (double)n;
     double var = (DET ? __ldcg(sums + c + i) : slot_total(sums, 2 * c, c + i)) / (double)n - m * m;
     if (var < 0.0) var = 0.0;
@@ -324,8 +330,8 @@ k_bn_fwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
 
 // ---- backward in ONE launch: reductions, grid barrier, dx (+ d_gamma / d_beta by CTA 0)
 // (DET: as in k_bn_fwd_fused)
-template <int VEC, bool DET>
-__global__ void __launch_bounds__(kThreads)
+template <int VEC, bool DET, int NT = kThreads>
+__global__ void __launch_bounds__(NT)
 k_bn_bwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int c_lo, const float* __restrict__ dy,
                float* __restrict__ dx, float* __restrict__ dx_hi, int64_t n, int c,
                const float* __restrict__ gamma, const float* __restrict__ beta,
@@ -335,9 +341,9 @@ k_bn_bwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
                int round_flags, const float* __restrict__ add, int64_t add_ld, int* err) {
   mm3d_griddep_launch();
   mm3d_griddep_wait();
-  zero_other(other, other_words);
+  zero_other<NT>(other, other_words);
   const int cv = c / VEC;
-  const int rows_pass = kThreads / cv;
+  const int rows_pass = NT / cv;
   const int r = threadIdx.x / cv, v = threadIdx.x - r * cv;
   const int64_t stride = (int64_t)gridDim.x * rows_pass;
   // x may be given as two column blocks [x | x_hi] (JoinTable without materialising the concatenation): this
@@ -397,21 +403,21 @@ k_bn_bwd_fused(const float* __restrict__ x, const float* __restrict__ x_hi, int 
         }
       }
     }
-    if (DET) block_flush<VEC, true>(s, q, c, cv, rows_pass, r, v, rows);
-    else block_flush<VEC>(s, q, c, cv, rows_pass, r, v, sums + (blockIdx.x % kSlots) * 2 * c);
+    if (DET) block_flush<VEC, true, NT>(s, q, c, cv, rows_pass, r, v, rows);
+    else block_flush<VEC, false, NT>(s, q, c, cv, rows_pass, r, v, sums + (blockIdx.x % kSlots) * 2 * c);
   }
   grid_arrive_and_wait(sync, err);
   if (DET) {
-    det_totals(rows, sums, 2 * c);
+    det_totals<NT>(rows, sums, 2 * c);
     grid_arrive_and_wait(sync + kSlots + 1, err);
   }
   // totals over the slot copies -> shared memory (block_flush's use of the buffer is over)
   double* s_tot = s_acc;
   __syncthreads();
-  for (int i = threadIdx.x; i < 2 * c; i += kThreads) s_tot[i] = DET ? __ldcg(sums + i) : slot_total(sums, 2 * c, i);
+  for (int i = threadIdx.x; i < 2 * c; i += NT) s_tot[i] = DET ? __ldcg(sums + i) : slot_total(sums, 2 * c, i);
   __syncthreads();
   if (blockIdx.x == 0)  // (frozen affine parameters: NULL gradient pointers)
-    for (int i = threadIdx.x; i < c; i += kThreads) {
+    for (int i = threadIdx.x; i < c; i += NT) {
       if (d_beta) d_beta[i] = (float)s_tot[i];
       if (d_gamma) d_gamma[i] = (float)s_tot[c + i];
     }
@@ -494,9 +500,9 @@ static int bn_per_sm_cap() {
   return v >= 1 && v <= 8 ? v : 2;
 }
 
-template <bool DET, typename Kernel>
+template <bool DET, int NT, typename Kernel>
 int bn_grid(Kernel kernel, int64_t n, int cv, size_t smem) {
-  const int rows_pass = kThreads / cv;
+  const int rows_pass = NT / cv;
   int64_t g = mm3d_cdiv(n, (int64_t)rows_pass * 4);  // >= 4 rows per thread when there is enough work
   if (g < 1) g = 1;
   // the query is cached per device and kernel instantiation for the 16 KB upper bound of these kernels' dynamic
@@ -506,7 +512,7 @@ int bn_grid(Kernel kernel, int64_t n, int cv, size_t smem) {
   int& slot = cached[mm3d_device_slot()];
   int per_sm = smem <= kSmemBound ? slot : 0;
   if (per_sm == 0) {
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, smem <= kSmemBound ? kSmemBound : smem) != cudaSuccess || per_sm < 1) {
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, NT, smem <= kSmemBound ? kSmemBound : smem) != cudaSuccess || per_sm < 1) {
       (void)cudaGetLastError();
       per_sm = 1;
     }
@@ -544,16 +550,20 @@ static int bn_det_capacity(size_t ws_bytes) {
 
 #define BN_DISPATCH(KERNEL, ...)                                                        \
   do {                                                                                  \
-    const int grid = mm3d_grid(n, kThreads / cv);                                       \
+    const int grid = mm3d_grid(n, nt / cv);                                             \
     if (vec4) KERNEL<4><<<grid, kThreads, smem, stream>>>(__VA_ARGS__);                 \
-    else      KERNEL<1><<<grid, kThreads, smem, stream>>>(__VA_ARGS__);                 \
+    else if (nt == kThreads) KERNEL<1><<<grid, kThreads, smem, stream>>>(__VA_ARGS__);  \
+    else KERNEL<1, kWideThreads><<<grid, kWideThreads, smem, stream>>>(__VA_ARGS__);    \
   } while (0)
 #define BN_DISPATCH_PDL(KERNEL, DET, ...)                                                                        \
   do {                                                                                                           \
-    if (vec4) { const int grid = bn_grid<DET>(KERNEL<4, DET>, n, cv, smem);                                      \
+    if (vec4) { const int grid = bn_grid<DET, kThreads>(KERNEL<4, DET>, n, cv, smem);                            \
                 MM3D_CUDA(mm3d_launch_pdl(KERNEL<4, DET>, dim3(grid), dim3(kThreads), smem, stream, __VA_ARGS__)); } \
-    else      { const int grid = bn_grid<DET>(KERNEL<1, DET>, n, cv, smem);                                      \
+    else if (nt == kThreads) { const int grid = bn_grid<DET, kThreads>(KERNEL<1, DET>, n, cv, smem);             \
                 MM3D_CUDA(mm3d_launch_pdl(KERNEL<1, DET>, dim3(grid), dim3(kThreads), smem, stream, __VA_ARGS__)); } \
+    else      { const int grid = bn_grid<DET, kWideThreads>(KERNEL<1, DET, kWideThreads>, n, cv, smem);          \
+                MM3D_CUDA(mm3d_launch_pdl(KERNEL<1, DET, kWideThreads>, dim3(grid), dim3(kWideThreads), smem, stream, \
+                                          __VA_ARGS__)); }                                                       \
   } while (0)
 
 // parity == NULL: the workspace is not known to be clean: zero it, use region 0.  Otherwise it is all zero (the kernels
@@ -569,7 +579,8 @@ static int bn_fwd(const float* x, const float* x_hi, int c_lo, float* y, int64_t
   MM3D_REQUIRE(c > 0 && n >= 0, MM3D_ERR_INVALID, "bad sizes");
   const bool vec4 = (c % 4 == 0) && (c_lo % 4 == 0) && ((((uintptr_t)x | (uintptr_t)x_hi | (uintptr_t)y) & 15) == 0);
   const int cv = vec4 ? c / 4 : c;
-  MM3D_REQUIRE(cv <= kThreads, MM3D_ERR_UNSUPPORTED, "BatchNorm with %d channels not supported", c);
+  const int nt = (!vec4 && cv > kThreads) ? kWideThreads : kThreads;
+  MM3D_REQUIRE(cv <= nt, MM3D_ERR_UNSUPPORTED, "BatchNorm with %d channels not supported", c);
   MM3D_REQUIRE(ws_bytes >= mm3d_bnrelu_workspace_bytes_ex(c, det ? MM3D_DETERMINISTIC : 0) && ws, MM3D_ERR_WORKSPACE,
                "bnrelu workspace too small");
   MM3D_REQUIRE(!x_hi || (training && c_lo > 0 && c_lo < c), MM3D_ERR_INVALID, "split input needs training mode and 0 < c_lo < c");
@@ -585,8 +596,8 @@ static int bn_fwd(const float* x, const float* x_hi, int c_lo, float* y, int64_t
   unsigned int* sync = (unsigned int*)(sums + (det ? 2 : kSlots * 2) * c);
   double* rows = det ? (double*)((char*)ws + 2 * region) : nullptr;
   const int other_words = (int)(region / 8);
-  const size_t smem = sizeof(double) * 2 * c > sizeof(float) * 2 * (kThreads / cv) * (size_t)c
-                          ? sizeof(double) * 2 * c : sizeof(float) * 2 * (kThreads / cv) * (size_t)c;
+  const size_t smem = sizeof(double) * 2 * c > sizeof(float) * 2 * (nt / cv) * (size_t)c
+                          ? sizeof(double) * 2 * c : sizeof(float) * 2 * (nt / cv) * (size_t)c;
   if (training) {
     MM3D_REQUIRE(save_mean && save_invstd && running_mean && running_var, MM3D_ERR_INVALID, "training needs stat buffers");
     if (!parity) MM3D_CUDA(cudaMemsetAsync(ws, 0, 2 * region, stream));
@@ -625,7 +636,8 @@ static int bn_bwd(const float* x, const float* x_hi, int c_lo, const float* dy, 
   const bool vec4 = (c % 4 == 0) && (c_lo % 4 == 0) && (!add || add_ld % 4 == 0) &&
                     ((((uintptr_t)x | (uintptr_t)x_hi | (uintptr_t)dy | (uintptr_t)dx | (uintptr_t)dx_hi | (uintptr_t)add) & 15) == 0);
   const int cv = vec4 ? c / 4 : c;
-  MM3D_REQUIRE(cv <= kThreads, MM3D_ERR_UNSUPPORTED, "BatchNorm with %d channels not supported", c);
+  const int nt = (!vec4 && cv > kThreads) ? kWideThreads : kThreads;
+  MM3D_REQUIRE(cv <= nt, MM3D_ERR_UNSUPPORTED, "BatchNorm with %d channels not supported", c);
   MM3D_REQUIRE(ws_bytes >= mm3d_bnrelu_workspace_bytes_ex(c, det ? MM3D_DETERMINISTIC : 0) && ws, MM3D_ERR_WORKSPACE,
                "bnrelu workspace too small");
   if (n == 0) {
@@ -641,8 +653,8 @@ static int bn_bwd(const float* x, const float* x_hi, int c_lo, const float* dy, 
   double* rows = det ? (double*)((char*)ws + 2 * region) : nullptr;
   const int other_words = (int)(region / 8);
   if (!parity) MM3D_CUDA(cudaMemsetAsync(ws, 0, 2 * region, stream));
-  const size_t smem = sizeof(double) * 2 * c > sizeof(float) * 2 * (kThreads / cv) * (size_t)c
-                          ? sizeof(double) * 2 * c : sizeof(float) * 2 * (kThreads / cv) * (size_t)c;
+  const size_t smem = sizeof(double) * 2 * c > sizeof(float) * 2 * (nt / cv) * (size_t)c
+                          ? sizeof(double) * 2 * c : sizeof(float) * 2 * (nt / cv) * (size_t)c;
   if (det)
     BN_DISPATCH_PDL(k_bn_bwd_fused, true, x, x_hi, c_lo, dy, dx, dx_hi, n, c, gamma, beta, save_mean, save_invstd, leakiness,
                     sums, sync, rows, other, other_words, d_gamma, d_beta, training, round_flags, add, add_ld,

@@ -62,6 +62,13 @@ static inline int mm3d_device_slot() {
 
 static inline int64_t mm3d_cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 static inline size_t mm3d_align(size_t x, size_t a = 256) { return (x + a - 1) / a * a; }
+// Layers wider than a kernel takes run as slices of shapes it does: `c` channels cut into ceil(c / max) near-equal
+// slices whose starts are multiples of q (max a multiple of q).  The width of every slice but the last; one slice
+// of the whole width when c <= max.
+static inline int mm3d_slice_step(int c, int max, int q) {
+  const int n = (int)mm3d_cdiv(c, max);
+  return (int)mm3d_cdiv(mm3d_cdiv(c, n), q) * q;
+}
 
 // grid for a grid-stride kernel over n items: enough CTAs to cover n once, capped at a few
 // waves of the 148 SMs so tiny levels do not launch thousands of empty CTAs.

@@ -37,12 +37,16 @@ __global__ void k_weight_transpose(const float* __restrict__ w, float* __restric
 }
 
 // Epi: empty (the default kernel) or one ConvEpi (the inference form: the value goes to its destinations, not to `out`)
-template <int CPL, class... Epi>
+// kStrided: a column slice of a wider layer, W rows ld_w and out / add rows ld_out floats apart (otherwise both c_out;
+// the layers of up to 256 columns keep the code they have without slicing)
+template <int CPL, bool kStrided, class... Epi>
 __global__ void __launch_bounds__(kFwdThreads)
 k_conv_fwd_simt(const float* __restrict__ in, float* __restrict__ out, const float* __restrict__ W,
                 const int32_t* __restrict__ tbl, int64_t tbl_stride, const uint8_t* __restrict__ onehot_off,
-                int64_t n_out, int c_in, int c_out, int K, const float* add, const __grid_constant__ Epi... epi) {
+                int64_t n_out, int c_in, int c_out, int ld_w, int ld_out, int K, const float* add,
+                const __grid_constant__ Epi... epi) {
   extern __shared__ __align__(16) float s_rows[];  // [kWarps][kRows][c_in]
+  if constexpr (!kStrided) ld_w = ld_out = c_out;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* a = s_rows + (size_t)warp * kRows * c_in;
   const bool vec = (c_in & 3) == 0;
@@ -75,7 +79,7 @@ k_conv_fwd_simt(const float* __restrict__ in, float* __restrict__ out, const flo
         }
       }
       __syncwarp();
-      const float* Wk = W + (int64_t)k * c_in * c_out;
+      const float* Wk = W + (int64_t)k * c_in * ld_w;
       if (vec) {
         for (int ci = 0; ci < c_in; ci += 4) {
           float w[4][CPL];
@@ -84,7 +88,7 @@ k_conv_fwd_simt(const float* __restrict__ in, float* __restrict__ out, const flo
 #pragma unroll
             for (int j = 0; j < CPL; ++j) {
               const int co = lane + 32 * j;
-              w[q][j] = co < c_out ? __ldg(Wk + (int64_t)(ci + q) * c_out + co) : 0.f;
+              w[q][j] = co < c_out ? __ldg(Wk + (int64_t)(ci + q) * ld_w + co) : 0.f;
             }
 #pragma unroll
           for (int r = 0; r < kRows; ++r) {
@@ -106,7 +110,7 @@ k_conv_fwd_simt(const float* __restrict__ in, float* __restrict__ out, const flo
 #pragma unroll
           for (int j = 0; j < CPL; ++j) {
             const int co = lane + 32 * j;
-            w[j] = co < c_out ? __ldg(Wk + (int64_t)ci * c_out + co) : 0.f;
+            w[j] = co < c_out ? __ldg(Wk + (int64_t)ci * ld_w + co) : 0.f;
           }
 #pragma unroll
           for (int r = 0; r < kRows; ++r) {
@@ -127,7 +131,7 @@ k_conv_fwd_simt(const float* __restrict__ in, float* __restrict__ out, const flo
         for (int j = 0; j < CPL; ++j) {
           const int co = lane + 32 * j;
           if (co < c_out) {
-            const int64_t o = (j0 + r) * c_out + co;
+            const int64_t o = (j0 + r) * ld_out + co;
             if constexpr (sizeof...(Epi) > 0) {
               const float v[1] = {add ? add[o] + acc[r][j] : acc[r][j]};
               (epi_store<1>(epi, j0 + r, co, v), ...);
@@ -145,13 +149,16 @@ k_conv_fwd_simt(const float* __restrict__ in, float* __restrict__ out, const flo
 constexpr int kWgThreads = 256;  // 16 (ci groups) x 16 (co groups)
 constexpr int kPairBatch = 32;
 constexpr int kMaxTI = 12;       // c_in  <= 192
-constexpr int kMaxTJ = 8;        // c_out <= 128
+constexpr int kMaxTJ = 8;        // c_out <= 128 (wider layers: tiles of at most that, mm3d_conv_wgrad_simt)
+constexpr int kSimtWide = 512;   // the widest layer either kernel takes, as slices
 
-template <int TI, int TJ>
+// kStrided: a tile of a wider layer, rows ld_in / ld_dout floats apart, dW[k][ci][co] at dW + k dw_k + ci dw_ld + co
+// (otherwise c_in, c_out, c_in c_out and c_out: the layers of up to (192, 128) channels keep their code)
+template <int TI, int TJ, bool kStrided = false>
 __global__ void __launch_bounds__(kWgThreads)
 k_conv_wgrad_simt(const float* __restrict__ in, const float* __restrict__ dout, float* __restrict__ dW,
                   const int32_t* __restrict__ tbl, int64_t tbl_stride, const uint8_t* __restrict__ onehot_off,
-                  int64_t n_out, int c_in, int c_out, int rows_per_chunk) {
+                  int64_t n_out, int c_in, int c_out, int ld_in, int ld_dout, int64_t dw_k, int dw_ld, int rows_per_chunk) {
   extern __shared__ __align__(16) float s_wg[];  // A[kPairBatch][c_in] | D[kPairBatch][c_out]
   __shared__ int s_pair_in[kWgThreads], s_pair_out[kWgThreads];
   __shared__ int s_warp_cnt[kWgThreads / 32];
@@ -193,11 +200,11 @@ k_conv_wgrad_simt(const float* __restrict__ in, const float* __restrict__ dout, 
       const int nb_pairs = total - b0 < kPairBatch ? total - b0 : kPairBatch;
       // stage the batch: pair p is copied by 8 lanes, 16-byte pieces of the input row and then of
       // the d_out row interleaved over the lanes, four loads in flight per thread
-      if (((c_in | c_out) & 3) == 0) {
+      if ((((kStrided ? ld_in | ld_dout : 0) | c_in | c_out) & 3) == 0) {
         const int p = threadIdx.x >> 3, l8 = threadIdx.x & 7;
         if (p < nb_pairs) {
-          const float4* src_a = reinterpret_cast<const float4*>(in + (int64_t)s_pair_in[b0 + p] * c_in);
-          const float4* src_d = reinterpret_cast<const float4*>(dout + (base + s_pair_out[b0 + p]) * c_out);
+          const float4* src_a = reinterpret_cast<const float4*>(in + (int64_t)s_pair_in[b0 + p] * (kStrided ? ld_in : c_in));
+          const float4* src_d = reinterpret_cast<const float4*>(dout + (base + s_pair_out[b0 + p]) * (kStrided ? ld_dout : c_out));
           float4* dst_a = reinterpret_cast<float4*>(sA + p * c_in);
           float4* dst_d = reinterpret_cast<float4*>(sD + p * c_out);
           const int qa = c_in >> 2, qt = (c_in + c_out) >> 2;
@@ -219,8 +226,8 @@ k_conv_wgrad_simt(const float* __restrict__ in, const float* __restrict__ dout, 
         }
       } else {
         for (int p = warp; p < nb_pairs; p += kWgThreads / 32) {
-          const float* src_a = in + (int64_t)s_pair_in[b0 + p] * c_in;
-          const float* src_d = dout + (base + s_pair_out[b0 + p]) * c_out;
+          const float* src_a = in + (int64_t)s_pair_in[b0 + p] * (kStrided ? ld_in : c_in);
+          const float* src_d = dout + (base + s_pair_out[b0 + p]) * (kStrided ? ld_dout : c_out);
           for (int c = lane; c < c_in; c += 32) sA[p * c_in + c] = __ldg(src_a + c);
           for (int c = lane; c < c_out; c += 32) sD[p * c_out + c] = __ldg(src_d + c);
         }
@@ -240,7 +247,7 @@ k_conv_wgrad_simt(const float* __restrict__ in, const float* __restrict__ dout, 
       __syncthreads();
     }
   }
-  float* dWk = dW + (int64_t)k * c_in * c_out;
+  float* dWk = kStrided ? dW + k * dw_k : dW + (int64_t)k * c_in * c_out;
 #pragma unroll
   for (int i = 0; i < TI; ++i) {
     const int ci = ty + 16 * i;
@@ -248,7 +255,7 @@ k_conv_wgrad_simt(const float* __restrict__ in, const float* __restrict__ dout, 
 #pragma unroll
       for (int jj = 0; jj < TJ; ++jj) {
         const int co = tx + 16 * jj;
-        if (co < c_out && acc[i][jj] != 0.f) atomicAdd(dWk + (int64_t)ci * c_out + co, acc[i][jj]);
+        if (co < c_out && acc[i][jj] != 0.f) atomicAdd(dWk + (int64_t)ci * (kStrided ? dw_ld : c_out) + co, acc[i][jj]);
       }
     }
   }
@@ -257,11 +264,12 @@ k_conv_wgrad_simt(const float* __restrict__ in, const float* __restrict__ dout, 
 template <int TI>
 int launch_wgrad_tj(int tj, dim3 grid, size_t smem, cudaStream_t stream, const float* in, const float* dout,
                     float* dW, const int32_t* tbl, int64_t tbl_stride, const uint8_t* onehot_off, int64_t n_out,
-                    int c_in, int c_out, int rows_per_chunk) {
+                    int c_in, int c_out, int ld_in, int ld_dout, int64_t dw_k, int dw_ld, int rows_per_chunk) {
 #define WG_CASE(TJ)                                                                                          \
   case TJ:                                                                                                   \
     k_conv_wgrad_simt<TI, TJ><<<grid, kWgThreads, smem, stream>>>(in, dout, dW, tbl, tbl_stride, onehot_off,   \
-                                                                 n_out, c_in, c_out, rows_per_chunk);        \
+                                                                 n_out, c_in, c_out, ld_in, ld_dout, dw_k,   \
+                                                                 dw_ld, rows_per_chunk);                     \
     return 0;
   switch (tj) {
     WG_CASE(1) WG_CASE(2) WG_CASE(3) WG_CASE(4) WG_CASE(5) WG_CASE(6) WG_CASE(7) WG_CASE(8)
@@ -283,8 +291,8 @@ int mm3d_conv_fwd_simt(const float* in, int64_t n_in, int c_in, float* out, int6
                        const uint8_t* onehot_off, int flags, void* ws, size_t ws_bytes, cudaStream_t stream,
                        const float* add, const ConvEpi* epi) {
   (void)n_in;
-  MM3D_REQUIRE(c_out <= 32 * 8, MM3D_ERR_UNSUPPORTED, "SIMT conv: c_out %d > 256", c_out);
-  MM3D_REQUIRE(c_in <= 384, MM3D_ERR_UNSUPPORTED, "SIMT conv: c_in %d > 384", c_in);
+  MM3D_REQUIRE(c_out <= kSimtWide, MM3D_ERR_UNSUPPORTED, "SIMT conv: c_out %d > %d", c_out, kSimtWide);
+  MM3D_REQUIRE(c_in <= kSimtWide, MM3D_ERR_UNSUPPORTED, "SIMT conv: c_in %d > %d", c_in, kSimtWide);
   if (n_out == 0) return MM3D_OK;
   const float* W = weight;
   if (flags & (MM3D_CONV_TRANSPOSE_W | MM3D_CONV_MIRROR_K)) {
@@ -296,36 +304,61 @@ int mm3d_conv_fwd_simt(const float* in, int64_t n_in, int c_in, float* out, int6
         weight, wt, K, c_in, c_out, (flags & MM3D_CONV_MIRROR_K) ? 1 : 0);
     W = wt;
   }
-  const int cpl = (c_out + 31) / 32;
+  // (input rows of more than 384 channels need more than the default 48 KB of dynamic shared memory)
   const size_t smem = sizeof(float) * kWarps * kRows * (size_t)c_in;
+  const bool big = smem > 48 * 1024;
+  using FwdK = void (*)(const float*, float*, const float*, const int32_t*, int64_t, const uint8_t*, int64_t, int, int, int,
+                        int, int, const float*);
+  using FwdEpiK = void (*)(const float*, float*, const float*, const int32_t*, int64_t, const uint8_t*, int64_t, int, int,
+                           int, int, int, const float*, ConvEpi);
   const int grid = mm3d_grid(mm3d_cdiv(n_out, kRows) * 32, kFwdThreads, 16);
-#define FWD_CASE(CPL)                                                                                       \
+  // output columns beyond 256 (8 per lane): column slices, each reading its columns of W and writing its columns of out
+  const int step = mm3d_slice_step(c_out, 32 * 8, 16);
+  int launches = W == weight ? 0 : 1;
+  for (int co0 = 0; co0 < c_out; co0 += step, ++launches) {
+    const int w = c_out - co0 < step ? c_out - co0 : step;
+    const float* a = add ? add + co0 : nullptr;
+    float* o = out ? out + co0 : nullptr;
+    ConvEpi e;
+    if (epi) e = epi_columns(*epi, co0);
+#define FWD_CASE(CPL, ST)                                                                                   \
   case CPL:                                                                                                 \
-    if (epi)                                                                                                \
-      k_conv_fwd_simt<CPL, ConvEpi><<<grid, kFwdThreads, smem, stream>>>(in, out, W, tbl, tbl_stride, onehot_off, \
-                                                                        n_out, c_in, c_out, K, add, *epi);       \
-    else                                                                                                    \
-      k_conv_fwd_simt<CPL><<<grid, kFwdThreads, smem, stream>>>(in, out, W, tbl, tbl_stride, onehot_off, n_out, \
-                                                               c_in, c_out, K, add);                             \
+    if (epi) {                                                                                              \
+      if (big) MM3D_CUDA(cudaFuncSetAttribute((const void*)(FwdEpiK)k_conv_fwd_simt<CPL, ST, ConvEpi>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+      k_conv_fwd_simt<CPL, ST, ConvEpi><<<grid, kFwdThreads, smem, stream>>>(in, o, W + co0, tbl, tbl_stride, onehot_off, \
+                                                                        n_out, c_in, w, c_out, c_out, K, a, e);   \
+    } else {                                                                                                \
+      if (big) MM3D_CUDA(cudaFuncSetAttribute((const void*)(FwdK)k_conv_fwd_simt<CPL, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+      k_conv_fwd_simt<CPL, ST><<<grid, kFwdThreads, smem, stream>>>(in, o, W + co0, tbl, tbl_stride, onehot_off, n_out, \
+                                                               c_in, w, c_out, c_out, K, a);                      \
+    }                                                                                                       \
     break;
-  switch (cpl) {
-    FWD_CASE(1) FWD_CASE(2) FWD_CASE(3) FWD_CASE(4) FWD_CASE(5) FWD_CASE(6) FWD_CASE(7) FWD_CASE(8)
-    default: MM3D_REQUIRE(false, MM3D_ERR_UNSUPPORTED, "SIMT conv: c_out %d", c_out);
-  }
+    if (w == c_out) {
+      switch ((w + 31) / 32) {
+        FWD_CASE(1, false) FWD_CASE(2, false) FWD_CASE(3, false) FWD_CASE(4, false)
+        FWD_CASE(5, false) FWD_CASE(6, false) FWD_CASE(7, false) FWD_CASE(8, false)
+        default: MM3D_REQUIRE(false, MM3D_ERR_UNSUPPORTED, "SIMT conv: c_out %d", c_out);
+      }
+    } else {  // (the last slice of 257..272 columns is 113..128 wide, so every width has its instantiation)
+      switch ((w + 31) / 32) {
+        FWD_CASE(1, true) FWD_CASE(2, true) FWD_CASE(3, true) FWD_CASE(4, true)
+        FWD_CASE(5, true) FWD_CASE(6, true) FWD_CASE(7, true) FWD_CASE(8, true)
+        default: MM3D_REQUIRE(false, MM3D_ERR_UNSUPPORTED, "SIMT conv: c_out %d", c_out);
+      }
+    }
 #undef FWD_CASE
-  mm3d_count_launches(W == weight ? 1 : 2);
+  }
+  mm3d_count_launches(launches);
   MM3D_CHECK_LAUNCH("mm3d_conv_fwd_simt");
   return MM3D_OK;
 }
 
-int mm3d_conv_wgrad_simt(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out, int c_out,
-                         float* d_weight, int K, const int32_t* tbl, int64_t tbl_stride,
-                         const uint8_t* onehot_off, int accumulate, cudaStream_t stream) {
-  (void)n_in;
-  MM3D_REQUIRE(c_in <= 16 * kMaxTI && c_out <= 16 * kMaxTJ, MM3D_ERR_UNSUPPORTED,
-               "SIMT wgrad: channels (%d,%d) beyond (192,128)", c_in, c_out);
-  if (!accumulate) MM3D_CUDA(cudaMemsetAsync(d_weight, 0, sizeof(float) * (size_t)K * c_in * c_out, stream));
-  if (n_out == 0) return MM3D_OK;
+// one launch: input channels [0, c_in) of rows ld_in floats apart, output channels [0, c_out) of rows ld_dout apart,
+// dW[k][ci][co] at d_weight + k * dw_k + ci * dw_ld + co
+static int wgrad_simt_tile(const float* in, int ld_in, int c_in, const float* d_out, int ld_dout, int c_out, int64_t n_out,
+                           float* d_weight, int64_t dw_k, int dw_ld, int K, const int32_t* tbl, int64_t tbl_stride,
+                           const uint8_t* onehot_off, cudaStream_t stream) {
+  const bool strided = ld_in != c_in || ld_dout != c_out;
   int ti = (c_in + 15) / 16, tj = (c_out + 15) / 16;
   if (ti == 9 || ti == 11) ++ti;  // only even tile heights are instantiated above 8
   // Row chunks of 2048: the pairs of a 3^3 table are very unevenly spread over the offsets (the
@@ -337,10 +370,26 @@ int mm3d_conv_wgrad_simt(const float* in, int64_t n_in, int c_in, const float* d
   dim3 grid((unsigned)chunks, (unsigned)K);
   const size_t smem = sizeof(float) * kPairBatch * (size_t)(c_in + c_out);
   int miss = 1;
+  if (strided) {
+    // the tiles of a wider layer: register tiles of 4, 8 or 12 x 4 or 8 (the kernel masks the channels past c_in /
+    // c_out), six instantiations instead of another eighty
+#define WG_S(TI, TJ)                                                                                          \
+  k_conv_wgrad_simt<TI, TJ, true><<<grid, kWgThreads, smem, stream>>>(                                         \
+      in, d_out, d_weight, tbl, tbl_stride, onehot_off, n_out, c_in, c_out, ld_in, ld_dout, dw_k, dw_ld, rows_per_chunk)
+    const int si = ti <= 4 ? 4 : ti <= 8 ? 8 : 12;
+    if (tj <= 4) {
+      if (si == 4) WG_S(4, 4); else if (si == 8) WG_S(8, 4); else WG_S(12, 4);
+    } else {
+      if (si == 4) WG_S(4, 8); else if (si == 8) WG_S(8, 8); else WG_S(12, 8);
+    }
+#undef WG_S
+    mm3d_count_launches(1);
+    return MM3D_OK;
+  }
 #define WG_TI(TI)                                                                                           \
   case TI:                                                                                                  \
     miss = launch_wgrad_tj<TI>(tj, grid, smem, stream, in, d_out, d_weight, tbl, tbl_stride, onehot_off,     \
-                               n_out, c_in, c_out, rows_per_chunk);                                         \
+                               n_out, c_in, c_out, ld_in, ld_dout, dw_k, dw_ld, rows_per_chunk);            \
     break;
   switch (ti) {
     WG_TI(1) WG_TI(2) WG_TI(3) WG_TI(4) WG_TI(5) WG_TI(6) WG_TI(7) WG_TI(8) WG_TI(10) WG_TI(12)
@@ -348,6 +397,27 @@ int mm3d_conv_wgrad_simt(const float* in, int64_t n_in, int c_in, const float* d
 #undef WG_TI
   MM3D_REQUIRE(miss == 0, MM3D_ERR_UNSUPPORTED, "SIMT wgrad: no kernel for channels (%d,%d)", c_in, c_out);
   mm3d_count_launches(1);
+  return MM3D_OK;
+}
+
+int mm3d_conv_wgrad_simt(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out, int c_out,
+                         float* d_weight, int K, const int32_t* tbl, int64_t tbl_stride,
+                         const uint8_t* onehot_off, int accumulate, cudaStream_t stream) {
+  (void)n_in;
+  MM3D_REQUIRE(c_in <= kSimtWide && c_out <= kSimtWide, MM3D_ERR_UNSUPPORTED,
+               "SIMT wgrad: channels (%d,%d) beyond (%d,%d)", c_in, c_out, kSimtWide, kSimtWide);
+  if (!accumulate) MM3D_CUDA(cudaMemsetAsync(d_weight, 0, sizeof(float) * (size_t)K * c_in * c_out, stream));
+  if (n_out == 0) return MM3D_OK;
+  // Channels beyond (192, 128): tiles of at most that, each its own launch adding into its block of d_weight
+  const int si = mm3d_slice_step(c_in, 16 * kMaxTI, 16), sj = mm3d_slice_step(c_out, 16 * kMaxTJ, 16);
+  for (int ci0 = 0; ci0 < c_in; ci0 += si)
+    for (int co0 = 0; co0 < c_out; co0 += sj) {
+      const int rc = wgrad_simt_tile(in + ci0, c_in, c_in - ci0 < si ? c_in - ci0 : si, d_out + co0, c_out,
+                                     c_out - co0 < sj ? c_out - co0 : sj, n_out, d_weight + (int64_t)ci0 * c_out + co0,
+                                     (int64_t)c_in * c_out, c_out, K, tbl, tbl_stride, onehot_off, stream);
+      if (rc) return rc;
+    }
   MM3D_CHECK_LAUNCH("mm3d_conv_wgrad_simt");
   return MM3D_OK;
 }
+

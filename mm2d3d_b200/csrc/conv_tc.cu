@@ -55,6 +55,9 @@ struct TcParams {
   const int32_t* tbl;
   int64_t tstride;
   int c_in, c_out, K;
+  int ld_in;    // row stride of `in` / `in_lo` in 4-byte units (c_in, or c_in / 2 for BF16, unless a channel slice)
+  int ld_out;   // row stride of `out` / `add` in floats (c_out unless a column slice)
+  int img_nb, img_rows;  // block stride of the weight image: its K-blocks per offset and rows per block (nb, n_pad unless sliced)
   int nb;       // K-blocks per offset = ceil(c_in / 32)
   int last_w;   // 16-byte chunks of an offset's last block (8, or 4 when c_in % 32 == 16)
   int S;        // ring stages = producer warps
@@ -302,9 +305,9 @@ k_conv_tc(const __grid_constant__ P p) {
       const bool tma = p.use_tma && w == 8;
       if (lane == 0) {  // this K-block's weight block rides on the same barrier as the gathered rows
         mbar_arrive_expect_tx(a_full(s), (uint32_t)(1 + p.x3) * b_bytes + (tma ? (uint32_t)kStageBytes : 0u));
-        bulk_g2s(b_base + (uint32_t)s * b_stage, p.wimg + ((size_t)k * p.nb + j) * p.n_pad * kKBlock, b_bytes, a_full(s));
+        bulk_g2s(b_base + (uint32_t)s * b_stage, p.wimg + ((size_t)k * p.img_nb + j) * p.img_rows * kKBlock, b_bytes, a_full(s));
         if (p.x3)
-          bulk_g2s(b_base + (uint32_t)s * b_stage + b_stride, p.wimg_lo + ((size_t)k * p.nb + j) * p.n_pad * kKBlock, b_bytes, a_full(s));
+          bulk_g2s(b_base + (uint32_t)s * b_stage + b_stride, p.wimg_lo + ((size_t)k * p.img_nb + j) * p.img_rows * kKBlock, b_bytes, a_full(s));
       }
       if (tma) {
         // One tile::gather4 per lane: rows 4 lane .. 4 lane + 3 of the K-block (128 bytes each, swizzled by the TMA
@@ -316,8 +319,8 @@ k_conv_tc(const __grid_constant__ P p) {
       } else {
         asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(ent + (uint32_t)lane * 16u), "r"(e.x), "r"(e.y), "r"(e.z), "r"(e.w) : "memory");
         __syncwarp();
-        // (addresses in 4-byte units: a K-block is 128 bytes of a row in both element types; BF16 rows are c_in / 2 units)
-        const uint32_t row_units = p.bf16 ? (uint32_t)p.c_in >> 1 : (uint32_t)p.c_in;
+        // (addresses in 4-byte units: a K-block is 128 bytes of a row in both element types)
+        const uint32_t row_units = (uint32_t)p.ld_in;
         const float* src0 = p.in + j * kKBlock;
         if (w == 8)      gather_block<8, false>(stage, ent, p.in, src0, row_units, lane);
         else if (w == 4) gather_block<4, false>(stage, ent, p.in, src0, row_units, lane);
@@ -363,8 +366,8 @@ k_conv_tc(const __grid_constant__ P p) {
         }
         if constexpr (std::is_same<P, TcEpiParams>::value) {
           if (row >= 0) {
-            const float* add = p.add ? p.add + (int64_t)row * p.c_out + c0 : nullptr;
-            if ((p.c_out & 3) == 0) {
+            const float* add = p.add ? p.add + (int64_t)row * p.ld_out + c0 : nullptr;
+            if (((p.c_out | p.ld_out) & 3) == 0) {
 #pragma unroll
               for (int jj = 0; jj < 16; jj += 4)
                 if (c0 + jj < p.c_out) {
@@ -385,14 +388,14 @@ k_conv_tc(const __grid_constant__ P p) {
             }
           }
         } else if (row >= 0) {
-          float* dst = p.out + (int64_t)row * p.c_out + c0;
-          if ((p.c_out & 3) == 0) {
+          float* dst = p.out + (int64_t)row * p.ld_out + c0;
+          if (((p.c_out | p.ld_out) & 3) == 0) {
 #pragma unroll
             for (int jj = 0; jj < 16; jj += 4)
               if (c0 + jj < p.c_out) {
                 float4 o = make_float4(acc[jj], acc[jj + 1], acc[jj + 2], acc[jj + 3]);
                 if (p.add) {  // (each row is owned by one thread: a plain read-modify-write when add == out)
-                  const float4 t = *reinterpret_cast<const float4*>(p.add + (int64_t)row * p.c_out + c0 + jj);
+                  const float4 t = *reinterpret_cast<const float4*>(p.add + (int64_t)row * p.ld_out + c0 + jj);
                   o.x += t.x; o.y += t.y; o.z += t.z; o.w += t.w;
                 }
                 *reinterpret_cast<float4*>(dst + jj) = o;
@@ -400,7 +403,7 @@ k_conv_tc(const __grid_constant__ P p) {
           } else {
 #pragma unroll
             for (int jj = 0; jj < 16; ++jj)
-              if (c0 + jj < p.c_out) dst[jj] = p.add ? p.add[(int64_t)row * p.c_out + c0 + jj] + acc[jj] : acc[jj];
+              if (c0 + jj < p.c_out) dst[jj] = p.add ? p.add[(int64_t)row * p.ld_out + c0 + jj] + acc[jj] : acc[jj];
           }
         }
       }
@@ -534,11 +537,19 @@ bool mm3d_encode_rows_tmap(CUtensorMap* tm, const float* base, int64_t rows, int
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+// One launch takes up to kSliceIn input channels (8 K-blocks: the item's 3-bit block index) and kSliceOut output
+// columns (the double-buffered accumulator in 512 TMEM columns).  Wider layers, up to kWide channels on either side,
+// run as slices (mm3d_conv_fwd_tc_img): output-column slices of near-equal multiples of 16, each a contiguous row
+// range of every block of the full-width weight image; input-channel slices of kSliceIn that accumulate through the
+// epilogue's addend.  The reference widths are one slice, the same launch as without slicing.
+constexpr int kSliceIn = 256, kSliceOut = 256, kWide = 512;
+
+// geometry of the full-width weight image
 static int tc_geometry(int c_in, int c_out, int K, int* nb, int* n_pad, int bf16 = 0) {
   *nb = bf16 ? (c_in + 63) / 64 : (c_in + 31) / 32;
   *n_pad = (c_out + 15) / 16 * 16;
   // input rows are cut into 128-byte blocks with an optional 64-byte tail
-  return (*n_pad <= 256 && (c_in % 16) == 0 && c_in <= 256 && K <= 32) ? 0 : 1;
+  return (*n_pad <= kWide && (c_in % 16) == 0 && c_in <= kWide && K <= 32) ? 0 : 1;
 }
 
 // 1 when the tcgen05 kernel handles this shape
@@ -671,37 +682,18 @@ static int set_conv_tc_attributes() {
   return MM3D_OK;
 }
 
-// the convolution proper, from a prebuilt weight image
-// wimg_lo != NULL: the TF32x3 form -- `in` carries a lo plane n_in * c_in floats behind the hi one, wimg_lo is the image of
-// the weights' TF32 remainder, and every item is three products (one launch, one gather of both planes)
-// epi != NULL: the inference form -- the epilogue writes to epi's destinations; `out` is not written
-int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
-                         const float* wimg, int K, const void* plan, int64_t plan_cap, const float* add, cudaStream_t stream,
-                         const float* wimg_lo, int bf16, const ConvEpi* epi) {
-  int nb, n_pad;
-  MM3D_REQUIRE(!(bf16 && wimg_lo), MM3D_ERR_INVALID, "tcgen05 conv: BF16 and TF32x3 exclude each other");
-  MM3D_REQUIRE(tc_geometry(c_in, c_out, K, &nb, &n_pad, bf16) == 0, MM3D_ERR_UNSUPPORTED,
-               "tcgen05 conv: unsupported shape c_in %d c_out %d K %d", c_in, c_out, K);
-  MM3D_REQUIRE(n_out < (1ll << 31) && n_in * (int64_t)c_in < (1ll << 32), MM3D_ERR_UNSUPPORTED,
-               "tcgen05 conv: tensor too large for 32-bit element offsets");
-  MM3D_REQUIRE(plan && plan_cap >= n_out, MM3D_ERR_INVALID, "tcgen05 conv: needs a row plan covering n_out rows");
-  MM3D_REQUIRE((((uintptr_t)in | (uintptr_t)out | (uintptr_t)wimg | (uintptr_t)add) & 15) == 0, MM3D_ERR_INVALID,
-               "tcgen05 conv: pointers must be 16-byte aligned");
-  if (epi && (c_out & 3) == 0) {  // the epilogue stores whole float4s (BF16 planes: 8-byte groups of four)
-    MM3D_REQUIRE(epi->n >= 1 && epi->n <= kEpiDsts, MM3D_ERR_INVALID, "tcgen05 conv: %d epilogue destinations", epi->n);
-    for (int i = 0; i < epi->n; ++i) {
-      const EpiDst& d = epi->d[i];
-      const uintptr_t a = (d.store == 4 ? 0 : (uintptr_t)d.p) | (d.store == 2 ? (uintptr_t)d.p2 : 0);
-      MM3D_REQUIRE((d.ld & 3) == 0 && (a & 15) == 0 && (d.store < 3 || ((uintptr_t)d.p2 & 7) == 0), MM3D_ERR_INVALID,
-                   "tcgen05 conv: epilogue destination %d not aligned for vector stores (ld %d)", i, d.ld);
-    }
-  }
-  if (n_out == 0) return MM3D_OK;
-  const Mm3dPlanView pv = mm3d_plan_view(plan, plan_cap);
+// One launch over a slice: input channels [ci0, ci0 + c_in) of rows ld_in units apart (in / in_lo at ci0), output
+// columns [co0, co0 + c_out) of rows ld_out floats apart (out / add / wimg / wimg_lo / epi already at the slice)
+static int conv_tc_launch(const float* in, const float* in_lo, int ld_in, int64_t n_in, int c_in, float* out, int ld_out,
+                          int64_t n_out, int c_out, const float* wimg, const float* wimg_lo, int img_nb, int img_rows, int K,
+                          const Mm3dPlanView& pv, const float* add, cudaStream_t stream, int bf16, const ConvEpi* epi,
+                          bool whole) {
+  const int nb = bf16 ? (c_in + 63) / 64 : (c_in + 31) / 32, n_pad = (c_out + 15) / 16 * 16;
   TcParams p;
   p.in = in; p.out = out; p.wimg = wimg;
   p.perm = pv.perm; p.tile_mask = pv.tile_mask; p.order = pv.order; p.tbl = pv.tbl; p.tstride = pv.stride;
   p.c_in = c_in; p.c_out = c_out; p.K = K; p.nb = nb;
+  p.ld_in = ld_in; p.ld_out = ld_out; p.img_nb = img_nb; p.img_rows = img_rows;
   // chunks of an offset's last block: TF32 rows are whole 64-byte pieces, BF16 rows whole 32-byte pieces
   p.last_w = bf16 ? ((c_in % 64) ? (c_in % 64) / 8 : 8) : ((c_in % 32) == 16 ? 4 : 8);
   p.bf16 = bf16;
@@ -710,7 +702,7 @@ int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, in
   p.err = mm3d_device_err_flag();
   p.add = add;
   p.x3 = wimg_lo ? 1 : 0;
-  p.in_lo = in + n_in * (int64_t)c_in;
+  p.in_lo = in_lo;
   p.wimg_lo = wimg_lo;
 #ifdef MM3D_TRACE
   p.trace = g_trace;
@@ -723,7 +715,7 @@ int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, in
   // for 64+ input channels and slower for 32 (the TMA unit takes ~4 cycles per 128-byte row and is shared by the SM's
   // CTAs), 1 % slower over the whole step -- kept selectable for that comparison (DESIGN.md section 7).
   static const bool want_tma = [] { const char* e = getenv("MM3D_TC_GATHER"); return e && strcmp(e, "tma") == 0; }();
-  if (want_tma && !wimg_lo && !bf16 && n_in > 0 && n_in < (1ll << 31) - 1) {
+  if (want_tma && whole && !wimg_lo && !bf16 && n_in > 0 && n_in < (1ll << 31) - 1) {
     p.use_tma = mm3d_encode_rows_tmap(&p.tmap, in, n_in, c_in, /*atom32=*/false) ? 1 : 0;
   }
   const uint32_t b_stride = ((uint32_t)n_pad * 128u + 1023u) & ~1023u;
@@ -779,6 +771,58 @@ int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, in
       MM3D_CUDA(mm3d_launch_pdl(k_conv_tc<TcParams>, dim3(grid), dim3(kThreads), smem, stream, p));
     }
     mm3d_count_launches(1);
+  }
+  return MM3D_OK;
+}
+
+// the convolution proper, from a prebuilt weight image
+// wimg_lo != NULL: the TF32x3 form -- `in` carries a lo plane n_in * c_in floats behind the hi one, wimg_lo is the image of
+// the weights' TF32 remainder, and every item is three products (one launch, one gather of both planes)
+// epi != NULL: the inference form -- the epilogue writes to epi's destinations; `out` is not written,
+// except for the partial sums of the input-channel slices before the last when c_in > kSliceIn
+int mm3d_conv_fwd_tc_img(const float* in, int64_t n_in, int c_in, float* out, int64_t n_out, int c_out,
+                         const float* wimg, int K, const void* plan, int64_t plan_cap, const float* add, cudaStream_t stream,
+                         const float* wimg_lo, int bf16, const ConvEpi* epi) {
+  int nb, n_pad;
+  MM3D_REQUIRE(!(bf16 && wimg_lo), MM3D_ERR_INVALID, "tcgen05 conv: BF16 and TF32x3 exclude each other");
+  MM3D_REQUIRE(tc_geometry(c_in, c_out, K, &nb, &n_pad, bf16) == 0, MM3D_ERR_UNSUPPORTED,
+               "tcgen05 conv: unsupported shape c_in %d c_out %d K %d", c_in, c_out, K);
+  MM3D_REQUIRE(n_out < (1ll << 31) && n_in * (int64_t)c_in < (1ll << 32), MM3D_ERR_UNSUPPORTED,
+               "tcgen05 conv: tensor too large for 32-bit element offsets");
+  MM3D_REQUIRE(plan && plan_cap >= n_out, MM3D_ERR_INVALID, "tcgen05 conv: needs a row plan covering n_out rows");
+  MM3D_REQUIRE((((uintptr_t)in | (uintptr_t)out | (uintptr_t)wimg | (uintptr_t)add) & 15) == 0, MM3D_ERR_INVALID,
+               "tcgen05 conv: pointers must be 16-byte aligned");
+  if (epi && (c_out & 3) == 0) {  // the epilogue stores whole float4s (BF16 planes: 8-byte groups of four)
+    MM3D_REQUIRE(epi->n >= 1 && epi->n <= kEpiDsts, MM3D_ERR_INVALID, "tcgen05 conv: %d epilogue destinations", epi->n);
+    for (int i = 0; i < epi->n; ++i) {
+      const EpiDst& d = epi->d[i];
+      const uintptr_t a = (d.store == 4 ? 0 : (uintptr_t)d.p) | (d.store == 2 ? (uintptr_t)d.p2 : 0);
+      MM3D_REQUIRE((d.ld & 3) == 0 && (a & 15) == 0 && (d.store < 3 || ((uintptr_t)d.p2 & 7) == 0), MM3D_ERR_INVALID,
+                   "tcgen05 conv: epilogue destination %d not aligned for vector stores (ld %d)", i, d.ld);
+    }
+  }
+  if (n_out == 0) return MM3D_OK;
+  const Mm3dPlanView pv = mm3d_plan_view(plan, plan_cap);
+  const int col_step = mm3d_slice_step(c_out, kSliceOut, 16);
+  const int units = bf16 ? 2 : 1;  // channels per 4-byte unit of `in`
+  const int per_blk = bf16 ? 2 * kKBlock : kKBlock;
+  MM3D_REQUIRE(!epi || c_in <= kSliceIn || out, MM3D_ERR_INVALID,
+               "tcgen05 conv: the inference form of c_in %d > %d needs `out` for the partial sums", c_in, kSliceIn);
+  for (int co0 = 0; co0 < c_out; co0 += col_step) {
+    const int w = c_out - co0 < col_step ? c_out - co0 : col_step;
+    ConvEpi e;
+    if (epi) e = epi_columns(*epi, co0);
+    for (int ci0 = 0; ci0 < c_in; ci0 += kSliceIn) {
+      const int cw = c_in - ci0 < kSliceIn ? c_in - ci0 : kSliceIn;
+      const bool last = ci0 + cw == c_in;
+      // input slices after the first add to the partial sum in `out`; only the last one runs the inference epilogue
+      const float* a = ci0 ? out + co0 : add ? add + co0 : nullptr;
+      const size_t img_off = ((size_t)(ci0 / per_blk) * n_pad + co0) * kKBlock;
+      int rc = conv_tc_launch(in + ci0 / units, in + n_in * (int64_t)c_in + ci0, c_in / units, n_in, cw,
+                              out ? out + co0 : nullptr, c_out, n_out, w, wimg + img_off, wimg_lo ? wimg_lo + img_off : nullptr,
+                              nb, n_pad, K, pv, a, stream, bf16, epi && last ? &e : nullptr, w == c_out && cw == c_in);
+      if (rc) return rc;
+    }
   }
   MM3D_CHECK_LAUNCH("mm3d_conv_fwd_tc");
   return MM3D_OK;

@@ -47,6 +47,9 @@ struct WgParams {
   const int32_t* tbl;
   int64_t tstride;
   int c_in, c_out, K;
+  int ld_in, ld_dout;  // row strides of `in` / `dout` in 4-byte units (c_in, c_out; halved for BF16 planes; wider for a slice)
+  int dw_ld;           // dW[k] row stride (c_out unless a slice)
+  int64_t dw_k;        // dW offset stride (c_in * c_out unless a slice)
   int nmb;          // M-blocks per offset: 1, or 2 when c_in > 128
   int cm;           // input channels per M-block = c_in / nmb
   int nbi;          // 32-channel shared-memory blocks of one item = ceil(cm / 32)
@@ -211,6 +214,8 @@ struct WgReduceParams {
   float* dw;
   int64_t slab_cta;
   int c_in, c_out, K, accumulate, groups;
+  int dw_ld;
+  int64_t dw_k;
   uint32_t gmask[32];  // as WgParams::gmask
 };
 
@@ -233,7 +238,8 @@ k_wgrad_reduce(const WgReduceParams r) {
       const float4 v = __ldcs(reinterpret_cast<const float4*>(src + (int64_t)b * r.slab_cta));
       s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
     }
-    float4* d = reinterpret_cast<float4*>(r.dw + 4 * i);
+    const int ci = (int)e / r.c_out, co = (int)e - ci * r.c_out;  // (a slice's per_k is at most 256 x 256)
+    float4* d = reinterpret_cast<float4*>(r.dw + k * r.dw_k + (int64_t)ci * r.dw_ld + co);
     if (r.accumulate) {
       const float4 o = *d;
       s = make_float4(o.x + s.x, o.y + s.y, o.z + s.z, o.w + s.w);
@@ -384,7 +390,7 @@ k_wgrad_tc(const WgParams p) {
         const int buf = (int)(gi % (uint32_t)p.gbufs);
         if (!mbar_wait(g_empty(buf), ((gi / (uint32_t)p.gbufs) & 1u) ^ 1u, abort_flag)) goto done;
         const uint32_t gb = g_base + (uint32_t)buf * g_bytes;
-        gather_rows16(gb, row0, pr, p.dout, (uint32_t)p.c_out, p.gblocks, p.g_last_w == 4, lane);
+        gather_rows16(gb, row0, pr, p.dout, (uint32_t)p.ld_dout, p.gblocks, p.g_last_w == 4, lane);
         cp_async_arrive(g_full(buf));
         ++gi;
       }
@@ -393,7 +399,7 @@ k_wgrad_tc(const WgParams p) {
       if (!mbar_wait(a_empty(s), ((n_item / (uint32_t)S) & 1u) ^ 1u, abort_flag)) goto done;
       TRACE(warp, n_item, 2);
       const uint32_t stage = a_base + (uint32_t)s * a_bytes;
-      gather_rows16(stage, row0, e, p.in + h * p.cm, (uint32_t)p.c_in, p.nbi, p.last_w == 4, lane);
+      gather_rows16(stage, row0, e, p.in + h * p.cm, (uint32_t)p.ld_in, p.nbi, p.last_w == 4, lane);
       cp_async_arrive(a_full(s));
       TRACE(warp, n_item, 3);
       e = en;
@@ -434,7 +440,7 @@ k_wgrad_tc(const WgParams p) {
       const int kidx = __popc(gmask & ((1u << k) - 1u));
       for (int h = 0; h < p.nmb; ++h) {
         const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + (uint32_t)((kidx * p.nmb + h) * p.c_out);
-        float* dst = p.dw + ((int64_t)k * p.c_in + h * p.cm + ci) * p.c_out;
+        float* dst = p.dw + k * p.dw_k + (int64_t)(h * p.cm + ci) * p.dw_ld;
         for (int c0 = 0; c0 < p.c_out; c0 += 16) {
           float acc[16];
           tmem_ld16(taddr + (uint32_t)c0, acc);
@@ -750,9 +756,9 @@ k_wgrad_tc_rings(const WgParams p) {
       __syncwarp();
       for (int jb = 0; jb < p.nbi; ++jb) {
         // (BF16: plain 128-byte swizzle, rows of c_in / 2 four-byte units, the last block's missing chunks zero-filled)
-        if (p.bf16) gather_block<8, false>(stage + (uint32_t)jb * kBlockBytes, ent, p.in, p.in + jb * 32, (uint32_t)p.c_in >> 1, lane, jb == p.nbi - 1 ? p.last_w : 8);
-        else if (jb == p.nbi - 1 && p.last_w == 4) gather_block<4, true>(stage + (uint32_t)jb * kBlockBytes, ent, p.in, p.in + jb * 32, (uint32_t)p.c_in, lane);
-        else gather_block<8, true>(stage + (uint32_t)jb * kBlockBytes, ent, p.in, p.in + jb * 32, (uint32_t)p.c_in, lane);
+        if (p.bf16) gather_block<8, false>(stage + (uint32_t)jb * kBlockBytes, ent, p.in, p.in + jb * 32, (uint32_t)p.ld_in, lane, jb == p.nbi - 1 ? p.last_w : 8);
+        else if (jb == p.nbi - 1 && p.last_w == 4) gather_block<4, true>(stage + (uint32_t)jb * kBlockBytes, ent, p.in, p.in + jb * 32, (uint32_t)p.ld_in, lane);
+        else gather_block<8, true>(stage + (uint32_t)jb * kBlockBytes, ent, p.in, p.in + jb * 32, (uint32_t)p.ld_in, lane);
       }
       cp_async_arrive(a_full(warp));
       __syncwarp();  // the entry row is rewritten by the next item
@@ -782,9 +788,9 @@ k_wgrad_tc_rings(const WgParams p) {
       __syncwarp();
       const uint32_t gb = g_base + (uint32_t)buf * g_bytes;
       for (int jb = 0; jb < p.gblocks; ++jb) {
-        if (p.bf16) gather_block<8, false>(gb + (uint32_t)jb * kBlockBytes, ent, p.dout, p.dout + jb * 32, (uint32_t)p.c_out >> 1, lane, jb == p.gblocks - 1 ? p.g_last_w : 8);
-        else if (jb == p.gblocks - 1 && p.g_last_w == 4) gather_block<4, true>(gb + (uint32_t)jb * kBlockBytes, ent, p.dout, p.dout + jb * 32, (uint32_t)p.c_out, lane);
-        else gather_block<8, true>(gb + (uint32_t)jb * kBlockBytes, ent, p.dout, p.dout + jb * 32, (uint32_t)p.c_out, lane);
+        if (p.bf16) gather_block<8, false>(gb + (uint32_t)jb * kBlockBytes, ent, p.dout, p.dout + jb * 32, (uint32_t)p.ld_dout, lane, jb == p.gblocks - 1 ? p.g_last_w : 8);
+        else if (jb == p.gblocks - 1 && p.g_last_w == 4) gather_block<4, true>(gb + (uint32_t)jb * kBlockBytes, ent, p.dout, p.dout + jb * 32, (uint32_t)p.ld_dout, lane);
+        else gather_block<8, true>(gb + (uint32_t)jb * kBlockBytes, ent, p.dout, p.dout + jb * 32, (uint32_t)p.ld_dout, lane);
       }
       cp_async_arrive(g_full(buf));
       __syncwarp();
@@ -819,7 +825,7 @@ k_wgrad_tc_rings(const WgParams p) {
       const int k = __ffs(rem) - 1;
       const int kidx = __popc(gmask & ((1u << k) - 1u));
       const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + (uint32_t)(kidx * p.c_out);
-      float* dst = p.dw + ((int64_t)k * p.c_in + ci) * p.c_out;
+      float* dst = p.dw + k * p.dw_k + (int64_t)ci * p.dw_ld;
       for (int c0 = 0; c0 < p.c_out; c0 += 16) {
         float acc[16];
         tmem_ld16(taddr + (uint32_t)c0, acc);
@@ -905,11 +911,35 @@ int* mm3d_device_err_flag();  // conv_tc.cu
 long long* mm3d_debug_trace_ptr();  // conv_tc.cu
 #endif
 
-int mm3d_conv_wgrad_tc_supported(int c_in, int c_out, int K) {
+// one launch's shape (wgrad_tc_slice)
+static int wgrad_slice_supported(int c_in, int c_out, int K) {
   if ((c_in % 16) != 0 || c_in < 16 || c_in > 256 || (c_out % 16) != 0 || c_out < 16 || c_out > 256 || K > 32) return 0;
   const int nmb = c_in > 128 ? 2 : 1;
   if (nmb == 2 && (c_in % 32) != 0) return 0;  // halves must stay whole 64-byte pieces
   return nmb * c_out <= 512;
+}
+
+// Layers wider than 256 channels on either side (up to 512) run as (input slice) x (output slice) launches, each a
+// shape wgrad_slice_supported takes, each writing its own block of dW: output slices of near-equal multiples of 16,
+// input slices of 256 channels and a remainder (cut at 128 when it is not a whole number of 64-byte M-block halves).
+// The shapes of 256 channels or fewer are one launch, as without slicing.
+constexpr int kWgSlice = 256, kWgWide = 512;
+static int wgrad_in_slice(int rem) {
+  if (rem > kWgSlice) return kWgSlice;
+  return (rem <= 128 || rem % 32 == 0) ? rem : 128;
+}
+static bool wgrad_sliced(int c_in, int c_out) { return c_in > kWgSlice || c_out > kWgSlice; }
+
+int mm3d_conv_wgrad_tc_supported(int c_in, int c_out, int K) {
+  if (!wgrad_sliced(c_in, c_out)) return wgrad_slice_supported(c_in, c_out, K);
+  if (c_in > kWgWide || c_out > kWgWide || (c_out % 16) != 0) return 0;
+  const int co_step = mm3d_slice_step(c_out, kWgSlice, 16);
+  for (int ci0 = 0, w; ci0 < c_in; ci0 += w) {
+    w = wgrad_in_slice(c_in - ci0);
+    for (int co0 = 0; co0 < c_out; co0 += co_step)
+      if (!wgrad_slice_supported(w, c_out - co0 < co_step ? c_out - co0 : co_step, K)) return 0;
+  }
+  return 1;
 }
 
 // offsets per group: as many (offset, M-block) accumulators of c_out TMEM columns as fit the 512 columns
@@ -928,40 +958,37 @@ static int wgrad_ctas(int c_in, int c_out, int K) {
 // Deterministic variant's workspace: the group -> first-CTA table (256 bytes), then one slab of gk * c_in * c_out floats
 // per CTA (at most 512 TMEM columns x 128 lanes = 256 KB).  Independent of the row count; 0 for shapes the kernels do
 // not take.
-size_t mm3d_conv_wgrad_tc_slab_bytes(int c_in, int c_out, int K) {
-  if (!mm3d_conv_wgrad_tc_supported(c_in, c_out, K)) return 0;
+static size_t wgrad_slice_slab_bytes(int c_in, int c_out, int K) {
   return 256 + (size_t)wgrad_ctas(c_in, c_out, K) * wgrad_group_size(c_in, c_out, K) * c_in * c_out * sizeof(float);
 }
+// (sliced layers: the largest slice's, the slices run one after the other through the same workspace)
+size_t mm3d_conv_wgrad_tc_slab_bytes(int c_in, int c_out, int K) {
+  if (!mm3d_conv_wgrad_tc_supported(c_in, c_out, K)) return 0;
+  if (!wgrad_sliced(c_in, c_out)) return wgrad_slice_slab_bytes(c_in, c_out, K);
+  size_t most = 0;
+  const int co_step = mm3d_slice_step(c_out, kWgSlice, 16);
+  for (int ci0 = 0, w; ci0 < c_in; ci0 += w) {
+    w = wgrad_in_slice(c_in - ci0);
+    for (int co0 = 0; co0 < c_out; co0 += co_step) {
+      const size_t b = wgrad_slice_slab_bytes(w, c_out - co0 < co_step ? c_out - co0 : co_step, K);
+      if (b > most) most = b;
+    }
+  }
+  return most;
+}
 
-// bf16 != 0: `in` / `d_out` point at BF16 planes ([rows, c] bfloat16); only shapes the two-ring kernel takes
-// (c_in <= 128), MM3D_ERR_UNSUPPORTED otherwise (the caller then runs the TF32 kernel on the FP32 planes)
-// slab != NULL: the deterministic variant (slab_bytes >= mm3d_conv_wgrad_tc_slab_bytes): every launch is followed by
-// k_wgrad_reduce, which adds that launch's slabs into d_weight, so the pieces of a long tile list reduce in piece order
-int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out, int c_out,
-                       float* d_weight, int K, const void* plan, int64_t plan_cap, int accumulate,
-                       cudaStream_t stream, int bf16, void* slab, size_t slab_bytes) {
-  MM3D_REQUIRE(mm3d_conv_wgrad_tc_supported(c_in, c_out, K), MM3D_ERR_UNSUPPORTED,
-               "tcgen05 wgrad: unsupported shape c_in %d c_out %d K %d", c_in, c_out, K);
-  MM3D_REQUIRE(n_out < (1ll << 31) && n_in * (int64_t)c_in < (1ll << 32) && n_out * (int64_t)c_out < (1ll << 32),
-               MM3D_ERR_UNSUPPORTED, "tcgen05 wgrad: tensor too large for 32-bit element offsets");
-  MM3D_REQUIRE(plan && plan_cap >= n_out, MM3D_ERR_INVALID, "tcgen05 wgrad: needs a row plan covering n_out rows");
-  MM3D_REQUIRE((((uintptr_t)in | (uintptr_t)d_out | (uintptr_t)d_weight) & 15) == 0, MM3D_ERR_INVALID,
-               "tcgen05 wgrad: pointers must be 16-byte aligned");
+// One launch (and the deterministic variant's reductions) over a slice: input channels of rows ld_in units apart,
+// output channels of rows ld_dout units apart, dW block (k, ci, co) at d_weight + k * dw_k + ci * dw_ld + co
+static int wgrad_tc_slice(const float* in, int ld_in, int c_in, const float* d_out, int ld_dout, int64_t n_out, int c_out,
+                          float* d_weight, int64_t dw_k, int dw_ld, int K, const Mm3dPlanView& pv, int accumulate,
+                          cudaStream_t stream, int bf16, void* slab) {
   const bool det = slab != nullptr;
-  MM3D_REQUIRE(!det || slab_bytes >= mm3d_conv_wgrad_tc_slab_bytes(c_in, c_out, K), MM3D_ERR_WORKSPACE,
-               "deterministic wgrad: workspace %zu bytes < %zu (mm3d_conv_wgrad_workspace_bytes)", slab_bytes,
-               mm3d_conv_wgrad_tc_slab_bytes(c_in, c_out, K));
-  MM3D_REQUIRE(((uintptr_t)slab & 15) == 0, MM3D_ERR_INVALID, "deterministic wgrad: workspace must be 16-byte aligned");
-  // (the deterministic variant's reduction overwrites d_weight itself when !accumulate)
-  if (!accumulate && (!det || n_out == 0))
-    MM3D_CUDA(cudaMemsetAsync(d_weight, 0, sizeof(float) * (size_t)K * c_in * c_out, stream));
-  if (n_out == 0) return MM3D_OK;
-  const Mm3dPlanView pv = mm3d_plan_view(plan, plan_cap);
   WgParams p;
   p.in = in; p.dout = d_out; p.dw = d_weight;
   p.perm = pv.perm; p.tile_mask = pv.tile_mask; p.order = pv.order; p.off_tiles = pv.off_tiles; p.tbl = pv.tbl;
   p.tstride = pv.stride;
   p.c_in = c_in; p.c_out = c_out; p.K = K;
+  p.ld_in = ld_in; p.ld_dout = ld_dout; p.dw_k = dw_k; p.dw_ld = dw_ld;
   p.nmb = c_in > 128 ? 2 : 1;
   p.cm = c_in / p.nmb;
   p.bf16 = bf16;
@@ -1049,6 +1076,7 @@ int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_o
   if (det) {
     rp.slab = p.slab; rp.cta0 = p.slab_cta0; rp.dw = d_weight; rp.slab_cta = p.slab_cta;
     rp.c_in = c_in; rp.c_out = c_out; rp.K = K; rp.groups = groups;
+    rp.dw_k = dw_k; rp.dw_ld = dw_ld;
     for (int g = 0; g < 32; ++g) rp.gmask[g] = g < groups ? p.gmask[g] : 0u;
   }
   const int reduce_grid = (int)mm3d_cdiv((int64_t)K * c_in * c_out / 4, 256);
@@ -1133,5 +1161,49 @@ int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_o
     if (det) reduce(start == 0);
   }
   MM3D_CHECK_LAUNCH("mm3d_conv_wgrad_tc");
+  return MM3D_OK;
+}
+
+// bf16 != 0: `in` / `d_out` point at BF16 planes ([rows, c] bfloat16); only shapes the two-ring kernel takes
+// (c_in <= 128), MM3D_ERR_UNSUPPORTED otherwise (the caller then runs the TF32 kernel on the FP32 planes)
+// slab != NULL: the deterministic variant (slab_bytes >= mm3d_conv_wgrad_tc_slab_bytes): every launch is followed by
+// k_wgrad_reduce, which adds that launch's slabs into d_weight, so the pieces of a long tile list reduce in piece order
+// (and the slices of a wide layer in slice order)
+int mm3d_conv_wgrad_tc(const float* in, int64_t n_in, int c_in, const float* d_out, int64_t n_out, int c_out,
+                       float* d_weight, int K, const void* plan, int64_t plan_cap, int accumulate,
+                       cudaStream_t stream, int bf16, void* slab, size_t slab_bytes) {
+  MM3D_REQUIRE(mm3d_conv_wgrad_tc_supported(c_in, c_out, K), MM3D_ERR_UNSUPPORTED,
+               "tcgen05 wgrad: unsupported shape c_in %d c_out %d K %d", c_in, c_out, K);
+  MM3D_REQUIRE(n_out < (1ll << 31) && n_in * (int64_t)c_in < (1ll << 32) && n_out * (int64_t)c_out < (1ll << 32),
+               MM3D_ERR_UNSUPPORTED, "tcgen05 wgrad: tensor too large for 32-bit element offsets");
+  MM3D_REQUIRE(plan && plan_cap >= n_out, MM3D_ERR_INVALID, "tcgen05 wgrad: needs a row plan covering n_out rows");
+  MM3D_REQUIRE((((uintptr_t)in | (uintptr_t)d_out | (uintptr_t)d_weight) & 15) == 0, MM3D_ERR_INVALID,
+               "tcgen05 wgrad: pointers must be 16-byte aligned");
+  const bool det = slab != nullptr;
+  MM3D_REQUIRE(!det || slab_bytes >= mm3d_conv_wgrad_tc_slab_bytes(c_in, c_out, K), MM3D_ERR_WORKSPACE,
+               "deterministic wgrad: workspace %zu bytes < %zu (mm3d_conv_wgrad_workspace_bytes)", slab_bytes,
+               mm3d_conv_wgrad_tc_slab_bytes(c_in, c_out, K));
+  MM3D_REQUIRE(((uintptr_t)slab & 15) == 0, MM3D_ERR_INVALID, "deterministic wgrad: workspace must be 16-byte aligned");
+  // the BF16 form only where every slice has one M-block (decided before anything runs: the caller falls back to the
+  // TF32 kernel for the whole layer)
+  if (bf16 && (c_in > 128 || getenv("MM3D_WGRAD_NO_BF16"))) return MM3D_ERR_UNSUPPORTED;
+  // (the deterministic variant's reduction overwrites d_weight itself when !accumulate)
+  if (!accumulate && (!det || n_out == 0))
+    MM3D_CUDA(cudaMemsetAsync(d_weight, 0, sizeof(float) * (size_t)K * c_in * c_out, stream));
+  if (n_out == 0) return MM3D_OK;
+  const Mm3dPlanView pv = mm3d_plan_view(plan, plan_cap);
+  const int units = bf16 ? 2 : 1;  // channels per 4-byte unit of the operands
+  const int co_step = wgrad_sliced(c_in, c_out) ? mm3d_slice_step(c_out, kWgSlice, 16) : c_out;
+  for (int ci0 = 0, w; ci0 < c_in; ci0 += w) {
+    w = wgrad_sliced(c_in, c_out) ? wgrad_in_slice(c_in - ci0) : c_in;
+    for (int co0 = 0; co0 < c_out; co0 += co_step) {
+      const int wo = c_out - co0 < co_step ? c_out - co0 : co_step;
+      // (slices write disjoint blocks of d_weight: each honours `accumulate` as the whole layer would)
+      const int rc = wgrad_tc_slice(in + ci0 / units, c_in / units, w, d_out + co0 / units, c_out / units, n_out, wo,
+                                    d_weight + (int64_t)ci0 * c_out + co0, (int64_t)c_in * c_out, c_out, K, pv,
+                                    accumulate || !det, stream, bf16, slab);
+      if (rc) return rc;
+    }
+  }
   return MM3D_OK;
 }

@@ -88,3 +88,17 @@ __device__ __forceinline__ void epi_store(const ConvEpi& e, int64_t row, int c, 
   for (int i = 0; i < kEpiDsts; ++i)
     if (i < e.n) epi_store_one<VEC>(e.d[i], row, c, v);
 }
+
+// the destinations of e from column c0 on: the epilogue of a column slice (the wide layers' slicing) indexes its own
+// columns from 0
+inline ConvEpi epi_columns(const ConvEpi& e, int c0) {
+  ConvEpi r = e;
+  for (int i = 0; i < r.n; ++i) {
+    EpiDst& d = r.d[i];
+    if (d.p) d.p += c0;
+    if (d.store == 2) d.p2 = reinterpret_cast<float*>(d.p2) + c0;
+    if (d.store >= 3) d.p2 = reinterpret_cast<__nv_bfloat16*>(d.p2) + c0;
+    if (d.mean) { d.mean += c0; d.scale += c0; d.beta += c0; }
+  }
+  return r;
+}

@@ -119,6 +119,7 @@ struct Net {
   std::vector<LevelMeta> lv;
   std::vector<LevelBufs> b;
   float *V, *Vp, *Z, *s_head;
+  float* wide_sum = nullptr;  // inference forward: partial sums of the tcgen05 input-channel slices (c_in > 256)
   float *d_Z, *d_R0, *d_X0, *d_Vp;        // backward: gradients w.r.t. Z, R_0, X_0 (operand form) and Vp
   float *d_wp = nullptr, *d_V = nullptr;  // backward, padded stem input only: gradients w.r.t. wp and V
   int head, n_params;                     // the head BatchNorm's first parameter slot; the number of slots
@@ -1008,6 +1009,13 @@ size_t infer_layout(Net& net, InferLayout& IL, void* ws) {
     }
   }
   net.Z = a.f(n0, net.m);
+  // A tensor-core convolution of more than 256 input channels runs as input slices whose partial sum goes through
+  // memory before the last slice's epilogue: one buffer of the largest such output.  Every convolution producing level
+  // l's rows has at most planes(l) output and 2 planes(l) input channels.
+  int64_t wide = 0;
+  for (int l = 0; l < net.L && net.mode != MM3D_MODE_FP32; ++l)
+    if (2 * net.planes(l) > 256 && net.lv[l].n * net.planes(l) > wide) wide = net.lv[l].n * net.planes(l);
+  net.wide_sum = wide ? a.f(wide, 1) : nullptr;
   net.img_ws_bytes = img_region_bytes(net, false);
   net.img_ws = a.bytes(net.img_ws_bytes);
   net.wp = net.cin_k != net.cin ? a.f(27, (int64_t)net.cin_k * net.m) : nullptr;
@@ -1105,7 +1113,8 @@ struct Infer {
     if (abl_skip("conv")) return;
     const Table t = table(c, kind, l);
     if (const float* im = find_img(c, w)) {
-      EX(conv_img(c, in, t.n_in, c_in, nullptr, t.n_out, c_out, im, find_img_lo(c, w), t.K, t.plan, t.cap, add, &e));
+      EX(conv_img(c, in, t.n_in, c_in, c_in > 256 ? net.wide_sum : nullptr, t.n_out, c_out, im, find_img_lo(c, w), t.K, t.plan,
+                  t.cap, add, &e));
     } else if (net.x3() || net.bf16()) {
       mm3d_set_error("unet: conv c_in %d c_out %d has no tensor-core weight image in this mode", c_in, c_out);
       if (c.rc == 0) c.rc = MM3D_ERR_UNSUPPORTED;
