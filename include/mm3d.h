@@ -125,6 +125,15 @@ MM3D_API int mm3d_coarsen(const uint64_t* fine_keys, const int32_t* n_fine_dev, 
 MM3D_API int mm3d_build_nbr27(const uint64_t* keys, const int32_t* n_dev, int64_t n_cap, int spatial_size,
                      const uint64_t* hash_keys, const int32_t* hash_vals, int64_t hash_cap,
                      int32_t* nbr_tbl, int64_t tbl_stride, mm3d_stream_t stream);
+/* Row boundaries of batch groups (grouped BatchNorm statistics, mm3d_unet_topo_forward_grouped): the structure holds
+ * `groups` batches one after the other, group k's scans with batch indices in [batch_start[k], batch_start[k + 1])
+ * (device int64 [groups + 1]), and its points before group k + 1's.  keys: HOST array of the levels' device key arrays,
+ * counts: device int32, level l's row count at counts[l].  Writes the device int32 bounds[levels][groups + 1], level l's
+ * group k = rows [bounds[l (groups + 1) + k], ... + 1).  One launch, no host synchronisation. */
+#define MM3D_MAX_GROUP_LEVELS 16
+MM3D_API int mm3d_group_bounds(const uint64_t* const* keys, const int32_t* counts, int levels, const int64_t* batch_start,
+                      int groups, int32_t* bounds, mm3d_stream_t stream);
+
 
 /* Row plan of a rule table, used by the tensor-core convolution modes: the table's output rows
  * ordered by neighbour mask (stable radix sort per 8192-row chunk), the table permuted into that
@@ -299,6 +308,26 @@ MM3D_API int mm3d_bnrelu_bwd_ex(const float* x, const float* dy, float* dx, int6
                        const float* beta, const float* save_mean, const float* save_invstd,
                        float* d_gamma, float* d_beta, float leakiness, int training,
                        void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags);
+/* Grouped BatchNorm statistics: the rows are `groups` consecutive ranges [bounds[k], bounds[k + 1]) (bounds: HOST
+ * array of groups + 1 row indices, 0 = bounds[0] <= ... <= bounds[groups] = n), and a training forward normalises each
+ * range as if it were its own mm3d_bnrelu_fwd_ex call, in range order: its own batch mean and biased variance, its own
+ * row of save_mean / save_invstd (both [groups][c]) and its own running-statistics update (unbiased with the range's
+ * row count; an empty range changes nothing).  The backward's dx is per range; d_gamma / d_beta total all rows.  Eval
+ * mode (training = 0) normalises with the running statistics, so the groups change nothing there (save_* are then [c]).
+ * 1 <= groups <= MM3D_BN_MAX_GROUPS; with groups = 1 the launches, workspace and results are those of the _ex
+ * functions.  ws: mm3d_bnrelu_workspace_bytes_grouped(c, groups, flags) (0 = bad arguments). */
+#define MM3D_BN_MAX_GROUPS 8
+MM3D_API size_t mm3d_bnrelu_workspace_bytes_grouped(int c, int groups, int flags);
+MM3D_API int mm3d_bnrelu_fwd_grouped(const float* x, float* y, int64_t n, int c, const float* gamma, const float* beta,
+                            float* running_mean, float* running_var, float* save_mean, float* save_invstd,
+                            float eps, float momentum, float leakiness, int training,
+                            void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags, int groups,
+                            const int64_t* bounds);
+MM3D_API int mm3d_bnrelu_bwd_grouped(const float* x, const float* dy, float* dx, int64_t n, int c, const float* gamma,
+                            const float* beta, const float* save_mean, const float* save_invstd,
+                            float* d_gamma, float* d_beta, float leakiness, int training,
+                            void* ws, size_t ws_bytes, mm3d_stream_t stream, int flags, int groups,
+                            const int64_t* bounds);
 
 /* ------------------------------------------------------------------------------------------
  * 2D->3D lift (replaces the per-sample advanced indexing of 2d_net/model.py:131-137):
@@ -476,6 +505,36 @@ MM3D_API int mm3d_unet_topo_backward_ex(int in_channels, int m, int num_planes, 
                                float* d_feats, void* const* params, void* const* grads, void* act, size_t act_bytes,
                                void* tmp, size_t tmp_bytes, void* scratch, size_t scratch_bytes,
                                const mm3d_unet_mask* mask, mm3d_stream_t stream, int flags);
+/* Grouped BatchNorm statistics (mm3d_bnrelu_fwd_grouped): several batches through one structure, one forward and one
+ * backward, each normalised as if it had been its own call.  The rows of every level are `groups` consecutive ranges,
+ * bounds: HOST int64 [num_planes][groups + 1], level l's group k = rows [bounds[l (groups + 1) + k], ... + 1), each
+ * level's running from 0 to its row count.  A training forward is then the same as one mm3d_unet_topo_forward_ex call
+ * per group, in group order: every BatchNorm normalises a group's rows with that group's statistics and updates the
+ * running statistics once per group.  The backward gives each group's feature gradient as its own call would and the
+ * parameter (and mask) gradients summed over the groups.  Eval mode: the groups change nothing.  1 <= groups <=
+ * MM3D_BN_MAX_GROUPS; groups == 1 (bounds may then be NULL) is the _ex call.  The saved statistics grow to [groups][C]:
+ * act and scratch come from the _grouped queries (mm3d_unet_topo_bwd_bytes does not depend on the groups). */
+typedef struct {
+  int groups;
+  const int64_t* bounds;
+} mm3d_unet_groups;
+MM3D_API size_t mm3d_unet_topo_act_bytes_grouped(int in_channels, int m, int num_planes, int block_reps, int residual,
+                                        int mode, const int64_t* level_desc, int64_t n_points, int groups);
+MM3D_API size_t mm3d_unet_topo_scratch_bytes_grouped(int in_channels, int m, int num_planes, int block_reps, int residual,
+                                            int mode, int flags, int groups);
+MM3D_API int mm3d_unet_topo_forward_grouped(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                   int training, float eps, float momentum, const int64_t* level_desc, int64_t n_points,
+                                   const int32_t* p2v, const int32_t* npts, const int32_t* vox_start,
+                                   const int32_t* vox_pts, const float* feats, float* out, void* const* params, void* act,
+                                   size_t act_bytes, void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask,
+                                   mm3d_stream_t stream, int flags, const mm3d_unet_groups* groups);
+MM3D_API int mm3d_unet_topo_backward_grouped(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                    int training, const int64_t* level_desc, int64_t n_points, const int32_t* p2v,
+                                    const int32_t* npts, const int32_t* vox_start, const int32_t* vox_pts,
+                                    const float* d_out, float* d_feats, void* const* params, void* const* grads, void* act,
+                                    size_t act_bytes, void* tmp, size_t tmp_bytes, void* scratch, size_t scratch_bytes,
+                                    const mm3d_unet_mask* mask, mm3d_stream_t stream, int flags,
+                                    const mm3d_unet_groups* groups);
 /* Inference forward: the eval-mode forward (BatchNorm with the running statistics, training = 0) without anything a
  * backward would read.  Every BatchNorm+ReLU is applied in the epilogue of the convolution that produces its input and
  * the JoinTable concatenations are never materialised; the output is the same bits as mm3d_unet_topo_forward_ex with

@@ -19,7 +19,15 @@ class UnetMask(C.Structure):
     _fields_ = [("wb", C.c_void_p), ("s", C.c_void_p), ("feats", C.c_void_p), ("d_wb", C.c_void_p),
                 ("ws", C.c_void_p), ("ws_bytes", C.c_size_t)]
 
+
+class UnetGroups(C.Structure):
+    """``mm3d_unet_groups`` of ``include/mm3d.h``."""
+    _fields_ = [("groups", C.c_int), ("bounds", C.c_void_p)]
+
+
 LEVEL_DESC_WORDS = 10
+BN_MAX_GROUPS = 8        # MM3D_BN_MAX_GROUPS: batch groups of one grouped call
+MAX_GROUP_LEVELS = 16    # MM3D_MAX_GROUP_LEVELS
 
 MODE_FP32, MODE_TF32, MODE_BF16, MODE_TF32X3 = 0, 1, 2, 3
 MODES = {"fp32": MODE_FP32, "tf32": MODE_TF32, "bf16": MODE_BF16, "tf32x3": MODE_TF32X3}
@@ -123,6 +131,16 @@ SIGNATURES = {
                                         _p, _sz, _p, _p, _i]),
     "mm3d_unet_topo_infer_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _p, _i64, _i]),
     "mm3d_unet_topo_infer": (_i, [_i, _i, _i, _i, _i, _i, _f, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p, _p, _i]),
+    "mm3d_group_bounds": (_i, [_p, _p, _i, _p, _i, _p, _p]),
+    "mm3d_bnrelu_workspace_bytes_grouped": (_sz, [_i, _i, _i]),
+    "mm3d_bnrelu_fwd_grouped": (_i, [_p, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _f, _f, _f, _i, _p, _sz, _p, _i, _i, _p]),
+    "mm3d_bnrelu_bwd_grouped": (_i, [_p, _p, _p, _i64, _i, _p, _p, _p, _p, _p, _p, _f, _i, _p, _sz, _p, _i, _i, _p]),
+    "mm3d_unet_topo_act_bytes_grouped": (_sz, [_i, _i, _i, _i, _i, _i, _p, _i64, _i]),
+    "mm3d_unet_topo_scratch_bytes_grouped": (_sz, [_i, _i, _i, _i, _i, _i, _i, _i]),
+    "mm3d_unet_topo_forward_grouped": (_i, [_i, _i, _i, _i, _i, _i, _i, _f, _f, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p,
+                                            _sz, _p, _p, _i, _p]),
+    "mm3d_unet_topo_backward_grouped": (_i, [_i, _i, _i, _i, _i, _i, _i, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p,
+                                             _sz, _p, _sz, _p, _p, _i, _p]),
 }
 
 class PlanDesc(C.Structure):

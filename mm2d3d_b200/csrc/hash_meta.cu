@@ -306,7 +306,49 @@ int carve_ws(void* ws, size_t ws_bytes, int64_t n_cap, int64_t hash_cap, UniqueW
   return MM3D_OK;
 }
 
+// Group row boundaries (grouped BatchNorm statistics): several batches built as one structure, group k's scans with
+// batch indices [batch_start[k], batch_start[k + 1]).  Its points precede group k + 1's and every level numbers its rows
+// by first occurrence, so each group is one contiguous row range at every level and "batch >= batch_start[k]" is false
+// then true along the rows: boundary k is the first row where it holds (a binary search).  blockIdx.x = level.
+struct GroupLevels {
+  const uint64_t* keys[MM3D_MAX_GROUP_LEVELS];
+};
+__global__ void k_group_bounds(const __grid_constant__ GroupLevels lv, const int32_t* __restrict__ counts,
+                               const int64_t* __restrict__ batch_start, int groups, int32_t* __restrict__ bounds) {
+  mm3d_griddep_wait();
+  const int l = blockIdx.x;
+  const int64_t n = counts[l];
+  for (int k = threadIdx.x; k <= groups; k += blockDim.x) {
+    int64_t lo = 0, hi = n;  // boundary k in [lo, hi]
+    if (k == 0) hi = 0;
+    else if (k < groups) {
+      const int64_t b = batch_start[k];
+      while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if ((int64_t)(lv.keys[l][mid] >> 48) >= b) hi = mid;
+        else lo = mid + 1;
+      }
+    }
+    bounds[l * (groups + 1) + k] = (int32_t)hi;
+  }
+}
+
 }  // namespace
+
+// bounds[l (groups + 1) + k]: the first row of group k at level l (bounds[.. + groups] = the level's row count)
+extern "C" int mm3d_group_bounds(const uint64_t* const* keys, const int32_t* counts, int levels, const int64_t* batch_start,
+                                 int groups, int32_t* bounds, mm3d_stream_t stream) {
+  MM3D_REQUIRE(levels >= 1 && levels <= MM3D_MAX_GROUP_LEVELS && groups >= 1 && keys && counts && bounds &&
+                   (groups == 1 || batch_start),
+               MM3D_ERR_INVALID, "group_bounds: bad arguments");
+  GroupLevels lv{};
+  for (int l = 0; l < levels; ++l) lv.keys[l] = keys[l];
+  MM3D_CUDA(mm3d_launch_pdl(k_group_bounds, dim3(levels), dim3(32), 0, (cudaStream_t)stream, lv, counts, batch_start, groups,
+                            bounds));
+  mm3d_count_launches(1);
+  MM3D_CHECK_LAUNCH("mm3d_group_bounds");
+  return MM3D_OK;
+}
 
 extern "C" int64_t mm3d_hash_capacity(int64_t n) {
   int64_t want = 2 * (n > 16 ? n : 16);

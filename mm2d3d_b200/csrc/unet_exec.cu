@@ -35,12 +35,13 @@
 int mm3d_bnrelu_fwd_impl(const float* x, const float* x_hi, int c_lo, float* y, int64_t n, int c, const float* gamma,
                          const float* beta, float* running_mean, float* running_var, float* save_mean,
                          float* save_invstd, float eps, float momentum, float leakiness, int training, void* ws,
-                         size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream, int det);
+                         size_t ws_bytes, int* parity, int round_tf32, cudaStream_t stream, int det, int groups,
+                         const int64_t* bounds);
 int mm3d_bnrelu_bwd_impl(const float* x, const float* x_hi, int c_lo, const float* dy, float* dx, float* dx_hi,
                          int64_t n, int c, const float* gamma, const float* beta, const float* save_mean,
                          const float* save_invstd, float* d_gamma, float* d_beta, float leakiness, int training,
                          void* ws, size_t ws_bytes, int* parity, int round_flags, const float* add, int64_t add_ld,
-                         cudaStream_t stream, int det);
+                         cudaStream_t stream, int det, int groups, const int64_t* bounds);
 
 // conv_tc.cu
 size_t mm3d_conv_tc_workspace_bytes(int c_in, int c_out, int K);
@@ -91,7 +92,7 @@ struct ConvInfo {
 struct BlockBufs {
   int a, b;
   int pidx;            // first parameter slot
-  float *A, *s1;       // first BatchNorm's output (operand form) and its save_mean | save_invstd ([2][a])
+  float *A, *s1;       // first BatchNorm's output (operand form) and its save_mean | save_invstd ([2][G][a])
   float *H, *A2, *s2;  // residual: first SMC's output, second BatchNorm's output (operand form), its save
   float* out;          // [n, b]
   // backward: gradients w.r.t. A, A2, H (operand form), the NetworkInNetwork's input, and the block's input (operand
@@ -102,7 +103,7 @@ struct BlockBufs {
 struct LevelBufs {
   float *X, *Y, *B, *E, *F, *J, *R;
   float* Jop;           // NiN shortcut: J in operand form (== J in FP32 mode)
-  float *s_dn, *s_up;   // BN save_mean | save_invstd ([2][C])
+  float *s_dn, *s_up;   // BN save_mean | save_invstd ([2][G][C])
   void* id_plan;        // NiN shortcut: identity row plan of the level's rows (capacity n)
   int dn, up;           // first parameter slot of the down and the up branch (BatchNorm, then the convolution at + 4)
   std::vector<BlockBufs> pre, post;
@@ -116,6 +117,10 @@ struct Net {
   int reps, res;         // blocks per pre / post group; residual blocks
   int mode;
   int flags;  // MM3D_DETERMINISTIC or 0
+  // grouped BatchNorm statistics: G row groups, level l's group k = rows [gb[l (G + 1) + k], gb[l (G + 1) + k + 1]);
+  // every saved statistic is [G][C] (mean) then [G][C] (invstd)
+  int G = 1;
+  std::vector<int64_t> gb;
   std::vector<LevelMeta> lv;
   std::vector<LevelBufs> b;
   float *V, *Vp, *Z, *s_head;
@@ -137,6 +142,7 @@ struct Net {
   int64_t n_points;
   bool det() const { return (flags & MM3D_DETERMINISTIC) != 0; }
   int planes(int l) const { return m * (l + 1); }
+  const int64_t* bounds(int l) const { return G > 1 ? gb.data() + (size_t)l * (G + 1) : nullptr; }
   // TF32x3 mode: every tensor a convolution gathers carries a hi and a lo plane ([rows, c] floats each)
   // BF16 mode: an FP32 plane (TF32-rounded: the weight-gradient operand) and a BF16 plane behind it (what forward and
   // dgrad gather; it only fills the first half of its plane)
@@ -175,14 +181,14 @@ struct Carve {
     bn(a);
     conv(27, a, b, 1);
     k.A = act.f(n, (int64_t)a * pl);
-    k.s1 = act.f(2, a);
+    k.s1 = act.f(2 * net.G, a);
     k.d_A = tmp.f(n, a);
     if (net.res) {
       bn(b);
       conv(27, b, b, 1);
       k.H = act.f(n, b);
       k.A2 = act.f(n, (int64_t)b * pl);
-      k.s2 = act.f(2, b);
+      k.s2 = act.f(2 * net.G, b);
       k.d_A2 = tmp.f(n, b);
       k.d_H = tmp.f(n, (int64_t)b * pl);
     }
@@ -210,14 +216,14 @@ struct Carve {
     B.dn = bn(p);
     conv(8, p, q, 0);
     B.B = act.f(n, (int64_t)p * pl);
-    B.s_dn = act.f(2, p);
+    B.s_dn = act.f(2 * net.G, p);
     B.d_B = tmp.f(n, p);
     B.d_Xn = tmp.f(nc, (int64_t)q * pl);
     level(l + 1, B.d_Xn);
     B.up = bn(q);
     conv(8, q, p, 0);
     B.E = act.f(nc, (int64_t)q * pl);
-    B.s_up = act.f(2, q);
+    B.s_up = act.f(2 * net.G, q);
     B.d_Rn = tmp.f(nc, (int64_t)q * pl);
     B.d_E = tmp.f(nc, q);
     B.F = act.f(n, p);
@@ -254,7 +260,7 @@ struct Carve {
     net.head = bn(net.m);
     net.n_params = pi;
     net.Z = act.f(n0, net.m);
-    net.s_head = act.f(2, net.m);
+    net.s_head = act.f(2 * net.G, net.m);
     net.d_Z = tmp.f(n0, net.m);
     net.d_R0 = tmp.f(n0, (int64_t)net.m * pl);
   }
@@ -284,12 +290,13 @@ void carve_scratch(Net& net, Bump& bp) {
   net.conv_ws = bp.bytes(conv);
   net.img_ws_bytes = img_region_bytes(net);
   net.img_ws = bp.bytes(net.img_ws_bytes);
-  net.bn_ws_bytes = mm3d_bnrelu_workspace_bytes(2 * net.m * net.L);
+  // (the groups' accumulators side by side: G times the widest layer's)
+  net.bn_ws_bytes = mm3d_bnrelu_workspace_bytes(2 * net.m * net.L * net.G);
   net.bn_ws = bp.bytes(net.bn_ws_bytes);
   net.wp = net.cin_k != net.cin ? bp.f(27, (int64_t)net.cin_k * net.m) : nullptr;
   if (!net.det()) return;
   // (behind the default layout, which stays as it is; the default BatchNorm workspace is then unused)
-  net.bn_ws_bytes = mm3d_bnrelu_workspace_bytes_ex(2 * net.m * net.L, MM3D_DETERMINISTIC);
+  net.bn_ws_bytes = mm3d_bnrelu_workspace_bytes_ex(2 * net.m * net.L * net.G, MM3D_DETERMINISTIC);
   net.bn_ws = bp.bytes(net.bn_ws_bytes);
   size_t wg = 0;
   for (const ConvInfo& ci : net.convs) {  // (0 for a convolution without a deterministic form: it keeps the default)
@@ -502,23 +509,27 @@ float* Gp(Ctx& c, int i) { return (float*)c.grads[i]; }
 // tensor core's truncation of the low mantissa bits is exact.  `to_conv`: the output feeds a convolution.
 bool tc_mode(const Ctx& c) { return c.net->mode != MM3D_MODE_FP32; }
 
-void bn_fwd(Ctx& c, int pidx, const float* x, float* y, int64_t n, int ch, float* save, const float* x_hi = nullptr,
+// l: the level whose rows x holds (its group boundaries)
+void bn_fwd(Ctx& c, int pidx, int l, const float* x, float* y, int64_t n, int ch, float* save, const float* x_hi = nullptr,
             int c_lo = 0, bool to_conv = true) {
   if (abl_skip("bn")) return;
+  const Net& net = *c.net;
   EX(mm3d_bnrelu_fwd_impl(x, x_hi, c_lo, y, n, ch, P(c, pidx), P(c, pidx + 1), (float*)c.params[pidx + 2], (float*)c.params[pidx + 3],
-                          save, save + ch, c.eps, c.momentum, 0.f, c.training, c.net->bn_ws, c.net->bn_ws_bytes, &c.bn_parity,
-                          tc_mode(c) && to_conv ? c.net->rmode() : 0, c.stream, c.net->det()));
+                          save, save + (int64_t)net.G * ch, c.eps, c.momentum, 0.f, c.training, net.bn_ws, net.bn_ws_bytes,
+                          &c.bn_parity, tc_mode(c) && to_conv ? net.rmode() : 0, c.stream, net.det(), net.G, net.bounds(l)));
 }
 // round: bit 0 = dx (its low column block when split) feeds a convolution as d_out, bit 1 = dx_hi does
 // add (rows add_ld floats apart): another gradient of the same tensor, summed into dx before it is stored;
 // add_lo: `add` is a TF32x3 operand whose lo plane (n * add_ld floats behind) is summed too
-void bn_bwd(Ctx& c, int pidx, const float* x, const float* dy, float* dx, int64_t n, int ch, const float* save,
+void bn_bwd(Ctx& c, int pidx, int l, const float* x, const float* dy, float* dx, int64_t n, int ch, const float* save,
             int round, const float* x_hi = nullptr, int c_lo = 0, float* dx_hi = nullptr, const float* add = nullptr,
             int64_t add_ld = 0, bool add_lo = false) {
   if (abl_skip("bn")) return;
-  const int flags = tc_mode(c) ? (round | (c.net->x3() ? 4 : c.net->bf16() ? 8 : 0) | (add_lo ? 16 : 0)) : 0;
-  EX(mm3d_bnrelu_bwd_impl(x, x_hi, c_lo, dy, dx, dx_hi, n, ch, P(c, pidx), P(c, pidx + 1), save, save + ch, Gp(c, pidx), Gp(c, pidx + 1), 0.f,
-                          c.training, c.net->bn_ws, c.net->bn_ws_bytes, &c.bn_parity, flags, add, add_ld, c.stream, c.net->det()));
+  const Net& net = *c.net;
+  const int flags = tc_mode(c) ? (round | (net.x3() ? 4 : net.bf16() ? 8 : 0) | (add_lo ? 16 : 0)) : 0;
+  EX(mm3d_bnrelu_bwd_impl(x, x_hi, c_lo, dy, dx, dx_hi, n, ch, P(c, pidx), P(c, pidx + 1), save, save + (int64_t)net.G * ch,
+                          Gp(c, pidx), Gp(c, pidx + 1), 0.f, c.training, net.bn_ws, net.bn_ws_bytes, &c.bn_parity, flags, add,
+                          add_ld, c.stream, net.det(), net.G, net.bounds(l)));
 }
 // NIN: NetworkInNetwork, a K = 1 convolution over the level's identity row plan
 enum Kind { SMC, DOWN, UP, NIN };
@@ -735,13 +746,13 @@ void block_fwd(Ctx& c, int l, const BlockBufs& k, const float* x, bool join) {
     const bool split = (p & 3) == 0 && c.training;  // JoinTable never materialised: BatchNorm reads [Y | F] directly
     // the shortcut gathers J: it is written (the BatchNorm of an unsplit join reads the unrounded J)
     if (!split || o) launch_join(c, B.Y, B.F, n, p, split ? B.Jop : B.J);
-    if (split) bn_fwd(c, bn1, B.Y, k.A, n, 2 * p, k.s1, B.F, p);
-    else bn_fwd(c, bn1, B.J, k.A, n, 2 * p, k.s1);
+    if (split) bn_fwd(c, bn1, l, B.Y, k.A, n, 2 * p, k.s1, B.F, p);
+    else bn_fwd(c, bn1, l, B.J, k.A, n, 2 * p, k.s1);
     if (o && tc_mode(c))  // J in operand form (rounded; + second plane)
       launch_pad_cols(c, split ? B.Jop : B.J, n, 2 * p, B.Jop, 2 * p, net.rmode());
     MARK("bn_fwd post", l);
   } else {
-    bn_fwd(c, bn1, x, k.A, n, k.a, k.s1);
+    bn_fwd(c, bn1, l, x, k.A, n, k.a, k.s1);
     MARK("bn_fwd block", l);
   }
   if (!net.res) {
@@ -750,7 +761,7 @@ void block_fwd(Ctx& c, int l, const BlockBufs& k, const float* x, bool join) {
     return;
   }
   conv_fwd(c, SMC, l, k.A, k.a, k.H, k.b, P(c, bn1 + 4));
-  bn_fwd(c, bn1 + 5, k.H, k.A2, n, k.b, k.s2);
+  bn_fwd(c, bn1 + 5, l, k.H, k.A2, n, k.b, k.s2);
   if (o) {  // NetworkInNetwork shortcut writes `out`, the second convolution adds onto it
     conv_fwd(c, NIN, l, B.Jop, k.a, k.out, k.b, P(c, k.pidx));
     conv_fwd(c, SMC, l, k.A2, k.b, k.out, k.b, P(c, bn1 + 9), k.out);
@@ -772,12 +783,12 @@ void level_fwd(Ctx& c, int l) {
   }
   if (l + 1 < net.L) {
     const int q = net.planes(l + 1);
-    bn_fwd(c, B.dn, B.Y, B.B, n, p, B.s_dn);
+    bn_fwd(c, B.dn, l, B.Y, B.B, n, p, B.s_dn);
     MARK("bn_fwd dn", l);
     conv_fwd(c, DOWN, l, B.B, p, net.b[l + 1].X, q, P(c, B.dn + 4));
     MARK("down_fwd", l);
     level_fwd(c, l + 1);
-    bn_fwd(c, B.up, net.b[l + 1].R, B.E, net.lv[l + 1].n, q, B.s_up);
+    bn_fwd(c, B.up, l + 1, net.b[l + 1].R, B.E, net.lv[l + 1].n, q, B.s_up);
     MARK("bn_fwd up", l);
     conv_fwd(c, UP, l, B.E, q, B.F, p, P(c, B.up + 4));
     MARK("up_fwd", l);
@@ -801,7 +812,7 @@ void block_bwd(Ctx& c, int l, const BlockBufs& k, const float* x, const float* d
     conv_bwd(c, SMC, l, k.A, k.a, d_o, k.b, P(c, k.pidx + 4), k.d_A, Gp(c, k.pidx + 4));
   } else {
     conv_bwd(c, SMC, l, k.A2, k.b, d_o, k.b, P(c, bn1 + 9), k.d_A2, Gp(c, bn1 + 9));
-    bn_bwd(c, bn1 + 5, k.H, k.d_A2, k.d_H, n, k.b, k.s2, 1);
+    bn_bwd(c, bn1 + 5, l, k.H, k.d_A2, k.d_H, n, k.b, k.s2, 1);
     conv_bwd(c, SMC, l, k.A, k.a, k.d_H, k.b, P(c, bn1 + 4), k.d_A, Gp(c, bn1 + 4));
     if (o) {
       conv_bwd(c, NIN, l, B.Jop, k.a, d_o, k.b, P(c, k.pidx), k.d_S, Gp(c, k.pidx));
@@ -815,15 +826,15 @@ void block_bwd(Ctx& c, int l, const BlockBufs& k, const float* x, const float* d
   }
   MARK("block conv bwd", l);
   if (!join) {
-    bn_bwd(c, bn1, x, k.d_A, k.d_x, n, k.a, k.s1, 1, nullptr, 0, nullptr, add, add_ld, add_lo);
+    bn_bwd(c, bn1, l, x, k.d_A, k.d_x, n, k.a, k.s1, 1, nullptr, 0, nullptr, add, add_ld, add_lo);
     MARK("bn_bwd block", l);
     return;
   }
   const int p = k.b;
   if ((p & 3) == 0 && c.training) {  // as in the forward: [Y | F] was never concatenated
-    bn_bwd(c, bn1, B.Y, k.d_A, B.d_J, n, 2 * p, k.s1, 2, B.F, p, B.d_F, add, add_ld);  // d_F is the deconvolution's d_out
+    bn_bwd(c, bn1, l, B.Y, k.d_A, B.d_J, n, 2 * p, k.s1, 2, B.F, p, B.d_F, add, add_ld);  // d_F is the deconvolution's d_out
   } else {
-    bn_bwd(c, bn1, B.J, k.d_A, B.d_J, n, 2 * p, k.s1, 0, nullptr, 0, nullptr, add, add_ld);  // (eval-mode backward: d_F stays unrounded)
+    bn_bwd(c, bn1, l, B.J, k.d_A, B.d_J, n, 2 * p, k.s1, 0, nullptr, 0, nullptr, add, add_ld);  // (eval-mode backward: d_F stays unrounded)
     // d_F = d_J[:, p:]; the skip half is combined with the branch gradient further down
     if (n && !c.rc) {
       if (mm3d_launch_pdl(k_copy_cols, dim3(mm3d_grid(n * p / 4 + 1, 256)), dim3(256), 0, c.stream, (const float*)B.d_J, n, 2 * p, B.d_F, p, 0, p, p) != cudaSuccess) c.rc = MM3D_ERR_CUDA;
@@ -852,7 +863,7 @@ void level_bwd(Ctx& c, int l, const float* d_R) {
     block_bwd(c, l, B.post[0], nullptr, d_o, true);
     conv_bwd(c, UP, l, B.E, q, B.d_F, p, P(c, B.up + 4), B.d_E, Gp(c, B.up + 4));
     MARK("up_dgrad", l);
-    bn_bwd(c, B.up, net.b[l + 1].R, B.d_E, B.d_Rn, nc, q, B.s_up, 1);
+    bn_bwd(c, B.up, l + 1, net.b[l + 1].R, B.d_E, B.d_Rn, nc, q, B.s_up, 1);
     MARK("bn_bwd up", l);
     level_bwd(c, l + 1, B.d_Rn);
     conv_bwd(c, DOWN, l, B.B, p, B.d_Xn, q, P(c, B.dn + 4), B.d_B, Gp(c, B.dn + 4));
@@ -860,7 +871,7 @@ void level_bwd(Ctx& c, int l, const float* d_R) {
     // d_Y = d_J[:, :p] (the skip half of the join's gradient) + the branch gradient: summed inside the BatchNorm
     // backward of the down-branch, stored rounded (it is the pre-block convolution's d_out)
     const bool split = (p & 3) == 0 && c.training;
-    bn_bwd(c, B.dn, B.Y, B.d_B, B.d_Yskip, n, p, B.s_dn, 1, nullptr, 0, nullptr, B.d_J, split ? p : 2 * p);
+    bn_bwd(c, B.dn, l, B.Y, B.d_B, B.d_Yskip, n, p, B.s_dn, 1, nullptr, 0, nullptr, B.d_J, split ? p : 2 * p);
     MARK("bn_bwd dn", l);
     d_Y = B.d_Yskip;
   }
@@ -871,7 +882,7 @@ void level_bwd(Ctx& c, int l, const float* d_R) {
 }
 
 int fill_net(Net& net, int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
-             const int64_t* level_desc, int64_t n_points, int flags = 0) {
+             const int64_t* level_desc, int64_t n_points, int flags = 0, const mm3d_unet_groups* groups = nullptr) {
   MM3D_REQUIRE((flags & ~MM3D_DETERMINISTIC) == 0, MM3D_ERR_INVALID, "unet: unknown flags %#x", flags);
   MM3D_REQUIRE(num_planes >= 1 && num_planes <= 16 && m > 0 && in_channels > 0, MM3D_ERR_INVALID, "bad network shape");
   MM3D_REQUIRE(block_reps >= 1 && block_reps <= 16 && (residual == 0 || residual == 1), MM3D_ERR_INVALID,
@@ -888,6 +899,21 @@ int fill_net(Net& net, int in_channels, int m, int num_planes, int block_reps, i
     const int64_t* d = level_desc + MM3D_LEVEL_DESC_WORDS * l;
     net.lv[l] = LevelMeta{d[0], (const int32_t*)d[1], d[2], (const int32_t*)d[3], (const uint8_t*)d[4], (const int32_t*)d[5],
                           (const void*)d[6], (const void*)d[7], (const void*)d[8], d[9]};
+  }
+  if (groups) {  // (a NULL bounds array only sizes: the queries)
+    MM3D_REQUIRE(groups->groups >= 1 && groups->groups <= MM3D_BN_MAX_GROUPS, MM3D_ERR_INVALID,
+                 "unet: %d groups (1..%d supported)", groups->groups, MM3D_BN_MAX_GROUPS);
+    net.G = groups->groups;
+    if (groups->bounds && net.G > 1) {
+      net.gb.assign(groups->bounds, groups->bounds + (size_t)num_planes * (net.G + 1));
+      for (int l = 0; l < num_planes && level_desc; ++l) {
+        const int64_t* b = net.gb.data() + (size_t)l * (net.G + 1);
+        MM3D_REQUIRE(b[0] == 0 && b[net.G] == net.lv[l].n, MM3D_ERR_INVALID,
+                     "unet: level %d's group boundaries must run from 0 to its %lld rows", l, (long long)net.lv[l].n);
+        for (int k = 1; k <= net.G; ++k)
+          MM3D_REQUIRE(b[k] >= b[k - 1], MM3D_ERR_INVALID, "unet: level %d's group boundaries decrease", l);
+      }
+    }
   }
   return MM3D_OK;
 }
@@ -1175,11 +1201,16 @@ MM3D_API int64_t mm3d_unet_topo_num_params(int num_planes, int block_reps, int r
 }
 MM3D_API int64_t mm3d_unet_num_params(int num_planes) { return mm3d_unet_topo_num_params(num_planes, 1, 0); }
 
+MM3D_API size_t mm3d_unet_topo_act_bytes_grouped(int in_channels, int m, int num_planes, int block_reps, int residual,
+                                                 int mode, const int64_t* level_desc, int64_t n_points, int groups) {
+  Net net;
+  const mm3d_unet_groups g{groups, nullptr};
+  if (!level_desc || fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points, 0, &g)) return 0;
+  return lay_out(net, nullptr, nullptr, nullptr).act + 256;
+}
 MM3D_API size_t mm3d_unet_topo_act_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
                                          const int64_t* level_desc, int64_t n_points) {
-  Net net;
-  if (!level_desc || fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points)) return 0;
-  return lay_out(net, nullptr, nullptr, nullptr).act + 256;
+  return mm3d_unet_topo_act_bytes_grouped(in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points, 1);
 }
 MM3D_API size_t mm3d_unet_act_bytes(int in_channels, int m, int num_planes, int mode, const int64_t* level_desc,
                                     int64_t n_points) {
@@ -1197,11 +1228,16 @@ MM3D_API size_t mm3d_unet_bwd_bytes(int in_channels, int m, int num_planes, int 
   return mm3d_unet_topo_bwd_bytes(in_channels, m, num_planes, 1, 0, mode, level_desc, n_points);
 }
 
+MM3D_API size_t mm3d_unet_topo_scratch_bytes_grouped(int in_channels, int m, int num_planes, int block_reps, int residual,
+                                                     int mode, int flags, int groups) {
+  Net net;
+  const mm3d_unet_groups g{groups, nullptr};
+  if (fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, nullptr, 0, flags, &g)) return 0;
+  return lay_out(net, nullptr, nullptr, nullptr).scratch;  // (independent of the row counts)
+}
 MM3D_API size_t mm3d_unet_topo_scratch_bytes_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
                                                int flags) {
-  Net net;
-  if (fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, nullptr, 0, flags)) return 0;
-  return lay_out(net, nullptr, nullptr, nullptr).scratch;  // (independent of the row counts)
+  return mm3d_unet_topo_scratch_bytes_grouped(in_channels, m, num_planes, block_reps, residual, mode, flags, 1);
 }
 MM3D_API size_t mm3d_unet_topo_scratch_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode) {
   return mm3d_unet_topo_scratch_bytes_ex(in_channels, m, num_planes, block_reps, residual, mode, 0);
@@ -1210,18 +1246,20 @@ MM3D_API size_t mm3d_unet_scratch_bytes(int in_channels, int m, int num_planes, 
   return mm3d_unet_topo_scratch_bytes(in_channels, m, num_planes, 1, 0, mode);
 }
 
-MM3D_API int mm3d_unet_topo_forward_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
-                                       int training, float eps, float momentum, const int64_t* level_desc, int64_t n_points,
-                                       const int32_t* p2v, const int32_t* npts, const int32_t* vox_start,
-                                       const int32_t* vox_pts, const float* feats, float* out, void* const* params, void* act,
-                                       size_t act_bytes, void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask,
-                                       mm3d_stream_t stream_, int flags) {
+MM3D_API int mm3d_unet_topo_forward_grouped(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                            int training, float eps, float momentum, const int64_t* level_desc,
+                                            int64_t n_points, const int32_t* p2v, const int32_t* npts,
+                                            const int32_t* vox_start, const int32_t* vox_pts, const float* feats, float* out,
+                                            void* const* params, void* act, size_t act_bytes, void* scratch,
+                                            size_t scratch_bytes, const mm3d_unet_mask* mask, mm3d_stream_t stream_, int flags,
+                                            const mm3d_unet_groups* groups) {
+  MM3D_REQUIRE(!groups || groups->groups == 1 || groups->bounds, MM3D_ERR_INVALID, "unet forward: groups without boundaries");
   MM3D_REQUIRE(level_desc, MM3D_ERR_INVALID, "unet forward: no level descriptors");
   MM3D_REQUIRE(!mask || (mask->wb && (n_points == 0 || mask->s)), MM3D_ERR_INVALID, "unet forward: incomplete mask descriptor");
   MM3D_REQUIRE(!(flags & MM3D_DETERMINISTIC) || (vox_start && vox_pts), MM3D_ERR_INVALID,
                "unet forward: the deterministic mode needs the voxels' point lists (mm3d_point_csr)");
   Net net;
-  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points, flags);
+  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points, flags, groups);
   if (rc) return rc;
   const Sizes need = lay_out(net, act, nullptr, scratch);  // (no backward temporaries)
   MM3D_REQUIRE(act_bytes >= need.act, MM3D_ERR_WORKSPACE, "activation workspace too small: need %zu have %zu", need.act, act_bytes);
@@ -1238,11 +1276,22 @@ MM3D_API int mm3d_unet_topo_forward_ex(int in_channels, int m, int num_planes, i
   conv_fwd(c, SMC, 0, net.Vp, net.cin_k, net.b[0].X, m, w_stem);
   MARK("stem fwd", -1);
   level_fwd(c, 0);
-  bn_fwd(c, net.head, net.b[0].R, net.Z, n0, m, net.s_head, nullptr, 0, /*to_conv=*/false);
+  bn_fwd(c, net.head, 0, net.b[0].R, net.Z, n0, m, net.s_head, nullptr, 0, /*to_conv=*/false);
   MARK("bn_fwd head", -1);
   EX(mm3d_output_fwd(net.Z, p2v, n_points, m, out, c.stream));
   MARK("output_fwd", -1);
   return c.rc;
+}
+
+MM3D_API int mm3d_unet_topo_forward_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                       int training, float eps, float momentum, const int64_t* level_desc, int64_t n_points,
+                                       const int32_t* p2v, const int32_t* npts, const int32_t* vox_start,
+                                       const int32_t* vox_pts, const float* feats, float* out, void* const* params, void* act,
+                                       size_t act_bytes, void* scratch, size_t scratch_bytes, const mm3d_unet_mask* mask,
+                                       mm3d_stream_t stream_, int flags) {
+  return mm3d_unet_topo_forward_grouped(in_channels, m, num_planes, block_reps, residual, mode, training, eps, momentum,
+                                        level_desc, n_points, p2v, npts, vox_start, vox_pts, feats, out, params, act,
+                                        act_bytes, scratch, scratch_bytes, mask, stream_, flags, nullptr);
 }
 
 MM3D_API int mm3d_unet_topo_forward(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
@@ -1264,12 +1313,14 @@ MM3D_API int mm3d_unet_forward(int in_channels, int m, int num_planes, int mode,
 }
 
 // grads: same slot order as params (running-stat slots ignored); d_feats may be NULL.
-MM3D_API int mm3d_unet_topo_backward_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
-                                        int training, const int64_t* level_desc, int64_t n_points, const int32_t* p2v,
-                                        const int32_t* npts, const int32_t* vox_start, const int32_t* vox_pts,
-                                        const float* d_out, float* d_feats, void* const* params, void* const* grads, void* act,
-                                        size_t act_bytes, void* tmp, size_t tmp_bytes, void* scratch, size_t scratch_bytes,
-                                        const mm3d_unet_mask* mask, mm3d_stream_t stream_, int flags) {
+MM3D_API int mm3d_unet_topo_backward_grouped(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                             int training, const int64_t* level_desc, int64_t n_points, const int32_t* p2v,
+                                             const int32_t* npts, const int32_t* vox_start, const int32_t* vox_pts,
+                                             const float* d_out, float* d_feats, void* const* params, void* const* grads,
+                                             void* act, size_t act_bytes, void* tmp, size_t tmp_bytes, void* scratch,
+                                             size_t scratch_bytes, const mm3d_unet_mask* mask, mm3d_stream_t stream_,
+                                             int flags, const mm3d_unet_groups* groups) {
+  MM3D_REQUIRE(!groups || groups->groups == 1 || groups->bounds, MM3D_ERR_INVALID, "unet backward: groups without boundaries");
   MM3D_REQUIRE(level_desc, MM3D_ERR_INVALID, "unet backward: no level descriptors");
   MM3D_REQUIRE(!mask || (mask->wb && mask->d_wb && mask->ws && (n_points == 0 || (mask->s && mask->feats))), MM3D_ERR_INVALID,
                "unet backward: incomplete mask descriptor");
@@ -1279,7 +1330,7 @@ MM3D_API int mm3d_unet_topo_backward_ex(int in_channels, int m, int num_planes, 
                MM3D_ERR_WORKSPACE, "unet backward: the deterministic mode's mask workspace needs %d doubles",
                MM3D_DET_CTAS * (in_channels + 1));
   Net net;
-  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points, flags);
+  int rc = fill_net(net, in_channels, m, num_planes, block_reps, residual, mode, level_desc, n_points, flags, groups);
   if (rc) return rc;
   const Sizes need = lay_out(net, act, tmp, scratch);
   MM3D_REQUIRE(act_bytes >= need.act, MM3D_ERR_WORKSPACE, "activation workspace too small: need %zu have %zu", need.act, act_bytes);
@@ -1324,7 +1375,7 @@ MM3D_API int mm3d_unet_topo_backward_ex(int in_channels, int m, int num_planes, 
   else
     EX(mm3d_output_bwd(d_out, p2v, n_points, n0, m, net.d_Z, c.stream));
   MARK("output_bwd", -1);
-  bn_bwd(c, net.head, net.b[0].R, net.d_Z, net.d_R0, n0, m, net.s_head, 1);
+  bn_bwd(c, net.head, 0, net.b[0].R, net.d_Z, net.d_R0, n0, m, net.s_head, 1);
   MARK("bn_bwd head", -1);
   level_bwd(c, 0, net.d_R0);
   // stem
@@ -1356,6 +1407,17 @@ MM3D_API int mm3d_unet_topo_backward_ex(int in_channels, int m, int num_planes, 
   join_side(c);  // everything after this call on `stream` sees the weight gradients
   MARK("join wgrad stream", -1);
   return c.rc;
+}
+
+MM3D_API int mm3d_unet_topo_backward_ex(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,
+                                        int training, const int64_t* level_desc, int64_t n_points, const int32_t* p2v,
+                                        const int32_t* npts, const int32_t* vox_start, const int32_t* vox_pts,
+                                        const float* d_out, float* d_feats, void* const* params, void* const* grads, void* act,
+                                        size_t act_bytes, void* tmp, size_t tmp_bytes, void* scratch, size_t scratch_bytes,
+                                        const mm3d_unet_mask* mask, mm3d_stream_t stream_, int flags) {
+  return mm3d_unet_topo_backward_grouped(in_channels, m, num_planes, block_reps, residual, mode, training, level_desc,
+                                         n_points, p2v, npts, vox_start, vox_pts, d_out, d_feats, params, grads, act,
+                                         act_bytes, tmp, tmp_bytes, scratch, scratch_bytes, mask, stream_, flags, nullptr);
 }
 
 MM3D_API size_t mm3d_unet_topo_infer_bytes(int in_channels, int m, int num_planes, int block_reps, int residual, int mode,

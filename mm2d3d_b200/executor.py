@@ -20,6 +20,10 @@ autograd would not record -- grad mode off, or no input of the call (features, R
 requiring a gradient -- runs ``mm3d_unet_topo_infer`` instead: every BatchNorm+ReLU in the epilogue of the convolution that produces its input, no
 JoinTable copies, a workspace of only what the forward writes, no autograd node.  The output is the same bits as the
 eval forward through ``UNetSCNFn`` (which ``net(x).detach()`` with grad mode on still runs).
+
+Grouped BatchNorm statistics (``UNetSCN.forward_groups`` / ``prepare_groups``, :func:`run_groups`): several batches
+through one structure (``metadata.group_coords``), one forward and one backward; in training mode the executor's
+``mm3d_unet_topo_*_grouped`` calls normalise each group's rows with the group's own statistics, level by level.
 """
 from __future__ import annotations
 
@@ -31,7 +35,7 @@ import torch
 from . import _lib
 from . import functional as F
 from ._lib import check, lib
-from .metadata import Metadata
+from .metadata import Metadata, group_coords
 
 
 def collect_slots(net):
@@ -151,6 +155,16 @@ def _level_desc(meta: Metadata, num_planes: int, spatial0: int, plans: bool):
     return desc
 
 
+def _unet_groups(meta: Metadata, num_planes: int):
+    """(``mm3d_unet_groups``, its bounds array) of a grouped structure's first ``num_planes`` levels."""
+    G = meta.groups
+    flat = [b for lv in meta.group_bounds()[:num_planes] for b in lv]
+    if len(flat) != num_planes * (G + 1):
+        raise ValueError("UNetSCN: the grouped structure has fewer levels than the network")
+    bounds = (C.c_int64 * len(flat))(*flat)
+    return _lib.UnetGroups(G, C.addressof(bounds)), bounds
+
+
 class UNetSCNFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, feats, meta, cfg, mask_w, mask_b, *slots):
@@ -168,13 +182,20 @@ class UNetSCNFn(torch.autograd.Function):
         wb = _mask_wb(in_ch, mask_w, mask_b) if masked else None  # (checked before anything is allocated)
         n_points = meta.n_points
         desc = _level_desc(meta, L, spatial0, plans=mode != _lib.MODE_FP32)
+        # a structure of several batch groups (UNetSCN.forward_groups), training mode: every BatchNorm per group
+        groups = _unet_groups(meta, L) if training and meta.groups > 1 else None
+        G = meta.groups if groups is not None else 1
         with torch.cuda.device(dev):
             # sticky device-error words (mapped host memory): whatever a kernel of an earlier call raised surfaces
             # here -- no synchronisation, a few nanoseconds
             _lib.raise_device_errors("UNetSCN.forward")
-            act_bytes = lib.mm3d_unet_topo_act_bytes(in_ch, m, L, reps, res, mode, desc, n_points)
+            if groups is None:
+                act_bytes = lib.mm3d_unet_topo_act_bytes(in_ch, m, L, reps, res, mode, desc, n_points)
+                scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes_ex(in_ch, m, L, reps, res, mode, flags), dev)
+            else:
+                act_bytes = lib.mm3d_unet_topo_act_bytes_grouped(in_ch, m, L, reps, res, mode, desc, n_points, G)
+                scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes_grouped(in_ch, m, L, reps, res, mode, flags, G), dev)
             act = torch.empty(act_bytes, dtype=torch.uint8, device=dev)
-            scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes_ex(in_ch, m, L, reps, res, mode, flags), dev)
             out = torch.empty(n_points, m, dtype=torch.float32, device=dev)
             vox_start, vox_pts = meta.point_csr() if det else (None, None)
             params = (C.c_void_p * len(slots))(*[t.data_ptr() for t in slots])
@@ -182,7 +203,14 @@ class UNetSCNFn(torch.autograd.Function):
             if masked:
                 gate = torch.empty(max(n_points, 1), dtype=torch.float32, device=dev)
                 mask = C.byref(_lib.UnetMask(wb.data_ptr(), gate.data_ptr(), None, None, None, 0))
-            if det:
+            if groups is not None:
+                check(lib.mm3d_unet_topo_forward_grouped(in_ch, m, L, reps, res, mode, int(training), eps, momentum, desc,
+                                                         n_points, meta.p2v_ptr, meta.npts_ptr, _lib.ptr(vox_start),
+                                                         _lib.ptr(vox_pts), feats.data_ptr(), out.data_ptr(), params,
+                                                         act.data_ptr(), act_bytes, scr.data_ptr(), scr.numel(), mask,
+                                                         _lib.stream_ptr(), flags, C.byref(groups[0])),
+                      "mm3d_unet_topo_forward_grouped")
+            elif det:
                 check(lib.mm3d_unet_topo_forward_ex(in_ch, m, L, reps, res, mode, int(training), eps, momentum, desc, n_points,
                                                     meta.p2v_ptr, meta.npts_ptr, vox_start.data_ptr(), vox_pts.data_ptr(),
                                                     feats.data_ptr(), out.data_ptr(), params, act.data_ptr(), act_bytes,
@@ -195,6 +223,7 @@ class UNetSCNFn(torch.autograd.Function):
                                                  _lib.stream_ptr()), "mm3d_unet_topo_forward")
         ctx.meta, ctx.cfg, ctx.desc, ctx.act, ctx.slots = meta, cfg, desc, act, slots
         ctx.flags = flags  # the backward keeps the forward's choice
+        ctx.groups = groups
         ctx.feats_shape = feats.shape
         ctx.mask = (feats, wb, gate, mask_w.shape, mask_b.shape) if masked else None
         return out
@@ -229,7 +258,12 @@ class UNetSCNFn(torch.autograd.Function):
                 d_feats.zero_()
             tmp_bytes = lib.mm3d_unet_topo_bwd_bytes(in_ch, m, L, reps, res, mode, desc, n_points)
             tmp = torch.empty(tmp_bytes, dtype=torch.uint8, device=dev)
-            scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes_ex(in_ch, m, L, reps, res, mode, flags), dev)
+            groups = ctx.groups
+            if groups is None:
+                scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes_ex(in_ch, m, L, reps, res, mode, flags), dev)
+            else:
+                scr = F.scratch(lib.mm3d_unet_topo_scratch_bytes_grouped(in_ch, m, L, reps, res, mode, flags,
+                                                                         groups[0].groups), dev)
             params = (C.c_void_p * len(slots))(*[t.data_ptr() for t in slots])
             gp = (C.c_void_p * len(slots))(*gptrs)
             mask, d_mw, d_mb = None, None, None
@@ -242,7 +276,15 @@ class UNetSCNFn(torch.autograd.Function):
                                              mws.numel() * 8))
                 d_mw, d_mb = d_wb[:in_ch].reshape(w_shape), d_wb[in_ch:].reshape(b_shape)
             d_feats_ptr = d_feats.data_ptr() if need_feats else None
-            if flags:
+            if groups is not None:
+                vox_start, vox_pts = meta.point_csr() if flags else (None, None)
+                check(lib.mm3d_unet_topo_backward_grouped(in_ch, m, L, reps, res, mode, int(training), desc, n_points,
+                                                          meta.p2v_ptr, meta.npts_ptr, _lib.ptr(vox_start),
+                                                          _lib.ptr(vox_pts), d_out.data_ptr(), d_feats_ptr, params, gp,
+                                                          act.data_ptr(), act.numel(), tmp.data_ptr(), tmp_bytes,
+                                                          scr.data_ptr(), scr.numel(), mask, _lib.stream_ptr(), flags,
+                                                          C.byref(groups[0])), "mm3d_unet_topo_backward_grouped")
+            elif flags:
                 vox_start, vox_pts = meta.point_csr()
                 check(lib.mm3d_unet_topo_backward_ex(in_ch, m, L, reps, res, mode, int(training), desc, n_points, meta.p2v_ptr,
                                                      meta.npts_ptr, vox_start.data_ptr(), vox_pts.data_ptr(), d_out.data_ptr(),
@@ -262,11 +304,12 @@ class PreparedScans:
     typically on a side stream while the previous step still computes, the way a prefetching data loader prepares
     the next batch.  Pass it to ``UNetSCN.forward`` in place of the coordinate tensor."""
 
-    __slots__ = ("meta", "event", "stream", "mode", "spatial0", "levels", "points")
+    __slots__ = ("meta", "event", "stream", "mode", "spatial0", "levels", "points", "sizes")
 
-    def __init__(self, meta, mode, spatial0, levels, points=None):
+    def __init__(self, meta, mode, spatial0, levels, points=None, sizes=None):
         self.meta, self.mode, self.spatial0, self.levels = meta, mode, spatial0, levels
         self.points = points  # augment.PointStructure when the batch was prepared from raw float points
+        self.sizes = sizes  # prepare_groups: the groups' point counts (None: one batch)
         self.stream = torch.cuda.current_stream(meta.device)
         self.event = torch.cuda.Event()
         self.event.record(self.stream)
@@ -312,6 +355,22 @@ def prepare(net, coords, wait=False):
         if F.deterministic():  # the voxels' point lists too, one step ahead like the rest of the structure
             meta.point_csr()
         return PreparedScans(meta, F.DEFAULT_MODE, spatial0, L)
+
+
+def prepare_groups(net, coords_list, wait=False):
+    """:func:`prepare` for several batch groups (``UNetSCN.forward_groups``): one structure build of the groups one
+    after the other, their row boundaries at every level computed on the device and read back with the row counts."""
+    if not isinstance(coords_list, (list, tuple)) or not all(isinstance(c, torch.Tensor) and c.is_cuda for c in coords_list):
+        raise RuntimeError("UNetSCN.prepare_groups: a list of CUDA coordinate tensors expected -- mm2d3d_b200 has no "
+                           "CPU path")
+    spatial0 = int(net.layer1.spatial_size[0])
+    L = net._num_planes
+    with torch.cuda.device(coords_list[0].device):
+        coords, batch_start = group_coords(coords_list)
+        meta = Metadata(coords, spatial0, L, plans=F.DEFAULT_MODE != "fp32", defer_sync=not wait, batch_start=batch_start)
+        if F.deterministic():
+            meta.point_csr()
+        return PreparedScans(meta, F.DEFAULT_MODE, spatial0, L, sizes=[int(c.shape[0]) for c in coords_list])
 
 
 def prepare_points(net, points, sample_offsets, rot, transl_u, scale, wait=False):
@@ -384,9 +443,8 @@ def infer(feats, meta, cfg, mask_w, mask_b, slots):
     return out
 
 
-def run(net, coords, feats, rgb_mask=None):
-    if not feats.is_cuda:
-        raise RuntimeError("UNetSCN: features must be a CUDA tensor -- mm2d3d_b200 has no CPU path")
+def _resolve(net, coords, feats):
+    """The structure of a forward: a prepared one (waited for on this stream) or one built now from ``coords``."""
     spatial0 = int(net.layer1.spatial_size[0])
     L = net._num_planes
     if isinstance(coords, PreparedScans):
@@ -403,6 +461,53 @@ def run(net, coords, feats, rgb_mask=None):
         if coords.device != feats.device:
             coords = coords.to(feats.device, non_blocking=True)
         meta = Metadata(coords, spatial0, L, plans=F.DEFAULT_MODE != "fp32")
+    return meta
+
+
+def run(net, coords, feats, rgb_mask=None):
+    if not feats.is_cuda:
+        raise RuntimeError("UNetSCN: features must be a CUDA tensor -- mm2d3d_b200 has no CPU path")
+    if isinstance(coords, PreparedScans) and coords.sizes is not None:
+        raise ValueError("UNetSCN: a structure from prepare_groups goes to forward_groups")
+    return _run(net, _resolve(net, coords, feats), feats, rgb_mask)
+
+
+def group_structure(net, coords, feats):
+    """(structure, the groups' point counts) of ``UNetSCN.forward_groups``: a structure from :func:`prepare_groups`
+    (waited for on this stream), or one built now from the list of the groups' coordinate tensors."""
+    if isinstance(coords, PreparedScans):
+        if coords.sizes is None:
+            raise ValueError("UNetSCN.forward_groups: the prepared structure is not grouped (use prepare_groups)")
+        check_group_feats(coords.sizes, feats)
+        return _resolve(net, coords, feats[0]), coords.sizes
+    sizes = [int(c.shape[0]) for c in coords]
+    check_group_feats(sizes, feats)
+    with torch.cuda.device(feats[0].device):
+        c, batch_start = group_coords(coords, feats[0].device)
+        meta = Metadata(c, int(net.layer1.spatial_size[0]), net._num_planes, plans=F.DEFAULT_MODE != "fp32",
+                        batch_start=batch_start)
+    return meta, sizes
+
+
+def run_groups(net, meta, sizes, feats, rgb_mask=None):
+    """``UNetSCN.forward_groups`` on the executor: one forward over the groups' structure (training mode: every
+    BatchNorm per group), the output split back into the groups (views of one tensor)."""
+    return list(_run(net, meta, torch.cat(list(feats)), rgb_mask).split(sizes))
+
+
+def check_group_feats(sizes, feats):
+    if len(feats) != len(sizes):
+        raise ValueError(f"UNetSCN.forward_groups: {len(sizes)} coordinate groups but {len(feats)} feature groups")
+    for k, (n, f) in enumerate(zip(sizes, feats)):
+        if not isinstance(f, torch.Tensor) or not f.is_cuda:
+            raise RuntimeError("UNetSCN: features must be a CUDA tensor -- mm2d3d_b200 has no CPU path")
+        if f.dim() != 2 or f.shape[0] != n:
+            raise ValueError(f"UNetSCN.forward_groups: group {k} has {n} points but features of shape {tuple(f.shape)}")
+
+
+def _run(net, meta, feats, rgb_mask):
+    spatial0 = int(net.layer1.spatial_size[0])
+    L = net._num_planes
     if feats.shape[0] < meta.n_points:
         raise ValueError(f"UNetSCN: {feats.shape[0]} feature rows for {meta.n_points} points")
     bn0 = net.layer4

@@ -8,6 +8,7 @@ argument, defaulting to the module-level :data:`DEFAULT_MODE`.
 """
 from __future__ import annotations
 
+import ctypes as C
 import warnings
 
 import torch
@@ -275,17 +276,29 @@ class TableConvFn(torch.autograd.Function):
 class BatchNormReLUFn(torch.autograd.Function):
     @staticmethod
     @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
-    def forward(ctx, x, gamma, beta, running_mean, running_var, eps, momentum, leakiness, training):
+    def forward(ctx, x, gamma, beta, running_mean, running_var, eps, momentum, leakiness, training, bounds=None):
+        """``bounds``: the row boundaries of batch groups (``Metadata.group_bounds``), each normalised with its own
+        statistics in training mode (``mm3d_bnrelu_fwd_grouped``); ``None`` = one group."""
         _require_cuda(x, "BatchNormReLU")
         x = _f32c(x)
         n, c = x.shape
         y = torch.empty_like(x)
-        save = torch.empty(2, c, dtype=torch.float32, device=x.device)
+        grouped = bounds is not None and len(bounds) > 2 and training
+        G = len(bounds) - 1 if grouped else 1
+        save = torch.empty(2, G, c, dtype=torch.float32, device=x.device)
         # deterministic: every reduction over rows (the training forward's statistics, and every backward: d_gamma /
         # d_beta are row sums in eval mode too) in its fixed-order form
         det = deterministic()
         with torch.cuda.device(x.device):
-            if det and training:
+            if grouped:
+                flags = _lib.DETERMINISTIC if det else 0
+                b = (C.c_int64 * (G + 1))(*bounds)
+                ws = scratch(lib.mm3d_bnrelu_workspace_bytes_grouped(c, G, flags), x.device)
+                check(lib.mm3d_bnrelu_fwd_grouped(ptr(x), ptr(y), n, c, ptr(gamma), ptr(beta), ptr(running_mean),
+                                                  ptr(running_var), ptr(save[0]), ptr(save[1]), eps, momentum, leakiness, 1,
+                                                  ptr(ws), ws.numel(), _lib.stream_ptr(), flags, G, b),
+                      "mm3d_bnrelu_fwd_grouped")
+            elif det and training:
                 ws = scratch(lib.mm3d_bnrelu_workspace_bytes_ex(c, _lib.DETERMINISTIC), x.device)
                 check(lib.mm3d_bnrelu_fwd_ex(ptr(x), ptr(y), n, c, ptr(gamma), ptr(beta), ptr(running_mean),
                                              ptr(running_var), ptr(save[0]), ptr(save[1]), eps, momentum, leakiness, 1,
@@ -298,6 +311,7 @@ class BatchNormReLUFn(torch.autograd.Function):
                                           ws.numel(), _lib.stream_ptr()), "mm3d_bnrelu_fwd")
         ctx.save_for_backward(x, gamma, beta, save)
         ctx.leak, ctx.training, ctx.det = leakiness, bool(training), det
+        ctx.bounds = tuple(bounds) if grouped else None
         return y
 
     @staticmethod
@@ -309,7 +323,16 @@ class BatchNormReLUFn(torch.autograd.Function):
         dx = torch.empty_like(x)
         dgb = torch.empty(2, c, dtype=torch.float32, device=x.device)
         with torch.cuda.device(x.device):
-            if ctx.det:
+            if ctx.bounds is not None:
+                G = len(ctx.bounds) - 1
+                flags = _lib.DETERMINISTIC if ctx.det else 0
+                b = (C.c_int64 * (G + 1))(*ctx.bounds)
+                ws = scratch(lib.mm3d_bnrelu_workspace_bytes_grouped(c, G, flags), x.device)
+                check(lib.mm3d_bnrelu_bwd_grouped(ptr(x), ptr(dy), ptr(dx), n, c, ptr(gamma), ptr(beta), ptr(save[0]),
+                                                  ptr(save[1]), ptr(dgb[0]), ptr(dgb[1]), ctx.leak, int(ctx.training),
+                                                  ptr(ws), ws.numel(), _lib.stream_ptr(), flags, G, b),
+                      "mm3d_bnrelu_bwd_grouped")
+            elif ctx.det:
                 ws = scratch(lib.mm3d_bnrelu_workspace_bytes_ex(c, _lib.DETERMINISTIC), x.device)
                 check(lib.mm3d_bnrelu_bwd_ex(ptr(x), ptr(dy), ptr(dx), n, c, ptr(gamma), ptr(beta), ptr(save[0]),
                                              ptr(save[1]), ptr(dgb[0]), ptr(dgb[1]), ctx.leak, int(ctx.training), ptr(ws),
@@ -320,7 +343,7 @@ class BatchNormReLUFn(torch.autograd.Function):
                 check(lib.mm3d_bnrelu_bwd(ptr(x), ptr(dy), ptr(dx), n, c, ptr(gamma), ptr(beta), ptr(save[0]), ptr(save[1]),
                                           ptr(dgb[0]), ptr(dgb[1]), ctx.leak, int(ctx.training), ptr(ws), ws.numel(),
                                           _lib.stream_ptr()), "mm3d_bnrelu_bwd")
-        return dx, dgb[0], dgb[1], None, None, None, None, None, None
+        return dx, dgb[0], dgb[1], None, None, None, None, None, None, None
 
 
 # ----------------------------------------------------------------------------- 2D -> 3D lift

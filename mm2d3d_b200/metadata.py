@@ -12,6 +12,8 @@ tensor views are only materialised for inspection (tests, debugging).
 """
 from __future__ import annotations
 
+import ctypes as C
+
 import torch
 
 from . import _lib
@@ -41,7 +43,7 @@ class Metadata:
     _side = {}  # per-device side stream for the neighbour tables
 
     def __init__(self, coords: torch.Tensor, spatial_size: int, prebuild_levels: int = 1, plans: bool = False,
-                 defer_sync: bool = False, points=None):
+                 defer_sync: bool = False, points=None, batch_start=None):
         """``defer_sync``: enqueue the build and an asynchronous read-back of the row counts, but do not wait for
         them; :meth:`finish` (called by every accessor that needs a row count) does.  Lets a caller enqueue a build
         on a side stream and keep launching other work.
@@ -50,8 +52,15 @@ class Metadata:
         dict of device tensors ``points [N,3] f32, offsets [B+1] i64, rot [B,9] f32, u [B,3] f64 or None, keep [N] u8,
         min_value [B,3] f32, offset [B,3] f64`` and the float ``scale`` (see ``augment.voxelize_points``).  If the
         batch holds a point outside the receptive field :attr:`dropped` is set once the counts are known and the
-        structure must not be used."""
+        structure must not be used.
+
+        ``batch_start`` (see :func:`group_coords`): the coordinates are several batch groups one after the other, group
+        k's scans with batch indices ``[batch_start[k], batch_start[k + 1])`` (device int64 ``[G + 1]``).  Every level
+        of the pre-built pyramid then also gets its group row boundaries (:meth:`group_bounds`), computed on the device
+        and read back with the row counts."""
         self.dropped = False
+        self.groups = 1 if batch_start is None else int(batch_start.numel()) - 1
+        self._group_bounds = None
         self._points = points  # (keeps the build's input tensors alive)
         if points is not None:
             if coords is not None:
@@ -83,7 +92,9 @@ class Metadata:
 
         with torch.cuda.device(self.device):
             stream = _lib.stream_ptr()
-            self._counts = torch.zeros(self.MAX_LEVELS + 1, dtype=torch.int32, device=self.device)
+            # row counts, status word, then (groups) each level's group boundaries
+            n_bounds = self.MAX_LEVELS * (self.groups + 1) if batch_start is not None else 0
+            self._counts = torch.zeros(self.MAX_LEVELS + 1 + n_bounds, dtype=torch.int32, device=self.device)
             if points is not None:
                 B = int(points["offsets"].numel()) - 1
                 ws_bytes = lib.mm3d_voxelize_points_workspace_bytes(n, B)
@@ -139,8 +150,13 @@ class Metadata:
                 # hardware hands out CTAs in index order, so the second wave should be the light ones
                 specs = [("smc", s) for s in sizes] + [("down", s) for s in sizes[:-1]] + [("up", s) for s in sizes[:-1]]
                 self.build_plans(specs)
+            if batch_start is not None:
+                self._batch_start = batch_start  # (kept alive until the launch is done)
+                keys = (C.c_void_p * L)(*[lv.ptr(lv.o_keys) for lv in self._order])
+                check(lib.mm3d_group_bounds(keys, cp, L, batch_start.data_ptr(), self.groups,
+                                            cp + 4 * (self.MAX_LEVELS + 1), stream), "mm3d_group_bounds")
             if defer_sync:
-                host = torch.empty(self.MAX_LEVELS + 1, dtype=torch.int32, pin_memory=True)
+                host = torch.empty(self._counts.numel(), dtype=torch.int32, pin_memory=True)
                 host.copy_(self._counts, non_blocking=True)
                 ev = torch.cuda.Event()
                 ev.record()
@@ -210,6 +226,24 @@ class Metadata:
         for lv in self._order:
             if lv.n is None:
                 lv.n = int(host[lv.count_slot])
+        if self.groups > 1 or host.numel() > self.MAX_LEVELS + 1:
+            g1 = self.groups + 1
+            b = host[self.MAX_LEVELS + 1:].view(self.MAX_LEVELS, g1)
+            self._group_bounds = [tuple(int(v) for v in b[lv.count_slot]) for lv in self._order]
+
+    def group_bounds(self, spatial_size=None):
+        """Group row boundaries (a structure built from :func:`group_coords`): per pre-built level, shallow to deep, a
+        tuple of ``groups + 1`` row indices -- group k = rows ``[b[k], b[k + 1])``; with ``spatial_size`` that level's
+        tuple only.  ``None`` for an ungrouped structure."""
+        self.finish()
+        if self._group_bounds is None:
+            return None
+        if spatial_size is None:
+            return self._group_bounds
+        lv = self.levels[int(spatial_size)]
+        if lv.count_slot >= len(self._group_bounds):
+            raise ValueError(f"no group boundaries for spatial size {spatial_size} (not a pre-built level)")
+        return self._group_bounds[lv.count_slot]
 
     def record_stream(self, stream):
         """Tell the caching allocator that ``stream`` uses this structure's buffers (needed when the structure
@@ -394,3 +428,33 @@ class Metadata:
         off = self._lv_view(fine, fine.o_off, torch.uint8, fine.n)
         child = self._lv_view(fine, fine.o_child, torch.int32, 8 * fine.tstride).view(8, fine.tstride)
         return parent, off, child[:, :coarse.n].t().contiguous()
+
+
+def group_coords(coords_list, device=None):
+    """Concatenate the coordinates of several batch groups into one structure's input, keeping the groups apart:
+    group k's batch column (each group's starting from 0) is offset by the scans of the groups before it.  The offsets
+    are computed on the device (no host synchronisation).  Returns ``(coords [sum N_k, 4] int64, batch_start int64
+    [G + 1])`` for ``Metadata(..., batch_start=...)``."""
+    if not isinstance(coords_list, (list, tuple)) or not coords_list:
+        raise ValueError("group_coords: a non-empty list of [N, 4] coordinate tensors expected")
+    if len(coords_list) > _lib.BN_MAX_GROUPS:
+        raise ValueError(f"group_coords: {len(coords_list)} groups; at most {_lib.BN_MAX_GROUPS} are supported")
+    cs = []
+    for c in coords_list:
+        if not isinstance(c, torch.Tensor) or c.dim() != 2 or c.shape[1] != 4:
+            raise ValueError("group_coords: every group's coordinates must be a tensor [N, 4] = (x, y, z, batch)")
+        if device is not None and c.device != torch.device(device):
+            c = c.to(device, non_blocking=True)
+        cs.append(c.to(torch.int64))
+    dev = cs[0].device
+    if any(c.device != dev for c in cs):
+        raise ValueError("group_coords: the groups' coordinates are on different devices")
+    # scans per group = its largest batch index + 1 (0 for an empty group), summed up on the device
+    counts = [c[:, 3].max().reshape(1) + 1 if c.shape[0] else torch.zeros(1, dtype=torch.int64, device=dev) for c in cs]
+    batch_start = torch.cat([torch.zeros(1, dtype=torch.int64, device=dev), torch.cat(counts).cumsum(0)])
+    out = torch.cat(cs)
+    row = cs[0].shape[0]
+    for k in range(1, len(cs)):  # (device scalars: no host synchronisation)
+        out[row:row + cs[k].shape[0], 3] += batch_start[k]
+        row += cs[k].shape[0]
+    return out, batch_start

@@ -235,8 +235,11 @@ class BatchNormLeakyReLU(nn.Module):
         self.register_buffer("running_var", torch.ones(nPlanes))
 
     def forward(self, x):
+        # a structure of several batch groups (UNetSCN.forward_groups): each group normalised with its own statistics
+        meta = x.metadata
+        bounds = meta.group_bounds(_ss(x)) if self.training and getattr(meta, "groups", 1) > 1 else None
         y = F.BatchNormReLUFn.apply(x.features, self.weight, self.bias, self.running_mean, self.running_var,
-                                    float(self.eps), float(self.momentum), float(self.leakiness), self.training)
+                                    float(self.eps), float(self.momentum), float(self.leakiness), self.training, bounds)
         return SparseConvNetTensor(y, x.metadata, x.spatial_size)
 
     def extra_repr(self):

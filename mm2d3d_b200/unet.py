@@ -115,6 +115,81 @@ class UNetSCN(nn.Module):
             raise RuntimeError("UNetSCN.prepare_points needs the fused executor (native backend, fused=True)")
         return executor.prepare_points(self, points, sample_offsets, rot, transl_u, scale, wait)
 
+    def prepare_groups(self, coords, wait=False):
+        """:meth:`prepare` for :meth:`forward_groups`: one structure build for several batch groups (a list of
+        coordinate tensors, each group's batch column starting from 0), enqueued on the current stream."""
+        from . import executor
+        self._check_groups(coords)
+        if len(coords) == 1:
+            return self.prepare(coords[0], wait)
+        if not (self.fused and self._native and executor.fusable(self)):
+            raise RuntimeError("UNetSCN.prepare_groups needs the fused executor (native backend, fused=True)")
+        return executor.prepare_groups(self, coords, wait)
+
+    def forward_groups(self, coords, feats, rgb_mask=None):
+        """Several batches through one structure build, one forward and one backward: ``coords`` a list of
+        ``[N_g, 4]`` coordinate tensors (each group's batch column starting from 0) or what :meth:`prepare_groups`
+        returned, ``feats`` the list of the groups' ``[N_g, C]`` features.  Returns the list of the groups' ``[N_g, m]``
+        outputs (views of one tensor).  The result is that of ``[self([coords[g], feats[g]]) for g in groups]`` run in
+        that order: in training mode every BatchNorm normalises each group with the group's own batch statistics and
+        updates the running statistics once per group, in group order; feature gradients are per group, parameter
+        (and RGB-mask) gradients the sums over the groups, in one flat gradient tensor.  In eval mode the groups change
+        nothing: coordinate lists then run as plain calls, a prepared structure as one eval forward over it.  At most
+        8 groups (``MM3D_BN_MAX_GROUPS``); the two-domain step of MM2D3D needs 2.  A prepared structure takes the
+        same path as coordinates: the executor when it takes the network, else module by module."""
+        from . import executor
+        feats = list(feats) if isinstance(feats, (list, tuple)) else feats
+        if not isinstance(feats, list):
+            raise ValueError("UNetSCN.forward_groups: feats must be a list of the groups' feature tensors")
+        if isinstance(coords, executor.PreparedScans):
+            if coords.sizes is None:  # (prepare_groups of one group: the plain path)
+                if len(feats) != 1:
+                    raise ValueError(f"UNetSCN.forward_groups: 1 coordinate group but {len(feats)} feature groups")
+                return [self([coords, feats[0]], rgb_mask)]
+        else:
+            self._check_groups(coords)
+            if len(coords) != len(feats):
+                raise ValueError(f"UNetSCN.forward_groups: {len(coords)} coordinate groups but {len(feats)} feature "
+                                 "groups")
+            if len(coords) == 1:  # one group is a plain call
+                return [self([coords[0], feats[0]], rgb_mask)]
+            if not self.training:
+                # eval mode normalises with the running statistics: the groups change nothing, and plain calls give
+                # each group the bits of its own call (a shared structure tiles the convolutions' rows differently)
+                out = torch.cat([self([c, x], rgb_mask) for c, x in zip(coords, feats)])
+                return list(out.split([int(c.shape[0]) for c in coords]))
+        if not self._native:
+            raise RuntimeError("UNetSCN.forward_groups needs the native backend")
+        rgb_mask = self._mask_pair(rgb_mask)
+        meta, sizes = executor.group_structure(self, coords, feats)
+        if self.fused and executor.fusable(self) and (rgb_mask is None or self.in_channels == 3):
+            return executor.run_groups(self, meta, sizes, feats, rgb_mask)
+        # module by module over the groups' structure: every BatchNorm finds the groups in the metadata
+        from . import functional as F
+        from .scn import SparseConvNetTensor
+        x = torch.cat(feats)
+        if rgb_mask is not None:
+            from .heads import rgb_mask as _mask
+            x = _mask(x, rgb_mask[0], rgb_mask[1])
+        y = SparseConvNetTensor(F.InputLayerFn.apply(x, meta, self.layer1.mode), meta, self.layer1.spatial_size)
+        for layer in (self.layer2, self.layer3, self.layer4, self.layer5):
+            y = layer(y)
+        return list(y.split(sizes))
+
+    @staticmethod
+    def _check_groups(coords):
+        from ._lib import BN_MAX_GROUPS
+        if not isinstance(coords, (list, tuple)) or not coords:
+            raise ValueError("UNetSCN.forward_groups: a non-empty list of the groups' coordinate tensors expected")
+        if len(coords) > BN_MAX_GROUPS:
+            raise ValueError(f"UNetSCN.forward_groups: {len(coords)} groups; at most {BN_MAX_GROUPS} are supported")
+
+    @staticmethod
+    def _mask_pair(rgb_mask):
+        if rgb_mask is not None and not isinstance(rgb_mask, (tuple, list)):
+            return (rgb_mask.weight, rgb_mask.bias)
+        return rgb_mask
+
     def forward(self, x, rgb_mask=None):
         """``x = [coords, feats]`` as in the reference.  ``rgb_mask``: an ``nn.Linear(in_channels, 1)`` (or its
         ``(weight, bias)``) -- the prologue of ``Net3DSeg.forward`` (``3d_net/model.py:46-48``,
